@@ -2,7 +2,7 @@
 """bench.py -- VLQ hot path on B200: search QPS (+ encode Mvec/s) for BASELINE.json configs[1]
 (C=2^16 centroids, 32 neighbour lines, PQ m=16, synthetic SIFT-shaped 10M x 128 per GPU).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (one process per GPU under torchrun for N>1)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   our arm (one process per GPU under torchrun for N>1)
   python bench.py --impl reference [...]                          CPU arm: the reference's CPU code (IndexFlatL2 /
                                                                   ProductQuantizer from oracle/_ref) for the stock
                                                                   pieces + the oracle port for the VLQ-only search
@@ -31,7 +31,9 @@ if ROOT not in sys.path:
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline device loop and of the e2e loop (the --sweep points and the "
+                         "configs[3]-density scan stage time a fixed 3 and 5 steps)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "imipq"],
                     help="b200: this framework; reference: the CPU arm of the same metric; imipq: the reference's IMI-PQ "
@@ -67,7 +69,12 @@ def parse():
     ap.add_argument("--sweep", action="store_true",
                     help="also report recall@1/10/100 and QPS over nprobe = 1..64 with w1 = 4*nprobe (BASELINE configs[2])")
     ap.add_argument("--quick", action="store_true", help="small sizes (for debugging the script itself)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the search result of the last step (distances float32, labels "
+                         "float64) as DIR/<name>.npy, at most 64 MB in all, to compare two builds output for output")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the result of the GPU search path: --impl b200 only")
     if a.quick:
         a.n, a.nlist, a.nq, a.kc = 400_000, 4096, 2000, 1 << 14
     return a
@@ -411,6 +418,27 @@ def workload_config(a, n_gpus):
     }
 
 
+DUMP_LIMIT_BYTES = 64_000_000  # all files together, .npy headers included
+NPY_HEADER_BYTES = 128  # numpy pads a 2-D float array's header to 128 bytes
+
+
+def dump_outputs(path, D, I):
+    """--dump-outputs: the (distances, labels) a GpuIndexIVFPQ::search caller receives, as float32 / float64 .npy files.
+    Labels fit float64 exactly (< 2^53).  A result larger than 64 MB (10^6 bytes each) is cut to a fixed, seeded sample of query rows,
+    whose indices go to query_rows.npy."""
+    D = D.cpu().numpy().astype(np.float32)
+    I = I.cpu().numpy().astype(np.float64)
+    nq, k = D.shape
+    rows = max(1, (DUMP_LIMIT_BYTES - 3 * NPY_HEADER_BYTES) // (k * (4 + 8) + 8))
+    os.makedirs(path, exist_ok=True)
+    if nq > rows:
+        sel = np.sort(np.random.default_rng(0).choice(nq, rows, replace=False))
+        D, I = D[sel], I[sel]
+        np.save(os.path.join(path, "query_rows.npy"), sel.astype(np.float64))
+    np.save(os.path.join(path, "distances.npy"), D)
+    np.save(os.path.join(path, "labels.npy"), I)
+
+
 # ------------------------------------------------------------------------------------------------------- our arm
 def run_b200(a):
     import torch
@@ -711,6 +739,8 @@ def run_b200(a):
             D, I = fullD, fullI
         else:
             D, I = step_nccl(xq)
+    if rank == 0 and a.dump_outputs:
+        dump_outputs(a.dump_outputs, D, I)
     ops_matches = None
     if world == 1:  # the C++ API and the C-ABI tile loop of ops.search must agree bit for bit
         Do_, Io_ = ops_search(xq)

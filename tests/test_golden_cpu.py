@@ -59,3 +59,18 @@ def test_search(oracle, g):
     Dc, Ic, _, _, nsc = oracle.search(*args, P=int(g["P"]), W=int(g["W"]), k=int(g["k"]), cap=3, want_debug=True)
     assert np.array_equal(Ic, g["search_cap3_I"]) and np.array_equal(nsc, g["search_cap3_nscan"])
     assert (nsc <= 3 * int(g["W"])).all()
+
+
+def test_lambda0_search_vs_reference_ivfpq(oracle, g):
+    """With a single lambda level == 0 the VLQ anchor is the centroid, so searching all lines of the P probed centroids
+    is IndexIVFPQ with nprobe = P: the reference's IndexIVFPQ results with the fixture's codebooks are stored."""
+    C, E, P, k = int(g["C"]), int(g["E"]), int(g["P"]), int(g["k"])
+    xb, xq = g["xb"].astype(np.float32), g["xq"].astype(np.float32)
+    lcb = np.zeros(1, np.float32)
+    enc = oracle.encode_all(xb, g["cent"], g["edge"], g["edge_d2"], lcb, g["pq"])
+    offsets, perm = oracle.build_lists(enc["list"], C * E)
+    D, I = oracle.search(xq, g["cent"], g["edge"], g["edge_d2"], lcb, g["pq"], offsets, enc["codes"][perm],
+                         enc["lamq"][perm], perm.astype(np.int64), P=P, W=P * E, k=k, cap=1 << 20)
+    qn = np.sum(xq.astype(np.float64) ** 2, axis=1, keepdims=True)
+    np.testing.assert_allclose(D + qn, g["ref_ivfpq_D"], rtol=2e-4)
+    assert (I == g["ref_ivfpq_I"]).mean() > 0.97

@@ -122,6 +122,10 @@ def test_knn_graph_matches_oracle(ops, cuda, oracle, small_model, g):
         # mismatches must be distance ties
         for c, e in np.argwhere(~same):
             assert abs(ed2[c, e] - do[c, e]) <= 1e-5 * abs(do[c, e]) + 1e-3
+    # the fixture's graph (the loop's last case) against the reference's IndexFlatL2 search of the centroids against
+    # themselves, stored in the fixture (column 0 is the centroid itself)
+    assert (edge == g["ref_graph_I"][:, 1:]).mean() > 0.995
+    np.testing.assert_allclose(ed2, g["ref_graph_D"][:, 1:], rtol=1e-3, atol=1e-2)
 
 
 # ------------------------------------------------------------------------------------------------ encode (a5-a8)
@@ -204,6 +208,7 @@ def test_line_encode_golden(ops, cuda, g):
     assert (N(enc.lamq)[ok] == g["lamq"][ok]).mean() > 0.998
     ok &= N(enc.lamq) == g["lamq"]
     assert (N(enc.codes)[ok] == g["codes"][ok]).mean() > 0.9995
+    assert (N(enc.codes)[ok] == g["ref_pq_codes"][ok]).mean() > 0.998  # the reference's ProductQuantizer::compute_codes
 
 
 def test_line_stage_only_mode(ops, cuda, oracle, small_model):

@@ -6,10 +6,14 @@ keeps ALL lines of the probed centroids (w1 = nprobe * nedge) is exactly IndexIV
 assignment, same residual PQ codes, same ADC distances (up to ||q||^2, which the GPU search path omits like the
 reference's GPU path, gpu/impl/Distance.cu:287-290).
 """
+import os
+
 import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "vlq_small.npz")
 
 
 @pytest.fixture(scope="module")
@@ -65,6 +69,40 @@ def test_gpu_vlq_lambda0_equals_reference_ivfpq(cuda, ref, d, C, E, M, P):
     np.testing.assert_allclose((D + qn)[same], Dr[same], rtol=2e-4)
     overlap = np.mean([len(set(a) & set(b)) / k for a, b in zip(I, Ir)])
     assert overlap > 0.99
+
+
+def test_gpu_vlq_lambda0_equals_stored_reference_ivfpq(cuda):
+    """The same lambda == 0 identity on the golden fixture (tests/golden/vlq_small.npz), where the reference's
+    IndexFlatL2 assignment and IndexIVFPQ search results with the fixture's codebooks are stored: runs without the
+    reference library."""
+    from vector_line_quantization_b200 import index as vi
+
+    g = dict(np.load(GOLD))
+    d, C, E, M, P, k = (int(g[key]) for key in ("d", "C", "E", "M", "P", "k"))
+    xb, xq = g["xb"].astype(np.float32), g["xq"].astype(np.float32)
+    res = vi.StandardGpuResources(0)
+    idx = vi.GpuIndexIVFPQ(res, d, C, M, 8, E, 1)
+    idx.setCodebooks(g["cent"], g["edge"], g["edge_d2"], np.zeros(1, np.float32), g["pq"])
+    idx.add(xb)
+    # encode parity: the E line lists of centroid c hold the vectors IndexFlatL2 assigned to c, up to near-ties
+    assign = np.full(len(xb), -1, np.int64)
+    for c in range(C):
+        for e in range(E):
+            _, las, ids = idx.getList(c * E + e)
+            assert np.all(las == 0)
+            assign[ids] = c
+    assert np.all(assign >= 0)
+    for i in np.nonzero(assign != g["ref_flat_assign_I"])[0]:
+        da, db = (np.sum((xb[i].astype(np.float64) - g["cent"][c]) ** 2) for c in (assign[i], g["ref_flat_assign_I"][i]))
+        assert abs(da - db) <= 1e-5 * max(da, db), (int(i), da, db)
+    idx.setNumProbes(P)
+    idx.w1_ = P * E
+    idx.setListCap(1 << 20)
+    D, I = idx.search(xq, k)
+    qn = np.sum(xq.astype(np.float64) ** 2, axis=1, keepdims=True)
+    same = I == g["ref_ivfpq_I"]
+    assert same.mean() > 0.97
+    np.testing.assert_allclose((D + qn)[same], g["ref_ivfpq_D"][same], rtol=2e-4)
 
 
 @pytest.mark.gpu
