@@ -190,6 +190,25 @@ int vlq_coarse_select_lines_exact(const float* q, int64_t nq, int d, const float
                                   int E, int W, int* out_coarse, int* out_list, float* out_term1, float* out_term6,
                                   vlq_stream_t stream);
 
+/* a11 + a12 for one query tile, the route chosen here: the one entry the index's search and the Python operator layer
+ *     call.  Outputs as vlq_coarse_select_lines (out_coarse nullable [nq][P]); 1 <= P <= min(C, VLQ_MAX_K).
+ *     vlq_coarse_route (have_pack: cent_pack of vlq_tc_pack_centroids will be passed):
+ *       0  no pack:                                        vlq_l2_distances + vlq_select_rows + vlq_select_lines
+ *       1  tcgen05 matrix:                                 vlq_l2_distances_tc (+ bucket minima) + vlq_coarse_select_lines
+ *       2  matrix-free (vlq_coarse_exact_preferred):       vlq_l2_bucket_min_tc + vlq_coarse_select_lines_exact
+ *     The environment switches VLQ_COARSE_MATRIX (route 1) and VLQ_COARSE_EXACT (route 2 wherever supported) are read on
+ *     every call (tests and tuning only).  The workspace (vlq_coarse_lines_workspace_bytes, which applies the same rule;
+ *     256-byte aligned, as the device allocators return it) holds only what the route uses: the distance tile [nq][C]
+ *     (routes 0, 1), the bucket minima and the vlq_l2_tc_workspace_bytes block (routes 1, 2), the top-P of route 0.
+ *     Too small: VLQ_EWORKSPACE.  q (routes 1, 2) and cent (route 2) 16-byte aligned.  Every argument is checked before
+ *     the first launch. */
+int vlq_coarse_route(int d, int C, int P, int E, int W, int have_pack);
+size_t vlq_coarse_lines_workspace_bytes(int64_t nq, int d, int C, int P, int E, int W, int have_pack);
+int vlq_coarse_lines(const float* q, int64_t nq, int d, const float* cent, const float* cnorm, const void* cent_pack,
+                     float scale, int C, int P, const int* edge, const float* edge_d2, int E, int W, int* out_coarse,
+                     int* out_list, float* out_term1, float* out_term6, void* workspace, size_t workspace_bytes,
+                     vlq_stream_t stream);
+
 /* candidate lists (f4): ids of the entries of the W selected lines of every query in line order, first k of them, -1
    padded -- the recall-of-the-candidate-list tool GpuIndexIVFPQ::search1 / IVFPQ::queryGraph1
    (gpu/GpuIndexIVFPQ.cu:1646-1670, gpu/impl/IVFPQ.cu:778-870: a host loop over listOffsetToUserIndex_ there) */

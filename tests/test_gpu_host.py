@@ -111,7 +111,7 @@ def _build(vi, res, m, xb, chunks=2):
     return idx
 
 
-def test_vlq_index_matches_oracle(vi, res, oracle, small_model, tmp_path):
+def test_vlq_index_matches_oracle(vi, res, oracle, small_model, tmp_path, monkeypatch):
     m = small_model
     idx = _build(vi, res, m, m["xb"], chunks=3)
     assert idx.ntotal == len(m["xb"])
@@ -130,8 +130,57 @@ def test_vlq_index_matches_oracle(vi, res, oracle, small_model, tmp_path):
         assert (codes == enc["codes"][want]).mean() > 0.99 and (las == enc["lamq"][want]).mean() > 0.99
     assert mism <= 2
     # search: the oracle gets the index exactly as the device stored it (dumped through the reference's .db* files), so
-    # only the query path differs; every differing id must be a float64 near-tie (tests/parity_util.py)
-    _search_vs_oracle_same_index(idx, oracle, m, m["xq"], 16, 128, 20, tmp_path)
+    # only the query path differs; every differing id must be a float64 near-tie (tests/parity_util.py).  The coarse
+    # route is chosen per call: at C = 256, P = 16, W = 128 the default is the tcgen05 matrix route, and
+    # VLQ_COARSE_EXACT selects the matrix-free one
+    for switch, route in ((None, 1), ("VLQ_COARSE_MATRIX", 1), ("VLQ_COARSE_EXACT", 2)):
+        with monkeypatch.context() as mp:
+            if switch:
+                mp.setenv(switch, "1")
+            assert _coarse_route(m, 16, 128) == route
+            _search_vs_oracle_same_index(idx, oracle, m, m["xq"], 16, 128, 20, tmp_path)
+
+
+def _coarse_route(m, P, W):
+    from vector_line_quantization_b200 import _abi
+
+    return _abi.lib().vlq_coarse_route(m["d"], m["C"], P, m["E"], W, 1)
+
+
+def test_search_matrix_free_odd_tile_cap(vi, res, oracle, small_model, tmp_path):
+    """nlist = 100000, nprobe = 1, w1_ = 256: the matrix-free route with a query tile cap of 3355 rows (odd), where
+    per-tile buffers carved back to back once put the bucket minima off their 16-byte boundary and search() failed.
+    The host search must equal ops.search bit for bit and match the oracle."""
+    import torch
+
+    from vector_line_quantization_b200 import data, ops
+
+    d, C, E, M, P, W, k = 128, 100000, 8, 16, 1, 256, 20
+    dev = torch.device("cuda:0")
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)  # noqa: E731
+    cent = t(data.sift_like(C, seed=11))
+    edge, ed2 = ops.knn_graph(cent, E)
+    m = dict(d=d, C=C, E=E, M=M, cent=cent.cpu().numpy(), edge=edge.cpu().numpy(), edge_d2=ed2.cpu().numpy(),
+             lambda_cb=small_model["lambda_cb"], pq=small_model["pq"])
+    assert _coarse_route(m, P, W) == 2
+    xb = data.sift_like(200000, seed=12)
+    xq = data.sift_like(32, seed=13)
+    idx = vi.GpuIndexIVFPQ(res, d, C, M, 8, E, len(m["lambda_cb"]))
+    idx.setCodebooks(m["cent"], m["edge"], m["edge_d2"], m["lambda_cb"], m["pq"])
+    idx.add(xb)
+    _search_vs_oracle_same_index(idx, oracle, m, xq, P, W, k, tmp_path)
+    D, I = idx.search(xq, k)
+    # the same index through the operator layer: tensor-core assignment, line encode, list build, search
+    pack = ops.CentPack(cent)
+    lcb, pq = t(m["lambda_cb"]), t(m["pq"])
+    x = t(xb)
+    A, _ = ops.l2_assign_tc(x, pack, want_dist=False)
+    enc = ops.line_encode(x, A, cent, edge, ed2, lcb, pq)
+    lists = ops.build_lists(C * E, M, enc.list, enc.codes, enc.lamq, enc.kappa,
+                            torch.arange(len(xb), dtype=torch.int64, device=dev))
+    Do, Io = ops.search(t(xq), cent, pack.cnorm, edge, ed2, lcb, pq, lists, P, W, k, pack=pack,
+                        list_len_hint=len(xb) // (C * E))
+    assert np.array_equal(Do.cpu().numpy(), D) and np.array_equal(Io.cpu().numpy(), I)
 
 
 def _dump_index(idx, m, tmp_path):
@@ -178,7 +227,7 @@ def _search_vs_oracle_same_index(idx, oracle, m, xq, P, W, k, tmp_path, model=No
     cent = t(mm["cent"])
     pack = ops.CentPack(cent)
     qd = t(xq)
-    stage = ops.CoarseStage(cent, pack.cnorm, t(mm["edge"]), t(mm["edge_d2"]), P, W, len(xq), pack)  # the host's dispatch
+    stage = ops.CoarseStage(cent, pack.cnorm, t(mm["edge"]), t(mm["edge_d2"]), P, W, len(xq), pack)  # the host's route
     lst, _, _ = stage.run(qd)
     same_lines = check_lines(lst.cpu().numpy(), lines, xq, mm)
     # strict for every query: against the oracle's scan of the device's own line choice

@@ -45,6 +45,9 @@ SIGNATURES = {
     "vlq_coarse_exact_supported": (_i, [_i, _i, _i, _i, _i]),
     "vlq_coarse_exact_preferred": (_i, [_i, _i, _i, _i, _i]),
     "vlq_coarse_select_lines_exact": (_i, [_p, _l, _i, _p, _p, _p, _i, _i, _i, _p, _p, _i, _i, _p, _p, _p, _p, _p]),
+    "vlq_coarse_route": (_i, [_i, _i, _i, _i, _i, _i]),
+    "vlq_coarse_lines_workspace_bytes": (_z, [_l, _i, _i, _i, _i, _i, _i]),
+    "vlq_coarse_lines": (_i, [_p, _l, _i, _p, _p, _p, _f, _i, _i, _p, _p, _i, _i, _p, _p, _p, _p, _p, _z, _p]),
     "vlq_gather_candidates": (_i, [_p, _l, _i, _p, _p, _l, _p, _p]),
     "vlq_scan_topk_workspace_bytes": (_z, [_l, _i]),
     "vlq_scan_topk": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _z, _p]),

@@ -1171,7 +1171,7 @@ int vlq_coarse_select_lines(const float* D, int64_t nq, int64_t ldD, const float
   const int cap = select_capacity(kmax, Q_THREADS, Q_BATCH, total);
   const size_t smem = ((select_smem_bytes(cap) + 15) & ~size_t(15)) + 2 * VLQ_MAX_K * sizeof(int);
   // fast path (coarse_select.cuh): the keys of each selection fit R per thread in registers
-  static const bool generic_only = getenv("VLQ_COARSE_GENERIC") != nullptr;  // tests: force the general kernel
+  const bool generic_only = getenv("VLQ_COARSE_GENERIC") != nullptr;  // read per call: tests force the general kernel
   const int need = nb > P * E ? (nb > P * 32 ? nb : P * 32) : (P * E > P * 32 ? P * E : P * 32);
   if (!generic_only && need <= 16 * csl::NT && W <= 1024 && nb % 4 == 0 && (reinterpret_cast<uintptr_t>(bucket_min) & 15) == 0) {
     const int R = need <= 8 * csl::NT ? 8 : 16;
@@ -1233,6 +1233,86 @@ int vlq_coarse_select_lines_exact(const float* q, int64_t nq, int d, const float
                bucket_min, nb, C, P, edge, edge_d2, E, W, out_coarse, out_list, out_term1, out_term6);
   }
   return last_error();
+}
+
+int vlq_coarse_route(int d, int C, int P, int E, int W, int have_pack) {
+  if (!have_pack) return 0;
+  if (getenv("VLQ_COARSE_MATRIX")) return 1;
+  if (getenv("VLQ_COARSE_EXACT")) return vlq_coarse_exact_supported(d, C, P, E, W) ? 2 : 1;
+  return vlq_coarse_exact_preferred(d, C, P, E, W) ? 2 : 1;
+}
+
+}  // extern "C"
+
+// Byte offsets of the arrays of the vlq_coarse_lines workspace: only those the route uses, each on a 256-byte boundary.
+struct CoarseWorkspace {
+  size_t D = 0, bmin = 0, tc = 0, cval = 0, cidx = 0, end = 0;
+};
+
+static CoarseWorkspace coarse_workspace(int route, int64_t nq, int d, int C, int P) {
+  const size_t n = nq > 0 ? (size_t)nq : 0;
+  CoarseWorkspace w;
+  auto take = [&w](size_t bytes) {
+    const size_t at = w.end;
+    w.end += (bytes + 255) & ~size_t(255);
+    return at;
+  };
+  if (route != 2) w.D = take(n * C * sizeof(float));
+  if (route != 0) {
+    w.bmin = take(n * vlq_tc_num_buckets(C) * sizeof(float));
+    w.tc = take(vlq_l2_tc_workspace_bytes(nq, d, C));
+  } else {
+    w.cval = take(n * P * sizeof(float));
+    w.cidx = take(n * P * sizeof(int));
+  }
+  return w;
+}
+
+extern "C" {
+
+size_t vlq_coarse_lines_workspace_bytes(int64_t nq, int d, int C, int P, int E, int W, int have_pack) {
+  return coarse_workspace(vlq_coarse_route(d, C, P, E, W, have_pack), nq, d, C, P).end;
+}
+
+int vlq_coarse_lines(const float* q, int64_t nq, int d, const float* cent, const float* cnorm, const void* cent_pack,
+                     float scale, int C, int P, const int* edge, const float* edge_d2, int E, int W, int* out_coarse,
+                     int* out_list, float* out_term1, float* out_term6, void* workspace, size_t workspace_bytes,
+                     vlq_stream_t stream) {
+  if (nq < 0 || d <= 0 || C <= 0 || P <= 0 || P > VLQ_MAX_K || P > C || E <= 0 || W <= 0 || W > VLQ_MAX_K)
+    return VLQ_EINVAL;
+  if (nq == 0) return VLQ_OK;
+  if (!q || !cent || !cnorm || !edge || !edge_d2 || !out_list || !out_term1 || !out_term6 || !workspace)
+    return VLQ_EINVAL;
+  const int route = vlq_coarse_route(d, C, P, E, W, cent_pack != nullptr);
+  // the tensor-core sweep reads q, the matrix-free select reads q and cent, in 16-byte vectors
+  const uintptr_t vec = reinterpret_cast<uintptr_t>(q) | (route == 2 ? reinterpret_cast<uintptr_t>(cent) : 0);
+  if ((route != 0 && (vec & 15)) || (reinterpret_cast<uintptr_t>(workspace) & 255)) return VLQ_EINVAL;
+  const CoarseWorkspace w = coarse_workspace(route, nq, d, C, P);
+  if (workspace_bytes < w.end) return VLQ_EWORKSPACE;
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  float* D = reinterpret_cast<float*>(ws + w.D);
+  float* bmin = reinterpret_cast<float*>(ws + w.bmin);
+  const int nb = vlq_tc_num_buckets(C);
+  const size_t tc_bytes = vlq_l2_tc_workspace_bytes(nq, d, C);
+  int rc;
+  if (route == 2) {
+    rc = vlq_l2_bucket_min_tc(q, nq, d, cent_pack, scale, C, bmin, ws + w.tc, tc_bytes, stream);
+    if (rc) return rc;
+    return vlq_coarse_select_lines_exact(q, nq, d, cent, cnorm, bmin, nb, C, P, edge, edge_d2, E, W, out_coarse,
+                                         out_list, out_term1, out_term6, stream);
+  }
+  if (route == 1) {
+    rc = vlq_l2_distances_tc(q, nq, d, cent_pack, scale, C, D, C, bmin, ws + w.tc, tc_bytes, stream);
+    if (rc) return rc;
+    return vlq_coarse_select_lines(D, nq, C, bmin, nb, C, P, edge, edge_d2, E, W, out_coarse, out_list, out_term1,
+                                   out_term6, stream);
+  }
+  int* cidx = out_coarse ? out_coarse : reinterpret_cast<int*>(ws + w.cidx);
+  rc = vlq_l2_distances(q, nq, d, cent, cnorm, C, D, C, stream);
+  if (rc) return rc;
+  rc = vlq_select_rows(D, nq, C, C, P, nullptr, reinterpret_cast<float*>(ws + w.cval), cidx, stream);
+  if (rc) return rc;
+  return vlq_select_lines(D, nq, C, cidx, P, edge, edge_d2, E, W, out_list, out_term1, out_term6, stream);
 }
 
 // term-3 tables of the batch (+ 256 spare bytes)

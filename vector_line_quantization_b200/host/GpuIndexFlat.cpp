@@ -152,24 +152,16 @@ void GpuIndexFlat::assignDevice(const float* dx, Index::idx_t n, int* dLabels, f
   }
 }
 
-void GpuIndexFlat::distancesDevice(const float* dx, Index::idx_t n, float* dD, Index::idx_t ldD, float* bucketMin) const {
+void GpuIndexFlat::distancesDevice(const float* dx, Index::idx_t n, float* dD, Index::idx_t ldD) const {
   vlq_stream_t st = resources_->getDefaultStream();
   if (pack_.get()) {
     const size_t ws = vlq_l2_tc_workspace_bytes(n, d, (int)ntotal);
     scratch_.reserve(ws);
-    VLQ_CALL(vlq_l2_distances_tc(dx, n, d, pack_.get(), packScale_, (int)ntotal, dD, ldD, bucketMin, scratch_.get(),
+    VLQ_CALL(vlq_l2_distances_tc(dx, n, d, pack_.get(), packScale_, (int)ntotal, dD, ldD, nullptr, scratch_.get(),
                                  scratch_.bytes(), st));
   } else {
-    VLQ_THROW_IF_NOT_MSG(bucketMin == nullptr, "bucket minima are produced by the tensor-core path only");
     VLQ_CALL(vlq_l2_distances(dx, n, d, vecs_.as<float>(), norms_.as<float>(), (int)ntotal, dD, ldD, st));
   }
-}
-
-void GpuIndexFlat::bucketMinDevice(const float* dx, Index::idx_t n, float* bucketMin) const {
-  VLQ_THROW_IF_NOT_MSG(pack_.get() != nullptr, "bucket minima are produced by the tensor-core path only");
-  vlq_stream_t st = resources_->getDefaultStream();
-  scratch_.reserve(vlq_l2_tc_workspace_bytes(n, d, (int)ntotal));
-  VLQ_CALL(vlq_l2_bucket_min_tc(dx, n, d, pack_.get(), packScale_, (int)ntotal, bucketMin, scratch_.get(), scratch_.bytes(), st));
 }
 
 void GpuIndexFlat::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const {

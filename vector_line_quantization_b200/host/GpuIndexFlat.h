@@ -63,10 +63,7 @@ class GpuIndexFlat : public faiss::Index {
   /// nearest stored vector for device rows: device in / device out (the entry the encode path uses)
   void assignDevice(const float* dx, Index::idx_t n, int* dLabels, float* dDist, bool addXnorm) const;
   /// distance matrix D = ||c||^2 - 2 x.c for device rows (no ||x||^2, reference gpu/impl/Distance.cu:287-290)
-  /// bucketMin (nullable, tensor-core path only): [n][vlq_tc_num_buckets(ntotal)] minima of 32-column buckets of D
-  void distancesDevice(const float* dx, Index::idx_t n, float* dD, Index::idx_t ldD, float* bucketMin = nullptr) const;
-  /// tensor-core sweep WITHOUT the distance matrix: only the minima of the 32-column buckets, [n][vlq_tc_num_buckets]
-  void bucketMinDevice(const float* dx, Index::idx_t n, float* bucketMin) const;
+  void distancesDevice(const float* dx, Index::idx_t n, float* dD, Index::idx_t ldD) const;
 
  private:
   void refreshDerived_();

@@ -133,9 +133,6 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   void commit_() const;  ///< merge pending entries into the CSR lists (lazy: first search / list access after adds)
   void ensurePending_(size_t extra);
   void addTiles_(Index::idx_t n, const void* x, bool isU8, const long* xids);
-  bool coarseMatrixFree_(int P, int W) const;
-  void coarseLines_(const float* q, Index::idx_t m, int P, int W, DeviceBuffer& dmat, float* cval, int* cidx, float* bmin,
-                    int* lline, float* t1, float* t6) const;
   void installLists_(const std::vector<int>& counts, const std::vector<uint8_t>& codes, const std::vector<uint8_t>& las,
                      const std::vector<long>& ids);
 

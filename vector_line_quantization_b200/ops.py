@@ -6,8 +6,6 @@ include/vlq_b200.h.
 """
 from collections import namedtuple
 
-import os
-
 import torch
 
 from . import _abi
@@ -170,20 +168,23 @@ def rotate_codes(offsets, codes, inverse=False):
     return torch.gather(codes, 1, idx).contiguous()
 
 
+def _lines_out(nq, W, dev, out):
+    """(list int32, term1 f32, term6 f32) [nq][W] destinations of a line selection: `out` checked, or new tensors"""
+    if out is not None:
+        lst, t1, t6 = out
+        assert lst.shape == (nq, W) and lst.is_contiguous() and t1.is_contiguous() and t6.is_contiguous()
+        return out
+    return (torch.empty((nq, W), dtype=torch.int32, device=dev), torch.empty((nq, W), dtype=torch.float32, device=dev),
+            torch.empty((nq, W), dtype=torch.float32, device=dev))
+
+
 def select_lines(D, coarse_ids, edge, edge_d2, W, out=None):
     """query-time line selection (a12): -> (list int32 [nq][W], term1, term6 f32 [nq][W])"""
     D = _chk(D, torch.float32, "D")
     coarse_ids = _chk(coarse_ids, torch.int32, "coarse_ids")
     nq, P = coarse_ids.shape
     E = edge.shape[1]
-    dev = D.device
-    if out is not None:
-        lst, t1, t6 = out
-        assert lst.shape == (nq, W) and lst.is_contiguous() and t1.is_contiguous() and t6.is_contiguous()
-    else:
-        lst = torch.empty((nq, W), dtype=torch.int32, device=dev)
-        t1 = torch.empty((nq, W), dtype=torch.float32, device=dev)
-        t6 = torch.empty((nq, W), dtype=torch.float32, device=dev)
+    lst, t1, t6 = _lines_out(nq, W, D.device, out)
     _abi.call("vlq_select_lines", _ptr(D), nq, D.stride(0), _ptr(coarse_ids), P, _ptr(edge), _ptr(edge_d2), E, W,
               _ptr(lst), _ptr(t1), _ptr(t6), _stream())
     return lst, t1, t6
@@ -293,37 +294,29 @@ def coarse_lines(q, cent, cnorm, edge, edge_d2, P, W, tile=5120, pack=None, out=
 
 
 class CoarseStage:
-    """a11 + a12 for one query tile -- the dispatch GpuIndexIVFPQ::coarseLines_ makes.  With a CentPack and a small
-    nprobe (vlq_coarse_exact_preferred) the distance matrix is never written: the tcgen05 sweep emits the bucket minima
-    only and vlq_coarse_select_lines_exact re-evaluates the columns it needs; otherwise vlq_l2_distances_tc +
-    vlq_coarse_select_lines (VLQ_COARSE_MATRIX=1 forces this route, VLQ_COARSE_EXACT=1 the other wherever it is
-    supported).  Without a pack: fp32 matrix + select_rows + select_lines."""
+    """a11 + a12 for query tiles of at most `tile` rows through vlq_coarse_lines, the entry GpuIndexIVFPQ::search calls:
+    it picks the route (vlq_coarse_route) and lays out the workspace.  .exact: the matrix-free route (route 2)."""
 
     def __init__(self, cent, cnorm, edge, edge_d2, P, W, tile, pack=None):
         self.cent, self.cnorm, self.edge, self.edge_d2, self.pack = cent, cnorm, edge, edge_d2, pack
         self.C, self.d = cent.shape
         self.P, self.W = min(P, self.C), W
-        dev = cent.device
-        fn = "vlq_coarse_exact_supported" if os.environ.get("VLQ_COARSE_EXACT") else "vlq_coarse_exact_preferred"
-        self.exact = (pack is not None and os.environ.get("VLQ_COARSE_MATRIX") is None and
-                      bool(getattr(_abi.lib(), fn)(self.d, self.C, self.P, edge.shape[1], W)))
-        self.Dbuf = None if self.exact else torch.empty((tile, self.C), dtype=torch.float32, device=dev)
-        self.bbuf = torch.empty((tile, num_buckets(self.C)), dtype=torch.float32, device=dev) if pack is not None else None
+        args = (self.d, self.C, self.P, edge.shape[1], W, int(pack is not None))
+        self.exact = _abi.lib().vlq_coarse_route(*args) == 2
+        self.ws = torch.empty(_abi.lib().vlq_coarse_lines_workspace_bytes(tile, *args), dtype=torch.uint8,
+                              device=cent.device)
 
     def run(self, qt, out=None, want_coarse=False):
-        m = qt.shape[0]
-        if self.exact:
-            l2_bucket_min_tc(qt, self.pack, self.bbuf[:m])
-            return coarse_select_lines_exact(qt, self.cent, self.cnorm, self.bbuf[:m], self.P, self.edge, self.edge_d2,
-                                             self.W, want_coarse=want_coarse, out=out)
-        if self.pack is not None:
-            D = l2_distances_tc(qt, self.pack, out=self.Dbuf[:m], bucket_min=self.bbuf[:m])
-            return coarse_select_lines(D, self.bbuf[:m], self.C, self.P, self.edge, self.edge_d2, self.W,
-                                       want_coarse=want_coarse, out=out)
-        D = l2_distances(qt, self.cent, self.cnorm, out=self.Dbuf[:m])
-        _, cid = select_rows(D, self.P)
-        r = select_lines(D, cid, self.edge, self.edge_d2, self.W, out=out)
-        return (*r, cid) if want_coarse else r
+        qt = _chk(qt, torch.float32, "q")
+        nq = qt.shape[0]
+        lst, t1, t6 = _lines_out(nq, self.W, qt.device, out)
+        cid = torch.empty((nq, self.P), dtype=torch.int32, device=qt.device) if want_coarse else None
+        pack = self.pack
+        _abi.call("vlq_coarse_lines", _ptr(qt), nq, self.d, _ptr(self.cent), _ptr(self.cnorm),
+                  0 if pack is None else _ptr(pack.buf), 1.0 if pack is None else pack.scale, self.C, self.P,
+                  _ptr(self.edge), _ptr(self.edge_d2), self.edge.shape[1], self.W, _ptr(cid), _ptr(lst), _ptr(t1),
+                  _ptr(t6), _ptr(self.ws), self.ws.numel(), _stream())
+        return (lst, t1, t6, cid) if want_coarse else (lst, t1, t6)
 
 
 def scan_lines(q, pq, lambda_cb, lines, edge_d2, lists, k, cap=1024, tile=5120, out=None, list_len_hint=None):
@@ -435,15 +428,8 @@ def coarse_select_lines_exact(q, cent, cnorm, bucket_min, P, edge, edge_d2, W, w
     q = _chk(q, torch.float32, "q")
     nq, d = q.shape
     C, E = cent.shape[0], edge.shape[1]
-    dev = q.device
-    if out is not None:
-        lst, t1, t6 = out
-        assert lst.shape == (nq, W) and lst.is_contiguous() and t1.is_contiguous() and t6.is_contiguous()
-    else:
-        lst = torch.empty((nq, W), dtype=torch.int32, device=dev)
-        t1 = torch.empty((nq, W), dtype=torch.float32, device=dev)
-        t6 = torch.empty((nq, W), dtype=torch.float32, device=dev)
-    cid = torch.empty((nq, P), dtype=torch.int32, device=dev) if want_coarse else None
+    lst, t1, t6 = _lines_out(nq, W, q.device, out)
+    cid = torch.empty((nq, P), dtype=torch.int32, device=q.device) if want_coarse else None
     _abi.call("vlq_coarse_select_lines_exact", _ptr(q), nq, d, _ptr(cent), _ptr(cnorm), _ptr(bucket_min),
               bucket_min.shape[1], C, P, _ptr(edge), _ptr(edge_d2), E, W, _ptr(cid), _ptr(lst), _ptr(t1), _ptr(t6),
               _stream())
@@ -458,15 +444,8 @@ def coarse_select_lines(D, bucket_min, C, P, edge, edge_d2, W, want_coarse=False
     """fused top-P (through the bucket minima) + line selection (a11 + a12); out = (list, term1, term6) destinations"""
     nq = D.shape[0]
     E = edge.shape[1]
-    dev = D.device
-    if out is not None:
-        lst, t1, t6 = out
-        assert lst.shape == (nq, W) and lst.is_contiguous() and t1.is_contiguous() and t6.is_contiguous()
-    else:
-        lst = torch.empty((nq, W), dtype=torch.int32, device=dev)
-        t1 = torch.empty((nq, W), dtype=torch.float32, device=dev)
-        t6 = torch.empty((nq, W), dtype=torch.float32, device=dev)
-    cid = torch.empty((nq, P), dtype=torch.int32, device=dev) if want_coarse else None
+    lst, t1, t6 = _lines_out(nq, W, D.device, out)
+    cid = torch.empty((nq, P), dtype=torch.int32, device=D.device) if want_coarse else None
     _abi.call("vlq_coarse_select_lines", _ptr(D), nq, D.stride(0), _ptr(bucket_min), bucket_min.shape[1], C, P,
               _ptr(edge), _ptr(edge_d2), E, W, _ptr(cid), _ptr(lst), _ptr(t1), _ptr(t6), _stream())
     return (lst, t1, t6, cid) if want_coarse else (lst, t1, t6)
