@@ -151,6 +151,23 @@ int vlq_build_lists(int64_t nlists, int M,
                     int64_t* out_offsets, uint8_t* out_codes, uint8_t* out_lamq, float* out_kappa, int64_t* out_ids,
                     void* workspace, size_t workspace_bytes, vlq_stream_t stream);
 
+/* a9 (removal): stable compaction of the CSR slab above, the survivors keeping their order inside their list (the
+ *     reference's IndexIVF::remove_ids, IndexIVF.cpp, swaps each removed entry with the last of its list instead).
+ *     An entry is removed iff range_lo <= id < range_hi OR id is in batch[0 .. n_batch), sorted ascending (duplicates
+ *     allowed; range_lo >= range_hi: no range).  offsets[nlists] must equal n.
+ *     pass 1 (plan) writes out_offsets[nlists + 1] of the survivors; out_offsets[nlists] = survivor count, which the
+ *     caller reads to size the new slab.  pass 2 (apply) gathers the survivors into out_* and re-rotates every code word
+ *     to its new list position; it reads the workspace pass 1 wrote, unchanged in between.  out_* must be non-NULL when
+ *     n > 0.  The workspace holds the keep mask (n / 8 bytes) and one int64 per 8192 entries; nlists does not enter it. */
+size_t vlq_remove_ids_workspace_bytes(int64_t n, int64_t nlists);
+int vlq_remove_ids_plan(int64_t nlists, int64_t n, const int64_t* offsets, const int64_t* ids, int64_t range_lo,
+                        int64_t range_hi, const int64_t* batch, int64_t n_batch, int64_t* out_offsets, void* workspace,
+                        size_t workspace_bytes, vlq_stream_t stream);
+int vlq_remove_ids_apply(int64_t nlists, int M, int64_t n, const int64_t* offsets, const uint8_t* codes,
+                         const uint8_t* lamq, const float* kappa, const int64_t* ids, const int64_t* out_offsets,
+                         uint8_t* out_codes, uint8_t* out_lamq, float* out_kappa, int64_t* out_ids,
+                         const void* workspace, size_t workspace_bytes, vlq_stream_t stream);
+
 /* a9 (loader): per-entry kappa = ||p||^2 + 2 anchor.p for list-major entries that arrive without it, i.e. lists read
  *     from the reference's .dbIdx/.dbcodes/.dbcount/.dblas files (gpu/GpuIndexIVFPQ.cu:1813-2010). */
 int vlq_recompute_kappa(int64_t n, int64_t nlists, const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq,

@@ -26,6 +26,10 @@ int vlq_host_index_add(void* index, long n, const float* x);
 int vlq_host_index_add_with_ids(void* index, long n, const float* x, const long* ids);
 int vlq_host_index_search(void* index, long n, const float* x, long k, float* distances, long* labels);
 int vlq_host_index_reset(void* index);
+/* Index::remove_ids with IDSelectorRange [imin, imax) / IDSelectorBatch (ids in host or device memory); *nremoved gets
+   the number of entries removed.  GpuIndexIVFPQ and GpuIndexIMIPQ implement it; other indexes fail (-1). */
+int vlq_host_index_remove_ids_range(void* index, long imin, long imax, long* nremoved);
+int vlq_host_index_remove_ids_batch(void* index, long n, const long* ids, long* nremoved);
 long vlq_host_index_ntotal(void* index);
 int vlq_host_index_is_trained(void* index);
 

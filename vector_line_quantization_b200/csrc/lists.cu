@@ -385,6 +385,164 @@ gather_candidates_kernel(const int* __restrict__ line_list, int W, const int64_t
   for (int64_t i = tot + threadIdx.x; i < k; i += 256) out[q * k + i] = -1;
 }
 
+// ------------------------------------------------------------------------------------------------ entry removal
+// Stable stream compaction of the slab (IndexIVF::remove_ids, but the survivors keep their order).  The slab is cut into
+// tiles of REM_TILE entries, one block each; word w of a tile is the keep mask of its entries 32 w .. 32 w + 31.  Because
+// the slab is list-major, the global survivor prefix of an entry is its destination, and the survivor prefix at
+// offsets[l] is the new offsets[l].  Workspace: the keep mask (n / 8 bytes) and one int64 per tile.
+constexpr int REM_WORDS = SCAN_THREADS;  // one mask word per thread
+constexpr int REM_TILE = REM_WORDS * kWarp;
+constexpr int REM_LISTS = 1024;          // list starts a tile of the apply pass keeps in shared memory
+
+__device__ __forceinline__ bool removed_id(int64_t id, int64_t lo, int64_t hi, const int64_t* __restrict__ batch,
+                                           int64_t nb) {
+  if (id >= lo && id < hi) return true;
+  if (nb == 0 || id < batch[0] || id > batch[nb - 1]) return false;
+  int64_t a = 0, b = nb;  // lower bound of id in the sorted batch
+  while (a < b) {
+    const int64_t mid = (a + b) >> 1;
+    if (batch[mid] < id) a = mid + 1; else b = mid;
+  }
+  return batch[a] == id;
+}
+
+// largest l in [lo, hi] with offsets[l] <= p (offsets[lo] <= p)
+__device__ __forceinline__ int64_t list_of(const int64_t* offsets, int64_t lo, int64_t hi, int64_t p) {
+  while (lo < hi) {
+    const int64_t mid = (lo + hi + 1) >> 1;
+    if (offsets[mid] <= p) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// pass 1: keep mask, survivors per tile (tile_sums), and for every list that starts inside the tile its survivor prefix
+// relative to the tile (rem_offsets_kernel adds the tile's base once the tile totals are scanned)
+__global__ void __launch_bounds__(SCAN_THREADS)
+rem_mark_kernel(int64_t n, int64_t nlists, const int64_t* __restrict__ offsets, const int64_t* __restrict__ ids,
+                int64_t lo, int64_t hi, const int64_t* __restrict__ batch, int64_t nb, uint32_t* __restrict__ mask,
+                int64_t* __restrict__ tile_sums, int64_t* __restrict__ out_offsets) {
+  __shared__ uint32_t sword[REM_WORDS];
+  __shared__ int64_t spre[REM_WORDS];
+  __shared__ int64_t wsum[SCAN_THREADS / kWarp];
+  __shared__ int64_t total;
+  const int lane = threadIdx.x % kWarp, warp = threadIdx.x / kWarp;
+  const int64_t base = (int64_t)blockIdx.x * REM_TILE;
+#pragma unroll 4
+  for (int it = 0; it < REM_WORDS / (SCAN_THREADS / kWarp); it++) {
+    const int w = it * (SCAN_THREADS / kWarp) + warp;
+    const int64_t e = base + (int64_t)w * kWarp + lane;
+    const bool keep = e < n && !removed_id(ids[e], lo, hi, batch, nb);
+    const uint32_t bits = __ballot_sync(kFull, keep);
+    if (lane == 0) {
+      sword[w] = bits;
+      mask[(int64_t)blockIdx.x * REM_WORDS + w] = bits;
+    }
+  }
+  __syncthreads();
+  spre[threadIdx.x] = block_exscan(__popc(sword[threadIdx.x]), &total, wsum);
+  if (threadIdx.x == 0) {
+    tile_sums[blockIdx.x] = total;
+    if (blockIdx.x == 0) tile_sums[gridDim.x] = 0;  // the exclusive scan leaves the survivor count here
+  }
+  __syncthreads();
+  // lists l with base <= offsets[l] < min(base + REM_TILE, n); lists starting at n are finished by rem_offsets_kernel
+  const int64_t end = min(base + REM_TILE, n);
+  int64_t a = 0, b = nlists;  // first l with offsets[l] >= base
+  while (a < b) {
+    const int64_t mid = (a + b) >> 1;
+    if (offsets[mid] < base) a = mid + 1; else b = mid;
+  }
+  for (int64_t l = a + threadIdx.x; l < nlists; l += SCAN_THREADS) {
+    const int64_t p = offsets[l];
+    if (p >= end) break;
+    const int r = (int)(p - base);
+    out_offsets[l] = spre[r / kWarp] + __popc(sword[r / kWarp] & ((1u << (r % kWarp)) - 1u));
+  }
+}
+
+// tile_sums holds the exclusive prefix of the tile totals (tile_sums[ntiles] = survivor count)
+__global__ void rem_offsets_kernel(int64_t n, int64_t nlists, const int64_t* __restrict__ offsets,
+                                   const int64_t* __restrict__ tile_sums, int64_t ntiles,
+                                   int64_t* __restrict__ out_offsets) {
+  for (int64_t l = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; l <= nlists; l += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t p = l < nlists ? offsets[l] : n;
+    out_offsets[l] = p < n ? out_offsets[l] + tile_sums[p / REM_TILE] : tile_sums[ntiles];
+  }
+}
+
+// pass 2: the in-tile prefix is rebuilt from the mask; every survivor is copied to its prefix and its code word re-rotated
+// from its old list position p to its new one p' (store_code_rotated by (p' - p) mod M)
+__global__ void __launch_bounds__(SCAN_THREADS)
+rem_apply_kernel(int64_t n, int64_t nlists, int M, const int64_t* __restrict__ offsets,
+                 const int64_t* __restrict__ out_offsets, const uint32_t* __restrict__ mask,
+                 const int64_t* __restrict__ tile_sums, ConstListArrays src, ListArrays dst) {
+  __shared__ uint32_t sword[REM_WORDS];
+  __shared__ int64_t spre[REM_WORDS];
+  __shared__ int64_t soff[REM_LISTS], sout[REM_LISTS];
+  __shared__ int64_t wsum[SCAN_THREADS / kWarp];
+  __shared__ int64_t total;
+  const int lane = threadIdx.x % kWarp, warp = threadIdx.x / kWarp;
+  const int64_t base = (int64_t)blockIdx.x * REM_TILE;
+  const int64_t last = min(base + REM_TILE, n) - 1;
+  const uint32_t mine = mask[(int64_t)blockIdx.x * REM_WORDS + threadIdx.x];
+  sword[threadIdx.x] = mine;
+  spre[threadIdx.x] = block_exscan(__popc(mine), &total, wsum) + tile_sums[blockIdx.x];  // syncs the block
+  if (total == 0) return;  // uniform
+  // the lists the tile spans: [l0, l1]
+  const int64_t l0 = list_of(offsets, 0, nlists - 1, base);
+  const int64_t l1 = list_of(offsets, l0, nlists - 1, last);
+  const bool cached = l1 - l0 < REM_LISTS;
+  if (cached) {
+    for (int64_t i = threadIdx.x; i <= l1 - l0; i += SCAN_THREADS) {
+      soff[i] = offsets[l0 + i];
+      sout[i] = out_offsets[l0 + i];
+    }
+  }
+  __syncthreads();
+#pragma unroll 2
+  for (int it = 0; it < REM_WORDS / (SCAN_THREADS / kWarp); it++) {
+    const int w = it * (SCAN_THREADS / kWarp) + warp;
+    const uint32_t bits = sword[w];
+    if (!((bits >> lane) & 1u)) continue;
+    const int64_t e = base + (int64_t)w * kWarp + lane;
+    const int64_t o = spre[w] + __popc(bits & ((1u << lane) - 1u));
+    int64_t ob, nb;
+    if (cached) {
+      const int64_t i = list_of(soff, 0, l1 - l0, e);
+      ob = soff[i];
+      nb = sout[i];
+    } else {
+      const int64_t l = list_of(offsets, l0, l1, e);
+      ob = offsets[l];
+      nb = out_offsets[l];
+    }
+    int64_t rot = ((o - nb) - (e - ob)) % M;  // new position - old position (<= 0)
+    if (rot < 0) rot += M;
+    store_code_rotated(dst.codes + o * M, src.codes + e * M, M, rot);
+    dst.lamq[o] = src.lamq[e];
+    dst.kappa[o] = src.kappa[e];
+    dst.ids[o] = src.ids[e];
+  }
+}
+
+struct RemWs {
+  uint32_t* mask;      // [ntiles * REM_WORDS]
+  int64_t* tile_sums;  // [ntiles + 1]
+  int64_t ntiles;
+  size_t bytes;
+};
+static RemWs carve_rem(void* ws, int64_t n) {
+  auto align = [](size_t v) { return (v + 255) & ~size_t(255); };
+  RemWs w{};
+  w.ntiles = div_up(n, REM_TILE);
+  unsigned char* p = static_cast<unsigned char*>(ws);
+  size_t off = 0;
+  w.mask = reinterpret_cast<uint32_t*>(p + off); off = align(off + sizeof(uint32_t) * REM_WORDS * w.ntiles);
+  w.tile_sums = reinterpret_cast<int64_t*>(p + off); off = align(off + sizeof(int64_t) * (w.ntiles + 1));
+  w.bytes = off;
+  return w;
+}
+
 }  // namespace vlq
 
 using namespace vlq;
@@ -467,6 +625,46 @@ extern "C" int vlq_build_lists(int64_t nlists, int M, int64_t n_old, const int64
   if (n_new > 0) {
     VLQ_LAUNCH(gather_new_kernel, wide, 256, 0, st, w.perm, nlists, new_list, w.new_base, oo, out_offsets, nsrc, dst, M);
   }
+  return last_error();
+}
+
+extern "C" size_t vlq_remove_ids_workspace_bytes(int64_t n, int64_t /*nlists*/) {
+  return carve_rem(nullptr, n < 0 ? 0 : n).bytes;
+}
+
+extern "C" int vlq_remove_ids_plan(int64_t nlists, int64_t n, const int64_t* offsets, const int64_t* ids,
+                                   int64_t range_lo, int64_t range_hi, const int64_t* batch, int64_t n_batch,
+                                   int64_t* out_offsets, void* workspace, size_t workspace_bytes, vlq_stream_t stream) {
+  if (nlists < 1 || n < 0 || n_batch < 0 || !offsets || !out_offsets || !workspace) return VLQ_EINVAL;
+  if ((n > 0 && !ids) || (n_batch > 0 && !batch)) return VLQ_EINVAL;
+  RemWs w = carve_rem(workspace, n);
+  if (workspace_bytes < w.bytes) return VLQ_EWORKSPACE;
+  cudaStream_t st = as_stream(stream);
+  if (n == 0) {
+    VLQ_CUDA_TRY(cudaMemsetAsync(out_offsets, 0, sizeof(int64_t) * (nlists + 1), st));
+    return VLQ_OK;
+  }
+  VLQ_LAUNCH(rem_mark_kernel, (unsigned)w.ntiles, SCAN_THREADS, 0, st, n, nlists, offsets, ids, range_lo, range_hi, batch,
+             n_batch, w.mask, w.tile_sums, out_offsets);
+  VLQ_LAUNCH(scan_tile_offsets_kernel, 1, SCAN_THREADS, 0, st, w.tile_sums, w.ntiles + 1);
+  const int64_t lgrid = div_up(nlists + 1, 256);
+  const unsigned grid = (unsigned)(lgrid < 148 * 8 ? lgrid : 148 * 8);
+  VLQ_LAUNCH(rem_offsets_kernel, grid, 256, 0, st, n, nlists, offsets, w.tile_sums, w.ntiles, out_offsets);
+  return last_error();
+}
+
+extern "C" int vlq_remove_ids_apply(int64_t nlists, int M, int64_t n, const int64_t* offsets, const uint8_t* codes,
+                                    const uint8_t* lamq, const float* kappa, const int64_t* ids, const int64_t* out_offsets,
+                                    uint8_t* out_codes, uint8_t* out_lamq, float* out_kappa, int64_t* out_ids,
+                                    const void* workspace, size_t workspace_bytes, vlq_stream_t stream) {
+  if (nlists < 1 || M < 1 || M > 64 || n < 0 || !offsets || !out_offsets || !workspace) return VLQ_EINVAL;
+  if (n > 0 && (!codes || !lamq || !kappa || !ids || !out_codes || !out_lamq || !out_kappa || !out_ids)) return VLQ_EINVAL;
+  RemWs w = carve_rem(const_cast<void*>(workspace), n);
+  if (workspace_bytes < w.bytes) return VLQ_EWORKSPACE;
+  if (n == 0) return VLQ_OK;
+  VLQ_LAUNCH(rem_apply_kernel, (unsigned)w.ntiles, SCAN_THREADS, 0, as_stream(stream), n, nlists, M, offsets,
+             out_offsets, w.mask, w.tile_sums, ConstListArrays{codes, lamq, kappa, ids},
+             ListArrays{out_codes, out_lamq, out_kappa, out_ids});
   return last_error();
 }
 

@@ -1,5 +1,7 @@
 #include "GpuIndexIMIPQ.h"
 
+#include "ListRemoval.h"
+
 #include <algorithm>
 #include <cstring>
 
@@ -185,6 +187,16 @@ void GpuIndexIMIPQ::commit_() const {
   lIds_.swap(nIds);
   nListed_ = (size_t)last;  // rows without a cell (NaN input) are dropped, as in the VLQ index
   nPending_ = 0;
+}
+
+// same slab as the VLQ index (zero lambda bytes): the same compaction (host/ListRemoval.cpp)
+long GpuIndexIMIPQ::remove_ids(const IDSelector& sel) {
+  DeviceScope scope(resources_->getDevice());
+  commit_();
+  const long removed = removeFromLists(resources_, sel, (int64_t)K_ * K_, M_,
+                                       ListSlab{lOffsets_, lCodes_, lLamq_, lKappa_, lIds_, nListed_});
+  ntotal -= removed;
+  return removed;
 }
 
 int GpuIndexIMIPQ::getListLength(long cell) const {

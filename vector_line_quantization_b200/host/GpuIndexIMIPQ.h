@@ -10,6 +10,7 @@
 #pragma once
 #include <vector>
 
+#include "AuxIndexStructures.h"
 #include "GpuIndexFlat.h"
 #include "ProductQuantizer.h"
 
@@ -26,6 +27,8 @@ class GpuIndexIMIPQ : public faiss::Index {
   void add_with_ids(Index::idx_t n, const float* x, const long* xids) override;
   void search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const override;
   void reset() override;
+  /// IndexIVF::remove_ids for IDSelectorRange / IDSelectorBatch, as GpuIndexIVFPQ::remove_ids (survivors keep their order)
+  long remove_ids(const IDSelector& sel) override;
 
   void setNumProbes(int nprobe);  ///< cells visited per query, 1 .. 1024
   int getNumProbes() const { return nprobe_; }

@@ -1,5 +1,7 @@
 #include "GpuIndexIVFPQ.h"
 
+#include "ListRemoval.h"
+
 #include <algorithm>
 #include <cfloat>
 #include <cmath>
@@ -303,6 +305,16 @@ void GpuIndexIVFPQ::commit_() const {
     capPending_ = 0;
     reserveVecs_ = 0;
   }
+}
+
+// IndexIVF::remove_ids: pending adds take part, then the slab is compacted on the device (host/ListRemoval.cpp)
+long GpuIndexIVFPQ::remove_ids(const IDSelector& sel) {
+  DeviceScope scope(ivfConfig_.device);
+  commit_();
+  const long removed = removeFromLists(resources_, sel, (int64_t)nlist_ * numedge_, subQuantizers_,
+                                       ListSlab{lOffsets_, lCodes_, lLamq_, lKappa_, lIds_, nListed_});
+  ntotal -= removed;
+  return removed;
 }
 
 // searchImpl_ -> IVFPQ::queryGraph (gpu/GpuIndexIVFPQ.cu:1400-1464, gpu/impl/IVFPQ.cu:685-775).  The coarse stage of a

@@ -9,6 +9,7 @@
 #include <string>
 #include <vector>
 
+#include "AuxIndexStructures.h"
 #include "GpuIndexFlat.h"
 #include "IndexIVFPQ.h"
 #include "ProductQuantizer.h"
@@ -79,6 +80,10 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   void add_with_ids_u8(Index::idx_t n, const uint8_t* x, const long* xids);
   void search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const override;
   void reset() override;
+  /// IndexIVF::remove_ids for IDSelectorRange / IDSelectorBatch (any other selector throws), on the device: pending adds
+  /// are committed first, then the lists are compacted.  Survivors keep their order inside a list, so the index equals
+  /// one that never received the removed vectors (IndexIVF swaps in the last entry of the list instead).
+  long remove_ids(const IDSelector& sel) override;
 
   void reserveMemory(size_t numVecs);
   void setPrecomputedCodes(bool) {}

@@ -11,6 +11,8 @@ namespace faiss {
 
 enum MetricType { METRIC_INNER_PRODUCT = 0, METRIC_L2 = 1 };
 
+struct IDSelector;
+
 /// user-facing errors (reference FaissAssert.h:54-91 throws; invariants abort)
 class FaissException : public std::exception {
  public:
@@ -58,6 +60,10 @@ struct Index {
   virtual void reconstruct_n(idx_t i0, idx_t ni, float* recons) const {
     for (idx_t i = 0; i < ni; i++) reconstruct(i0 + i, recons + i * d);
   }
+
+  /// remove the entries whose id the selector holds; returns how many were removed (reference Index.h remove_ids;
+  /// selectors in AuxIndexStructures.h)
+  virtual long remove_ids(const IDSelector& /*sel*/) { VLQ_THROW_MSG("remove_ids not implemented for this type of index"); }
 
   /// labels of the k nearest neighbours (= search without the distances; reference Index.cpp:23-29)
   void assign(idx_t n, const float* x, idx_t* labels, idx_t k = 1);

@@ -2,7 +2,9 @@
 
 #include <cstring>
 #include <string>
+#include <vector>
 
+#include "AuxIndexStructures.h"
 #include "Clustering.h"
 #include "GpuIndexIMIPQ.h"
 #include "GpuIndexIVFPQ.h"
@@ -56,6 +58,22 @@ int vlq_host_index_search(void* index, long n, const float* x, long k, float* di
   GUARD(I(index)->search(n, x, k, distances, labels))
 }
 int vlq_host_index_reset(void* index) { GUARD(I(index)->reset()) }
+int vlq_host_index_remove_ids_range(void* index, long imin, long imax, long* nremoved) {
+  GUARD(*nremoved = I(index)->remove_ids(IDSelectorRange(imin, imax)))
+}
+int vlq_host_index_remove_ids_batch(void* index, long n, const long* ids, long* nremoved) {
+  GUARD({
+    VLQ_THROW_IF_NOT_MSG(n >= 0 && (n == 0 || ids), "remove_ids: n must be >= 0 and ids non-null when n > 0");
+    std::vector<long> staged;
+    if (n > 0 && vlq_pointer_is_device(ids) == 1) {  // IDSelectorBatch sorts on the host
+      staged.resize((size_t)n);
+      VLQ_CALL(vlq_memcpy_d2h(staged.data(), ids, (size_t)n * sizeof(long), nullptr));
+      VLQ_CALL(vlq_stream_synchronize(nullptr));
+      ids = staged.data();
+    }
+    *nremoved = I(index)->remove_ids(IDSelectorBatch(n, ids));
+  })
+}
 long vlq_host_index_ntotal(void* index) { return I(index)->ntotal; }
 int vlq_host_index_is_trained(void* index) { return I(index)->is_trained ? 1 : 0; }
 

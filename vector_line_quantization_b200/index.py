@@ -128,12 +128,39 @@ class Index:
     def reset(self):
         _call("vlq_host_index_reset", self.h)
 
+    def remove_ids(self, sel):
+        """faiss Index.remove_ids: sel is an IDSelectorRange or an int64 id array (numpy or torch, host or device; any
+        order, duplicates allowed).  Returns the number of entries removed.  GpuIndexIVFPQ and GpuIndexIMIPQ implement
+        it; the survivors keep their order inside their lists."""
+        out = C.c_long()
+        if isinstance(sel, IDSelectorRange):
+            _call("vlq_host_index_remove_ids_range", self.h, C.c_long(sel.imin), C.c_long(sel.imax), C.byref(out))
+            return out.value
+        if _is_torch(sel):
+            import torch
+
+            sel = sel.reshape(-1)
+            if sel.is_cuda:
+                torch.cuda.current_stream(sel.device).synchronize()  # the host layer copies it on its own stream
+        else:
+            sel = np.asarray(sel).reshape(-1)
+        p, keep, _ = _in(sel, np.int64)
+        _call("vlq_host_index_remove_ids_batch", self.h, C.c_long(sel.shape[0]), p, C.byref(out))
+        return out.value
+
     def __del__(self):
         try:
             if self.h:
                 host().vlq_host_index_free(self.h)
         except Exception:
             pass
+
+
+class IDSelectorRange:
+    """the ids imin <= id < imax (faiss IDSelectorRange), for Index.remove_ids"""
+
+    def __init__(self, imin, imax):
+        self.imin, self.imax = int(imin), int(imax)
 
 
 def _reconstruct_n(self, i0, ni):

@@ -154,6 +154,39 @@ def build_lists(nlists, M, new_list, new_codes, new_lamq, new_kappa, new_ids, ol
     return out
 
 
+def remove_ids(lists, ids=None, id_range=None):
+    """remove the entries whose id is in `ids` (int64, any order, duplicates allowed) or in the half-open
+    id_range = (lo, hi) from CSR lists (vlq_remove_ids_plan + vlq_remove_ids_apply) -> (Lists, removed).
+    Survivors keep their order inside a list; their code words are re-rotated to their new positions.  The result is
+    a new Lists at its exact size (peak memory: old + new slab); `lists` is left as it is."""
+    offsets = _chk(lists.offsets, torch.int64, "offsets")
+    dev = offsets.device
+    nlists = offsets.shape[0] - 1
+    n = lists.ids.shape[0]
+    M = lists.codes.shape[1]
+    batch = None
+    if ids is not None:
+        batch = torch.unique(torch.as_tensor(ids, dtype=torch.int64).reshape(-1).to(dev))  # sorted, de-duplicated
+    lo, hi = (int(id_range[0]), int(id_range[1])) if id_range is not None else (0, 0)
+    wsb = _abi.lib().vlq_remove_ids_workspace_bytes(n, nlists)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+    out_off = torch.empty(nlists + 1, dtype=torch.int64, device=dev)
+    nb = 0 if batch is None else batch.numel()
+    _abi.call("vlq_remove_ids_plan", nlists, n, _ptr(offsets), _ptr(_chk(lists.ids, torch.int64, "ids")), lo, hi,
+              _ptr(batch) if nb else 0, nb, _ptr(out_off), _ptr(ws), wsb, _stream())
+    live = int(out_off[-1])
+    # at least one row each: the apply pass takes non-NULL destinations even when nothing survives
+    rows = max(live, 1)
+    out = Lists(out_off, torch.empty((rows, M), dtype=torch.uint8, device=dev),
+                torch.empty(rows, dtype=torch.uint8, device=dev), torch.empty(rows, dtype=torch.float32, device=dev),
+                torch.empty(rows, dtype=torch.int64, device=dev))
+    _abi.call("vlq_remove_ids_apply", nlists, M, n, _ptr(offsets), _ptr(_chk(lists.codes, torch.uint8, "codes")),
+              _ptr(_chk(lists.lamq, torch.uint8, "lamq")), _ptr(_chk(lists.kappa, torch.float32, "kappa")),
+              _ptr(lists.ids), _ptr(out_off), _ptr(out.codes), _ptr(out.lamq), _ptr(out.kappa), _ptr(out.ids),
+              _ptr(ws), wsb, _stream())
+    return Lists(out_off, *(t[:live] for t in out[1:])), n - live
+
+
 def rotate_codes(offsets, codes, inverse=False):
     """canonical list-major codes [n][M] -> the stored layout (or back with inverse=True): the entry at position pos of
     its list keeps stored[j] = code[(j + pos) mod M] (csrc/scan.cuh).  Plumbing for callers that assemble Lists by hand
