@@ -259,6 +259,35 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
                   size_t workspace_bytes, vlq_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
+ * a15-range  radius search over the selected lines: every entry the scan above would look at (the first min(len, cap)
+ *     entries of each of the W lines in line_list, -1 slots skipped) whose distance is below `radius` (strict), in
+ *     stream order: lines in slot order, then list position.   replaces IndexIVF::range_search (IndexIVF.cpp) for the
+ *     line lists, which the reference GPU index lacks.
+ *     dist = term1 + l*term6 + (l*l-l)*term5 + kappa_i - 2 q.p(code_i) + row_add[q]   (row_add nullable; pass ||q||^2 for
+ *     the full squared L2 when term1 excludes it, as the VLQ coarse stage does; NULL when term1 = ||q - c||^2, IMI-PQ),
+ *     evaluated in fp32 from term-3 tables in a fixed order, each operation rounded as written: both passes compute the
+ *     same bits, and results do not depend on the list lengths.  edge_d2 NULL = lambda-hat 0.
+ *     pass 1 (count) builds the term-3 tables of the nq queries into the workspace, counts the survivors of every query
+ *       and writes out_lims[nq + 1] (exclusive prefix; out_lims[nq] = total, which the caller reads to size its output).
+ *     pass 2 (gather) reads the workspace pass 1 wrote, unchanged in between, and writes the results of the queries
+ *       [q0, q1) to outD / outI at lims[q] - lims[q0]: a large tile can be gathered in parts.
+ *     M <= 64, d % M == 0, 1 <= nL <= 256, 1 <= W <= VLQ_MAX_K, 1 <= cap <= 2^20, W * cap < 2^31; a NaN radius is
+ *     VLQ_EINVAL; pq and workspace 16-byte aligned.  VLQ_EUNSUPPORTED where the term-3 kernels do not take the shape
+ *     (d % 4 != 0, or d > 200).  Every argument is checked before the first launch.
+ * ---------------------------------------------------------------------------------------------------------------- */
+size_t vlq_range_workspace_bytes(int64_t nq, int M, int W, int cap);
+int vlq_range_count(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                    const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                    const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
+                    const float* row_add, float radius, int64_t* out_lims, void* workspace, size_t workspace_bytes,
+                    vlq_stream_t stream);
+int vlq_range_gather(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                     const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                     const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
+                     const float* row_add, float radius, const int64_t* ids, const int64_t* lims, int64_t q0, int64_t q1,
+                     float* outD, int64_t* outI, const void* workspace, size_t workspace_bytes, vlq_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------------------------
  * a16 shard merge: k smallest of R*k candidates per query; D, I are [R][nq][k] (the all-gather layout); shards with
  *     fewer than k results pad with (FLT_MAX, -1), as vlq_scan_topk does.
  *     replaces GpuIndexIVFPQ::merge / mergekernel, gpu/GpuIndexIVFPQ.cu:1467-1591 (CPU twin MetaIndexes.cpp:290-347).

@@ -30,6 +30,15 @@ int vlq_host_index_reset(void* index);
    the number of entries removed.  GpuIndexIVFPQ and GpuIndexIMIPQ implement it; other indexes fail (-1). */
 int vlq_host_index_remove_ids_range(void* index, long imin, long imax, long* nremoved);
 int vlq_host_index_remove_ids_batch(void* index, long n, const long* ids, long* nremoved);
+/* Index::range_search: every stored vector with squared L2 distance < radius for each of the n queries (x host or
+   device).  *result receives a RangeSearchResult handle: vlq_host_range_result_total gives lims[n] (the number of
+   results), vlq_host_range_result_copy writes any of lims [n + 1], distances and labels [total] (host memory; NULL
+   skips one) and vlq_host_range_result_free releases it.  GpuIndexIVFPQ and GpuIndexIMIPQ implement it; other indexes
+   fail (-1) and leave *result NULL. */
+int vlq_host_index_range_search(void* index, long n, const float* x, float radius, void** result);
+int vlq_host_range_result_total(void* result, long* total);
+int vlq_host_range_result_copy(void* result, long* lims, float* distances, long* labels);
+int vlq_host_range_result_free(void* result);
 long vlq_host_index_ntotal(void* index);
 int vlq_host_index_is_trained(void* index);
 

@@ -54,6 +54,10 @@ SIGNATURES = {
     "vlq_gather_candidates": (_i, [_p, _l, _i, _p, _p, _l, _p, _p]),
     "vlq_scan_topk_workspace_bytes": (_z, [_l, _i]),
     "vlq_scan_topk": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _z, _p]),
+    "vlq_range_workspace_bytes": (_z, [_l, _i, _i, _i]),
+    "vlq_range_count": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i, _p, _f, _p, _p, _z, _p]),
+    "vlq_range_gather": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i, _p, _f, _p, _p, _l, _l,
+                              _p, _p, _p, _z, _p]),
     "vlq_merge_topk": (_i, [_p, _p, _i, _l, _i, _p, _p, _p]),
     "vlq_merge_topk_peers": (_i, [_p, _z, _z, _i, _l, _i, _p, _p, _p]),
     "vlq_gather_peer_slices": (_i, [_p, _i, _i, _p, _i, _l, _l, _p]),

@@ -543,6 +543,11 @@ static RemWs carve_rem(void* ws, int64_t n) {
   return w;
 }
 
+int launch_exclusive_scan_i64(int64_t* v, int64_t n, cudaStream_t st) {
+  VLQ_LAUNCH(scan_tile_offsets_kernel, 1, SCAN_THREADS, 0, st, v, n);
+  return last_error();
+}
+
 }  // namespace vlq
 
 using namespace vlq;

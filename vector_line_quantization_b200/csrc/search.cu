@@ -262,55 +262,6 @@ coarse_select_lines_kernel(const float* __restrict__ D, int64_t ldD, const float
 }
 
 // ------------------------------------------------------------------------------------------------ scan + top-k
-// PQ codes of one entry held in registers (16-byte / 8-byte vector loads for M = 16 / 8; byte loads otherwise)
-// `pos` = position of the entry inside its list: the stored bytes are rotated by pos mod M (scan.cuh) and adc() sums the
-// sub-quantizers in canonical order m = 0..M-1, the order of the reference and of the oracle.
-template <int M_T>
-struct CodeRegs {
-  uint32_t w[M_T == 16 ? 4 : (M_T == 8 ? 2 : 1)];
-  const uint8_t* ptr;
-  int rot;
-  __device__ __forceinline__ void load(const uint8_t* __restrict__ code_ptr, int pos) {
-    if constexpr (M_T == 16) {
-      const uint4 c = ld_nc_v4(code_ptr);
-      w[0] = c.x; w[1] = c.y; w[2] = c.z; w[3] = c.w;
-      rot = (16 - (pos & 15)) & 15;
-    } else if constexpr (M_T == 8) {
-      const uint2 c = ld_nc_v2(code_ptr);
-      w[0] = c.x; w[1] = c.y;
-      rot = (8 - (pos & 7)) & 7;
-    } else {
-      ptr = code_ptr;
-      rot = pos;
-    }
-  }
-  __device__ __forceinline__ float adc(const float* __restrict__ T3, int M, int ksub) const {
-    float acc = 0.f;
-    if constexpr (M_T == 16) {
-      uint32_t r[4] = {w[0], w[1], w[2], w[3]};
-      rot16(r, rot);
-#pragma unroll
-      for (int t = 0; t < 4; t++)
-#pragma unroll
-        for (int b = 0; b < 4; b++) acc += T3[(t * 4 + b) * 256 + ((r[t] >> (8 * b)) & 0xff)];
-    } else if constexpr (M_T == 8) {
-      uint32_t r[2] = {w[0], w[1]};
-      rot8(r, rot);
-#pragma unroll
-      for (int t = 0; t < 2; t++)
-#pragma unroll
-        for (int b = 0; b < 4; b++) acc += T3[(t * 4 + b) * 256 + ((r[t] >> (8 * b)) & 0xff)];
-    } else {
-      int j = (M - rot % M) % M;  // stored[j] = code[(j + pos) mod M]  =>  code[m] = stored[(m - pos) mod M]
-      for (int m = 0; m < M; m++) {
-        acc += T3[m * ksub + ptr[j]];
-        j = j + 1 == M ? 0 : j + 1;
-      }
-    }
-    return acc;
-  }
-};
-
 // LONG = false: the selected lists are walked as ONE flattened entry stream (lists of a handful of entries keep all
 //               lanes busy);  LONG = true: every warp owns whole lists (slot w -> warp w % 8) and strides their entries,
 //               so the per-list scalars are warp-uniform and nothing has to be searched per entry.
@@ -740,6 +691,26 @@ term3_reg_kernel(const float* __restrict__ q, int64_t nq, const float* __restric
     __syncthreads();
     buf ^= 1;
   }
+}
+
+static size_t term3_pq_smem_bytes(int d) { return ((size_t)256 * d + d) * sizeof(float); }  // codebook + one query
+
+bool term3_supported(int d, int M) { return d > 0 && M > 0 && d % M == 0 && d % 4 == 0 && term3_pq_smem_bytes(d) <= 200 * 1024; }
+
+// persistent CTAs (at most one per SM) walk the queries of the batch
+int launch_term3(const float* q, int64_t nq, int d, const float* pq, int M, float* t3, bool code_major, cudaStream_t st) {
+  const unsigned grid = (unsigned)(nq < 148 ? nq : 148);
+  const int dsub = d / M;
+  if (M == 16 && dsub == 8) {
+    VLQ_LAUNCH((term3_reg_kernel<16, 8>), grid, T3_THREADS, 0, st, q, nq, pq, t3, code_major);
+  } else if (M == 8 && dsub == 12) {
+    VLQ_LAUNCH((term3_reg_kernel<8, 12>), grid, T3_THREADS, 0, st, q, nq, pq, t3, code_major);
+  } else {
+    const size_t pq_smem = term3_pq_smem_bytes(d);
+    VLQ_CUDA_TRY(cudaFuncSetAttribute(term3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pq_smem));
+    VLQ_LAUNCH(term3_kernel, grid, T3_THREADS, pq_smem, st, q, nq, d, pq, M, dsub, t3, code_major);
+  }
+  return VLQ_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ asynchronous scan
@@ -1336,10 +1307,9 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
   a.sel_cap = select_capacity(k, Q_THREADS, Q_BATCH, (long long)W * cap);
   a.t3 = nullptr;
   const size_t t3_bytes = (size_t)nq * M * 256 * sizeof(float);
-  const size_t pq_smem = ((size_t)M * 256 * a.dsub + d) * sizeof(float);
   const bool long_lists = list_len_hint >= 24;  // average list length of the index: warp-per-list pays off
   const bool al16 = (reinterpret_cast<uintptr_t>(codes) % 16) == 0;
-  const bool have_t3 = workspace && workspace_bytes >= t3_bytes + 256 && pq_smem <= 200 * 1024 && d % 4 == 0 &&
+  const bool have_t3 = workspace && workspace_bytes >= t3_bytes + 256 && term3_supported(d, M) &&
                        ((reinterpret_cast<uintptr_t>(workspace) | reinterpret_cast<uintptr_t>(pq)) & 15) == 0;
   const bool use_async = long_lists && k <= kWarpSelMaxK && have_t3 && (M * 256) % 4 == 0;  // warp-autonomous scan
   // bank-skewed tables pay off once the lists are long enough to amortise the 64 KB table fill and the four extra
@@ -1373,15 +1343,8 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
   const bool skew = use_long || (use_async && al16 && (M == 16 || M == 8) && list_len_hint >= skew_min_len);
   if (have_t3) {
     float* t3 = static_cast<float*>(workspace);
-    const unsigned grid = (unsigned)(nq < 148 ? nq : 148);
-    if (M == 16 && a.dsub == 8) {
-      VLQ_LAUNCH((term3_reg_kernel<16, 8>), grid, T3_THREADS, 0, as_stream(stream), q, nq, pq, t3, skew);
-    } else if (M == 8 && a.dsub == 12) {
-      VLQ_LAUNCH((term3_reg_kernel<8, 12>), grid, T3_THREADS, 0, as_stream(stream), q, nq, pq, t3, skew);
-    } else {
-      VLQ_CUDA_TRY(cudaFuncSetAttribute(term3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pq_smem));
-      VLQ_LAUNCH(term3_kernel, grid, T3_THREADS, pq_smem, as_stream(stream), q, nq, d, pq, M, a.dsub, t3, skew);
-    }
+    const int rc = launch_term3(q, nq, d, pq, M, t3, skew, as_stream(stream));
+    if (rc) return rc;
     a.t3 = t3;
   }
   a.owner_cap = (int)((long long)W * cap < 4096 ? (long long)W * cap : 4096);

@@ -1,6 +1,7 @@
 #include "GpuIndexIMIPQ.h"
 
 #include "ListRemoval.h"
+#include "RangeSearch.h"
 
 #include <algorithm>
 #include <cstring>
@@ -197,6 +198,24 @@ long GpuIndexIMIPQ::remove_ids(const IDSelector& sel) {
                                        ListSlab{lOffsets_, lCodes_, lLamq_, lKappa_, lIds_, nListed_});
   ntotal -= removed;
   return removed;
+}
+
+// the cells of cellsDevice_ are the lines; term1 = ||q - c||^2 already makes the distances full ones (row_add NULL)
+void GpuIndexIMIPQ::range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const {
+  VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
+  DeviceScope scope(resources_->getDevice());
+  if (n > 0) commit_();
+  vlq_stream_t st = resources_->getDefaultStream();
+  const int W = nprobe_;
+  RangeLists lists{dPq_.as<float>(), M_, dLambda_.as<float>(), 1, nullptr, W, listCap_, lOffsets_.as<int64_t>(),
+                   lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), lKappa_.as<float>(), lIds_.as<int64_t>(), nListed_, false,
+                   4096};
+  rangeSearchLists(resources_, d, n, x, radius, lists,
+                   [&](const float* dq, Index::idx_t m, int* cells, float* t1, float* t6) {
+                     cellsDevice_(dq, m, W, cells, t1);
+                     VLQ_CALL(vlq_memset(t6, 0, (size_t)m * W * sizeof(float), st));
+                   },
+                   result);
 }
 
 int GpuIndexIMIPQ::getListLength(long cell) const {

@@ -29,6 +29,9 @@ class GpuIndexIMIPQ : public faiss::Index {
   void reset() override;
   /// IndexIVF::remove_ids for IDSelectorRange / IDSelectorBatch, as GpuIndexIVFPQ::remove_ids (survivors keep their order)
   long remove_ids(const IDSelector& sel) override;
+  /// Index::range_search: every entry of the nprobe cells (first listCap_ of each) with ||q - x||^2 < radius, cells in
+  /// the order of searchCells, then list position; the same distances as search()
+  void range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const override;
 
   void setNumProbes(int nprobe);  ///< cells visited per query, 1 .. 1024
   int getNumProbes() const { return nprobe_; }

@@ -1,6 +1,7 @@
 #include "GpuIndexIVFPQ.h"
 
 #include "ListRemoval.h"
+#include "RangeSearch.h"
 
 #include <algorithm>
 #include <cfloat>
@@ -315,6 +316,32 @@ long GpuIndexIVFPQ::remove_ids(const IDSelector& sel) {
                                        ListSlab{lOffsets_, lCodes_, lLamq_, lKappa_, lIds_, nListed_});
   ntotal -= removed;
   return removed;
+}
+
+// same lines as search(): the coarse stage of a tile is vlq_coarse_lines (host/RangeSearch.cpp runs the rest)
+void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const {
+  VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
+  VLQ_THROW_IF_NOT_MSG(w1_ >= 1 && w1_ <= VLQ_MAX_K, "w1_ must be in [1, 1024]");
+  DeviceScope scope(ivfConfig_.device);
+  if (n > 0) commit_();
+  vlq_stream_t st = resources_->getDefaultStream();
+  const int P = std::min(nprobe_, nlist_);
+  const int W = w1_;
+  const Index::idx_t tile = std::max<Index::idx_t>(64, std::min<Index::idx_t>(5120, ((Index::idx_t)5 << 26) / nlist_));
+  DeviceBuffer coarseWs;
+  RangeLists lists{dPq_.as<float>(), subQuantizers_, dLambda_.as<float>(), nLambda_, dEdgeDist_.as<float>(), W, listCap_,
+                   lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), lKappa_.as<float>(),
+                   lIds_.as<int64_t>(), nListed_, true, tile};
+  rangeSearchLists(resources_, d, n, x, radius, lists,
+                   [&](const float* dq, Index::idx_t m, int* lines, float* t1, float* t6) {
+                     coarseWs.reserve(vlq_coarse_lines_workspace_bytes(m, d, nlist_, P, numedge_, W,
+                                                                       quantizer_->devicePack() != nullptr));
+                     VLQ_CALL(vlq_coarse_lines(dq, m, d, quantizer_->deviceVectors(), quantizer_->deviceNorms(),
+                                               quantizer_->devicePack(), quantizer_->packScale(), nlist_, P,
+                                               dEdge_.as<int>(), dEdgeDist_.as<float>(), numedge_, W, nullptr, lines,
+                                               t1, t6, coarseWs.get(), coarseWs.bytes(), st));
+                   },
+                   result);
 }
 
 // searchImpl_ -> IVFPQ::queryGraph (gpu/GpuIndexIVFPQ.cu:1400-1464, gpu/impl/IVFPQ.cu:685-775).  The coarse stage of a

@@ -84,6 +84,10 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   /// are committed first, then the lists are compacted.  Survivors keep their order inside a list, so the index equals
   /// one that never received the removed vectors (IndexIVF swaps in the last entry of the list instead).
   long remove_ids(const IDSelector& sel) override;
+  /// Index::range_search: every entry that search() scans (the first min(len, listCap_) of each of the w1_ lines) with
+  /// full squared distance ||q - x||^2 < radius -- unlike search(), whose distances exclude ||q||^2, a radius needs
+  /// the full value.  Per query: lines in slot order, then list position.  Pending adds are committed first.
+  void range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const override;
 
   void reserveMemory(size_t numVecs);
   void setPrecomputedCodes(bool) {}

@@ -12,6 +12,7 @@ namespace faiss {
 enum MetricType { METRIC_INNER_PRODUCT = 0, METRIC_L2 = 1 };
 
 struct IDSelector;
+struct RangeSearchResult;
 
 /// user-facing errors (reference FaissAssert.h:54-91 throws; invariants abort)
 class FaissException : public std::exception {
@@ -64,6 +65,13 @@ struct Index {
   /// remove the entries whose id the selector holds; returns how many were removed (reference Index.h remove_ids;
   /// selectors in AuxIndexStructures.h)
   virtual long remove_ids(const IDSelector& /*sel*/) { VLQ_THROW_MSG("remove_ids not implemented for this type of index"); }
+
+  /// every stored vector closer than `radius` to each query (reference Index.h range_search; METRIC_L2: squared
+  /// distance < radius).  result->nq == n; the index fills lims, labels and distances (RangeSearchResult,
+  /// AuxIndexStructures.h)
+  virtual void range_search(idx_t /*n*/, const float* /*x*/, float /*radius*/, RangeSearchResult* /*result*/) const {
+    VLQ_THROW_MSG("range_search not implemented for this type of index");
+  }
 
   /// labels of the k nearest neighbours (= search without the distances; reference Index.cpp:23-29)
   void assign(idx_t n, const float* x, idx_t* labels, idx_t k = 1);

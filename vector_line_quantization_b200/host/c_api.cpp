@@ -74,6 +74,36 @@ int vlq_host_index_remove_ids_batch(void* index, long n, const long* ids, long* 
     *nremoved = I(index)->remove_ids(IDSelectorBatch(n, ids));
   })
 }
+int vlq_host_index_range_search(void* index, long n, const float* x, float radius, void** result) {
+  GUARD({
+    VLQ_THROW_IF_NOT_MSG(result != nullptr && n >= 0, "range_search: n must be >= 0 and result non-null");
+    *result = nullptr;
+    RangeSearchResult* r = new RangeSearchResult(n);
+    try {
+      I(index)->range_search(n, x, radius, r);
+    } catch (...) {
+      delete r;
+      throw;
+    }
+    *result = r;
+  })
+}
+static RangeSearchResult* R(void* h) {
+  if (!h) throw FaissException("null range search result");
+  return static_cast<RangeSearchResult*>(h);
+}
+int vlq_host_range_result_total(void* result, long* total) { GUARD(*total = (long)R(result)->lims[R(result)->nq]) }
+int vlq_host_range_result_copy(void* result, long* lims, float* distances, long* labels) {
+  GUARD({
+    const RangeSearchResult* r = R(result);
+    const size_t total = r->lims[r->nq];
+    if (lims)
+      for (size_t i = 0; i <= r->nq; i++) lims[i] = (long)r->lims[i];
+    if (distances && total) std::memcpy(distances, r->distances, total * sizeof(float));
+    if (labels && total) std::memcpy(labels, r->labels, total * sizeof(long));
+  })
+}
+int vlq_host_range_result_free(void* result) { GUARD(delete static_cast<RangeSearchResult*>(result)) }
 long vlq_host_index_ntotal(void* index) { return I(index)->ntotal; }
 int vlq_host_index_is_trained(void* index) { return I(index)->is_trained ? 1 : 0; }
 

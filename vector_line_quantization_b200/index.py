@@ -125,6 +125,26 @@ class Index:
         _call("vlq_host_index_search", self.h, C.c_long(n), p, C.c_long(k), pd, pi)
         return D, I
 
+    def range_search(self, x, radius):
+        """faiss Index.range_search: every stored vector with squared L2 distance < radius -> (lims int64 [n + 1],
+        D f32 [total], I int64 [total]) numpy arrays; the results of query i are D / I[lims[i]:lims[i + 1]].
+        x is numpy or torch (host or device).  GpuIndexIVFPQ and GpuIndexIMIPQ implement it."""
+        p, keep, _ = _in(x, np.float32)
+        n = x.shape[0]
+        res = C.c_void_p()
+        _call("vlq_host_index_range_search", self.h, C.c_long(n), p, C.c_float(radius), C.byref(res))
+        try:
+            total = C.c_long()
+            _call("vlq_host_range_result_total", res, C.byref(total))
+            lims = np.empty(n + 1, np.int64)
+            D = np.empty(total.value, np.float32)
+            I = np.empty(total.value, np.int64)
+            _call("vlq_host_range_result_copy", res, C.c_void_p(lims.ctypes.data), C.c_void_p(D.ctypes.data),
+                  C.c_void_p(I.ctypes.data))
+        finally:
+            host().vlq_host_range_result_free(res)
+        return lims, D, I
+
     def reset(self):
         _call("vlq_host_index_reset", self.h)
 

@@ -256,6 +256,70 @@ def scan_topk(q, pq, lambda_cb, line_list, term1, term6, edge_d2, lists, k, cap=
     return outD, outI
 
 
+def range_scan_lines(q, pq, lambda_cb, lines, edge_d2, lists, radius, cap=1024, row_add=None, tile=5120,
+                     stage_results=None):
+    """Radius search over the selected lines (a15-range, vlq_range_count + vlq_range_gather): every entry the scan would
+    look at whose distance (+ row_add[q], e.g. ||q||^2 for the full squared L2) is < radius, per query in stream order
+    (lines in slot order, then list position) -> (lims int64 [nq + 1], D f32 [total], I int64 [total]), CUDA tensors.
+    stage_results: gather each tile in query sub-ranges of at most this many results (one query at least)."""
+    q = _chk(q, torch.float32, "q")
+    pq = _chk(pq, torch.float32, "pq")
+    nq, d = q.shape
+    M = pq.shape[0]
+    lst, t1, t6 = lines
+    W = lst.shape[1]
+    dev = q.device
+    ed2 = None if edge_d2 is None else edge_d2.reshape(-1)
+    lims = [torch.zeros(1, dtype=torch.int64, device=dev)]
+    outD, outI = [], []
+    tile = _tile_rows(nq, tile)
+    ws = torch.empty(max(_abi.lib().vlq_range_workspace_bytes(tile, M, W, cap), 256), dtype=torch.uint8, device=dev)
+    lt = torch.empty(tile + 1, dtype=torch.int64, device=dev)
+    done = 0
+    for s in range(0, nq, tile):
+        e = min(nq, s + tile)
+        m = e - s
+        args = (_ptr(q[s:e]), m, d, _ptr(pq), M, _ptr(lambda_cb), lambda_cb.shape[0],
+                _ptr(_chk(lst[s:e], torch.int32, "line_list")), _ptr(t1[s:e]), _ptr(t6[s:e]), _ptr(ed2), W,
+                _ptr(lists.offsets), _ptr(lists.codes), _ptr(lists.lamq), _ptr(lists.kappa), cap,
+                _ptr(None if row_add is None else row_add[s:e]), float(radius))
+        _abi.call("vlq_range_count", *args, _ptr(lt), _ptr(ws), ws.numel(), _stream())
+        hl = lt[:m + 1].cpu()
+        total = int(hl[m])
+        D = torch.empty(max(total, 1), dtype=torch.float32, device=dev)
+        I = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
+        q0 = 0
+        while q0 < m:
+            q1 = q0 + 1
+            if stage_results is None:
+                q1 = m
+            while q1 < m and int(hl[q1 + 1] - hl[q0]) <= stage_results:
+                q1 += 1
+            o = int(hl[q0])
+            if int(hl[q1]) == o:  # no results in [q0, q1): nothing to write (and an empty slice has no address)
+                q0 = q1
+                continue
+            _abi.call("vlq_range_gather", *args, _ptr(lists.ids), _ptr(lt), q0, q1, _ptr(D[o:]), _ptr(I[o:]), _ptr(ws),
+                      ws.numel(), _stream())
+            q0 = q1
+        lims.append(hl[1:].to(dev) + done)
+        outD.append(D[:total])
+        outI.append(I[:total])
+        done += total
+    return torch.cat(lims), (torch.cat(outD) if outD else torch.empty(0, device=dev)), \
+        (torch.cat(outI) if outI else torch.empty(0, dtype=torch.int64, device=dev))
+
+
+def range_search(q, cent, cnorm, edge, edge_d2, lambda_cb, pq, lists, P, W, radius, cap=1024, tile=5120, pack=None,
+                 stage_results=None):
+    """Full radius query (a11 + a12 + a15-range) on resident tensors: the lines of ops.search, then every entry of them
+    with full squared distance ||q - x||^2 < radius -> (lims int64 [nq + 1], D f32 [total], I int64 [total])"""
+    q = _chk(q, torch.float32, "q")
+    lines = coarse_lines(q, cent, cnorm, edge, edge_d2, P, W, tile=tile, pack=pack)
+    return range_scan_lines(q, pq, lambda_cb, lines, edge_d2, lists, radius, cap=cap, row_add=row_norms(q), tile=tile,
+                            stage_results=stage_results)
+
+
 def merge_topk(D, I):
     """shard merge (a16): D, I are [R][nq][k] -> (nq,k)"""
     D = _chk(D, torch.float32, "D")
