@@ -272,8 +272,9 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
  *     pass 2 (gather) reads the workspace pass 1 wrote, unchanged in between, and writes the results of the queries
  *       [q0, q1) to outD / outI at lims[q] - lims[q0]: a large tile can be gathered in parts.
  *     M <= 64, d % M == 0, 1 <= nL <= 256, 1 <= W <= VLQ_MAX_K, 1 <= cap <= 2^20, W * cap < 2^31; a NaN radius is
- *     VLQ_EINVAL; pq and workspace 16-byte aligned.  VLQ_EUNSUPPORTED where the term-3 kernels do not take the shape
- *     (d % 4 != 0, or d > 200).  Every argument is checked before the first launch.
+ *     VLQ_EINVAL; pq and workspace 16-byte aligned.  VLQ_EUNSUPPORTED where the term-3 kernels do not take the shape:
+ *     d % 4 != 0, or the codebook plus one query (1028 d bytes) beyond 200 KiB of shared memory, i.e. d > 196 (GloVe-200
+ *     is refused).  Every argument is checked before the first launch.
  * ---------------------------------------------------------------------------------------------------------------- */
 size_t vlq_range_workspace_bytes(int64_t nq, int M, int W, int cap);
 int vlq_range_count(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,

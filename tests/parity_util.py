@@ -1,4 +1,4 @@
-"""Per-mismatch near-tie verification for the query path (north_star: "identical except documented near-ties,
+"""Per-mismatch near-tie verification for the encode and query paths (north_star: "identical except documented near-ties,
 relative distance gap < 1e-5").  Every id / line that differs from the oracle is re-evaluated in float64 from the
 codebooks and must be closer to the oracle's choice than REL_TIE; nothing is accepted as a fraction.
 
@@ -106,3 +106,111 @@ def check_topk(D, I, Do, Io, xq, m, entry_line, entry_lamq, entry_codes, same_li
     same = (I == Io) & (I >= 0)
     assert np.all(np.abs(D - Do)[same] <= rel_dist * (np.abs(Do) + qn[:, None])[same])
     return int(diff.sum()), int((~same_lines).sum())
+
+
+def _np(t):
+    return t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+
+
+def check_encode(enc, o, x, m):
+    """line_encode's outputs (enc, an ops.Encoded with residual) against the oracle's encode o of the same vectors x and
+    assignment: lines, lambda bytes and PQ codes identical except near-ties, each verified in float64; residuals close
+    wherever line and lambda byte agree.  Returns the mask of those vectors."""
+    lst, lam, lamq, codes = _np(enc.list), _np(enc.lam), _np(enc.lamq), _np(enc.codes)
+    n = x.shape[0]
+    same_line = lst == o["list"]
+    assert same_line.mean() > 0.999, same_line.mean()
+    # mismatching lines must be near-ties in point-to-line distance
+    x64, c64 = x.astype(np.float64), m["cent"].astype(np.float64)
+    E = m["edge"].shape[1]
+
+    def line_q2(i, l):
+        a = c64[l // E]
+        s = c64[m["edge"][l // E, l % E]]
+        t = np.dot(x64[i] - a, s - a) / np.dot(s - a, s - a)
+        return np.sum((x64[i] - (a + t * (s - a))) ** 2)
+
+    for i in np.nonzero(~same_line)[0]:
+        qa, qb = line_q2(i, lst[i]), line_q2(i, o["list"][i])
+        assert abs(qa - qb) <= 1e-4 * max(qa, qb) + 1e-6, (i, qa, qb)
+    ok = same_line
+    np.testing.assert_allclose(lam[ok], o["lam"][ok], rtol=1e-3, atol=1e-4)
+    same_lq = ok & (lamq == o["lamq"])
+    assert same_lq.sum() >= ok.sum() - max(2, n // 500)  # lambda exactly between two levels
+    # PQ codes identical wherever line and lambda level agree, except sub-space near-ties
+    cm = codes[same_lq] != o["codes"][same_lq]
+    assert cm.mean() < 2e-4, cm.mean()
+    M = codes.shape[1]
+    dsub = x.shape[1] // M
+    rows = np.nonzero(same_lq)[0]
+    for ri, mm in np.argwhere(cm):
+        i = rows[ri]
+        sub = o["residual"][i, mm * dsub:(mm + 1) * dsub].astype(np.float64)
+        da = np.sum((sub - m["pq"][mm, codes[i, mm]]) ** 2)
+        db = np.sum((sub - m["pq"][mm, o["codes"][i, mm]]) ** 2)
+        assert abs(da - db) <= REL_TIE * max(da, db) + 1e-9
+    res = _np(enc.residual)
+    np.testing.assert_allclose(res[same_lq], o["residual"][same_lq], rtol=1e-5, atol=1e-3)
+    return same_lq
+
+
+def scan_candidates(q, lines, term1, term6, t5, lambda_cb, pq, offsets, codes, lamq, kappa, ids, cap):
+    """float64 restatement of the scan distance of include/vlq_b200.h (vlq_scan_topk) from the kernel's own inputs:
+        dist = t1 + l t6 + (l^2 - l) t5 + kappa - 2 q.p(code),   l = lambda_cb[lamq]
+    over the entries the scan looks at: the first min(len, cap) entries of every selected line (-1 slots skipped), lines
+    in slot order, then list position.  t5: per list id (edge_d2 flattened), or None for 0.  codes: list-major and in
+    canonical sub-quantizer order (not rotated).  No VLQ geometry enters, so IMI-PQ inputs (t1 a full distance, t6 = 0,
+    no t5) work the same.  Returns per query (dist float64 [n_q], ids int64 [n_q]) in stream order."""
+    q = np.asarray(q, np.float64)
+    pq = np.asarray(pq, np.float64)
+    lcb = np.asarray(lambda_cb, np.float64)
+    M, _, dsub = pq.shape
+    out = []
+    for i in range(q.shape[0]):
+        T3 = -2.0 * np.einsum("mjt,mt->mj", pq, q[i].reshape(M, dsub))
+        d_parts, i_parts = [], []
+        for w, l in enumerate(lines[i]):
+            if l < 0:
+                continue
+            s = int(offsets[l])
+            e = s + min(int(offsets[l + 1]) - s, cap)
+            la = lcb[lamq[s:e]]
+            base = float(term1[i, w]) + la * float(term6[i, w]) + (la * la - la) * (0.0 if t5 is None else float(t5[l]))
+            d_parts.append(base + kappa[s:e].astype(np.float64) + T3[np.arange(M), codes[s:e]].sum(1))
+            i_parts.append(ids[s:e])
+        out.append((np.concatenate(d_parts) if d_parts else np.empty(0), np.concatenate(i_parts).astype(np.int64)
+                    if i_parts else np.empty(0, np.int64)))
+    return out
+
+
+def check_scan_topk(D, I, cands, k, qn, rel=REL_TIE, rel_dist=REL_DIST):
+    """a scan's top-k (D, I) [nq][k] against the float64 candidates of scan_candidates (qn: ||q||^2, the scale of the
+    cancelled term, as in check_topk):
+    * min(k, candidates) results, then (FLT_MAX, -1) padding; rows ascending;
+    * every returned distance within rel_dist of the float64 distance of its id;
+    * every rank whose id differs from the float64 top-k is a near-tie (rel);
+    * a float64 top-k id that is missing ties the k-th float64 distance."""
+    D, I = np.asarray(D), np.asarray(I)
+    fmax = np.finfo(np.float32).max
+    assert np.all(np.diff(D, axis=1) >= 0), "distances not ascending"
+    for i, (dc, ic) in enumerate(cands):
+        nv = min(k, len(ic))
+        assert np.all(I[i, :nv] >= 0) and np.all(I[i, nv:] == -1) and np.all(D[i, nv:] == fmax), ("padding", i, nv)
+        if nv == 0:
+            continue
+        scale = qn[i]
+        d64 = dict(zip(ic.tolist(), dc.tolist()))
+        got = np.array([d64[v] for v in I[i, :nv].tolist()])
+        err = np.abs(D[i, :nv] - got)
+        assert np.all(err <= rel_dist * (np.abs(got) + scale)), ("distance", i, float(err.max()))
+        order = np.argsort(dc, kind="stable")[:nv]
+        ref_i, ref_d = ic[order], dc[order]
+        r = np.nonzero(I[i, :nv] != ref_i)[0]
+        bad = np.abs(got[r] - ref_d[r]) > rel * (np.abs(ref_d[r]) + scale)
+        assert not bad.any(), ("unexplained id mismatch (query, rank, id, ref id, d64, ref d64)",
+                               [(i, int(x), int(I[i, x]), int(ref_i[x]), got[x], ref_d[x]) for x in r[bad][:5]])
+        missing = np.setdiff1d(ref_i, I[i, :nv])
+        if len(missing):
+            dm = np.array([d64[v] for v in missing.tolist()])
+            kth = ref_d[nv - 1]
+            assert np.all(np.abs(dm - kth) <= rel * (np.abs(kth) + scale)), ("missing id", i, missing[:5])

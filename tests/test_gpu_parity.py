@@ -8,6 +8,8 @@ import os
 import numpy as np
 import pytest
 
+from tests.parity_util import check_encode
+
 pytestmark = pytest.mark.gpu
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "vlq_small.npz")
@@ -141,50 +143,11 @@ def _encode_both(ops, cuda, oracle, x, m, use_oracle_assign=True):
     return enc, dict(A=A, list=lst, lam=lam, lamq=lamq, residual=r, codes=codes)
 
 
-def _check_encode(enc, o, x, m):
-    lst, lam, lamq, codes = N(enc.list), N(enc.lam), N(enc.lamq), N(enc.codes)
-    n = x.shape[0]
-    same_line = lst == o["list"]
-    assert same_line.mean() > 0.999, same_line.mean()
-    # mismatching lines must be near-ties in point-to-line distance
-    x64, c64 = x.astype(np.float64), m["cent"].astype(np.float64)
-    E = m["edge"].shape[1]
-
-    def line_q2(i, l):
-        a = c64[l // E]
-        s = c64[m["edge"][l // E, l % E]]
-        t = np.dot(x64[i] - a, s - a) / np.dot(s - a, s - a)
-        return np.sum((x64[i] - (a + t * (s - a))) ** 2)
-
-    for i in np.nonzero(~same_line)[0]:
-        qa, qb = line_q2(i, lst[i]), line_q2(i, o["list"][i])
-        assert abs(qa - qb) <= 1e-4 * max(qa, qb) + 1e-6, (i, qa, qb)
-    ok = same_line
-    np.testing.assert_allclose(lam[ok], o["lam"][ok], rtol=1e-3, atol=1e-4)
-    same_lq = ok & (lamq == o["lamq"])
-    assert same_lq.sum() >= ok.sum() - max(2, n // 500)  # lambda exactly between two levels
-    # PQ codes identical wherever line and lambda level agree, except sub-space near-ties
-    cm = codes[same_lq] != o["codes"][same_lq]
-    assert cm.mean() < 2e-4, cm.mean()
-    M = codes.shape[1]
-    dsub = x.shape[1] // M
-    rows = np.nonzero(same_lq)[0]
-    for ri, mm in np.argwhere(cm):
-        i = rows[ri]
-        sub = o["residual"][i, mm * dsub:(mm + 1) * dsub].astype(np.float64)
-        da = np.sum((sub - m["pq"][mm, codes[i, mm]]) ** 2)
-        db = np.sum((sub - m["pq"][mm, o["codes"][i, mm]]) ** 2)
-        assert abs(da - db) <= REL_TIE * max(da, db) + 1e-9
-    res = N(enc.residual)
-    np.testing.assert_allclose(res[same_lq], o["residual"][same_lq], rtol=1e-5, atol=1e-3)
-    return same_lq
-
-
 def test_line_encode_matches_oracle(ops, cuda, oracle, small_model):
     m = small_model
     x = m["xb"][:7001]  # ragged: not a multiple of the CTA's 16 warps
     enc, o = _encode_both(ops, cuda, oracle, x, m)
-    same = _check_encode(enc, o, x, m)
+    same = check_encode(enc, o, x, m)
     # kappa = ||p||^2 + 2 anchor.p  (DESIGN.md): check against float64
     kap = N(enc.kappa)
     E, M = m["E"], m["M"]
@@ -231,7 +194,7 @@ def test_line_encode_d96_m8_e64(ops, cuda, oracle):
     m = oracle.train_all(xt, nlist=128, E=64, M=8, nL=256, niter=5, pq_niter=5)
     x = data.deep_like(3000, kc=256, seed=6)
     enc, o = _encode_both(ops, cuda, oracle, x, m)
-    _check_encode(enc, o, x, m)
+    check_encode(enc, o, x, m)
 
 
 # ------------------------------------------------------------------------------------------------ lists (a9)

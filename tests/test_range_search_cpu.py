@@ -66,6 +66,7 @@ def test_count_argument_checks(lib):
     # shapes the term-3 kernels do not take
     assert count(lib, d=102, M=2) == VLQ_EUNSUPPORTED  # d % 4
     assert count(lib, d=256, M=32) == VLQ_EUNSUPPORTED  # codebook beyond the kernel's shared memory
+    assert count(lib, d=200, M=8) == VLQ_EUNSUPPORTED  # 1028 d = 205 600 B > 200 KiB: d <= 196 only
     # nq = 0 needs no inputs: only lims[0] = 0 is written (that reaches the device, so it is tested on the GPU)
 
 
@@ -80,6 +81,7 @@ def test_gather_argument_checks(lib):
         assert gather(lib, q0=q0, q1=q1) == VLQ_EINVAL, (q0, q1)
     assert gather(lib, ws_bytes=lib.vlq_range_workspace_bytes(100, 16, 64, 1024) - 1) == VLQ_EWORKSPACE
     assert gather(lib, d=102, M=2) == VLQ_EUNSUPPORTED
+    assert gather(lib, d=200, M=8) == VLQ_EUNSUPPORTED
     # an empty query range launches nothing, so its outputs may be NULL
     assert gather(lib, q0=7, q1=7, ids=None, lims=None, oD=None, oI=None) == 0
     assert gather(lib, nq=0, q=None, pq=None, lcb=None, lines=None, t1=None, t6=None, off=None, codes=None, lamq=None,
