@@ -168,6 +168,31 @@ int vlq_remove_ids_apply(int64_t nlists, int M, int64_t n, const int64_t* offset
                          uint8_t* out_codes, uint8_t* out_lamq, float* out_kappa, int64_t* out_ids,
                          const void* workspace, size_t workspace_bytes, vlq_stream_t stream);
 
+/* a9 (read-back): id lookup and decode of stored entries (Index::reconstruct / reconstruct_n / search_and_reconstruct,
+ *     IndexIVFPQ::reconstruct_from_offset in the reference).
+ *     vlq_lookup_ids: one pass over ids[n]; out_pos[slot] = the LOWEST slab index whose id maps to the slot, -1 if none;
+ *       *out_found (one int64 on the device) = the number of slots found.  keys == NULL: range mode, slot = id - range_lo
+ *       for range_lo <= id < range_lo + nslots.  keys != NULL: batch mode, keys[nslots] sorted ascending and unique, slot
+ *       = index of the id in keys.  There is no persistent id -> slab map: every call reads the ids once.
+ *     vlq_decode_entries (VLQ) / vlq_imi_decode_entries (IMI-PQ, nlists = 2^(2 nbits), cell l = i1 | i2 << nbits):
+ *       out_x[i][j] = anchor_j + pq[m][code_m][j - m dsub], m = j / dsub, of the entry at slab index pos[i] of list l
+ *       (offsets[l] <= pos[i] < offsets[l + 1]), its stored code bytes un-rotated by (pos[i] - offsets[l]) mod M;
+ *         VLQ anchor = (1 - lh) cent[l / E] + lh cent[edge[l]], lh = lambda_cb[lamq[pos[i]]]   (nlists = C E)
+ *         IMI anchor = [cb1[i1] | cb2[i2]]   (cb1, cb2: [2^nbits][d / 2])
+ *       fp32, each operation rounded as written (no fma contraction), summed in the order shown: a lambda codebook {0}
+ *       gives exactly c + p (IndexIVFPQ's decode).  pos[i] = -1 (or outside the slab) gives a row of NaN (all-ones bits)
+ *       and out_ids[i] = -1.  out_ids (nullable) = ids[pos[i]]; it may alias pos (the scan's slab-index output turned
+ *       into labels in place).  M <= 64, d % M == 0 (IMI: d even). */
+int vlq_lookup_ids(int64_t n, const int64_t* ids, int64_t range_lo, const int64_t* keys, int64_t nslots, int64_t* out_pos,
+                   int64_t* out_found, vlq_stream_t stream);
+int vlq_decode_entries(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets, const uint8_t* codes,
+                       const uint8_t* lamq, const int64_t* ids, int M, int d, const float* pq, const float* cent,
+                       const int* edge, int E, const float* lambda_cb, int nL, float* out_x, int64_t* out_ids,
+                       vlq_stream_t stream);
+int vlq_imi_decode_entries(int64_t n, const int64_t* pos, const int64_t* offsets, const uint8_t* codes,
+                           const int64_t* ids, int M, int d, const float* pq, const float* cb1, const float* cb2,
+                           int nbits, float* out_x, int64_t* out_ids, vlq_stream_t stream);
+
 /* a9 (loader): per-entry kappa = ||p||^2 + 2 anchor.p for list-major entries that arrive without it, i.e. lists read
  *     from the reference's .dbIdx/.dbcodes/.dbcount/.dblas files (gpu/GpuIndexIVFPQ.cu:1813-2010). */
 int vlq_recompute_kappa(int64_t n, int64_t nlists, const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq,
@@ -242,6 +267,9 @@ int vlq_gather_candidates(const int* line_list, int64_t nq, int W, const int64_t
  *     over the first min(len, cap) entries of each selected list; k smallest ascending, padded (FLT_MAX, -1).
  *     edge_d2 is indexed by list id (term5); NULL = 0 (an index whose lambda codebook is {0}: stock IVFPQ / IMI-PQ).
  *     k <= VLQ_MAX_K, W <= VLQ_MAX_K.
+ *     ids == NULL: outI receives each result's SLAB index (the entry's position in codes / lamq / kappa) instead of its
+ *     id; selection does not depend on ids, so distances and order are unchanged.  search_and_reconstruct decodes the
+ *     exact entries found this way (vlq_decode_entries), which ids alone cannot name when an id is stored twice.
  *     list_len_hint: average list length of the index (entries / lists; 0 = unknown).  >= 24 selects the
  *     warp-per-list walk (1B-scale lists), otherwise the flattened entry stream (lists of a few entries).  Results are
  *     identical either way.

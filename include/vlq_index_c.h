@@ -46,6 +46,12 @@ int vlq_host_index_is_trained(void* index);
 int vlq_host_flat_new(void* res, int d, int use_tensor_cores, void** out);
 int vlq_host_flat_assign(void* flat, long n, const float* x, int* labels);
 int vlq_host_index_reconstruct_n(void* index, long i0, long ni, float* recons); /* Index::reconstruct_n; throws (-1) where undecodable */
+/* Index::reconstruct_batch: the stored vectors of keys[0 .. n) (ids, any order) into recons [n][d]; a key without an
+   entry fails (-1) and nothing is written.  Index::search_and_reconstruct: search plus the vector behind every label,
+   recons [n][k][d], NaN rows for label -1.  Pointers may be host or device memory for GpuIndexIVFPQ / GpuIndexIMIPQ. */
+int vlq_host_index_reconstruct_batch(void* index, long n, const long* keys, float* recons);
+int vlq_host_index_search_and_reconstruct(void* index, long n, const float* x, long k, float* distances, long* labels,
+                                          float* recons);
 int vlq_host_flat_search_int(void* flat, long n, const float* x, long k, float* distances, int* labels); /* searchInt */
 /* assign1Base: device pointers only; line id (assign2 = A*numedge + e) and float lambda of every row */
 int vlq_host_flat_assign1_base(void* flat, long n, const float* d_input, const int* d_assign1, int* d_assign2,

@@ -42,6 +42,9 @@ SIGNATURES = {
     "vlq_remove_ids_workspace_bytes": (_z, [_l, _l]),
     "vlq_remove_ids_plan": (_i, [_l, _l, _p, _p, _l, _l, _p, _l, _p, _p, _z, _p]),
     "vlq_remove_ids_apply": (_i, [_l, _i, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _z, _p]),
+    "vlq_lookup_ids": (_i, [_l, _p, _l, _p, _l, _p, _p, _p]),
+    "vlq_decode_entries": (_i, [_l, _p, _l, _p, _p, _p, _p, _i, _i, _p, _p, _p, _i, _p, _i, _p, _p, _p]),
+    "vlq_imi_decode_entries": (_i, [_l, _p, _p, _p, _p, _i, _i, _p, _p, _p, _i, _p, _p, _p]),
     "vlq_recompute_kappa": (_i, [_l, _l, _p, _p, _p, _p, _i, _p, _i, _p, _p, _i, _p, _p]),
     "vlq_select_lines": (_i, [_p, _l, _l, _p, _i, _p, _p, _i, _i, _p, _p, _p, _p]),
     "vlq_coarse_select_lines": (_i, [_p, _l, _l, _p, _i, _i, _i, _p, _p, _i, _i, _p, _p, _p, _p, _p]),

@@ -394,16 +394,21 @@ constexpr int REM_WORDS = SCAN_THREADS;  // one mask word per thread
 constexpr int REM_TILE = REM_WORDS * kWarp;
 constexpr int REM_LISTS = 1024;          // list starts a tile of the apply pass keeps in shared memory
 
-__device__ __forceinline__ bool removed_id(int64_t id, int64_t lo, int64_t hi, const int64_t* __restrict__ batch,
-                                           int64_t nb) {
-  if (id >= lo && id < hi) return true;
-  if (nb == 0 || id < batch[0] || id > batch[nb - 1]) return false;
+// index of id in the sorted batch[0 .. nb), or -1
+__device__ __forceinline__ int64_t batch_slot(int64_t id, const int64_t* __restrict__ batch, int64_t nb) {
+  if (nb == 0 || id < batch[0] || id > batch[nb - 1]) return -1;
   int64_t a = 0, b = nb;  // lower bound of id in the sorted batch
   while (a < b) {
     const int64_t mid = (a + b) >> 1;
     if (batch[mid] < id) a = mid + 1; else b = mid;
   }
-  return batch[a] == id;
+  return batch[a] == id ? a : -1;
+}
+
+__device__ __forceinline__ bool removed_id(int64_t id, int64_t lo, int64_t hi, const int64_t* __restrict__ batch,
+                                           int64_t nb) {
+  if (id >= lo && id < hi) return true;
+  return batch_slot(id, batch, nb) >= 0;
 }
 
 // largest l in [lo, hi] with offsets[l] <= p (offsets[lo] <= p)
@@ -543,6 +548,128 @@ static RemWs carve_rem(void* ws, int64_t n) {
   return w;
 }
 
+// ------------------------------------------------------------------------------------------------ entry lookup / decode
+// Lookup: one pass over ids[n]; the slot of an id is id - lo (range) or its index in the sorted keys (batch), and the
+// slot keeps the lowest slab index that carries it (atomicMin: the result does not depend on the schedule).  There is
+// no id -> slab map to keep in step with add / remove_ids: a lookup costs one read of the ids.
+constexpr int64_t kNoPos = INT64_MAX;
+constexpr int LOOKUP_UNROLL = 4;
+
+__global__ void lookup_init_kernel(int64_t* __restrict__ out_pos, int64_t nslots,
+                                   unsigned long long* __restrict__ found) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nslots; i += stride) out_pos[i] = kNoPos;
+  if (blockIdx.x == 0 && threadIdx.x == 0) *found = 0;
+}
+
+__global__ void __launch_bounds__(SCAN_THREADS)
+lookup_mark_kernel(int64_t n, const int64_t* __restrict__ ids, int64_t lo, int64_t nslots,
+                   const int64_t* __restrict__ keys, int64_t* __restrict__ out_pos) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t e0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e0 < n; e0 += stride * LOOKUP_UNROLL) {
+    int64_t id[LOOKUP_UNROLL];
+#pragma unroll
+    for (int u = 0; u < LOOKUP_UNROLL; u++) {  // the loads of all four entries first
+      const int64_t e = e0 + u * stride;
+      id[u] = e < n ? ids[e] : 0;
+    }
+#pragma unroll
+    for (int u = 0; u < LOOKUP_UNROLL; u++) {
+      const int64_t e = e0 + u * stride;
+      if (e >= n) break;
+      int64_t slot;
+      if (keys) {
+        slot = batch_slot(id[u], keys, nslots);
+      } else {  // id - lo in unsigned arithmetic: no overflow for any lo <= id
+        slot = (id[u] >= lo && (uint64_t)id[u] - (uint64_t)lo < (uint64_t)nslots) ? id[u] - lo : -1;
+      }
+      if (slot >= 0) atomicMin(reinterpret_cast<long long*>(out_pos + slot), (long long)e);
+    }
+  }
+}
+
+__global__ void __launch_bounds__(SCAN_THREADS)
+lookup_finish_kernel(int64_t* __restrict__ out_pos, int64_t nslots, unsigned long long* __restrict__ found) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  unsigned long long cnt = 0;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nslots; i += stride) {
+    if (out_pos[i] == kNoPos) out_pos[i] = -1;
+    else cnt++;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(kFull, cnt, o);
+  if ((threadIdx.x % kWarp) == 0 && cnt) atomicAdd(found, cnt);
+}
+
+// Decode: x[j] = anchor[j] + pq[m][code_m][j - m dsub], m = j / dsub, one warp per entry with d spread over the lanes
+// (coarse rows and codebook rows are gathered through L2; the output row is one coalesced store).  The list of slab
+// index p is found by binary search over offsets; the stored code bytes are un-rotated by (p - offsets[l]) mod M.
+//   VLQ:    anchor = (1 - lh) c + lh s,  c = cent[l / E], s = cent[edge[l]], lh = lambda_cb[lamq[p]]
+//   IMI-PQ: anchor = [cb1[i1] | cb2[i2]],  l = i1 | i2 << nbits
+// fp32, every operation rounded as written (no contraction), in the order shown: lh = 0 gives exactly c + p.
+struct DecodeAnchor {
+  const float* cent;       // VLQ: [C][d]
+  const int* edge;         // VLQ: [nlists]
+  const uint8_t* lamq;     // VLQ: [n entries]
+  const float* lambda_cb;  // VLQ
+  int E;
+  const float* cb1;        // IMI: [K][d / 2]
+  const float* cb2;
+  int nbits;
+};
+
+template <bool IMI>
+__global__ void __launch_bounds__(SCAN_THREADS)
+decode_entries_kernel(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* __restrict__ offsets,
+                      const uint8_t* __restrict__ codes, const int64_t* __restrict__ ids, int M, int d,
+                      const float* __restrict__ pq, DecodeAnchor an, float* __restrict__ out_x, int64_t* out_ids) {
+  const int lane = threadIdx.x % kWarp;
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) / kWarp;
+  const int64_t nslab = offsets[nlists];
+  const int dsub = d / M;
+  for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / kWarp; r < n; r += nwarps) {
+    const int64_t p = pos[r];
+    __syncwarp();  // out_ids may alias pos: every lane has read pos[r] before lane 0 overwrites it
+    float* o = out_x + r * d;
+    if (p < 0 || p >= nslab) {
+      for (int j = lane; j < d; j += kWarp) o[j] = __uint_as_float(0xffffffffu);
+      if (out_ids && lane == 0) out_ids[r] = -1;
+      continue;
+    }
+    const int64_t l = list_of(offsets, 0, nlists - 1, p);
+    const int rot = (int)((p - offsets[l]) % M);
+    const uint8_t* cw = codes + p * M;
+    const float *a0, *a1;
+    float lh = 0.f, oml = 1.f;
+    if constexpr (IMI) {
+      const int h = d / 2;
+      a0 = an.cb1 + (l & ((1 << an.nbits) - 1)) * h;
+      a1 = an.cb2 + (l >> an.nbits) * h;
+    } else {
+      a0 = an.cent + (l / an.E) * d;
+      a1 = an.cent + (int64_t)an.edge[l] * d;
+      lh = an.lambda_cb[an.lamq[p]];
+      oml = __fsub_rn(1.f, lh);
+    }
+    for (int j = lane; j < d; j += kWarp) {
+      const int m = j / dsub;
+      int sb = m - rot;  // stored[(m - pos) mod M] = code[m]
+      if (sb < 0) sb += M;
+      const float pv = pq[((int64_t)m * 256 + cw[sb]) * dsub + (j - m * dsub)];
+      float a;
+      if constexpr (IMI) a = *(j < d / 2 ? a0 + j : a1 + (j - d / 2));
+      else a = __fadd_rn(__fmul_rn(oml, a0[j]), __fmul_rn(lh, a1[j]));
+      o[j] = __fadd_rn(a, pv);
+    }
+    if (out_ids && lane == 0) out_ids[r] = ids[p];
+  }
+}
+
+static unsigned grid_for(int64_t items, int per_block) {
+  const int64_t g = div_up(items, per_block);
+  return (unsigned)(g < 1 ? 1 : (g < 148 * 16 ? g : 148 * 16));
+}
+
 int launch_exclusive_scan_i64(int64_t* v, int64_t n, cudaStream_t st) {
   VLQ_LAUNCH(scan_tile_offsets_kernel, 1, SCAN_THREADS, 0, st, v, n);
   return last_error();
@@ -671,6 +798,62 @@ extern "C" int vlq_remove_ids_apply(int64_t nlists, int M, int64_t n, const int6
              out_offsets, w.mask, w.tile_sums, ConstListArrays{codes, lamq, kappa, ids},
              ListArrays{out_codes, out_lamq, out_kappa, out_ids});
   return last_error();
+}
+
+extern "C" int vlq_lookup_ids(int64_t n, const int64_t* ids, int64_t range_lo, const int64_t* keys, int64_t nslots,
+                              int64_t* out_pos, int64_t* out_found, vlq_stream_t stream) {
+  if (n < 0 || nslots < 0 || !out_found || (n > 0 && !ids) || (nslots > 0 && !out_pos)) return VLQ_EINVAL;
+  if (!keys && range_lo > INT64_MAX - nslots) return VLQ_EINVAL;
+  cudaStream_t st = as_stream(stream);
+  unsigned long long* found = reinterpret_cast<unsigned long long*>(out_found);
+  if (nslots == 0) {
+    VLQ_CUDA_TRY(cudaMemsetAsync(out_found, 0, sizeof(int64_t), st));
+    return VLQ_OK;
+  }
+  const unsigned sgrid = grid_for(nslots, SCAN_THREADS);
+  VLQ_LAUNCH(lookup_init_kernel, sgrid, SCAN_THREADS, 0, st, out_pos, nslots, found);
+  if (n > 0)
+    VLQ_LAUNCH(lookup_mark_kernel, grid_for(div_up(n, LOOKUP_UNROLL), SCAN_THREADS), SCAN_THREADS, 0, st, n, ids, range_lo,
+               nslots, keys, out_pos);
+  VLQ_LAUNCH(lookup_finish_kernel, sgrid, SCAN_THREADS, 0, st, out_pos, nslots, found);
+  return last_error();
+}
+
+static int decode_launch(bool imi, int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
+                         const uint8_t* codes, const int64_t* ids, int M, int d, const float* pq, const DecodeAnchor& an,
+                         float* out_x, int64_t* out_ids, vlq_stream_t stream) {
+  if (n < 0 || nlists < 1 || M < 1 || M > 64 || d < 1 || d % M != 0) return VLQ_EINVAL;
+  if (n > 0 && (!pos || !offsets || !codes || !pq || !out_x || (out_ids && !ids))) return VLQ_EINVAL;
+  if (n == 0) return VLQ_OK;
+  const unsigned grid = grid_for(n, SCAN_THREADS / kWarp);
+  if (imi)
+    VLQ_LAUNCH(decode_entries_kernel<true>, grid, SCAN_THREADS, 0, as_stream(stream), n, pos, nlists, offsets, codes, ids, M,
+               d, pq, an, out_x, out_ids);
+  else
+    VLQ_LAUNCH(decode_entries_kernel<false>, grid, SCAN_THREADS, 0, as_stream(stream), n, pos, nlists, offsets, codes, ids,
+               M, d, pq, an, out_x, out_ids);
+  return last_error();
+}
+
+extern "C" int vlq_decode_entries(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
+                                  const uint8_t* codes, const uint8_t* lamq, const int64_t* ids, int M, int d,
+                                  const float* pq, const float* cent, const int* edge, int E, const float* lambda_cb,
+                                  int nL, float* out_x, int64_t* out_ids, vlq_stream_t stream) {
+  if (E < 1 || nlists % E != 0 || nL < 1 || nL > 256) return VLQ_EINVAL;
+  if (n > 0 && (!lamq || !cent || !edge || !lambda_cb)) return VLQ_EINVAL;
+  DecodeAnchor an{};
+  an.cent = cent; an.edge = edge; an.lamq = lamq; an.lambda_cb = lambda_cb; an.E = E;
+  return decode_launch(false, n, pos, nlists, offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
+}
+
+extern "C" int vlq_imi_decode_entries(int64_t n, const int64_t* pos, const int64_t* offsets, const uint8_t* codes,
+                                      const int64_t* ids, int M, int d, const float* pq, const float* cb1,
+                                      const float* cb2, int nbits, float* out_x, int64_t* out_ids, vlq_stream_t stream) {
+  if (nbits < 1 || nbits > 15 || d % 2 != 0) return VLQ_EINVAL;
+  if (n > 0 && (!cb1 || !cb2)) return VLQ_EINVAL;
+  DecodeAnchor an{};
+  an.cb1 = cb1; an.cb2 = cb2; an.nbits = nbits;
+  return decode_launch(true, n, pos, (int64_t)1 << (2 * nbits), offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
 }
 
 extern "C" int vlq_gather_candidates(const int* line_list, int64_t nq, int W, const int64_t* offsets, const int64_t* ids,

@@ -495,7 +495,8 @@ __global__ void __launch_bounds__(NT, 2) scan_long_kernel(ScanArgs a, int look, 
     if (key != kKeyInf) {
       const uint32_t pay = key_payload(key);
       dv = key_val(key);
-      id = a.ids[desc[pay >> 20].st + (pay & 0xfffffu)];
+      const int64_t e = desc[pay >> 20].st + (pay & 0xfffffu);
+      id = a.ids ? a.ids[e] : e;
     }
     a.outD[qi * a.k + i] = dv;
     a.outI[qi * a.k + i] = id;

@@ -483,7 +483,8 @@ __global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel
         const int pos = (int)key_payload(mykey);
         const int lo = owner[pos];
         a.outD[qi * a.k + threadIdx.x] = ord2f((uint32_t)(mykey >> 32));
-        a.outI[qi * a.k + threadIdx.x] = a.ids[lstart[lo] + (pos - prefix[lo])];
+        const int64_t e = lstart[lo] + (pos - prefix[lo]);
+        a.outI[qi * a.k + threadIdx.x] = a.ids ? a.ids[e] : e;
       }
       return;
     }
@@ -494,7 +495,8 @@ __global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel
       const int pos = (int)key_payload(mykey);
       const int lo = owner[pos];
       a.outD[qi * a.k + rank] = ord2f((uint32_t)(mykey >> 32));
-      a.outI[qi * a.k + rank] = a.ids[lstart[lo] + (pos - prefix[lo])];
+      const int64_t e = lstart[lo] + (pos - prefix[lo]);
+      a.outI[qi * a.k + rank] = a.ids ? a.ids[e] : e;
     }
     return;
   }
@@ -582,7 +584,8 @@ __global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel
         if (prefix[mid] <= pos) lo = mid; else hi = mid;
       }
       dv = key_val(key);
-      id = a.ids[lstart[lo] + (pos - prefix[lo])];
+      const int64_t e = lstart[lo] + (pos - prefix[lo]);
+      id = a.ids ? a.ids[e] : e;
     }
     a.outD[qi * a.k + i] = dv;
     a.outI[qi * a.k + i] = id;
@@ -977,7 +980,8 @@ __global__ void __launch_bounds__(SKEW ? AQ_THREADS_SKEW : Q_THREADS, SKEW ? 2 :
         if (desc[mid].p0 <= pos) lo = mid; else hi = mid;
       }
       dv = key_val(key);
-      id = a.ids[desc[lo].st + (pos - desc[lo].p0)];
+      const int64_t e = desc[lo].st + (pos - desc[lo].p0);
+      id = a.ids ? a.ids[e] : e;
     }
     a.outD[qi * a.k + i] = dv;
     a.outI[qi * a.k + i] = id;

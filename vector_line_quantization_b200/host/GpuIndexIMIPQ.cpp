@@ -2,6 +2,7 @@
 
 #include "ListRemoval.h"
 #include "RangeSearch.h"
+#include "Reconstruct.h"
 
 #include <algorithm>
 #include <cstring>
@@ -218,6 +219,33 @@ void GpuIndexIMIPQ::range_search(Index::idx_t n, const float* x, float radius, R
                    result);
 }
 
+// ------------------------------------------------------------------------------------------------ read-back
+void GpuIndexIMIPQ::decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const {
+  VLQ_CALL(vlq_imi_decode_entries(n, pos, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lIds_.as<int64_t>(), M_, d,
+                                  dPq_.as<float>(), half_[0]->deviceVectors(), half_[1]->deviceVectors(), nbits_, out,
+                                  outIds, st));
+}
+
+void GpuIndexIMIPQ::readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const {
+  VLQ_THROW_IF_NOT_MSG(n == 0 || is_trained, "Index not trained");
+  if (n == 0) return;
+  DeviceScope scope(resources_->getDevice());
+  commit_();
+  reconstructIds(resources_, d, SlabIds{lIds_.as<int64_t>(), nListed_}, n, keys, i0, recons,
+                 [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
+                 recStage_);
+}
+
+void GpuIndexIMIPQ::reconstruct(Index::idx_t key, float* recons) const { readBack_(1, &key, 0, recons); }
+void GpuIndexIMIPQ::reconstruct_n(Index::idx_t i0, Index::idx_t ni, float* recons) const {
+  VLQ_THROW_IF_NOT_MSG(i0 >= 0 && ni >= 0, "reconstruct_n: i0 and ni must be >= 0");
+  readBack_(ni, nullptr, i0, recons);
+}
+void GpuIndexIMIPQ::reconstruct_batch(Index::idx_t n, const Index::idx_t* keys, float* recons) const {
+  VLQ_THROW_IF_NOT_MSG(n >= 0 && (n == 0 || keys), "reconstruct_batch: n must be >= 0 and keys non-null");
+  readBack_(n, keys, 0, recons);
+}
+
 int GpuIndexIMIPQ::getListLength(long cell) const {
   VLQ_THROW_IF_NOT(cell >= 0 && cell < (long)K_ * K_);
   DeviceScope scope(resources_->getDevice());
@@ -272,10 +300,28 @@ void GpuIndexIMIPQ::searchCells(Index::idx_t n, const float* x, int nprobe, floa
 
 // IndexIVFPQ::search with a MultiIndexQuantizer (IndexIVFPQ.cpp:1050-1100): cells -> scan of their lists -> top-k
 void GpuIndexIMIPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const {
+  DeviceScope scope(resources_->getDevice());
+  searchTiles_(n, x, k, distances, labels, false, nullptr);
+}
+
+// as GpuIndexIVFPQ::search_and_reconstruct: the scan reports slab indexes, the decode turns them into ids in place
+void GpuIndexIMIPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances,
+                                           Index::idx_t* labels, float* recons) const {
+  VLQ_THROW_IF_NOT_MSG(n == 0 || recons != nullptr, "search_and_reconstruct: recons is null");
+  DeviceScope scope(resources_->getDevice());
+  const TileEpilogue decode = [&](Index::idx_t row0, Index::idx_t m, float*, int64_t* dI, vlq_stream_t st) {
+    decodeToOutput(d, dI, (int64_t)m * k, recons + (size_t)row0 * k * d, dI,
+                   [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
+                   recStage_, st);
+  };
+  searchTiles_(n, x, k, distances, labels, true, &decode);
+}
+
+void GpuIndexIMIPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                                 bool slabIndex, const TileEpilogue* epilogue) const {
   VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
   VLQ_THROW_IF_NOT_MSG(k >= 1 && k <= VLQ_MAX_K, "k must be in [1, 1024]");
   if (n == 0) return;
-  DeviceScope scope(resources_->getDevice());
   commit_();
   vlq_stream_t st = resources_->getDefaultStream();
   const int W = nprobe_;
@@ -296,7 +342,9 @@ void GpuIndexIMIPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float
     cellsDevice_(dq, m, W, cells, t1);  // term1 = ||q - c||^2 in full: the results are full squared distances
     VLQ_CALL(vlq_scan_topk(dq, m, d, dPq_.as<float>(), M_, dLambda_.as<float>(), 1, cells, t1, t6, nullptr, W,
                            lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), lKappa_.as<float>(),
-                           lIds_.as<int64_t>(), (int)k, listCap_, hint, oD, oI, t3ws_.get(), t3ws_.bytes(), st));
+                           slabIndex ? nullptr : lIds_.as<int64_t>(), (int)k, listCap_, hint, oD, oI, t3ws_.get(),
+                           t3ws_.bytes(), st));
+    if (epilogue) (*epilogue)(s, m, oD, oI, st);
     fromDevice(distances + (size_t)s * k, oD, (size_t)m * k * sizeof(float), st);
     fromDevice(labels + (size_t)s * k, oI, (size_t)m * k * sizeof(int64_t), st);
     resources_->syncDefaultStream();

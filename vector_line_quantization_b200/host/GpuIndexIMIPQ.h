@@ -8,6 +8,7 @@
 // zero lambda codebook (the per-entry kappa replaces the use_precomputed_table = 2 tables, IndexIVFPQ.cpp:645-687).
 // search() returns full squared distances ||q - c - p||^2 like IndexIVFPQ::search.
 #pragma once
+#include <functional>
 #include <vector>
 
 #include "AuxIndexStructures.h"
@@ -32,6 +33,13 @@ class GpuIndexIMIPQ : public faiss::Index {
   /// Index::range_search: every entry of the nprobe cells (first listCap_ of each) with ||q - x||^2 < radius, cells in
   /// the order of searchCells, then list position; the same distances as search()
   void range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const override;
+  /// reconstruct / reconstruct_n / reconstruct_batch / search_and_reconstruct as GpuIndexIVFPQ's (keys are ids); the
+  /// decode is [cb1[i1] | cb2[i2]] + p(code) in fp32, IndexIVFPQ's decode with a MultiIndexQuantizer
+  void reconstruct(Index::idx_t key, float* recons) const override;
+  void reconstruct_n(Index::idx_t i0, Index::idx_t ni, float* recons) const override;
+  void reconstruct_batch(Index::idx_t n, const Index::idx_t* keys, float* recons) const override;
+  void search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                              float* recons) const override;
 
   void setNumProbes(int nprobe);  ///< cells visited per query, 1 .. 1024
   int getNumProbes() const { return nprobe_; }
@@ -46,6 +54,13 @@ class GpuIndexIMIPQ : public faiss::Index {
 
  private:
   void commit_() const;
+  /// the tile loop of search(): slabIndex makes the scan report slab indexes instead of ids; `epilogue` (nullable)
+  /// runs after each tile's scan on the device results (as GpuIndexIVFPQ::searchTiles_)
+  using TileEpilogue = std::function<void(Index::idx_t row0, Index::idx_t m, float* dD, int64_t* dI, vlq_stream_t st)>;
+  void searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                    bool slabIndex, const TileEpilogue* epilogue) const;
+  void decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const;
+  void readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const;
   void cellsDevice_(const float* dq, Index::idx_t m, int nprobe, int* dCells, float* dDist) const;
 
   GpuResources* resources_;
@@ -57,7 +72,7 @@ class GpuIndexIMIPQ : public faiss::Index {
   mutable size_t nListed_;
   mutable DeviceBuffer pCell_, pCodes_, pKappa_, pIds_;  // pending entries (arrival order)
   mutable size_t nPending_, capPending_;
-  mutable DeviceBuffer scratch_, work_, t3ws_;
+  mutable DeviceBuffer scratch_, work_, t3ws_, recStage_;
 };
 
 }  // namespace gpu

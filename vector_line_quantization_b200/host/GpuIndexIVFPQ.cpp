@@ -2,6 +2,7 @@
 
 #include "ListRemoval.h"
 #include "RangeSearch.h"
+#include "Reconstruct.h"
 
 #include <algorithm>
 #include <cfloat>
@@ -318,6 +319,34 @@ long GpuIndexIVFPQ::remove_ids(const IDSelector& sel) {
   return removed;
 }
 
+// ------------------------------------------------------------------------------------------------ read-back
+void GpuIndexIVFPQ::decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const {
+  VLQ_CALL(vlq_decode_entries(n, pos, (int64_t)nlist_ * numedge_, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(),
+                              lLamq_.as<uint8_t>(), lIds_.as<int64_t>(), subQuantizers_, d, dPq_.as<float>(),
+                              quantizer_->deviceVectors(), dEdge_.as<int>(), numedge_, dLambda_.as<float>(), nLambda_,
+                              out, outIds, st));
+}
+
+void GpuIndexIVFPQ::readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const {
+  VLQ_THROW_IF_NOT_MSG(n == 0 || is_trained, "Index not trained");
+  if (n == 0) return;
+  DeviceScope scope(ivfConfig_.device);
+  commit_();
+  reconstructIds(resources_, d, SlabIds{lIds_.as<int64_t>(), nListed_}, n, keys, i0, recons,
+                 [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
+                 recStage_);
+}
+
+void GpuIndexIVFPQ::reconstruct(Index::idx_t key, float* recons) const { readBack_(1, &key, 0, recons); }
+void GpuIndexIVFPQ::reconstruct_n(Index::idx_t i0, Index::idx_t ni, float* recons) const {
+  VLQ_THROW_IF_NOT_MSG(i0 >= 0 && ni >= 0, "reconstruct_n: i0 and ni must be >= 0");
+  readBack_(ni, nullptr, i0, recons);
+}
+void GpuIndexIVFPQ::reconstruct_batch(Index::idx_t n, const Index::idx_t* keys, float* recons) const {
+  VLQ_THROW_IF_NOT_MSG(n >= 0 && (n == 0 || keys), "reconstruct_batch: n must be >= 0 and keys non-null");
+  readBack_(n, keys, 0, recons);
+}
+
 // same lines as search(): the coarse stage of a tile is vlq_coarse_lines (host/RangeSearch.cpp runs the rest)
 void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const {
   VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
@@ -348,12 +377,32 @@ void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, R
 // query tile (a11 + a12: the line, term1, term6 of the W best lines of every query) is one vlq_coarse_lines call, which
 // picks the route (fp32 matrix, tcgen05 matrix, matrix-free) and lays out its workspace.
 void GpuIndexIVFPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const {
+  DeviceScope scope(ivfConfig_.device);
+  searchTiles_(n, x, k, distances, labels, false, nullptr);
+}
+
+// search() whose scan reports slab indexes: each tile's labels are decoded (vlq_decode_entries turns them into ids in
+// place) before the tile's results leave the device, so D and I are search()'s bits
+void GpuIndexIVFPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances,
+                                           Index::idx_t* labels, float* recons) const {
+  VLQ_THROW_IF_NOT_MSG(n == 0 || recons != nullptr, "search_and_reconstruct: recons is null");
+  DeviceScope scope(ivfConfig_.device);
+  const TileEpilogue decode = [&](Index::idx_t row0, Index::idx_t m, float*, int64_t* dI, vlq_stream_t st) {
+    decodeToOutput(d, dI, (int64_t)m * k, recons + (size_t)row0 * k * d, dI,
+                   [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
+                   recStage_, st);
+  };
+  searchTiles_(n, x, k, distances, labels, true, &decode);
+}
+
+void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                                 bool slabIndex, const TileEpilogue* epilogue) const {
   VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
   VLQ_THROW_IF_NOT_MSG(k >= 1 && k <= VLQ_MAX_K, "k must be in [1, 1024]");
   VLQ_THROW_IF_NOT_MSG(w1_ >= 1 && w1_ <= VLQ_MAX_K, "w1_ must be in [1, 1024]");
   if (n == 0) return;
-  DeviceScope scope(ivfConfig_.device);
   commit_();
+  const int64_t* ids = slabIndex ? nullptr : lIds_.as<int64_t>();
   vlq_stream_t st = resources_->getDefaultStream();
   const int P = std::min(nprobe_, nlist_);
   const int W = w1_;
@@ -435,9 +484,10 @@ void GpuIndexIVFPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float
       int64_t* oI = inPlace ? reinterpret_cast<int64_t*>(hI) : outI.as<int64_t>() + (size_t)s * k;
       VLQ_CALL(vlq_scan_topk(q, m, d, dPq_.as<float>(), M, dLambda_.as<float>(), nLambda_, lline, t1, t6,
                              dEdgeDist_.as<float>(), W, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(),
-                             lLamq_.as<uint8_t>(), lKappa_.as<float>(), lIds_.as<int64_t>(), (int)k, listCap_,
+                             lLamq_.as<uint8_t>(), lKappa_.as<float>(), ids, (int)k, listCap_,
                              (int)std::min<size_t>(nListed_ / populatedLists_, 1 << 20), oD, oI, t3ws_.get(),
                              t3ws_.bytes(), sb));
+      if (epilogue) (*epilogue)(p0 + s, m, oD, oI, sb);
       if (overlap) VLQ_CALL(vlq_event_record(evScan_[slot], sb));
       if (!inPlace) {
         VLQ_CALL(vlq_stream_wait(ds, sb));  // results of this tile are complete

@@ -6,6 +6,7 @@
 // fused scan + top-k).
 #pragma once
 #include <cstdint>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -88,6 +89,18 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   /// full squared distance ||q - x||^2 < radius -- unlike search(), whose distances exclude ||q||^2, a radius needs
   /// the full value.  Per query: lines in slot order, then list position.  Pending adds are committed first.
   void range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const override;
+  /// Index::reconstruct / reconstruct_n / reconstruct_batch, decoded on the device: keys are ids (as in
+  /// IndexIVFPQ::reconstruct_n, ids i0 .. i0 + ni - 1), in any order, duplicates allowed.  An id stored more than once
+  /// decodes the entry with the lowest slab index; a key without an entry throws before recons is written.  The decode
+  /// is anchor + p(code), anchor = (1 - lambda) c + lambda s in fp32 (a copyFrom index: c + p, IndexIVFPQ's own decode).
+  /// Pending adds are committed first.  keys / recons may be host or device memory.
+  void reconstruct(Index::idx_t key, float* recons) const override;
+  void reconstruct_n(Index::idx_t i0, Index::idx_t ni, float* recons) const override;
+  void reconstruct_batch(Index::idx_t n, const Index::idx_t* keys, float* recons) const override;
+  /// search() plus the decode of exactly the entry behind every result (the scan reports slab indexes, so a repeated id
+  /// is no ambiguity): distances and labels are bit-identical to search(); rows of label -1 are NaN.  recons [n][k][d].
+  void search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                              float* recons) const override;
 
   void reserveMemory(size_t numVecs);
   void setPrecomputedCodes(bool) {}
@@ -140,6 +153,14 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
  private:
   void uploadTables_();
   void commit_() const;  ///< merge pending entries into the CSR lists (lazy: first search / list access after adds)
+  /// the query tile pipeline of search(): slabIndex makes the scan report slab indexes instead of ids; `epilogue`
+  /// (nullable) runs on the scan stream after each tile's scan with (first row, rows, device D [m][k], device I [m][k],
+  /// stream), before the tile's results are copied out
+  using TileEpilogue = std::function<void(Index::idx_t row0, Index::idx_t m, float* dD, int64_t* dI, vlq_stream_t st)>;
+  void searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                    bool slabIndex, const TileEpilogue* epilogue) const;
+  void decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const;
+  void readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const;
   void ensurePending_(size_t extra);
   void addTiles_(Index::idx_t n, const void* x, bool isU8, const long* xids);
   void installLists_(const std::vector<int>& counts, const std::vector<uint8_t>& codes, const std::vector<uint8_t>& las,
@@ -161,7 +182,7 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   mutable DeviceBuffer pList_, pCodes_, pLamq_, pKappa_, pIds_;
   mutable size_t nPending_, capPending_;
   mutable vlq_event_t evCoarse_[2] = {nullptr, nullptr}, evScan_[2] = {nullptr, nullptr};  // search(): two-stream tile pipeline
-  mutable DeviceBuffer scratch_, scratchB_, qIn_, outD_, outI_, addIn_[2], addA_, addF32_, t3ws_;  // grow-only staging / workspace
+  mutable DeviceBuffer scratch_, scratchB_, qIn_, outD_, outI_, addIn_[2], addA_, addF32_, t3ws_, recStage_;  // grow-only staging / workspace
 };
 
 }  // namespace gpu

@@ -3,8 +3,10 @@
 // argument meaning, padding conventions (-1 labels / FLT_MAX distances) and error behaviour (FaissException for user
 // errors).  idx_t = long; matrices are row-major compact float32; pointers may be host or device.
 #pragma once
+#include <algorithm>
 #include <cstdio>
 #include <exception>
+#include <limits>
 #include <string>
 
 namespace faiss {
@@ -60,6 +62,21 @@ struct Index {
   /// stored vectors [i0, i0 + ni) (reference Index.cpp:54-59: one reconstruct per row unless overridden)
   virtual void reconstruct_n(idx_t i0, idx_t ni, float* recons) const {
     for (idx_t i = 0; i < ni; i++) reconstruct(i0 + i, recons + i * d);
+  }
+  /// stored vectors of keys[0 .. n) (reference Index.h reconstruct_batch: one reconstruct per key unless overridden)
+  virtual void reconstruct_batch(idx_t n, const idx_t* keys, float* recons) const {
+    for (idx_t i = 0; i < n; i++) reconstruct(keys[i], recons + i * d);
+  }
+  /// search, then the stored vector behind every label; rows of label -1 are NaN (reference Index.cpp
+  /// search_and_reconstruct).  recons is [n][k][d].
+  virtual void search_and_reconstruct(idx_t n, const float* x, idx_t k, float* distances, idx_t* labels,
+                                      float* recons) const {
+    search(n, x, k, distances, labels);
+    for (idx_t i = 0; i < n * k; i++) {
+      float* r = recons + i * d;
+      if (labels[i] < 0) std::fill(r, r + d, std::numeric_limits<float>::quiet_NaN());
+      else reconstruct(labels[i], r);
+    }
   }
 
   /// remove the entries whose id the selector holds; returns how many were removed (reference Index.h remove_ids;

@@ -117,6 +117,13 @@ int vlq_host_flat_new(void* res, int d, int use_tensor_cores, void** out) {
 }
 int vlq_host_flat_assign(void* flat, long n, const float* x, int* labels) { GUARD(F(flat)->assignFlat(n, x, labels, 1)) }
 int vlq_host_index_reconstruct_n(void* index, long i0, long ni, float* recons) { GUARD(I(index)->reconstruct_n(i0, ni, recons)) }
+int vlq_host_index_reconstruct_batch(void* index, long n, const long* keys, float* recons) {
+  GUARD(I(index)->reconstruct_batch(n, keys, recons))
+}
+int vlq_host_index_search_and_reconstruct(void* index, long n, const float* x, long k, float* distances, long* labels,
+                                          float* recons) {
+  GUARD(I(index)->search_and_reconstruct(n, x, k, distances, labels, recons))
+}
 int vlq_host_flat_search_int(void* flat, long n, const float* x, long k, float* distances, int* labels) {
   GUARD(F(flat)->searchInt(n, x, k, distances, labels))
 }

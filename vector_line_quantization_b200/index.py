@@ -183,6 +183,67 @@ class IDSelectorRange:
         self.imin, self.imax = int(imin), int(imax)
 
 
+def _sync_if_cuda(a):
+    if _is_torch(a) and a.is_cuda:
+        import torch
+
+        torch.cuda.current_stream(a.device).synchronize()  # the host layer reads it on its own stream
+
+
+def _ptr_of(a):
+    return C.c_void_p(a.data_ptr() if _is_torch(a) else a.ctypes.data)
+
+
+class _ReadBack:
+    """Decode of stored entries (GpuIndexIVFPQ, GpuIndexIMIPQ): keys are ids; a key without an entry raises
+    FaissException and writes nothing; an id stored more than once gives its entry with the lowest slab index.
+    numpy for host input, torch CUDA for device input (as Index.search)."""
+
+    def reconstruct_n(self, i0, ni, out=None):
+        """stored vectors of the ids i0 .. i0 + ni - 1 -> [ni][d] f32 (numpy, or `out`: a caller array, e.g. CUDA)"""
+        if out is None:
+            out = np.empty((ni, self.d), np.float32)
+        _call("vlq_host_index_reconstruct_n", self.h, C.c_long(i0), C.c_long(ni), _ptr_of(out))
+        return out
+
+    def reconstruct(self, key):
+        return self.reconstruct_batch(np.array([key], np.int64))[0]
+
+    def reconstruct_batch(self, keys):
+        """stored vectors of the ids `keys` (any order, duplicates allowed) -> [n][d] f32"""
+        if _is_torch(keys):
+            import torch
+
+            keys = keys.reshape(-1)
+            _sync_if_cuda(keys)
+            out = torch.empty((keys.shape[0], self.d), dtype=torch.float32, device=keys.device)
+        else:
+            keys = np.asarray(keys).reshape(-1)
+            out = np.empty((keys.shape[0], self.d), np.float32)
+        p, keep, _ = _in(keys, np.int64)
+        _call("vlq_host_index_reconstruct_batch", self.h, C.c_long(keys.shape[0]), p, _ptr_of(out))
+        return out
+
+    def search_and_reconstruct(self, x, k):
+        """-> (D [n][k], I [n][k], R [n][k][d]): search() and the stored vector behind every label (NaN rows for -1)"""
+        _sync_if_cuda(x)
+        p, keep, dev = _in(x, np.float32)
+        n = x.shape[0]
+        if dev:
+            import torch
+
+            D = torch.empty((n, k), dtype=torch.float32, device=x.device)
+            I = torch.empty((n, k), dtype=torch.int64, device=x.device)
+            R = torch.empty((n, k, self.d), dtype=torch.float32, device=x.device)
+        else:
+            D = np.empty((n, k), np.float32)
+            I = np.empty((n, k), np.int64)
+            R = np.empty((n, k, self.d), np.float32)
+        _call("vlq_host_index_search_and_reconstruct", self.h, C.c_long(n), p, C.c_long(k), _ptr_of(D), _ptr_of(I),
+              _ptr_of(R))
+        return D, I, R
+
+
 def _reconstruct_n(self, i0, ni):
     out = np.empty((ni, self.d), np.float32)
     _call("vlq_host_index_reconstruct_n", self.h, C.c_long(i0), C.c_long(ni), C.c_void_p(out.ctypes.data))
@@ -246,7 +307,7 @@ def kmeans(res, x, k, niter=10, seed=1234):
     return out
 
 
-class GpuIndexIVFPQ(Index):
+class GpuIndexIVFPQ(_ReadBack, Index):
     """The VLQ index: GpuIndexIVFPQ(res, d, nlist, M, bitsPerCode, nedge, nLambda) (gpu/GpuIndexIVFPQ.h:59-67)."""
 
     def __init__(self, res, d, nlist, M, bits=8, nedge=32, nLambda=256, use_tensor_cores=True):
@@ -420,7 +481,7 @@ class CpuIndexIVFPQ:
             pass
 
 
-class GpuIndexIMIPQ(Index):
+class GpuIndexIMIPQ(_ReadBack, Index):
     """IMI-PQ on the device (host/GpuIndexIMIPQ.h): MultiIndexQuantizer(d, 2, nbits_coarse) + IVFPQ over the K^2 cells"""
 
     def __init__(self, res, d, nbits_coarse, M, nbits=8):

@@ -187,6 +187,54 @@ def remove_ids(lists, ids=None, id_range=None):
     return Lists(out_off, *(t[:live] for t in out[1:])), n - live
 
 
+def lookup_ids(lists, keys=None, id_range=None):
+    """slab index of every wanted id (vlq_lookup_ids) -> (pos int64 CUDA tensor, found).  keys: sorted unique int64
+    keys (batch mode), pos[i] for keys[i]; id_range = (lo, hi): pos[i] for the id lo + i.  pos = the lowest slab index
+    holding the id, -1 where none does; found = the number of slots with an entry."""
+    offsets = _chk(lists.offsets, torch.int64, "offsets")
+    dev = offsets.device
+    n = lists.ids.shape[0]
+    if (keys is None) == (id_range is None):
+        raise ValueError("give exactly one of keys and id_range")
+    if keys is not None:
+        keys = _chk(torch.as_tensor(keys, dtype=torch.int64).reshape(-1).to(dev).contiguous(), torch.int64, "keys")
+        lo, nslots = 0, keys.numel()
+    else:
+        lo, nslots = int(id_range[0]), int(id_range[1]) - int(id_range[0])
+    pos = torch.empty(max(nslots, 0), dtype=torch.int64, device=dev)
+    found = torch.empty(1, dtype=torch.int64, device=dev)
+    _abi.call("vlq_lookup_ids", n, _ptr(_chk(lists.ids, torch.int64, "ids")) if n else 0, lo,
+              _ptr(keys) if keys is not None and nslots else 0, nslots, _ptr(pos), _ptr(found), _stream())
+    return pos, int(found)
+
+
+def decode_entries(lists, pos, pq, cent=None, edge=None, lambda_cb=None, cb=None, nbits=None, want_ids=False):
+    """stored vectors of the entries at the slab indexes pos (-1: a NaN row) -> x f32 [n][d] (, ids int64 [n]).
+    VLQ lists (vlq_decode_entries): cent [C][d], edge [C][E] (lists = C E), lambda_cb.  IMI-PQ lists
+    (vlq_imi_decode_entries): cb = (cb1, cb2), each [2^nbits][d / 2]."""
+    offsets = _chk(lists.offsets, torch.int64, "offsets")
+    pq = _chk(pq, torch.float32, "pq")
+    pos = _chk(pos, torch.int64, "pos")
+    M, d = pq.shape[0], pq.shape[0] * pq.shape[2]
+    n = pos.numel()
+    out = torch.empty((n, d), dtype=torch.float32, device=offsets.device)
+    oid = torch.empty(n, dtype=torch.int64, device=offsets.device) if want_ids else None
+    codes = _chk(lists.codes, torch.uint8, "codes")
+    ids = _chk(lists.ids, torch.int64, "ids")
+    if cb is None:
+        edge = _chk(edge, torch.int32, "edge")
+        lambda_cb = _chk(lambda_cb, torch.float32, "lambda_cb")
+        _abi.call("vlq_decode_entries", n, _ptr(pos), offsets.shape[0] - 1, _ptr(offsets), _ptr(codes),
+                  _ptr(_chk(lists.lamq, torch.uint8, "lamq")), _ptr(ids), M, d, _ptr(pq),
+                  _ptr(_chk(cent, torch.float32, "cent")), _ptr(edge), edge.shape[-1], _ptr(lambda_cb),
+                  lambda_cb.shape[0], _ptr(out), _ptr(oid), _stream())
+    else:
+        _abi.call("vlq_imi_decode_entries", n, _ptr(pos), _ptr(offsets), _ptr(codes), _ptr(ids), M, d, _ptr(pq),
+                  _ptr(_chk(cb[0], torch.float32, "cb1")), _ptr(_chk(cb[1], torch.float32, "cb2")), int(nbits),
+                  _ptr(out), _ptr(oid), _stream())
+    return (out, oid) if want_ids else out
+
+
 def rotate_codes(offsets, codes, inverse=False):
     """canonical list-major codes [n][M] -> the stored layout (or back with inverse=True): the entry at position pos of
     its list keeps stored[j] = code[(j + pos) mod M] (csrc/scan.cuh).  Plumbing for callers that assemble Lists by hand
@@ -227,8 +275,9 @@ _scan_ws = {}
 
 
 def scan_topk(q, pq, lambda_cb, line_list, term1, term6, edge_d2, lists, k, cap=1024, use_workspace=True,
-              list_len_hint=None, out=None):
-    """ADC scan of the selected lists fused with exact top-k (a13-a15): -> (D f32 [nq][k], I int64 [nq][k])"""
+              list_len_hint=None, out=None, slab_index=False):
+    """ADC scan of the selected lists fused with exact top-k (a13-a15): -> (D f32 [nq][k], I int64 [nq][k]).
+    slab_index=True: I holds each result's slab index (its row in lists.codes) instead of its id (ids = NULL)."""
     q = _chk(q, torch.float32, "q")
     pq = _chk(pq, torch.float32, "pq")
     nq, d = q.shape
@@ -251,8 +300,8 @@ def scan_topk(q, pq, lambda_cb, line_list, term1, term6, edge_d2, lists, k, cap=
             _scan_ws[q.device] = ws
     _abi.call("vlq_scan_topk", _ptr(q), nq, d, _ptr(pq), M, _ptr(lambda_cb), lambda_cb.shape[0],
               _ptr(_chk(line_list, torch.int32, "line_list")), _ptr(term1), _ptr(term6), _ptr(edge_d2), W,
-              _ptr(lists.offsets), _ptr(lists.codes), _ptr(lists.lamq), _ptr(lists.kappa), _ptr(lists.ids), k, cap,
-              int(hint), _ptr(outD), _ptr(outI), _ptr(ws), wsb, _stream())
+              _ptr(lists.offsets), _ptr(lists.codes), _ptr(lists.lamq), _ptr(lists.kappa),
+              0 if slab_index else _ptr(lists.ids), k, cap, int(hint), _ptr(outD), _ptr(outI), _ptr(ws), wsb, _stream())
     return outD, outI
 
 
