@@ -193,6 +193,22 @@ int vlq_imi_decode_entries(int64_t n, const int64_t* pos, const int64_t* offsets
                            const int64_t* ids, int M, int d, const float* pq, const float* cb1, const float* cb2,
                            int nbits, float* out_x, int64_t* out_ids, vlq_stream_t stream);
 
+/* a15-filter: search / range search restricted to an id selector (faiss SearchParameters::sel) without touching the scan
+ *     or range kernels.  Every distance they compute is (kappa_i + sum_m T3[m][code_im]) + (term1 + ...) with kappa read
+ *     through the one pointer they are given, so a filtered call hands them a masked copy:
+ *     vlq_filter_kappa: out_kappa[e] = member(ids[e]) ? kappa[e] (same bits) : +inf (0x7f800000), for e < n, where
+ *       member(id) = (range_lo <= id < range_hi) OR id in batch[0 .. n_batch) (sorted ascending, as
+ *       vlq_remove_ids_plan) OR bit (id & 7) of bitmap[id >> 3] (faiss IDSelectorBitmap order; an id outside
+ *       [0, 8 bitmap_bytes) is not in the bitmap), negated when invert != 0.  range_lo >= range_hi: no range.
+ *       A masked entry's distance is +inf: it ranks after every finite result and fails `dist < radius` at any radius.
+ *       n = 0 is a no-op; out_kappa must not alias kappa.
+ *     vlq_filter_results: D[i] = FLT_MAX, I[i] = -1 wherever D[i] is +inf in the rows x k results of a scan: a query
+ *       with fewer than k members among its candidates gets the usual padding.  Rows stay sorted. */
+int vlq_filter_kappa(int64_t n, const int64_t* ids, const float* kappa, int64_t range_lo, int64_t range_hi,
+                     const int64_t* batch, int64_t n_batch, const uint8_t* bitmap, int64_t bitmap_bytes, int invert,
+                     float* out_kappa, vlq_stream_t stream);
+int vlq_filter_results(int64_t rows, int k, float* D, int64_t* I, vlq_stream_t stream);
+
 /* a9 (loader): per-entry kappa = ||p||^2 + 2 anchor.p for list-major entries that arrive without it, i.e. lists read
  *     from the reference's .dbIdx/.dbcodes/.dbcount/.dblas files (gpu/GpuIndexIVFPQ.cu:1813-2010). */
 int vlq_recompute_kappa(int64_t n, int64_t nlists, const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq,

@@ -52,6 +52,24 @@ int vlq_host_index_reconstruct_n(void* index, long i0, long ni, float* recons); 
 int vlq_host_index_reconstruct_batch(void* index, long n, const long* keys, float* recons);
 int vlq_host_index_search_and_reconstruct(void* index, long n, const float* x, long k, float* distances, long* labels,
                                           float* recons);
+/* id selectors for filtered search (faiss IDSelectorRange [imin, imax) / IDSelectorBatch (ids host or device, any
+   order, duplicates allowed; copied) / IDSelectorBitmap (bit id & 7 of bitmap[id >> 3] over nbytes bytes; host or
+   device memory, borrowed) / IDSelectorNot (borrows sel)); is_member evaluates one on the host (a bitmap in host
+   memory).  Free each with vlq_host_selector_free after the calls that use it. */
+int vlq_host_selector_range_new(long imin, long imax, void** out);
+int vlq_host_selector_batch_new(long n, const long* ids, void** out);
+int vlq_host_selector_bitmap_new(long nbytes, const unsigned char* bitmap, void** out);
+int vlq_host_selector_not_new(void* sel, void** out);
+int vlq_host_selector_is_member(void* sel, long id, int* out);
+int vlq_host_selector_free(void* sel);
+/* search / range_search / search_and_reconstruct restricted to the ids `sel` holds (SearchParameters::sel; NULL:
+   unfiltered, the calls above).  GpuIndexIVFPQ and GpuIndexIMIPQ filter on the device: the candidates are the entries
+   the unfiltered call scans, members keep its distances, missing results are (FLT_MAX, -1) padding.  Other indexes
+   fail (-1) for a non-NULL selector. */
+int vlq_host_index_search_sel(void* index, long n, const float* x, long k, float* distances, long* labels, void* sel);
+int vlq_host_index_range_search_sel(void* index, long n, const float* x, float radius, void** result, void* sel);
+int vlq_host_index_search_and_reconstruct_sel(void* index, long n, const float* x, long k, float* distances,
+                                              long* labels, float* recons, void* sel);
 int vlq_host_flat_search_int(void* flat, long n, const float* x, long k, float* distances, int* labels); /* searchInt */
 /* assign1Base: device pointers only; line id (assign2 = A*numedge + e) and float lambda of every row */
 int vlq_host_flat_assign1_base(void* flat, long n, const float* d_input, const int* d_assign1, int* d_assign2,

@@ -45,6 +45,8 @@ SIGNATURES = {
     "vlq_lookup_ids": (_i, [_l, _p, _l, _p, _l, _p, _p, _p]),
     "vlq_decode_entries": (_i, [_l, _p, _l, _p, _p, _p, _p, _i, _i, _p, _p, _p, _i, _p, _i, _p, _p, _p]),
     "vlq_imi_decode_entries": (_i, [_l, _p, _p, _p, _p, _i, _i, _p, _p, _p, _i, _p, _p, _p]),
+    "vlq_filter_kappa": (_i, [_l, _p, _p, _l, _l, _p, _l, _p, _l, _i, _p, _p]),
+    "vlq_filter_results": (_i, [_l, _i, _p, _p, _p]),
     "vlq_recompute_kappa": (_i, [_l, _l, _p, _p, _p, _p, _i, _p, _i, _p, _p, _i, _p, _p]),
     "vlq_select_lines": (_i, [_p, _l, _l, _p, _i, _p, _p, _i, _i, _p, _p, _p, _p]),
     "vlq_coarse_select_lines": (_i, [_p, _l, _l, _p, _i, _i, _i, _p, _p, _i, _i, _p, _p, _p, _p, _p]),

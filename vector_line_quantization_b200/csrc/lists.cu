@@ -10,6 +10,8 @@
 //   3. scatter of the new entry ordinals with a per-list cursor (arbitrary order inside a list) ...
 //   4. ... made deterministic: each list segment is sorted by ordinal = arrival order (what push_back gives)
 //   5. old entries are copied to their new place; new entries are gathered behind them.
+#include <cfloat>
+
 #include "scan.cuh"
 
 namespace vlq {
@@ -665,6 +667,56 @@ decode_entries_kernel(int64_t n, const int64_t* pos, int64_t nlists, const int64
   }
 }
 
+// ------------------------------------------------------------------------------------------------ filtered search
+// Mask pass: out_kappa[e] = member(ids[e]) ? kappa[e] : +inf.  Every scan and range kernel reads kappa through the one
+// pointer it is given, so running them on out_kappa filters without touching them: a non-member's distance is +inf
+// (finite terms + inf), which ranks after every finite key and fails every `dist < radius` test.  Membership is
+// vlq_remove_ids_plan's (range OR sorted batch) OR a faiss IDSelectorBitmap bit, then optionally inverted.
+constexpr int FILTER_UNROLL = 4;
+constexpr uint32_t kInfBits = 0x7f800000u;
+
+// bit (id & 7) of bitmap[id >> 3]; ids outside [0, 8 nbytes) are not in the bitmap (negative ids wrap to huge)
+__device__ __forceinline__ bool bitmap_member(int64_t id, const uint8_t* __restrict__ bitmap, int64_t nbytes) {
+  const uint64_t u = (uint64_t)id;
+  return (u >> 3) < (uint64_t)nbytes && ((bitmap[u >> 3] >> (u & 7)) & 1u);
+}
+
+__global__ void __launch_bounds__(SCAN_THREADS)
+filter_kappa_kernel(int64_t n, const int64_t* __restrict__ ids, const float* __restrict__ kappa, int64_t lo, int64_t hi,
+                    const int64_t* __restrict__ batch, int64_t nb, const uint8_t* __restrict__ bitmap, int64_t nbytes,
+                    bool invert, float* __restrict__ out_kappa) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t e0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e0 < n; e0 += stride * FILTER_UNROLL) {
+    int64_t id[FILTER_UNROLL];
+    float kp[FILTER_UNROLL];
+#pragma unroll
+    for (int u = 0; u < FILTER_UNROLL; u++) {  // every load of the four entries first
+      const int64_t e = e0 + u * stride;
+      id[u] = e < n ? ids[e] : 0;
+      kp[u] = e < n ? kappa[e] : 0.f;
+    }
+#pragma unroll
+    for (int u = 0; u < FILTER_UNROLL; u++) {
+      const int64_t e = e0 + u * stride;
+      if (e >= n) break;
+      const bool member = removed_id(id[u], lo, hi, batch, nb) || bitmap_member(id[u], bitmap, nbytes);
+      out_kappa[e] = member != invert ? kp[u] : __uint_as_float(kInfBits);
+    }
+  }
+}
+
+// the padding of a query with fewer than k candidates: (+inf, id) results of masked entries become (FLT_MAX, -1)
+__global__ void __launch_bounds__(SCAN_THREADS)
+filter_results_kernel(int64_t total, float* __restrict__ D, int64_t* __restrict__ I) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+    if (__float_as_uint(D[i]) == kInfBits) {
+      D[i] = FLT_MAX;
+      I[i] = -1;
+    }
+  }
+}
+
 static unsigned grid_for(int64_t items, int per_block) {
   const int64_t g = div_up(items, per_block);
   return (unsigned)(g < 1 ? 1 : (g < 148 * 16 ? g : 148 * 16));
@@ -854,6 +906,26 @@ extern "C" int vlq_imi_decode_entries(int64_t n, const int64_t* pos, const int64
   DecodeAnchor an{};
   an.cb1 = cb1; an.cb2 = cb2; an.nbits = nbits;
   return decode_launch(true, n, pos, (int64_t)1 << (2 * nbits), offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
+}
+
+extern "C" int vlq_filter_kappa(int64_t n, const int64_t* ids, const float* kappa, int64_t range_lo, int64_t range_hi,
+                                const int64_t* batch, int64_t n_batch, const uint8_t* bitmap, int64_t bitmap_bytes,
+                                int invert, float* out_kappa, vlq_stream_t stream) {
+  if (n < 0 || n_batch < 0 || bitmap_bytes < 0) return VLQ_EINVAL;
+  if ((n > 0 && (!ids || !kappa || !out_kappa)) || (n_batch > 0 && !batch) || (bitmap_bytes > 0 && !bitmap))
+    return VLQ_EINVAL;
+  if (n == 0) return VLQ_OK;
+  VLQ_LAUNCH(filter_kappa_kernel, grid_for(div_up(n, FILTER_UNROLL), SCAN_THREADS), SCAN_THREADS, 0, as_stream(stream), n,
+             ids, kappa, range_lo, range_hi, batch, n_batch, bitmap, bitmap_bytes, invert != 0, out_kappa);
+  return last_error();
+}
+
+extern "C" int vlq_filter_results(int64_t rows, int k, float* D, int64_t* I, vlq_stream_t stream) {
+  if (rows < 0 || k < 1 || (rows > 0 && (!D || !I))) return VLQ_EINVAL;
+  if (rows == 0) return VLQ_OK;
+  const int64_t total = rows * k;
+  VLQ_LAUNCH(filter_results_kernel, grid_for(total, SCAN_THREADS), SCAN_THREADS, 0, as_stream(stream), total, D, I);
+  return last_error();
 }
 
 extern "C" int vlq_gather_candidates(const int* line_list, int64_t nq, int W, const int64_t* offsets, const int64_t* ids,

@@ -1,10 +1,12 @@
-// ID selectors of faiss::Index::remove_ids (reference AuxIndexStructures.h: IDSelector, IDSelectorRange,
-// IDSelectorBatch) and the result of faiss::Index::range_search (RangeSearchResult).  The device indexes cannot call a virtual is_member per entry: they recognise these two types and
-// hand the range bounds or the sorted id array to the compaction kernels (vlq_remove_ids_plan).  is_member stays for
-// host callers.
+// ID selectors of faiss::Index::remove_ids and of filtered search (reference AuxIndexStructures.h: IDSelector,
+// IDSelectorRange, IDSelectorBatch, IDSelectorBitmap, IDSelectorNot) and the result of faiss::Index::range_search
+// (RangeSearchResult).  The device indexes cannot call a virtual is_member per entry: they recognise these types and
+// hand the range bounds, the sorted id array or the bitmap to their kernels (vlq_remove_ids_plan takes Range and Batch,
+// vlq_filter_kappa all four).  is_member stays for host callers.
 #pragma once
 #include <algorithm>
 #include <cstddef>
+#include <cstdint>
 #include <cstring>
 #include <vector>
 
@@ -34,6 +36,25 @@ struct IDSelectorBatch : IDSelector {
     ids.erase(std::unique(ids.begin(), ids.end()), ids.end());
   }
   bool is_member(idx_t id) const override { return std::binary_search(ids.begin(), ids.end(), id); }
+};
+
+/// bit (id & 7) of bitmap[id >> 3] over n bytes (reference IDSelectorBitmap); ids outside [0, 8 n) are not members.
+/// The bitmap is borrowed, in host or device memory (the device search reads either; is_member needs host memory).
+struct IDSelectorBitmap : IDSelector {
+  size_t n;
+  const uint8_t* bitmap;
+  IDSelectorBitmap(size_t n_, const uint8_t* bitmap_) : n(n_), bitmap(bitmap_) {}
+  bool is_member(idx_t id) const override {
+    const uint64_t u = (uint64_t)id;  // a negative id wraps past the end
+    return (u >> 3) < n && ((bitmap[u >> 3] >> (u & 7)) & 1);
+  }
+};
+
+/// the complement of a borrowed selector (reference IDSelectorNot)
+struct IDSelectorNot : IDSelector {
+  const IDSelector* sel;
+  explicit IDSelectorNot(const IDSelector* sel_) : sel(sel_) {}
+  bool is_member(idx_t id) const override { return !sel->is_member(id); }
 };
 
 /// the results of range_search for nq queries (reference AuxIndexStructures.h): the results of query i are

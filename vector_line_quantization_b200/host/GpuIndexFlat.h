@@ -27,6 +27,7 @@ class GpuIndexFlat : public faiss::Index {
   void add(Index::idx_t n, const float* x) override;  ///< host or device pointer
   void reset() override;
   /// k <= 1024 (reference limit gpu/GpuIndexFlat.cu:226-232).  L2 distances include ||x||^2 (exact flag).
+  using Index::search;  // the SearchParameters overload: no filtering here (a selector throws)
   void search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const override;
 
   size_t getNumVecs() const { return (size_t)ntotal; }

@@ -3,6 +3,7 @@
 #include "ListRemoval.h"
 #include "RangeSearch.h"
 #include "Reconstruct.h"
+#include "SearchFilter.h"
 
 #include <algorithm>
 #include <cstring>
@@ -46,6 +47,7 @@ void GpuIndexIMIPQ::reset() {
   lLamq_.release();
   lKappa_.release();
   lIds_.release();
+  filtKappa_.release();
   pCell_.release();
   pCodes_.release();
   pKappa_.release();
@@ -203,14 +205,23 @@ long GpuIndexIMIPQ::remove_ids(const IDSelector& sel) {
 
 // the cells of cellsDevice_ are the lines; term1 = ||q - c||^2 already makes the distances full ones (row_add NULL)
 void GpuIndexIMIPQ::range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const {
+  range_search(n, x, radius, result, nullptr);
+}
+
+// as GpuIndexIVFPQ's: with a selector the range kernels read the masked kappa
+void GpuIndexIMIPQ::range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result,
+                                 const SearchParameters* params) const {
   VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
+  const IDSelector* sel = searchSelector(params);
+  if (sel) checkSearchSelector(sel);
   DeviceScope scope(resources_->getDevice());
   if (n > 0) commit_();
+  const float* kappa = lKappa_.as<float>();
+  if (sel && n > 0) kappa = maskKappa(resources_, *sel, lIds_.as<int64_t>(), kappa, nListed_, filtKappa_);
   vlq_stream_t st = resources_->getDefaultStream();
   const int W = nprobe_;
   RangeLists lists{dPq_.as<float>(), M_, dLambda_.as<float>(), 1, nullptr, W, listCap_, lOffsets_.as<int64_t>(),
-                   lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), lKappa_.as<float>(), lIds_.as<int64_t>(), nListed_, false,
-                   4096};
+                   lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), kappa, lIds_.as<int64_t>(), nListed_, false, 4096};
   rangeSearchLists(resources_, d, n, x, radius, lists,
                    [&](const float* dq, Index::idx_t m, int* cells, float* t1, float* t6) {
                      cellsDevice_(dq, m, W, cells, t1);
@@ -301,12 +312,23 @@ void GpuIndexIMIPQ::searchCells(Index::idx_t n, const float* x, int nprobe, floa
 // IndexIVFPQ::search with a MultiIndexQuantizer (IndexIVFPQ.cpp:1050-1100): cells -> scan of their lists -> top-k
 void GpuIndexIMIPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const {
   DeviceScope scope(resources_->getDevice());
-  searchTiles_(n, x, k, distances, labels, false, nullptr);
+  searchTiles_(n, x, k, distances, labels, false, nullptr, nullptr);
+}
+
+void GpuIndexIMIPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                           const SearchParameters* params) const {
+  DeviceScope scope(resources_->getDevice());
+  searchTiles_(n, x, k, distances, labels, false, nullptr, searchSelector(params));
 }
 
 // as GpuIndexIVFPQ::search_and_reconstruct: the scan reports slab indexes, the decode turns them into ids in place
 void GpuIndexIMIPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances,
                                            Index::idx_t* labels, float* recons) const {
+  search_and_reconstruct(n, x, k, distances, labels, recons, nullptr);
+}
+
+void GpuIndexIMIPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances,
+                                           Index::idx_t* labels, float* recons, const SearchParameters* params) const {
   VLQ_THROW_IF_NOT_MSG(n == 0 || recons != nullptr, "search_and_reconstruct: recons is null");
   DeviceScope scope(resources_->getDevice());
   const TileEpilogue decode = [&](Index::idx_t row0, Index::idx_t m, float*, int64_t* dI, vlq_stream_t st) {
@@ -314,15 +336,19 @@ void GpuIndexIMIPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index
                    [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
                    recStage_, st);
   };
-  searchTiles_(n, x, k, distances, labels, true, &decode);
+  searchTiles_(n, x, k, distances, labels, true, &decode, searchSelector(params));
 }
 
 void GpuIndexIMIPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
-                                 bool slabIndex, const TileEpilogue* epilogue) const {
+                                 bool slabIndex, const TileEpilogue* epilogue, const IDSelector* sel) const {
   VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
   VLQ_THROW_IF_NOT_MSG(k >= 1 && k <= VLQ_MAX_K, "k must be in [1, 1024]");
+  if (sel) checkSearchSelector(sel);
   if (n == 0) return;
   commit_();
+  // one stream: the mask pass precedes every scan of the call
+  const float* kappa = lKappa_.as<float>();
+  if (sel) kappa = maskKappa(resources_, *sel, lIds_.as<int64_t>(), kappa, nListed_, filtKappa_);
   vlq_stream_t st = resources_->getDefaultStream();
   const int W = nprobe_;
   const Index::idx_t tile = 4096;
@@ -341,9 +367,10 @@ void GpuIndexIMIPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
     const float* dq = static_cast<const float*>(toDevice(x + (size_t)s * d, (size_t)m * d * sizeof(float), stage, st));
     cellsDevice_(dq, m, W, cells, t1);  // term1 = ||q - c||^2 in full: the results are full squared distances
     VLQ_CALL(vlq_scan_topk(dq, m, d, dPq_.as<float>(), M_, dLambda_.as<float>(), 1, cells, t1, t6, nullptr, W,
-                           lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), lKappa_.as<float>(),
+                           lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), kappa,
                            slabIndex ? nullptr : lIds_.as<int64_t>(), (int)k, listCap_, hint, oD, oI, t3ws_.get(),
                            t3ws_.bytes(), st));
+    if (sel) VLQ_CALL(vlq_filter_results(m, (int)k, oD, oI, st));  // (+inf, id) of masked entries -> padding
     if (epilogue) (*epilogue)(s, m, oD, oI, st);
     fromDevice(distances + (size_t)s * k, oD, (size_t)m * k * sizeof(float), st);
     fromDevice(labels + (size_t)s * k, oI, (size_t)m * k * sizeof(int64_t), st);

@@ -40,6 +40,14 @@ class GpuIndexIMIPQ : public faiss::Index {
   void reconstruct_batch(Index::idx_t n, const Index::idx_t* keys, float* recons) const override;
   void search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
                               float* recons) const override;
+  /// filtered search / range_search / search_and_reconstruct as GpuIndexIVFPQ's: the candidates are the first listCap_
+  /// entries of the nprobe cells, restricted to the ids params->sel holds
+  void search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+              const SearchParameters* params) const override;
+  void range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result,
+                    const SearchParameters* params) const override;
+  void search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                              float* recons, const SearchParameters* params) const override;
 
   void setNumProbes(int nprobe);  ///< cells visited per query, 1 .. 1024
   int getNumProbes() const { return nprobe_; }
@@ -55,10 +63,10 @@ class GpuIndexIMIPQ : public faiss::Index {
  private:
   void commit_() const;
   /// the tile loop of search(): slabIndex makes the scan report slab indexes instead of ids; `epilogue` (nullable)
-  /// runs after each tile's scan on the device results (as GpuIndexIVFPQ::searchTiles_)
+  /// runs after each tile's scan on the device results; sel (nullable) filters (as GpuIndexIVFPQ::searchTiles_)
   using TileEpilogue = std::function<void(Index::idx_t row0, Index::idx_t m, float* dD, int64_t* dI, vlq_stream_t st)>;
   void searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
-                    bool slabIndex, const TileEpilogue* epilogue) const;
+                    bool slabIndex, const TileEpilogue* epilogue, const IDSelector* sel) const;
   void decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const;
   void readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const;
   void cellsDevice_(const float* dq, Index::idx_t m, int nprobe, int* dCells, float* dDist) const;
@@ -72,7 +80,7 @@ class GpuIndexIMIPQ : public faiss::Index {
   mutable size_t nListed_;
   mutable DeviceBuffer pCell_, pCodes_, pKappa_, pIds_;  // pending entries (arrival order)
   mutable size_t nPending_, capPending_;
-  mutable DeviceBuffer scratch_, work_, t3ws_, recStage_;
+  mutable DeviceBuffer scratch_, work_, t3ws_, recStage_, filtKappa_;  // filtKappa_: masked kappa of a filtered call
 };
 
 }  // namespace gpu

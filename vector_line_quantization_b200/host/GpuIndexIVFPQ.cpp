@@ -3,6 +3,7 @@
 #include "ListRemoval.h"
 #include "RangeSearch.h"
 #include "Reconstruct.h"
+#include "SearchFilter.h"
 
 #include <algorithm>
 #include <cfloat>
@@ -91,6 +92,7 @@ void GpuIndexIVFPQ::reset() {
   lLamq_.release();
   lKappa_.release();
   lIds_.release();
+  filtKappa_.release();
   nListed_ = 0;
   nPending_ = 0;
   ntotal = 0;
@@ -349,17 +351,27 @@ void GpuIndexIVFPQ::reconstruct_batch(Index::idx_t n, const Index::idx_t* keys, 
 
 // same lines as search(): the coarse stage of a tile is vlq_coarse_lines (host/RangeSearch.cpp runs the rest)
 void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result) const {
+  range_search(n, x, radius, result, nullptr);
+}
+
+// with a selector the range kernels read the masked kappa: a non-member's distance is +inf, never < radius
+void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result,
+                                 const SearchParameters* params) const {
   VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
   VLQ_THROW_IF_NOT_MSG(w1_ >= 1 && w1_ <= VLQ_MAX_K, "w1_ must be in [1, 1024]");
+  const IDSelector* sel = searchSelector(params);
+  if (sel) checkSearchSelector(sel);
   DeviceScope scope(ivfConfig_.device);
   if (n > 0) commit_();
+  const float* kappa = lKappa_.as<float>();
+  if (sel && n > 0) kappa = maskKappa(resources_, *sel, lIds_.as<int64_t>(), kappa, nListed_, filtKappa_);
   vlq_stream_t st = resources_->getDefaultStream();
   const int P = std::min(nprobe_, nlist_);
   const int W = w1_;
   const Index::idx_t tile = std::max<Index::idx_t>(64, std::min<Index::idx_t>(5120, ((Index::idx_t)5 << 26) / nlist_));
   DeviceBuffer coarseWs;
   RangeLists lists{dPq_.as<float>(), subQuantizers_, dLambda_.as<float>(), nLambda_, dEdgeDist_.as<float>(), W, listCap_,
-                   lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), lKappa_.as<float>(),
+                   lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), kappa,
                    lIds_.as<int64_t>(), nListed_, true, tile};
   rangeSearchLists(resources_, d, n, x, radius, lists,
                    [&](const float* dq, Index::idx_t m, int* lines, float* t1, float* t6) {
@@ -378,13 +390,24 @@ void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, R
 // picks the route (fp32 matrix, tcgen05 matrix, matrix-free) and lays out its workspace.
 void GpuIndexIVFPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const {
   DeviceScope scope(ivfConfig_.device);
-  searchTiles_(n, x, k, distances, labels, false, nullptr);
+  searchTiles_(n, x, k, distances, labels, false, nullptr, nullptr);
+}
+
+void GpuIndexIVFPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                           const SearchParameters* params) const {
+  DeviceScope scope(ivfConfig_.device);
+  searchTiles_(n, x, k, distances, labels, false, nullptr, searchSelector(params));
 }
 
 // search() whose scan reports slab indexes: each tile's labels are decoded (vlq_decode_entries turns them into ids in
 // place) before the tile's results leave the device, so D and I are search()'s bits
 void GpuIndexIVFPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances,
                                            Index::idx_t* labels, float* recons) const {
+  search_and_reconstruct(n, x, k, distances, labels, recons, nullptr);
+}
+
+void GpuIndexIVFPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances,
+                                           Index::idx_t* labels, float* recons, const SearchParameters* params) const {
   VLQ_THROW_IF_NOT_MSG(n == 0 || recons != nullptr, "search_and_reconstruct: recons is null");
   DeviceScope scope(ivfConfig_.device);
   const TileEpilogue decode = [&](Index::idx_t row0, Index::idx_t m, float*, int64_t* dI, vlq_stream_t st) {
@@ -392,17 +415,22 @@ void GpuIndexIVFPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index
                    [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
                    recStage_, st);
   };
-  searchTiles_(n, x, k, distances, labels, true, &decode);
+  searchTiles_(n, x, k, distances, labels, true, &decode, searchSelector(params));
 }
 
 void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
-                                 bool slabIndex, const TileEpilogue* epilogue) const {
+                                 bool slabIndex, const TileEpilogue* epilogue, const IDSelector* sel) const {
   VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
   VLQ_THROW_IF_NOT_MSG(k >= 1 && k <= VLQ_MAX_K, "k must be in [1, 1024]");
   VLQ_THROW_IF_NOT_MSG(w1_ >= 1 && w1_ <= VLQ_MAX_K, "w1_ must be in [1, 1024]");
+  if (sel) checkSearchSelector(sel);
   if (n == 0) return;
   commit_();
   const int64_t* ids = slabIndex ? nullptr : lIds_.as<int64_t>();
+  // filtered: the mask pass runs on the default stream here, before the first page; the scan stream waits for the
+  // default stream at every page start, so every scan reads the finished mask
+  const float* kappa = lKappa_.as<float>();
+  if (sel) kappa = maskKappa(resources_, *sel, lIds_.as<int64_t>(), kappa, nListed_, filtKappa_);
   vlq_stream_t st = resources_->getDefaultStream();
   const int P = std::min(nprobe_, nlist_);
   const int W = w1_;
@@ -451,7 +479,7 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
     }
     outD.reserve((size_t)pn * k * sizeof(float));
     outI.reserve((size_t)pn * k * sizeof(int64_t));
-    if (overlap) VLQ_CALL(vlq_stream_wait(sb, st));  // everything before this page (commit, earlier calls)
+    if (overlap) VLQ_CALL(vlq_stream_wait(sb, st));  // everything before this page (commit, mask pass, earlier calls)
     Index::idx_t ti = 0;
     for (Index::idx_t s = 0; s < pn; s += tile, ti++) {
       const Index::idx_t m = std::min(tile, pn - s);
@@ -484,9 +512,10 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
       int64_t* oI = inPlace ? reinterpret_cast<int64_t*>(hI) : outI.as<int64_t>() + (size_t)s * k;
       VLQ_CALL(vlq_scan_topk(q, m, d, dPq_.as<float>(), M, dLambda_.as<float>(), nLambda_, lline, t1, t6,
                              dEdgeDist_.as<float>(), W, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(),
-                             lLamq_.as<uint8_t>(), lKappa_.as<float>(), ids, (int)k, listCap_,
+                             lLamq_.as<uint8_t>(), kappa, ids, (int)k, listCap_,
                              (int)std::min<size_t>(nListed_ / populatedLists_, 1 << 20), oD, oI, t3ws_.get(),
                              t3ws_.bytes(), sb));
+      if (sel) VLQ_CALL(vlq_filter_results(m, (int)k, oD, oI, sb));  // (+inf, id) of masked entries -> padding
       if (epilogue) (*epilogue)(p0 + s, m, oD, oI, sb);
       if (overlap) VLQ_CALL(vlq_event_record(evScan_[slot], sb));
       if (!inPlace) {

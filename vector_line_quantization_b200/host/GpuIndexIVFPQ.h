@@ -101,6 +101,18 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   /// is no ambiguity): distances and labels are bit-identical to search(); rows of label -1 are NaN.  recons [n][k][d].
   void search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
                               float* recons) const override;
+  /// filtered search / range_search / search_and_reconstruct: params->sel (IDSelectorRange, IDSelectorBatch,
+  /// IDSelectorBitmap, or IDSelectorNot of one of them; any other type throws before anything is written) restricts the
+  /// candidates -- the entries the unfiltered call scans -- to the ids it holds.  A non-member keeps its place in the
+  /// listCap_ window of its line.  Members get the unfiltered call's distance bits; search pads with (FLT_MAX, -1),
+  /// range_search returns the unfiltered result without the non-members.  An entry whose true distance overflows to
+  /// +inf counts as not found.  No selector: the calls above.
+  void search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+              const SearchParameters* params) const override;
+  void range_search(Index::idx_t n, const float* x, float radius, RangeSearchResult* result,
+                    const SearchParameters* params) const override;
+  void search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
+                              float* recons, const SearchParameters* params) const override;
 
   void reserveMemory(size_t numVecs);
   void setPrecomputedCodes(bool) {}
@@ -155,10 +167,11 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   void commit_() const;  ///< merge pending entries into the CSR lists (lazy: first search / list access after adds)
   /// the query tile pipeline of search(): slabIndex makes the scan report slab indexes instead of ids; `epilogue`
   /// (nullable) runs on the scan stream after each tile's scan with (first row, rows, device D [m][k], device I [m][k],
-  /// stream), before the tile's results are copied out
+  /// stream), before the tile's results are copied out.  sel (nullable): the scan reads the masked kappa (filtKappa_)
+  /// and each tile's +inf results become padding (vlq_filter_results) before the epilogue.
   using TileEpilogue = std::function<void(Index::idx_t row0, Index::idx_t m, float* dD, int64_t* dI, vlq_stream_t st)>;
   void searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
-                    bool slabIndex, const TileEpilogue* epilogue) const;
+                    bool slabIndex, const TileEpilogue* epilogue, const IDSelector* sel) const;
   void decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const;
   void readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const;
   void ensurePending_(size_t extra);
@@ -182,7 +195,8 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   mutable DeviceBuffer pList_, pCodes_, pLamq_, pKappa_, pIds_;
   mutable size_t nPending_, capPending_;
   mutable vlq_event_t evCoarse_[2] = {nullptr, nullptr}, evScan_[2] = {nullptr, nullptr};  // search(): two-stream tile pipeline
-  mutable DeviceBuffer scratch_, scratchB_, qIn_, outD_, outI_, addIn_[2], addA_, addF32_, t3ws_, recStage_;  // grow-only staging / workspace
+  mutable DeviceBuffer scratch_, scratchB_, qIn_, outD_, outI_, addIn_[2], addA_, addF32_, t3ws_, recStage_,
+      filtKappa_;  // grow-only staging / workspace; filtKappa_: the masked kappa of a filtered call (4 B per entry)
 };
 
 }  // namespace gpu

@@ -36,6 +36,13 @@ class FaissException : public std::exception {
   } while (0)
 #define VLQ_THROW_IF_NOT(COND) VLQ_THROW_IF_NOT_MSG(COND, "'" #COND "' failed")
 
+/// per-call search options (reference Index.h SearchParameters): sel restricts the results to the ids it holds
+/// (nullptr: every id)
+struct SearchParameters {
+  IDSelector* sel = nullptr;
+  virtual ~SearchParameters() {}
+};
+
 struct Index {
   typedef long idx_t;
 
@@ -88,6 +95,24 @@ struct Index {
   /// AuxIndexStructures.h)
   virtual void range_search(idx_t /*n*/, const float* /*x*/, float /*radius*/, RangeSearchResult* /*result*/) const {
     VLQ_THROW_MSG("range_search not implemented for this type of index");
+  }
+
+  /// search / range_search / search_and_reconstruct with per-call parameters.  Without a selector (params or
+  /// params->sel null) these are the calls above; an index that cannot filter throws for a selector.
+  virtual void search(idx_t n, const float* x, idx_t k, float* distances, idx_t* labels,
+                      const SearchParameters* params) const {
+    VLQ_THROW_IF_NOT_MSG(!params || !params->sel, "search parameters not supported for this type of index");
+    search(n, x, k, distances, labels);
+  }
+  virtual void range_search(idx_t n, const float* x, float radius, RangeSearchResult* result,
+                            const SearchParameters* params) const {
+    VLQ_THROW_IF_NOT_MSG(!params || !params->sel, "search parameters not supported for this type of index");
+    range_search(n, x, radius, result);
+  }
+  virtual void search_and_reconstruct(idx_t n, const float* x, idx_t k, float* distances, idx_t* labels, float* recons,
+                                      const SearchParameters* params) const {
+    VLQ_THROW_IF_NOT_MSG(!params || !params->sel, "search parameters not supported for this type of index");
+    search_and_reconstruct(n, x, k, distances, labels, recons);
   }
 
   /// labels of the k nearest neighbours (= search without the distances; reference Index.cpp:23-29)

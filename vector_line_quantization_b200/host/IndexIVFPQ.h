@@ -18,6 +18,7 @@ struct IndexFlatL2 : Index {
     xb.insert(xb.end(), x, x + (size_t)n * d);
     ntotal += n;
   }
+  using Index::search;
   void search(idx_t, const float*, idx_t, float*, idx_t*) const override {
     VLQ_THROW_MSG("IndexFlatL2 is a container here: search with GpuIndexFlatL2");
   }
@@ -56,6 +57,7 @@ struct IndexIVFPQ : Index {
     if (own_fields) delete quantizer;
   }
   void add(idx_t, const float*) override { VLQ_THROW_MSG("IndexIVFPQ is a container here: add through GpuIndexIVFPQ"); }
+  using Index::search;
   void search(idx_t, const float*, idx_t, float*, idx_t*) const override {
     VLQ_THROW_MSG("IndexIVFPQ is a container here: search through GpuIndexIVFPQ");
   }

@@ -21,6 +21,7 @@ class IndexProxy : public faiss::Index {
   void reset() override;
   void train(Index::idx_t n, const float* x) override;
   void add(Index::idx_t n, const float* x) override;
+  using Index::search;  // the SearchParameters overload: no filtering here (a selector throws)
   void search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const override;
   size_t count() const { return indices_.size(); }
 
@@ -37,6 +38,7 @@ class IndexShards : public faiss::Index {
   void add_shard(Index* index);
   void train(idx_t n, const float* x) override;
   void add(idx_t n, const float* x) override;  ///< splits the rows evenly over the shards (MetaIndexes.cpp:402-440)
+  using Index::search;  // the SearchParameters overload: no filtering here (a selector throws)
   void search(idx_t n, const float* x, idx_t k, float* distances, idx_t* labels) const override;
   void reset() override;
   std::vector<Index*> shard_indexes;

@@ -124,6 +124,67 @@ int vlq_host_index_search_and_reconstruct(void* index, long n, const float* x, l
                                           float* recons) {
   GUARD(I(index)->search_and_reconstruct(n, x, k, distances, labels, recons))
 }
+
+/* ---- id selectors (filtered search) */
+static IDSelector* SEL(void* h) {
+  if (!h) throw FaissException("null selector");
+  return static_cast<IDSelector*>(h);
+}
+int vlq_host_selector_range_new(long imin, long imax, void** out) { GUARD(*out = new IDSelectorRange(imin, imax)) }
+int vlq_host_selector_batch_new(long n, const long* ids, void** out) {
+  GUARD({
+    VLQ_THROW_IF_NOT_MSG(n >= 0 && (n == 0 || ids), "selector: n must be >= 0 and ids non-null when n > 0");
+    std::vector<long> staged;
+    if (n > 0 && vlq_pointer_is_device(ids) == 1) {  // IDSelectorBatch sorts on the host
+      staged.resize((size_t)n);
+      VLQ_CALL(vlq_memcpy_d2h(staged.data(), ids, (size_t)n * sizeof(long), nullptr));
+      VLQ_CALL(vlq_stream_synchronize(nullptr));
+      ids = staged.data();
+    }
+    *out = new IDSelectorBatch(n, ids);
+  })
+}
+int vlq_host_selector_bitmap_new(long nbytes, const unsigned char* bitmap, void** out) {
+  GUARD({
+    VLQ_THROW_IF_NOT_MSG(nbytes >= 0 && (nbytes == 0 || bitmap), "selector: nbytes must be >= 0 and bitmap non-null");
+    *out = new IDSelectorBitmap((size_t)nbytes, bitmap);
+  })
+}
+int vlq_host_selector_not_new(void* sel, void** out) { GUARD(*out = new IDSelectorNot(SEL(sel))) }
+int vlq_host_selector_is_member(void* sel, long id, int* out) { GUARD(*out = SEL(sel)->is_member(id) ? 1 : 0) }
+int vlq_host_selector_free(void* sel) { GUARD(delete static_cast<IDSelector*>(sel)) }
+
+int vlq_host_index_search_sel(void* index, long n, const float* x, long k, float* distances, long* labels, void* sel) {
+  GUARD({
+    SearchParameters p;
+    p.sel = static_cast<IDSelector*>(sel);
+    I(index)->search(n, x, k, distances, labels, &p);
+  })
+}
+int vlq_host_index_range_search_sel(void* index, long n, const float* x, float radius, void** result, void* sel) {
+  GUARD({
+    VLQ_THROW_IF_NOT_MSG(result != nullptr && n >= 0, "range_search: n must be >= 0 and result non-null");
+    *result = nullptr;
+    SearchParameters p;
+    p.sel = static_cast<IDSelector*>(sel);
+    RangeSearchResult* r = new RangeSearchResult(n);
+    try {
+      I(index)->range_search(n, x, radius, r, &p);
+    } catch (...) {
+      delete r;
+      throw;
+    }
+    *result = r;
+  })
+}
+int vlq_host_index_search_and_reconstruct_sel(void* index, long n, const float* x, long k, float* distances,
+                                              long* labels, float* recons, void* sel) {
+  GUARD({
+    SearchParameters p;
+    p.sel = static_cast<IDSelector*>(sel);
+    I(index)->search_and_reconstruct(n, x, k, distances, labels, recons, &p);
+  })
+}
 int vlq_host_flat_search_int(void* flat, long n, const float* x, long k, float* distances, int* labels) {
   GUARD(F(flat)->searchInt(n, x, k, distances, labels))
 }

@@ -105,9 +105,12 @@ class Index:
         pi, ki, _ = _in(ids, np.int64)
         _call("vlq_host_index_add_with_ids", self.h, C.c_long(x.shape[0]), p, pi)
 
-    def search(self, x, k, out=None):
+    def search(self, x, k, out=None, sel=None):
         """-> (distances [n][k] f32, labels [n][k] i64), numpy for host input, torch CUDA for device input.
-        out=(D, I) reuses caller buffers (e.g. pinned torch tensors)."""
+        out=(D, I) reuses caller buffers (e.g. pinned torch tensors).  sel: restrict the results to these ids (see
+        _Selector; GpuIndexIVFPQ and GpuIndexIMIPQ), missing results padded with (FLT_MAX, -1)."""
+        if sel is not None:
+            _sync_if_cuda(x)
         p, keep, dev = _in(x, np.float32)
         n = x.shape[0]
         if out is not None:
@@ -122,17 +125,28 @@ class Index:
             I = np.empty((n, k), np.int64)
         pd = C.c_void_p(D.data_ptr() if _is_torch(D) else D.ctypes.data)
         pi = C.c_void_p(I.data_ptr() if _is_torch(I) else I.ctypes.data)
-        _call("vlq_host_index_search", self.h, C.c_long(n), p, C.c_long(k), pd, pi)
+        if sel is None:
+            _call("vlq_host_index_search", self.h, C.c_long(n), p, C.c_long(k), pd, pi)
+        else:
+            with _Selector(sel) as hs:
+                _call("vlq_host_index_search_sel", self.h, C.c_long(n), p, C.c_long(k), pd, pi, hs)
         return D, I
 
-    def range_search(self, x, radius):
+    def range_search(self, x, radius, sel=None):
         """faiss Index.range_search: every stored vector with squared L2 distance < radius -> (lims int64 [n + 1],
         D f32 [total], I int64 [total]) numpy arrays; the results of query i are D / I[lims[i]:lims[i + 1]].
-        x is numpy or torch (host or device).  GpuIndexIVFPQ and GpuIndexIMIPQ implement it."""
+        x is numpy or torch (host or device).  GpuIndexIVFPQ and GpuIndexIMIPQ implement it.  sel: only these ids
+        (see _Selector)."""
+        if sel is not None:
+            _sync_if_cuda(x)
         p, keep, _ = _in(x, np.float32)
         n = x.shape[0]
         res = C.c_void_p()
-        _call("vlq_host_index_range_search", self.h, C.c_long(n), p, C.c_float(radius), C.byref(res))
+        if sel is None:
+            _call("vlq_host_index_range_search", self.h, C.c_long(n), p, C.c_float(radius), C.byref(res))
+        else:
+            with _Selector(sel) as hs:
+                _call("vlq_host_index_range_search_sel", self.h, C.c_long(n), p, C.c_float(radius), C.byref(res), hs)
         try:
             total = C.c_long()
             _call("vlq_host_range_result_total", res, C.byref(total))
@@ -177,10 +191,92 @@ class Index:
 
 
 class IDSelectorRange:
-    """the ids imin <= id < imax (faiss IDSelectorRange), for Index.remove_ids"""
+    """the ids imin <= id < imax (faiss IDSelectorRange), for Index.remove_ids and filtered search"""
 
     def __init__(self, imin, imax):
         self.imin, self.imax = int(imin), int(imax)
+
+
+class IDSelectorBitmap:
+    """the ids whose bit (id & 7) of bitmap[id >> 3] is set (faiss IDSelectorBitmap); ids outside [0, 8 len(bitmap))
+    are not members.  bitmap: uint8 bytes, numpy (host) or a torch CUDA tensor (read on the device in place)."""
+
+    def __init__(self, bitmap):
+        if _is_torch(bitmap):
+            import torch
+
+            assert bitmap.dtype == torch.uint8
+            self.bitmap = bitmap.reshape(-1).contiguous()
+        else:
+            self.bitmap = np.ascontiguousarray(np.asarray(bitmap, np.uint8).reshape(-1))
+
+
+class IDSelectorNot:
+    """the ids `sel` does not hold (faiss IDSelectorNot); sel: any selector that filtered search accepts"""
+
+    def __init__(self, sel):
+        self.sel = sel
+
+
+class _Selector:
+    """context manager: a host-layer IDSelector handle for `sel` (IDSelectorRange, IDSelectorBitmap, IDSelectorNot, or
+    an int64 id array -- numpy or torch, any order, duplicates allowed: IDSelectorBatch), freed on exit"""
+
+    def __init__(self, sel):
+        self.sel = sel
+        self.handles = []
+        self.keep = []
+
+    def _new(self, fn, *args):
+        h = C.c_void_p()
+        self.handles.append(h)  # freed on exit even when a later step fails
+        _call(fn, *args, C.byref(h))
+        return h
+
+    def _make(self, sel):
+        if isinstance(sel, IDSelectorRange):
+            return self._new("vlq_host_selector_range_new", C.c_long(sel.imin), C.c_long(sel.imax))
+        if isinstance(sel, IDSelectorBitmap):
+            _sync_if_cuda(sel.bitmap)
+            self.keep.append(sel.bitmap)
+            return self._new("vlq_host_selector_bitmap_new", C.c_long(sel.bitmap.shape[0]), _ptr_of(sel.bitmap))
+        if isinstance(sel, IDSelectorNot):
+            return self._new("vlq_host_selector_not_new", self._make(sel.sel))
+        if _is_torch(sel) or isinstance(sel, (np.ndarray, list, tuple)):
+            ids = sel.reshape(-1) if _is_torch(sel) else np.asarray(sel).reshape(-1)
+            if not _is_torch(ids) and ids.size and not np.issubdtype(ids.dtype, np.integer):
+                raise TypeError("an id selector array must hold integers, not %s" % ids.dtype)
+            _sync_if_cuda(ids)
+            p, keep, _ = _in(ids, np.int64)
+            self.keep.append(keep)
+            return self._new("vlq_host_selector_batch_new", C.c_long(ids.shape[0]), p)
+        raise TypeError("unsupported selector %r: use IDSelectorRange, IDSelectorBitmap, IDSelectorNot or an int64 id "
+                        "array" % type(sel).__name__)
+
+    def __enter__(self):
+        try:
+            return self._make(self.sel)
+        except BaseException:
+            self.__exit__(None, None, None)
+            raise
+
+    def __exit__(self, *exc):
+        for h in reversed(self.handles):
+            if h:
+                host().vlq_host_selector_free(h)
+        self.handles = []
+        return False
+
+
+def selector_is_member(sel, ids):
+    """host-side membership (IDSelector::is_member) of every id in `ids` -> bool numpy array"""
+    out = C.c_int()
+    res = []
+    with _Selector(sel) as hs:
+        for i in np.asarray(ids, np.int64).reshape(-1):
+            _call("vlq_host_selector_is_member", hs, C.c_long(int(i)), C.byref(out))
+            res.append(bool(out.value))
+    return np.array(res, bool)
 
 
 def _sync_if_cuda(a):
@@ -224,8 +320,9 @@ class _ReadBack:
         _call("vlq_host_index_reconstruct_batch", self.h, C.c_long(keys.shape[0]), p, _ptr_of(out))
         return out
 
-    def search_and_reconstruct(self, x, k):
-        """-> (D [n][k], I [n][k], R [n][k][d]): search() and the stored vector behind every label (NaN rows for -1)"""
+    def search_and_reconstruct(self, x, k, sel=None):
+        """-> (D [n][k], I [n][k], R [n][k][d]): search() and the stored vector behind every label (NaN rows for -1).
+        sel: as in search()."""
         _sync_if_cuda(x)
         p, keep, dev = _in(x, np.float32)
         n = x.shape[0]
@@ -239,8 +336,13 @@ class _ReadBack:
             D = np.empty((n, k), np.float32)
             I = np.empty((n, k), np.int64)
             R = np.empty((n, k, self.d), np.float32)
-        _call("vlq_host_index_search_and_reconstruct", self.h, C.c_long(n), p, C.c_long(k), _ptr_of(D), _ptr_of(I),
-              _ptr_of(R))
+        if sel is None:
+            _call("vlq_host_index_search_and_reconstruct", self.h, C.c_long(n), p, C.c_long(k), _ptr_of(D), _ptr_of(I),
+                  _ptr_of(R))
+        else:
+            with _Selector(sel) as hs:
+                _call("vlq_host_index_search_and_reconstruct_sel", self.h, C.c_long(n), p, C.c_long(k), _ptr_of(D),
+                      _ptr_of(I), _ptr_of(R), hs)
         return D, I, R
 
 

@@ -235,6 +235,39 @@ def decode_entries(lists, pos, pq, cent=None, edge=None, lambda_cb=None, cb=None
     return (out, oid) if want_ids else out
 
 
+def filter_kappa(lists, id_range=None, ids=None, bitmap=None, invert=False, out=None):
+    """masked kappa of filtered search (vlq_filter_kappa) -> f32 CUDA tensor [n]: lists.kappa where the entry's id is a
+    member, +inf elsewhere.  member = id in the half-open id_range (lo, hi) OR in `ids` (int64, any order, duplicates
+    allowed) OR bit (id & 7) of bitmap[id >> 3] (uint8 tensor), negated with invert=True.  Pass the result as the
+    `kappa` of scan_topk / range_scan_lines."""
+    kappa = _chk(lists.kappa, torch.float32, "kappa")
+    dev = kappa.device
+    n = lists.ids.shape[0]
+    batch = None
+    if ids is not None:
+        batch = torch.unique(torch.as_tensor(ids, dtype=torch.int64).reshape(-1).to(dev))  # sorted, de-duplicated
+    nb = 0 if batch is None else batch.numel()
+    if bitmap is not None:
+        bitmap = _chk(torch.as_tensor(bitmap, dtype=torch.uint8).reshape(-1).to(dev).contiguous(), torch.uint8, "bitmap")
+    nbytes = 0 if bitmap is None else bitmap.numel()
+    lo, hi = (int(id_range[0]), int(id_range[1])) if id_range is not None else (0, 0)
+    if out is None:
+        out = torch.empty(n, dtype=torch.float32, device=dev)
+    _abi.call("vlq_filter_kappa", n, _ptr(_chk(lists.ids, torch.int64, "ids")) if n else 0, _ptr(kappa) if n else 0, lo,
+              hi, _ptr(batch) if nb else 0, nb, _ptr(bitmap) if nbytes else 0, nbytes, int(bool(invert)),
+              _ptr(out) if n else 0, _stream())
+    return out
+
+
+def filter_results(D, I):
+    """(+inf, id) results of a scan on masked kappa -> (FLT_MAX, -1) in place (vlq_filter_results); returns (D, I)"""
+    D = _chk(D, torch.float32, "D")
+    I = _chk(I, torch.int64, "I")
+    rows, k = D.shape
+    _abi.call("vlq_filter_results", rows, k, _ptr(D), _ptr(I), _stream())
+    return D, I
+
+
 def rotate_codes(offsets, codes, inverse=False):
     """canonical list-major codes [n][M] -> the stored layout (or back with inverse=True): the entry at position pos of
     its list keeps stored[j] = code[(j + pos) mod M] (csrc/scan.cuh).  Plumbing for callers that assemble Lists by hand
@@ -275,9 +308,10 @@ _scan_ws = {}
 
 
 def scan_topk(q, pq, lambda_cb, line_list, term1, term6, edge_d2, lists, k, cap=1024, use_workspace=True,
-              list_len_hint=None, out=None, slab_index=False):
+              list_len_hint=None, out=None, slab_index=False, kappa=None):
     """ADC scan of the selected lists fused with exact top-k (a13-a15): -> (D f32 [nq][k], I int64 [nq][k]).
-    slab_index=True: I holds each result's slab index (its row in lists.codes) instead of its id (ids = NULL)."""
+    slab_index=True: I holds each result's slab index (its row in lists.codes) instead of its id (ids = NULL).
+    kappa: per-entry kappa to read instead of lists.kappa (filter_kappa's mask)."""
     q = _chk(q, torch.float32, "q")
     pq = _chk(pq, torch.float32, "pq")
     nq, d = q.shape
@@ -300,17 +334,21 @@ def scan_topk(q, pq, lambda_cb, line_list, term1, term6, edge_d2, lists, k, cap=
             _scan_ws[q.device] = ws
     _abi.call("vlq_scan_topk", _ptr(q), nq, d, _ptr(pq), M, _ptr(lambda_cb), lambda_cb.shape[0],
               _ptr(_chk(line_list, torch.int32, "line_list")), _ptr(term1), _ptr(term6), _ptr(edge_d2), W,
-              _ptr(lists.offsets), _ptr(lists.codes), _ptr(lists.lamq), _ptr(lists.kappa),
+              _ptr(lists.offsets), _ptr(lists.codes), _ptr(lists.lamq),
+              _ptr(lists.kappa if kappa is None else _chk(kappa, torch.float32, "kappa")),
               0 if slab_index else _ptr(lists.ids), k, cap, int(hint), _ptr(outD), _ptr(outI), _ptr(ws), wsb, _stream())
     return outD, outI
 
 
 def range_scan_lines(q, pq, lambda_cb, lines, edge_d2, lists, radius, cap=1024, row_add=None, tile=5120,
-                     stage_results=None):
+                     stage_results=None, kappa=None):
     """Radius search over the selected lines (a15-range, vlq_range_count + vlq_range_gather): every entry the scan would
     look at whose distance (+ row_add[q], e.g. ||q||^2 for the full squared L2) is < radius, per query in stream order
     (lines in slot order, then list position) -> (lims int64 [nq + 1], D f32 [total], I int64 [total]), CUDA tensors.
-    stage_results: gather each tile in query sub-ranges of at most this many results (one query at least)."""
+    stage_results: gather each tile in query sub-ranges of at most this many results (one query at least).
+    kappa: per-entry kappa to read instead of lists.kappa (filter_kappa's mask)."""
+    if kappa is not None:
+        lists = lists._replace(kappa=_chk(kappa, torch.float32, "kappa"))
     q = _chk(q, torch.float32, "q")
     pq = _chk(pq, torch.float32, "pq")
     nq, d = q.shape
