@@ -1,6 +1,5 @@
 #include "GpuIndexIMIPQ.h"
 
-#include "ListRemoval.h"
 #include "RangeSearch.h"
 #include "Reconstruct.h"
 #include "SearchFilter.h"
@@ -13,7 +12,8 @@ namespace gpu {
 
 GpuIndexIMIPQ::GpuIndexIMIPQ(GpuResources* resources, int dims, int nbitsCoarse, int subQuantizers, int bitsPerCode)
     : Index(dims, faiss::METRIC_L2), listCap_(1 << 20), resources_(resources), nbits_(nbitsCoarse), K_(1 << nbitsCoarse),
-      M_(subQuantizers), bitsPerCode_(bitsPerCode), nprobe_(1), nListed_(0), nPending_(0), capPending_(0) {
+      M_(subQuantizers), bitsPerCode_(bitsPerCode), nprobe_(1),
+      lists_(resources, (int64_t)1 << (2 * nbitsCoarse), subQuantizers) {
   VLQ_THROW_IF_NOT_MSG(dims % 2 == 0 && dims % subQuantizers == 0 && (dims / 2) % (dims / subQuantizers) == 0,
                        "d must be even and every PQ sub-space must lie inside one half");
   VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8, "only 8-bit PQ codes (as the VLQ index)");
@@ -42,17 +42,7 @@ void GpuIndexIMIPQ::setNumProbes(int nprobe) {
 
 void GpuIndexIMIPQ::reset() {
   DeviceScope scope(resources_->getDevice());
-  lOffsets_.release();
-  lCodes_.release();
-  lLamq_.release();
-  lKappa_.release();
-  lIds_.release();
-  filtKappa_.release();
-  pCell_.release();
-  pCodes_.release();
-  pKappa_.release();
-  pIds_.release();
-  nListed_ = nPending_ = capPending_ = 0;
+  lists_.reset();
   ntotal = 0;
 }
 
@@ -128,22 +118,8 @@ void GpuIndexIMIPQ::add_with_ids(Index::idx_t n, const float* x, const long* xid
   DeviceScope scope(resources_->getDevice());
   vlq_stream_t st = resources_->getDefaultStream();
   const int h = d / 2;
-  if (nPending_ + (size_t)n > capPending_) {  // grow the pending arena (contents preserved)
-    const size_t cap = std::max(nPending_ + (size_t)n, 2 * capPending_);
-    DeviceBuffer c(cap * sizeof(int)), k(cap * (size_t)M_), kp(cap * sizeof(float)), id(cap * sizeof(int64_t));
-    if (nPending_) {
-      VLQ_CALL(vlq_memcpy_d2d(c.get(), pCell_.get(), nPending_ * sizeof(int), st));
-      VLQ_CALL(vlq_memcpy_d2d(k.get(), pCodes_.get(), nPending_ * (size_t)M_, st));
-      VLQ_CALL(vlq_memcpy_d2d(kp.get(), pKappa_.get(), nPending_ * sizeof(float), st));
-      VLQ_CALL(vlq_memcpy_d2d(id.get(), pIds_.get(), nPending_ * sizeof(int64_t), st));
-      resources_->syncDefaultStream();
-    }
-    pCell_.swap(c);
-    pCodes_.swap(k);
-    pKappa_.swap(kp);
-    pIds_.swap(id);
-    capPending_ = cap;
-  }
+  const DeviceLists::Slots out = lists_.makeRoom((size_t)n);
+  VLQ_CALL(vlq_memset(out.lamq, 0, (size_t)n, st));  // no lambda: every entry sits on its cell's centroid
   const Index::idx_t tile = 1 << 20;
   DeviceBuffer stage, halves((size_t)std::min(tile, n) * h * sizeof(float)), assign((size_t)std::min(tile, n) * sizeof(int) * 2);
   for (Index::idx_t s0 = 0; s0 < n; s0 += tile) {
@@ -156,49 +132,18 @@ void GpuIndexIMIPQ::add_with_ids(Index::idx_t n, const float* x, const long* xid
       half_[s]->assignDevice(halves.as<float>(), m, s ? a2 : a1, nullptr, false);
     }
     VLQ_CALL(vlq_imi_encode(dx, m, d, a1, a2, half_[0]->deviceVectors(), half_[1]->deviceVectors(), nbits_, dPq_.as<float>(),
-                            M_, pCell_.as<int>() + nPending_, pCodes_.as<uint8_t>() + nPending_ * (size_t)M_,
-                            pKappa_.as<float>() + nPending_, st));
-    VLQ_CALL(vlq_memcpy_h2d(pIds_.as<int64_t>() + nPending_, xids + s0, (size_t)m * sizeof(int64_t), st));
+                            M_, out.list + s0, out.codes + (size_t)s0 * M_, out.kappa + s0, st));
+    VLQ_CALL(vlq_memcpy_h2d(out.ids + s0, xids + s0, (size_t)m * sizeof(int64_t), st));
     resources_->syncDefaultStream();
-    nPending_ += (size_t)m;
+    lists_.appended((size_t)m);
   }
   ntotal += n;
 }
 
-// pending entries -> CSR lists over the K^2 cells (stable counting sort, vlq_build_lists; lambda bytes are all zero)
-void GpuIndexIMIPQ::commit_() const {
-  if (nPending_ == 0 && lOffsets_.bytes()) return;
-  vlq_stream_t st = resources_->getDefaultStream();
-  const int64_t L = (int64_t)K_ * K_;
-  const size_t tot = nListed_ + nPending_;
-  DeviceBuffer nOff((size_t)(L + 1) * sizeof(int64_t)), nCodes(std::max<size_t>(1, tot * M_)), nLamq(std::max<size_t>(1, tot)),
-      nKappa(std::max<size_t>(1, tot) * sizeof(float)), nIds(std::max<size_t>(1, tot) * sizeof(int64_t));
-  DeviceBuffer zeros(std::max<size_t>(1, nPending_));
-  VLQ_CALL(vlq_memset(zeros.get(), 0, zeros.bytes(), st));
-  DeviceBuffer ws(vlq_build_lists_workspace_bytes((int64_t)nPending_, L));
-  VLQ_CALL(vlq_build_lists(L, M_, (int64_t)nListed_, nListed_ ? lOffsets_.as<int64_t>() : nullptr, lCodes_.as<uint8_t>(),
-                           lLamq_.as<uint8_t>(), lKappa_.as<float>(), lIds_.as<int64_t>(), (int64_t)nPending_,
-                           pCell_.as<int>(), pCodes_.as<uint8_t>(), zeros.as<uint8_t>(), pKappa_.as<float>(),
-                           pIds_.as<int64_t>(), nOff.as<int64_t>(), nCodes.as<uint8_t>(), nLamq.as<uint8_t>(),
-                           nKappa.as<float>(), nIds.as<int64_t>(), ws.get(), ws.bytes(), st));
-  int64_t last = 0;
-  VLQ_CALL(vlq_memcpy_d2h(&last, nOff.as<int64_t>() + L, sizeof(int64_t), st));
-  resources_->syncDefaultStream();
-  lOffsets_.swap(nOff);
-  lCodes_.swap(nCodes);
-  lLamq_.swap(nLamq);
-  lKappa_.swap(nKappa);
-  lIds_.swap(nIds);
-  nListed_ = (size_t)last;  // rows without a cell (NaN input) are dropped, as in the VLQ index
-  nPending_ = 0;
-}
-
-// same slab as the VLQ index (zero lambda bytes): the same compaction (host/ListRemoval.cpp)
 long GpuIndexIMIPQ::remove_ids(const IDSelector& sel) {
   DeviceScope scope(resources_->getDevice());
   commit_();
-  const long removed = removeFromLists(resources_, sel, (int64_t)K_ * K_, M_,
-                                       ListSlab{lOffsets_, lCodes_, lLamq_, lKappa_, lIds_, nListed_});
+  const long removed = lists_.remove(sel);
   ntotal -= removed;
   return removed;
 }
@@ -216,12 +161,10 @@ void GpuIndexIMIPQ::range_search(Index::idx_t n, const float* x, float radius, R
   if (sel) checkSearchSelector(sel);
   DeviceScope scope(resources_->getDevice());
   if (n > 0) commit_();
-  const float* kappa = lKappa_.as<float>();
-  if (sel && n > 0) kappa = maskKappa(resources_, *sel, lIds_.as<int64_t>(), kappa, nListed_, filtKappa_);
+  const float* kappa = n > 0 ? lists_.kappa(sel) : nullptr;
   vlq_stream_t st = resources_->getDefaultStream();
   const int W = nprobe_;
-  RangeLists lists{dPq_.as<float>(), M_, dLambda_.as<float>(), 1, nullptr, W, listCap_, lOffsets_.as<int64_t>(),
-                   lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), kappa, lIds_.as<int64_t>(), nListed_, false, 4096};
+  RangeLists lists{dPq_.as<float>(), M_, dLambda_.as<float>(), 1, nullptr, W, listCap_, &lists_, kappa, false, 4096};
   rangeSearchLists(resources_, d, n, x, radius, lists,
                    [&](const float* dq, Index::idx_t m, int* cells, float* t1, float* t6) {
                      cellsDevice_(dq, m, W, cells, t1);
@@ -232,9 +175,8 @@ void GpuIndexIMIPQ::range_search(Index::idx_t n, const float* x, float radius, R
 
 // ------------------------------------------------------------------------------------------------ read-back
 void GpuIndexIMIPQ::decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const {
-  VLQ_CALL(vlq_imi_decode_entries(n, pos, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lIds_.as<int64_t>(), M_, d,
-                                  dPq_.as<float>(), half_[0]->deviceVectors(), half_[1]->deviceVectors(), nbits_, out,
-                                  outIds, st));
+  VLQ_CALL(vlq_imi_decode_entries(n, pos, lists_.offsets(), lists_.codes(), lists_.ids(), M_, d, dPq_.as<float>(),
+                                  half_[0]->deviceVectors(), half_[1]->deviceVectors(), nbits_, out, outIds, st));
 }
 
 void GpuIndexIMIPQ::readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const {
@@ -242,7 +184,7 @@ void GpuIndexIMIPQ::readBack_(Index::idx_t n, const Index::idx_t* keys, Index::i
   if (n == 0) return;
   DeviceScope scope(resources_->getDevice());
   commit_();
-  reconstructIds(resources_, d, SlabIds{lIds_.as<int64_t>(), nListed_}, n, keys, i0, recons,
+  reconstructIds(resources_, d, lists_, n, keys, i0, recons,
                  [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
                  recStage_);
 }
@@ -258,13 +200,9 @@ void GpuIndexIMIPQ::reconstruct_batch(Index::idx_t n, const Index::idx_t* keys, 
 }
 
 int GpuIndexIMIPQ::getListLength(long cell) const {
-  VLQ_THROW_IF_NOT(cell >= 0 && cell < (long)K_ * K_);
   DeviceScope scope(resources_->getDevice());
   commit_();
-  int64_t o[2];
-  VLQ_CALL(vlq_memcpy_d2h(o, lOffsets_.as<int64_t>() + cell, sizeof(o), resources_->getDefaultStream()));
-  resources_->syncDefaultStream();
-  return (int)(o[1] - o[0]);
+  return (int)lists_.listLength(cell);
 }
 
 // nprobe best cells of m device queries: half tables -> sorted prefixes -> hyperbola merge
@@ -346,13 +284,10 @@ void GpuIndexIMIPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
   if (sel) checkSearchSelector(sel);
   if (n == 0) return;
   commit_();
-  // one stream: the mask pass precedes every scan of the call
-  const float* kappa = lKappa_.as<float>();
-  if (sel) kappa = maskKappa(resources_, *sel, lIds_.as<int64_t>(), kappa, nListed_, filtKappa_);
+  const float* kappa = lists_.kappa(sel);  // one stream: the mask pass precedes every scan of the call
   vlq_stream_t st = resources_->getDefaultStream();
   const int W = nprobe_;
   const Index::idx_t tile = 4096;
-  DeviceBuffer stage;
   work_.reserve((size_t)tile * W * (sizeof(int) + 2 * sizeof(float)) + (size_t)tile * k * (sizeof(float) + sizeof(int64_t)));
   int* cells = work_.as<int>();
   float* t1 = reinterpret_cast<float*>(cells + (size_t)tile * W);
@@ -361,15 +296,14 @@ void GpuIndexIMIPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
   int64_t* oI = reinterpret_cast<int64_t*>(oD + (size_t)tile * k);
   t3ws_.reserve(vlq_scan_topk_workspace_bytes(tile, M_));
   VLQ_CALL(vlq_memset(t6, 0, (size_t)tile * W * sizeof(float), st));
-  const int hint = (int)std::min<size_t>(nListed_ / std::max<size_t>(1, (size_t)K_ * K_), 1 << 20);
+  const int hint = (int)std::min<size_t>(lists_.size() / std::max<size_t>(1, (size_t)K_ * K_), 1 << 20);
   for (Index::idx_t s = 0; s < n; s += tile) {
     const Index::idx_t m = std::min(tile, n - s);
-    const float* dq = static_cast<const float*>(toDevice(x + (size_t)s * d, (size_t)m * d * sizeof(float), stage, st));
+    const float* dq = static_cast<const float*>(toDevice(x + (size_t)s * d, (size_t)m * d * sizeof(float), qIn_, st));
     cellsDevice_(dq, m, W, cells, t1);  // term1 = ||q - c||^2 in full: the results are full squared distances
     VLQ_CALL(vlq_scan_topk(dq, m, d, dPq_.as<float>(), M_, dLambda_.as<float>(), 1, cells, t1, t6, nullptr, W,
-                           lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), kappa,
-                           slabIndex ? nullptr : lIds_.as<int64_t>(), (int)k, listCap_, hint, oD, oI, t3ws_.get(),
-                           t3ws_.bytes(), st));
+                           lists_.offsets(), lists_.codes(), lists_.lamq(), kappa, slabIndex ? nullptr : lists_.ids(),
+                           (int)k, listCap_, hint, oD, oI, t3ws_.get(), t3ws_.bytes(), st));
     if (sel) VLQ_CALL(vlq_filter_results(m, (int)k, oD, oI, st));  // (+inf, id) of masked entries -> padding
     if (epilogue) (*epilogue)(s, m, oD, oI, st);
     fromDevice(distances + (size_t)s * k, oD, (size_t)m * k * sizeof(float), st);

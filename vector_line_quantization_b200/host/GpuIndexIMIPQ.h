@@ -4,14 +4,16 @@
 // i.e. two k-means over the halves of the vectors (K = 2^nbitsCoarse centroids each), K^2 cells, residual PQ codes per
 // cell and a search that walks the nprobe cells with the smallest d1 + d2 (multi-sequence, IndexPQ.cpp:637-857).
 // Here the same index lives on the device: half assignments / half distance tables by the flat kernels, cell selection by
-// vlq_imi_top_cells, encode by vlq_imi_encode, lists = the CSR slab of the VLQ index, scan = vlq_scan_topk with a
-// zero lambda codebook (the per-entry kappa replaces the use_precomputed_table = 2 tables, IndexIVFPQ.cpp:645-687).
+// vlq_imi_top_cells, encode by vlq_imi_encode, lists = the CSR slab of the VLQ index (DeviceLists.h), scan =
+// vlq_scan_topk with a zero lambda codebook (the per-entry kappa replaces the use_precomputed_table = 2 tables,
+// IndexIVFPQ.cpp:645-687).
 // search() returns full squared distances ||q - c - p||^2 like IndexIVFPQ::search.
 #pragma once
 #include <functional>
 #include <vector>
 
 #include "AuxIndexStructures.h"
+#include "DeviceLists.h"
 #include "GpuIndexFlat.h"
 #include "ProductQuantizer.h"
 
@@ -61,7 +63,11 @@ class GpuIndexIMIPQ : public faiss::Index {
   int listCap_;              ///< entries scanned per cell at most (1 << 20: the CPU IndexIVFPQ has no cap)
 
  private:
-  void commit_() const;
+  /// the build workspace is a temporary: at K^2 lists it is too large to keep
+  void commit_() const {
+    DeviceBuffer ws;
+    lists_.commit(ws);
+  }
   /// the tile loop of search(): slabIndex makes the scan report slab indexes instead of ids; `epilogue` (nullable)
   /// runs after each tile's scan on the device results; sel (nullable) filters (as GpuIndexIVFPQ::searchTiles_)
   using TileEpilogue = std::function<void(Index::idx_t row0, Index::idx_t m, float* dD, int64_t* dI, vlq_stream_t st)>;
@@ -76,11 +82,9 @@ class GpuIndexIMIPQ : public faiss::Index {
   GpuIndexFlatL2* half_[2];    // the two coarse codebooks (K rows of d/2)
   std::vector<float> pqHost_;  // (M, 256, dsub)
   DeviceBuffer dPq_, dLambda_;
-  mutable DeviceBuffer lOffsets_, lCodes_, lLamq_, lKappa_, lIds_;  // CSR lists over the K^2 cells
-  mutable size_t nListed_;
-  mutable DeviceBuffer pCell_, pCodes_, pKappa_, pIds_;  // pending entries (arrival order)
-  mutable size_t nPending_, capPending_;
-  mutable DeviceBuffer scratch_, work_, t3ws_, recStage_, filtKappa_;  // filtKappa_: masked kappa of a filtered call
+  mutable DeviceLists lists_;  // over the K^2 cells
+  // grow-only; qIn_ stages host queries of search() (a cudaMalloc / cudaFree per call can cost more than the search)
+  mutable DeviceBuffer scratch_, work_, t3ws_, recStage_, qIn_;
 };
 
 }  // namespace gpu

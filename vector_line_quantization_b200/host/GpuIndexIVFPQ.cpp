@@ -1,6 +1,5 @@
 #include "GpuIndexIVFPQ.h"
 
-#include "ListRemoval.h"
 #include "RangeSearch.h"
 #include "Reconstruct.h"
 #include "SearchFilter.h"
@@ -55,8 +54,8 @@ GpuIndexIVFPQ::GpuIndexIVFPQ(GpuResources* resources, int dims, int nlist, int s
                              int nedge, int nLambda, faiss::MetricType metric, GpuIndexIVFPQConfig config)
     : GpuIndexIVF(resources, dims, metric, nlist, config), nLambda_(nLambda), numedge_(nedge), begin_(0), end_(nlist),
       w1_(256), edgeInfo_(nullptr), edgeDistInfo_(nullptr), lambdaInfo_(nullptr), constInfo_(nullptr), listCap_(VLQ_LIST_CAP),
-      ivfpqConfig_(config), subQuantizers_(subQuantizers), bitsPerCode_(bitsPerCode), reserveVecs_(0), nListed_(0), populatedLists_((size_t)nlist * nedge),
-      nPending_(0), capPending_(0) {
+      ivfpqConfig_(config), subQuantizers_(subQuantizers), bitsPerCode_(bitsPerCode),
+      lists_(resources, (int64_t)nlist * nedge, subQuantizers), populatedLists_((size_t)nlist * nedge) {
   VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8, "the scan kernels are written for 8-bit PQ codes");
   VLQ_THROW_IF_NOT_MSG(subQuantizers > 0 && subQuantizers <= 64 && dims % subQuantizers == 0,
                        "number of sub-quantizers must divide the dimension (and be <= 64)");
@@ -82,19 +81,9 @@ GpuIndexIVFPQ::~GpuIndexIVFPQ() {
   }
 }
 
-void GpuIndexIVFPQ::reserveMemory(size_t numVecs) { reserveVecs_ = numVecs; }
-
 void GpuIndexIVFPQ::reset() {
   DeviceScope scope(ivfConfig_.device);
-  resources_->syncDefaultStream();
-  lOffsets_.release();
-  lCodes_.release();
-  lLamq_.release();
-  lKappa_.release();
-  lIds_.release();
-  filtKappa_.release();
-  nListed_ = 0;
-  nPending_ = 0;
+  lists_.reset();
   ntotal = 0;
   populatedLists_ = (size_t)nlist_ * numedge_;
   begin_ = 0;
@@ -183,29 +172,6 @@ void GpuIndexIVFPQ::train(Index::idx_t n, const float* x) {
   is_trained = true;
 }
 
-void GpuIndexIVFPQ::ensurePending_(size_t extra) {
-  const size_t need = nPending_ + extra;
-  if (need <= capPending_) return;
-  vlq_stream_t st = resources_->getDefaultStream();
-  size_t cap = std::max(std::max(need, capPending_ * 2), std::max<size_t>(reserveVecs_, 1 << 16));
-  const int M = subQuantizers_;
-  DeviceBuffer nl(cap * sizeof(int)), nc(cap * M), nq(cap), nk(cap * sizeof(float)), ni(cap * sizeof(int64_t));
-  if (nPending_) {
-    VLQ_CALL(vlq_memcpy_d2d(nl.get(), pList_.get(), nPending_ * sizeof(int), st));
-    VLQ_CALL(vlq_memcpy_d2d(nc.get(), pCodes_.get(), nPending_ * M, st));
-    VLQ_CALL(vlq_memcpy_d2d(nq.get(), pLamq_.get(), nPending_, st));
-    VLQ_CALL(vlq_memcpy_d2d(nk.get(), pKappa_.get(), nPending_ * sizeof(float), st));
-    VLQ_CALL(vlq_memcpy_d2d(ni.get(), pIds_.get(), nPending_ * sizeof(int64_t), st));
-    resources_->syncDefaultStream();
-  }
-  pList_.swap(nl);
-  pCodes_.swap(nc);
-  pLamq_.swap(nq);
-  pKappa_.swap(nk);
-  pIds_.swap(ni);
-  capPending_ = cap;
-}
-
 // classifyAndAddVectors (gpu/GpuIndexIVFPQ.cu:577-908), entirely on the device: coarse NN -> fused line stage / lambda
 // quantiser / residual / PQ encode -> append to the pending arena.  Tiles of <= 512 Ki vectors like gpu/GpuIndex.cu:75-106.
 void GpuIndexIVFPQ::add_with_ids(Index::idx_t n, const float* x, const long* xids) { addTiles_(n, x, false, xids); }
@@ -219,7 +185,7 @@ void GpuIndexIVFPQ::addTiles_(Index::idx_t n, const void* xv, bool isU8, const l
   VLQ_THROW_IF_NOT(n > 0 && xv);
   DeviceScope scope(ivfConfig_.device);
   vlq_stream_t st = resources_->getDefaultStream();
-  ensurePending_((size_t)n);
+  const DeviceLists::Slots out = lists_.makeRoom((size_t)n);
   const Index::idx_t tile = (Index::idx_t)1 << 19;
   const int M = subQuantizers_;
   const size_t esz = isU8 ? 1 : sizeof(float);
@@ -250,20 +216,18 @@ void GpuIndexIVFPQ::addTiles_(Index::idx_t n, const void* xv, bool isU8, const l
     }
     dA.reserve((size_t)m * sizeof(int));
     quantizer_->assignDevice(dx, m, dA.as<int>(), nullptr, false);
-    const size_t o = nPending_;
     VLQ_CALL(vlq_line_encode(dx, m, d, dA.as<int>(), quantizer_->deviceVectors(), dEdge_.as<int>(),
                              dEdgeDist_.as<float>(), numedge_, dLambda_.as<float>(), nLambda_, dPq_.as<float>(), M,
-                             pList_.as<int>() + o, nullptr, pLamq_.as<uint8_t>() + o, pCodes_.as<uint8_t>() + o * M,
-                             pKappa_.as<float>() + o, nullptr, st));
+                             out.list + s, nullptr, out.lamq + s, out.codes + (size_t)s * M, out.kappa + s, nullptr, st));
     if (xids) {
       if (vlq_pointer_is_device(xids) == 1)
-        VLQ_CALL(vlq_memcpy_d2d(pIds_.as<int64_t>() + o, xids + s, (size_t)m * sizeof(int64_t), st));
+        VLQ_CALL(vlq_memcpy_d2d(out.ids + s, xids + s, (size_t)m * sizeof(int64_t), st));
       else
-        VLQ_CALL(vlq_memcpy_h2d(pIds_.as<int64_t>() + o, xids + s, (size_t)m * sizeof(int64_t), st));
+        VLQ_CALL(vlq_memcpy_h2d(out.ids + s, xids + s, (size_t)m * sizeof(int64_t), st));
     } else {
-      VLQ_CALL(vlq_iota_i64(pIds_.as<int64_t>() + o, m, (int64_t)(ntotal + s), st));
+      VLQ_CALL(vlq_iota_i64(out.ids + s, m, (int64_t)(ntotal + s), st));
     }
-    nPending_ += (size_t)m;
+    lists_.appended((size_t)m);
     if (s + tile < n) cur = stage(s + tile, slot ^ 1);  // overlaps the kernels just launched
     if (!onDevice) VLQ_CALL(vlq_stream_synchronize(cs));
     resources_->syncDefaultStream();  // the staging buffer of this tile is reused two tiles later
@@ -272,61 +236,20 @@ void GpuIndexIVFPQ::addTiles_(Index::idx_t n, const void* xv, bool isU8, const l
   ntotal += n;
 }
 
-void GpuIndexIVFPQ::commit_() const {
-  const int64_t L = (int64_t)nlist_ * numedge_;
-  if (nPending_ == 0 && lOffsets_.get()) return;
-  vlq_stream_t st = resources_->getDefaultStream();
-  const int M = subQuantizers_;
-  const size_t tot = nListed_ + nPending_;
-  DeviceBuffer no((size_t)(L + 1) * sizeof(int64_t)), nc(tot * M), nq(tot), nk(tot * sizeof(float)), ni(tot * sizeof(int64_t));
-  const size_t wsb = vlq_build_lists_workspace_bytes((int64_t)nPending_, L);
-  scratch_.reserve(wsb);
-  VLQ_CALL(vlq_build_lists(L, M, (int64_t)nListed_, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(),
-                           lKappa_.as<float>(), lIds_.as<int64_t>(), (int64_t)nPending_, pList_.as<int>(),
-                           pCodes_.as<uint8_t>(), pLamq_.as<uint8_t>(), pKappa_.as<float>(), pIds_.as<int64_t>(),
-                           no.as<int64_t>(), nc.as<uint8_t>(), nq.as<uint8_t>(), nk.as<float>(), ni.as<int64_t>(),
-                           scratch_.get(), scratch_.bytes(), st));
-  // vectors the encoder skipped (list id < 0) are not stored: the live count is offsets[L]
-  int64_t live = 0;
-  VLQ_CALL(vlq_memcpy_d2h(&live, no.as<int64_t>() + L, sizeof(int64_t), st));
-  resources_->syncDefaultStream();
-  lOffsets_.swap(no);
-  lCodes_.swap(nc);
-  lLamq_.swap(nq);
-  lKappa_.swap(nk);
-  lIds_.swap(ni);
-  nListed_ = (size_t)live;
-  nPending_ = 0;
-  // the pending arena has done its job: keep at most one add-chunk worth of it (a bulk load followed by searches would
-  // otherwise hold 33 B per vector next to the 29 B per vector of the lists)
-  const size_t keep = (size_t)1 << 21;
-  if (capPending_ > keep) {
-    pList_.release();
-    pCodes_.release();
-    pLamq_.release();
-    pKappa_.release();
-    pIds_.release();
-    capPending_ = 0;
-    reserveVecs_ = 0;
-  }
-}
-
-// IndexIVF::remove_ids: pending adds take part, then the slab is compacted on the device (host/ListRemoval.cpp)
+// IndexIVF::remove_ids: pending adds take part, then the slab is compacted on the device
 long GpuIndexIVFPQ::remove_ids(const IDSelector& sel) {
   DeviceScope scope(ivfConfig_.device);
   commit_();
-  const long removed = removeFromLists(resources_, sel, (int64_t)nlist_ * numedge_, subQuantizers_,
-                                       ListSlab{lOffsets_, lCodes_, lLamq_, lKappa_, lIds_, nListed_});
+  const long removed = lists_.remove(sel);
   ntotal -= removed;
   return removed;
 }
 
 // ------------------------------------------------------------------------------------------------ read-back
 void GpuIndexIVFPQ::decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const {
-  VLQ_CALL(vlq_decode_entries(n, pos, (int64_t)nlist_ * numedge_, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(),
-                              lLamq_.as<uint8_t>(), lIds_.as<int64_t>(), subQuantizers_, d, dPq_.as<float>(),
-                              quantizer_->deviceVectors(), dEdge_.as<int>(), numedge_, dLambda_.as<float>(), nLambda_,
-                              out, outIds, st));
+  VLQ_CALL(vlq_decode_entries(n, pos, lists_.nlists(), lists_.offsets(), lists_.codes(), lists_.lamq(), lists_.ids(),
+                              subQuantizers_, d, dPq_.as<float>(), quantizer_->deviceVectors(), dEdge_.as<int>(),
+                              numedge_, dLambda_.as<float>(), nLambda_, out, outIds, st));
 }
 
 void GpuIndexIVFPQ::readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const {
@@ -334,7 +257,7 @@ void GpuIndexIVFPQ::readBack_(Index::idx_t n, const Index::idx_t* keys, Index::i
   if (n == 0) return;
   DeviceScope scope(ivfConfig_.device);
   commit_();
-  reconstructIds(resources_, d, SlabIds{lIds_.as<int64_t>(), nListed_}, n, keys, i0, recons,
+  reconstructIds(resources_, d, lists_, n, keys, i0, recons,
                  [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
                  recStage_);
 }
@@ -363,16 +286,14 @@ void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, R
   if (sel) checkSearchSelector(sel);
   DeviceScope scope(ivfConfig_.device);
   if (n > 0) commit_();
-  const float* kappa = lKappa_.as<float>();
-  if (sel && n > 0) kappa = maskKappa(resources_, *sel, lIds_.as<int64_t>(), kappa, nListed_, filtKappa_);
+  const float* kappa = n > 0 ? lists_.kappa(sel) : nullptr;
   vlq_stream_t st = resources_->getDefaultStream();
   const int P = std::min(nprobe_, nlist_);
   const int W = w1_;
   const Index::idx_t tile = std::max<Index::idx_t>(64, std::min<Index::idx_t>(5120, ((Index::idx_t)5 << 26) / nlist_));
   DeviceBuffer coarseWs;
   RangeLists lists{dPq_.as<float>(), subQuantizers_, dLambda_.as<float>(), nLambda_, dEdgeDist_.as<float>(), W, listCap_,
-                   lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(), lLamq_.as<uint8_t>(), kappa,
-                   lIds_.as<int64_t>(), nListed_, true, tile};
+                   &lists_, kappa, true, tile};
   rangeSearchLists(resources_, d, n, x, radius, lists,
                    [&](const float* dq, Index::idx_t m, int* lines, float* t1, float* t6) {
                      coarseWs.reserve(vlq_coarse_lines_workspace_bytes(m, d, nlist_, P, numedge_, W,
@@ -426,11 +347,10 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
   if (sel) checkSearchSelector(sel);
   if (n == 0) return;
   commit_();
-  const int64_t* ids = slabIndex ? nullptr : lIds_.as<int64_t>();
+  const int64_t* ids = slabIndex ? nullptr : lists_.ids();
   // filtered: the mask pass runs on the default stream here, before the first page; the scan stream waits for the
   // default stream at every page start, so every scan reads the finished mask
-  const float* kappa = lKappa_.as<float>();
-  if (sel) kappa = maskKappa(resources_, *sel, lIds_.as<int64_t>(), kappa, nListed_, filtKappa_);
+  const float* kappa = lists_.kappa(sel);
   vlq_stream_t st = resources_->getDefaultStream();
   const int P = std::min(nprobe_, nlist_);
   const int W = w1_;
@@ -511,10 +431,9 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
       float* oD = inPlace ? hD : outD.as<float>() + (size_t)s * k;
       int64_t* oI = inPlace ? reinterpret_cast<int64_t*>(hI) : outI.as<int64_t>() + (size_t)s * k;
       VLQ_CALL(vlq_scan_topk(q, m, d, dPq_.as<float>(), M, dLambda_.as<float>(), nLambda_, lline, t1, t6,
-                             dEdgeDist_.as<float>(), W, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(),
-                             lLamq_.as<uint8_t>(), kappa, ids, (int)k, listCap_,
-                             (int)std::min<size_t>(nListed_ / populatedLists_, 1 << 20), oD, oI, t3ws_.get(),
-                             t3ws_.bytes(), sb));
+                             dEdgeDist_.as<float>(), W, lists_.offsets(), lists_.codes(), lists_.lamq(), kappa, ids,
+                             (int)k, listCap_, (int)std::min<size_t>(lists_.size() / populatedLists_, 1 << 20), oD, oI,
+                             t3ws_.get(), t3ws_.bytes(), sb));
       if (sel) VLQ_CALL(vlq_filter_results(m, (int)k, oD, oI, sb));  // (+inf, id) of masked entries -> padding
       if (epilogue) (*epilogue)(p0 + s, m, oD, oI, sb);
       if (overlap) VLQ_CALL(vlq_event_record(evScan_[slot], sb));
@@ -533,13 +452,9 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
 
 // ---------------------------------------------------------------------------------------------- list accessors
 int GpuIndexIVFPQ::getListLength(int listId) const {
-  VLQ_THROW_IF_NOT(listId >= 0 && listId < nlist_ * numedge_);
   DeviceScope scope(ivfConfig_.device);
   commit_();
-  int64_t o[2];
-  VLQ_CALL(vlq_memcpy_d2h(o, lOffsets_.as<int64_t>() + listId, sizeof(o), resources_->getDefaultStream()));
-  resources_->syncDefaultStream();
-  return (int)(o[1] - o[0]);
+  return (int)lists_.listLength(listId);
 }
 
 // Device lists keep the M code bytes of the entry at list position pos rotated by pos mod M (csrc/scan.cuh):
@@ -555,14 +470,14 @@ static void rotateListCodes(uint8_t* codes, size_t len, int M, bool toStored) {
 }
 
 template <typename T>
-static std::vector<T> fetchList(const DeviceBuffer& offsets, const DeviceBuffer& data, int listId, size_t per,
-                                GpuResources* res) {
+static std::vector<T> fetchList(const int64_t* offsets, const void* data, int listId, size_t per, GpuResources* res) {
   int64_t o[2];
-  VLQ_CALL(vlq_memcpy_d2h(o, offsets.as<int64_t>() + listId, sizeof(o), res->getDefaultStream()));
+  VLQ_CALL(vlq_memcpy_d2h(o, offsets + listId, sizeof(o), res->getDefaultStream()));
   res->syncDefaultStream();
   std::vector<T> out((size_t)(o[1] - o[0]) * per);
   if (!out.empty()) {
-    VLQ_CALL(vlq_memcpy_d2h(out.data(), data.as<T>() + (size_t)o[0] * per, out.size() * sizeof(T), res->getDefaultStream()));
+    VLQ_CALL(vlq_memcpy_d2h(out.data(), static_cast<const T*>(data) + (size_t)o[0] * per, out.size() * sizeof(T),
+                            res->getDefaultStream()));
     res->syncDefaultStream();
   }
   return out;
@@ -572,7 +487,8 @@ std::vector<unsigned char> GpuIndexIVFPQ::getListCodes(int listId) const {
   VLQ_THROW_IF_NOT(listId >= 0 && listId < nlist_ * numedge_);
   DeviceScope scope(ivfConfig_.device);
   commit_();
-  std::vector<unsigned char> codes = fetchList<unsigned char>(lOffsets_, lCodes_, listId, subQuantizers_, resources_);
+  std::vector<unsigned char> codes =
+      fetchList<unsigned char>(lists_.offsets(), lists_.codes(), listId, subQuantizers_, resources_);
   rotateListCodes(codes.data(), codes.size() / subQuantizers_, subQuantizers_, false);
   return codes;
 }
@@ -580,13 +496,13 @@ std::vector<unsigned char> GpuIndexIVFPQ::getListLambdas(int listId) const {
   VLQ_THROW_IF_NOT(listId >= 0 && listId < nlist_ * numedge_);
   DeviceScope scope(ivfConfig_.device);
   commit_();
-  return fetchList<unsigned char>(lOffsets_, lLamq_, listId, 1, resources_);
+  return fetchList<unsigned char>(lists_.offsets(), lists_.lamq(), listId, 1, resources_);
 }
 std::vector<long> GpuIndexIVFPQ::getListIndices(int listId) const {
   VLQ_THROW_IF_NOT(listId >= 0 && listId < nlist_ * numedge_);
   DeviceScope scope(ivfConfig_.device);
   commit_();
-  return fetchList<long>(lOffsets_, lIds_, listId, 1, resources_);
+  return fetchList<long>(lists_.offsets(), lists_.ids(), listId, 1, resources_);
 }
 
 void GpuIndexIVFPQ::merge(faiss::Index::idx_t* nns, float* dist, int k, int nq, int nprocess, float* distances,
@@ -645,13 +561,14 @@ void GpuIndexIVFPQ::writeDbToFile(const std::string& name) {  // .dbIdx .dbcodes
   vlq_stream_t st = resources_->getDefaultStream();
   const size_t L = (size_t)nlist_ * numedge_;
   std::vector<int64_t> off(L + 1);
-  std::vector<long> ids(nListed_);
-  std::vector<uint8_t> codes(nListed_ * subQuantizers_), las(nListed_);
-  VLQ_CALL(vlq_memcpy_d2h(off.data(), lOffsets_.get(), off.size() * sizeof(int64_t), st));
-  if (nListed_) {
-    VLQ_CALL(vlq_memcpy_d2h(ids.data(), lIds_.get(), ids.size() * sizeof(long), st));
-    VLQ_CALL(vlq_memcpy_d2h(codes.data(), lCodes_.get(), codes.size(), st));
-    VLQ_CALL(vlq_memcpy_d2h(las.data(), lLamq_.get(), las.size(), st));
+  const size_t n = lists_.size();
+  std::vector<long> ids(n);
+  std::vector<uint8_t> codes(n * subQuantizers_), las(n);
+  VLQ_CALL(vlq_memcpy_d2h(off.data(), lists_.offsets(), off.size() * sizeof(int64_t), st));
+  if (n) {
+    VLQ_CALL(vlq_memcpy_d2h(ids.data(), lists_.ids(), ids.size() * sizeof(long), st));
+    VLQ_CALL(vlq_memcpy_d2h(codes.data(), lists_.codes(), codes.size(), st));
+    VLQ_CALL(vlq_memcpy_d2h(las.data(), lists_.lamq(), las.size(), st));
   }
   resources_->syncDefaultStream();
   std::vector<int> counts(L);
@@ -676,27 +593,15 @@ void GpuIndexIVFPQ::installLists_(const std::vector<int>& counts, const std::vec
   for (size_t l = 0; l < L; l++) off[l + 1] = off[l] + counts[l];
   const size_t tot = (size_t)off[L];
   VLQ_THROW_IF_NOT(ids.size() == tot && las.size() == tot && codes.size() == tot * subQuantizers_);
-  reset();
-  lOffsets_.resize((L + 1) * sizeof(int64_t));
-  lCodes_.resize(std::max<size_t>(1, codes.size()));
-  lLamq_.resize(std::max<size_t>(1, tot));
-  lKappa_.resize(std::max<size_t>(1, tot) * sizeof(float));
-  lIds_.resize(std::max<size_t>(1, tot) * sizeof(int64_t));
-  VLQ_CALL(vlq_memcpy_h2d(lOffsets_.get(), off.data(), off.size() * sizeof(int64_t), st));
-  std::vector<uint8_t> stored;  // outlives the copy (freed after the stream sync below)
-  if (tot) {
-    stored = codes;
-    for (size_t l = 0; l < L; l++)
-      rotateListCodes(stored.data() + (size_t)off[l] * subQuantizers_, (size_t)counts[l], subQuantizers_, true);
-    VLQ_CALL(vlq_memcpy_h2d(lCodes_.get(), stored.data(), stored.size(), st));
-    VLQ_CALL(vlq_memcpy_h2d(lLamq_.get(), las.data(), tot, st));
-    VLQ_CALL(vlq_memcpy_h2d(lIds_.get(), ids.data(), tot * sizeof(int64_t), st));
-    VLQ_CALL(vlq_recompute_kappa((int64_t)tot, (int64_t)L, lOffsets_.as<int64_t>(), lCodes_.as<uint8_t>(),
-                                 lLamq_.as<uint8_t>(), quantizer_->deviceVectors(), d, dEdge_.as<int>(), numedge_,
-                                 dLambda_.as<float>(), dPq_.as<float>(), subQuantizers_, lKappa_.as<float>(), st));
-  }
+  std::vector<uint8_t> stored = codes;  // outlives the copy (freed after the stream sync below)
+  for (size_t l = 0; l < L; l++)
+    rotateListCodes(stored.data() + (size_t)off[l] * subQuantizers_, (size_t)counts[l], subQuantizers_, true);
+  float* kappa = lists_.install(off, stored, las, ids);
+  if (tot)
+    VLQ_CALL(vlq_recompute_kappa((int64_t)tot, (int64_t)L, lists_.offsets(), lists_.codes(), lists_.lamq(),
+                                 quantizer_->deviceVectors(), d, dEdge_.as<int>(), numedge_, dLambda_.as<float>(),
+                                 dPq_.as<float>(), subQuantizers_, kappa, st));
   resources_->syncDefaultStream();
-  nListed_ = tot;
   ntotal = (Index::idx_t)tot;
 }
 
@@ -869,7 +774,7 @@ void GpuIndexIVFPQ::search1(Index::idx_t n, const float* x, Index::idx_t k, floa
                               quantizer_->packScale(), nlist_, P, dEdge_.as<int>(), dEdgeDist_.as<float>(), numedge_, W,
                               nullptr, lline.as<int>(), t1.as<float>(), t6.as<float>(), coarseWs.get(), coarseWs.bytes(), st));
     int64_t* o = lOnDevice ? reinterpret_cast<int64_t*>(labels + (size_t)s * k) : out.as<int64_t>();
-    VLQ_CALL(vlq_gather_candidates(lline.as<int>(), m, W, lOffsets_.as<int64_t>(), lIds_.as<int64_t>(), (int64_t)k, o, st));
+    VLQ_CALL(vlq_gather_candidates(lline.as<int>(), m, W, lists_.offsets(), lists_.ids(), (int64_t)k, o, st));
     if (!lOnDevice) VLQ_CALL(vlq_memcpy_d2h(labels + (size_t)s * k, o, (size_t)m * k * sizeof(int64_t), st));
     resources_->syncDefaultStream();
   }

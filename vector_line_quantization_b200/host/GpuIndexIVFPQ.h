@@ -1,9 +1,8 @@
 // GpuIndexIVFPQ with the vector-line-quantization extension: the index class of the hot path
 // (reference gpu/GpuIndexIVF.{h,cu}, gpu/GpuIndexIVFPQ.{h,cu}; VLQ ctor gpu/GpuIndexIVFPQ.h:59-67, public VLQ members
 // :69-81).  Same constructor signature, member names and file formats; the implementation underneath is new:
-// inverted lists are one CSR slab on the device (codes + lambda byte + per-entry kappa + ids), adds are encoded and
-// appended entirely on the device, and search is four kernels per query tile (coarse GEMM, top-P, line selection,
-// fused scan + top-k).
+// inverted lists are one CSR slab on the device (DeviceLists.h), adds are encoded and appended entirely on the device,
+// and search is four kernels per query tile (coarse GEMM, top-P, line selection, fused scan + top-k).
 #pragma once
 #include <cstdint>
 #include <functional>
@@ -11,6 +10,7 @@
 #include <vector>
 
 #include "AuxIndexStructures.h"
+#include "DeviceLists.h"
 #include "GpuIndexFlat.h"
 #include "IndexIVFPQ.h"
 #include "ProductQuantizer.h"
@@ -114,7 +114,7 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   void search_and_reconstruct(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
                               float* recons, const SearchParameters* params) const override;
 
-  void reserveMemory(size_t numVecs);
+  void reserveMemory(size_t numVecs) { lists_.reserve(numVecs); }
   void setPrecomputedCodes(bool) {}
   bool getPrecomputedCodes() const { return true; }
   int getNumSubQuantizers() const { return subQuantizers_; }
@@ -164,17 +164,16 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
 
  private:
   void uploadTables_();
-  void commit_() const;  ///< merge pending entries into the CSR lists (lazy: first search / list access after adds)
+  void commit_() const { lists_.commit(scratch_); }  ///< lazy: first search / list access after adds
   /// the query tile pipeline of search(): slabIndex makes the scan report slab indexes instead of ids; `epilogue`
   /// (nullable) runs on the scan stream after each tile's scan with (first row, rows, device D [m][k], device I [m][k],
-  /// stream), before the tile's results are copied out.  sel (nullable): the scan reads the masked kappa (filtKappa_)
-  /// and each tile's +inf results become padding (vlq_filter_results) before the epilogue.
+  /// stream), before the tile's results are copied out.  sel (nullable): the scan reads the masked kappa and each
+  /// tile's +inf results become padding (vlq_filter_results) before the epilogue.
   using TileEpilogue = std::function<void(Index::idx_t row0, Index::idx_t m, float* dD, int64_t* dI, vlq_stream_t st)>;
   void searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
                     bool slabIndex, const TileEpilogue* epilogue, const IDSelector* sel) const;
   void decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const;
   void readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const;
-  void ensurePending_(size_t extra);
   void addTiles_(Index::idx_t n, const void* x, bool isU8, const long* xids);
   void installLists_(const std::vector<int>& counts, const std::vector<uint8_t>& codes, const std::vector<uint8_t>& las,
                      const std::vector<long>& ids);
@@ -183,20 +182,14 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   int subQuantizers_;
   int bitsPerCode_;
   std::vector<float> pqHost_;  // (M, 256, dsub)
-  mutable size_t reserveVecs_;  // bulk-load hint of reserveMemory(): consumed by the first commit
 
   // device tables
   DeviceBuffer dEdge_, dEdgeDist_, dLambda_, dPq_;
-  // CSR lists
-  mutable DeviceBuffer lOffsets_, lCodes_, lLamq_, lKappa_, lIds_;
-  mutable size_t nListed_;
+  mutable DeviceLists lists_;  // over the nlist * numedge lines
   size_t populatedLists_;  ///< lists that can hold entries (all of them; the slice of readDbFromFile(name, pronum, rank))
-  // pending (encoded, arrival order)
-  mutable DeviceBuffer pList_, pCodes_, pLamq_, pKappa_, pIds_;
-  mutable size_t nPending_, capPending_;
   mutable vlq_event_t evCoarse_[2] = {nullptr, nullptr}, evScan_[2] = {nullptr, nullptr};  // search(): two-stream tile pipeline
-  mutable DeviceBuffer scratch_, scratchB_, qIn_, outD_, outI_, addIn_[2], addA_, addF32_, t3ws_, recStage_,
-      filtKappa_;  // grow-only staging / workspace; filtKappa_: the masked kappa of a filtered call (4 B per entry)
+  mutable DeviceBuffer scratch_, scratchB_, qIn_, outD_, outI_, addIn_[2], addA_, addF32_, t3ws_,
+      recStage_;  // grow-only staging / workspace
 };
 
 }  // namespace gpu

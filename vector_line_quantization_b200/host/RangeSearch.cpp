@@ -24,7 +24,7 @@ void rangeSearchLists(GpuResources* res, int d, Index::idx_t n, const float* x, 
   std::fill(result->lims, result->lims + n + 1, (size_t)0);
   std::vector<float> hD;
   std::vector<int64_t> hI;
-  if (n > 0 && L.nListed > 0) {
+  if (n > 0 && L.lists->size() > 0) {
     vlq_stream_t st = res->getDefaultStream();
     const int W = L.W;
     const Index::idx_t tile = std::min(L.tile, n);
@@ -46,8 +46,8 @@ void rangeSearchLists(GpuResources* res, int d, Index::idx_t n, const float* x, 
       if (L.addQueryNorm) VLQ_CALL(vlq_row_norms(q, m, d, qn.as<float>(), st));
       const float* rowAdd = L.addQueryNorm ? qn.as<float>() : nullptr;
       VLQ_CALL(vlq_range_count(q, m, d, L.pq, L.M, L.lambdaCb, L.nLambda, lines.as<int>(), t1.as<float>(), t6.as<float>(),
-                               L.edgeDist, W, L.offsets, L.codes, L.lamq, L.kappa, L.cap, rowAdd, radius,
-                               lims.as<int64_t>(), ws.get(), ws.bytes(), st));
+                               L.edgeDist, W, L.lists->offsets(), L.lists->codes(), L.lists->lamq(), L.kappa, L.cap,
+                               rowAdd, radius, lims.as<int64_t>(), ws.get(), ws.bytes(), st));
       // the one host synchronisation of a tile: its result sizes decide the sub-ranges and the host arrays
       VLQ_CALL(vlq_memcpy_d2h(hl.data(), lims.get(), (size_t)(m + 1) * sizeof(int64_t), st));
       res->syncDefaultStream();
@@ -74,8 +74,9 @@ void rangeSearchLists(GpuResources* res, int d, Index::idx_t n, const float* x, 
         const int64_t cnt = hl[p.second] - hl[p.first];
         if (cnt == 0) continue;
         VLQ_CALL(vlq_range_gather(q, m, d, L.pq, L.M, L.lambdaCb, L.nLambda, lines.as<int>(), t1.as<float>(),
-                                  t6.as<float>(), L.edgeDist, W, L.offsets, L.codes, L.lamq, L.kappa, L.cap, rowAdd, radius,
-                                  L.ids, lims.as<int64_t>(), p.first, p.second, sD, sI, ws.get(), ws.bytes(), st));
+                                  t6.as<float>(), L.edgeDist, W, L.lists->offsets(), L.lists->codes(), L.lists->lamq(),
+                                  L.kappa, L.cap, rowAdd, radius, L.lists->ids(), lims.as<int64_t>(), p.first, p.second,
+                                  sD, sI, ws.get(), ws.bytes(), st));
         // stream order: the next gather overwrites the staging buffer only after these copies
         VLQ_CALL(vlq_memcpy_d2h(hD.data() + at + hl[p.first], sD, (size_t)cnt * sizeof(float), st));
         VLQ_CALL(vlq_memcpy_d2h(hI.data() + at + hl[p.first], sI, (size_t)cnt * sizeof(int64_t), st));

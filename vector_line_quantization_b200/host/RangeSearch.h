@@ -1,21 +1,20 @@
-// range_search over the CSR list slab that GpuIndexIVFPQ and GpuIndexIMIPQ share (offsets / codes / lamq / kappa / ids,
-// csrc/lists.cu).  Each index supplies its coarse stage (the W lines of every query of a tile with their term1 / term6);
-// per query tile the helper then counts the results on the device (vlq_range_count), reads the tile's lims (one host
-// synchronisation per tile: the result sizes decide the buffers), gathers the results in query sub-ranges that fit a
-// bounded device staging buffer (vlq_range_gather) and downloads them.  The result is assembled through
-// RangeSearchResult::do_allocation().
+// range_search over the lists of DeviceLists.h.  Each index supplies its coarse stage (the W lines of every query of a
+// tile with their term1 / term6); per query tile the helper then counts the results on the device (vlq_range_count),
+// reads the tile's lims (one host synchronisation per tile: the result sizes decide the buffers), gathers the results
+// in query sub-ranges that fit a bounded device staging buffer (vlq_range_gather) and downloads them.  The result is
+// assembled through RangeSearchResult::do_allocation().
 #pragma once
 #include <cstddef>
 #include <cstdint>
 #include <functional>
 
 #include "AuxIndexStructures.h"
-#include "GpuResources.h"
+#include "DeviceLists.h"
 
 namespace faiss {
 namespace gpu {
 
-/// the committed slab and the scan tables of an index (device pointers)
+/// the committed lists and the scan tables of an index (device pointers)
 struct RangeLists {
   const float* pq;        ///< (M, 256, d / M)
   int M;
@@ -24,12 +23,8 @@ struct RangeLists {
   const float* edgeDist;  ///< per-list squared edge length (term5); nullptr = 0 (IMI-PQ)
   int W;                  ///< lines per query
   int cap;                ///< entries scanned per line at most
-  const int64_t* offsets;
-  const uint8_t* codes;
-  const uint8_t* lamq;
-  const float* kappa;
-  const int64_t* ids;
-  size_t nListed;         ///< entries in the slab
+  const DeviceLists* lists;  ///< committed
+  const float* kappa;        ///< lists->kappa(sel) of the call
   bool addQueryNorm;      ///< term1 excludes ||q||^2 (the VLQ coarse stage): add it back for the full distance
   Index::idx_t tile;      ///< queries per coarse stage at most
 };

@@ -32,7 +32,7 @@ void decodeToOutput(int d, const int64_t* pos, int64_t n, float* recons, int64_t
   }
 }
 
-void reconstructIds(GpuResources* res, int d, const SlabIds& slab, Index::idx_t n, const Index::idx_t* keys,
+void reconstructIds(GpuResources* res, int d, const DeviceLists& lists, Index::idx_t n, const Index::idx_t* keys,
                     Index::idx_t i0, float* recons, const EntryDecoder& decode, DeviceBuffer& staging) {
   VLQ_THROW_IF_NOT_MSG(n >= 0, "reconstruct: n must be >= 0");
   if (n == 0) return;
@@ -59,7 +59,7 @@ void reconstructIds(GpuResources* res, int d, const SlabIds& slab, Index::idx_t 
     VLQ_CALL(vlq_memcpy_h2d(dKeys.get(), uk.data(), dKeys.bytes(), st));
   }
   DeviceBuffer dPos((size_t)nslots * sizeof(int64_t)), dFound(sizeof(int64_t));
-  VLQ_CALL(vlq_lookup_ids((int64_t)slab.nListed, slab.ids, keys ? 0 : i0, dKeys.as<int64_t>(), nslots,
+  VLQ_CALL(vlq_lookup_ids((int64_t)lists.size(), lists.ids(), keys ? 0 : i0, dKeys.as<int64_t>(), nslots,
                           dPos.as<int64_t>(), dFound.as<int64_t>(), st));
   int64_t found = 0;
   VLQ_CALL(vlq_memcpy_d2h(&found, dFound.get(), sizeof(int64_t), st));
