@@ -290,7 +290,8 @@ int vlq_gather_candidates(const int* line_list, int64_t nq, int W, const int64_t
  *     warp-per-list walk (1B-scale lists), otherwise the flattened entry stream (lists of a few entries).  Results are
  *     identical either way.
  *     workspace (optional, vlq_scan_topk_workspace_bytes): holds the term-3 tables of the batch, built by one
- *     persistent kernel with the PQ codebook in shared memory; with workspace == NULL every query CTA builds its own.
+ *     persistent kernel with the PQ codebook in shared memory, and the list of short-list queries too long for the
+ *     short-list kernel; with workspace == NULL every query CTA builds its own tables in the general kernel.
  *     The one exception to "never synchronises": the FIRST call of a process that selects the long-list kernel
  *     (list_len_hint >= 160) runs a one-thread probe kernel and copies 4 bytes back (base address of the dynamic shared
  *     memory, which that kernel folds into its load instructions); later calls only enqueue work.

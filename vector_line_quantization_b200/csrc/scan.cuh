@@ -25,7 +25,7 @@ struct ScanArgs {
   int k, cap;
   int sel_cap;
   int owner_cap;    // stream positions covered by the shared-memory owner table (0 = always binary search)
-  int no_small;     // tests (VLQ_SCAN_NO_SMALL): skip the register-resident small-query path of scan_topk_kernel
+  const int* qlist; // scan_topk_kernel: nullptr = query blockIdx.x; else {n, q_0 .. q_n-1}: CTA j < n scans q_j
   const float* t3;  // optional precomputed term-3 tables [nq][M*ksub] (term3_kernel); nullptr = build in the kernel
   float* outD;
   int64_t* outI;

@@ -262,12 +262,18 @@ coarse_select_lines_kernel(const float* __restrict__ D, int64_t ldD, const float
 }
 
 // ------------------------------------------------------------------------------------------------ scan + top-k
+// Distance of one scanned entry: (kappa + adc) + (t1 + l t6 + (l^2 - l) t5), l = lambda_cb[lamq].  Every block-synchronous
+// scan kernel evaluates it through this one expression, so they contract it into the same FMAs and agree bit for bit.
+__device__ __forceinline__ float entry_dist(float kp, float adc, float la, float t1, float t6, float t5) {
+  const float base_d = t1 + la * t6 + (la * la - la) * t5;
+  return (kp + adc) + base_d;
+}
+
 // LONG = false: the selected lists are walked as ONE flattened entry stream (lists of a handful of entries keep all
 //               lanes busy);  LONG = true: every warp owns whole lists (slot w -> warp w % 8) and strides their entries,
 //               so the per-list scalars are warp-uniform and nothing has to be searched per entry.
 template <int M_T, bool LONG>
-__global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel(ScanArgs a) {  // 3 CTAs per SM (80 registers); measured at C2 before the strided small-query path: 0.86 ms per 10 k queries, 2 CTAs 1.03, 4 CTAs (spills) 1.63 -- now 0.57
-  extern __shared__ __align__(16) unsigned char smem[];
+__device__ __forceinline__ void scan_query(const ScanArgs& a, const int64_t qi, unsigned char* smem) {
   // smem: [topk keys S*8 + 16][T3 M*ksub f32][lambda nL f32][per line: start i64, prefix i32 (W+1), t1, t6, t5 f32]
   const int M = a.M, ksub = a.ksub, dsub = a.dsub, W = a.W;
   BlockSelect<Q_THREADS> sel;
@@ -289,7 +295,6 @@ __global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel
   uint16_t* owner = reinterpret_cast<uint16_t*>(smem + off);  // [owner_cap] line slot of every stream position
 
   sel.init(smem, a.k, a.sel_cap, LONG ? 2 : Q_BATCH);
-  const int64_t qi = blockIdx.x;
   const float* qv = a.q + qi * a.d;
 
   // term3 table: T3[m][j] = -2 q_m . p_mj            (gpu/impl/IVFPQ.cu:1409-1432)
@@ -391,11 +396,7 @@ __global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel
           const int e = off_ + u * 32 + lane;
           const bool valid = e < len;
           float dist = 0.f;
-          if (valid) {
-            const float la = lcb[lq[u]];
-            const float base_d = t1 + la * t6 + (la * la - la) * t5;
-            dist = (kp[u] + cr[u].adc(T3, M, ksub)) + base_d;
-          }
+          if (valid) dist = entry_dist(kp[u], cr[u].adc(T3, M, ksub), lcb[lq[u]], t1, t6, t5);
           any |= sel.offer_f(valid, dist, (uint32_t)(p0 + e));
         }
         off_ += 64;
@@ -408,97 +409,6 @@ __global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel
     for (int w = threadIdx.x; w < W; w += Q_THREADS)
       for (int p = prefix[w]; p < prefix[w + 1]; p++) owner[p] = (uint16_t)w;
     __syncthreads();
-  }
-
-  // ---- small queries (a few thousand entries in all, the C2 regime): every distance of the query fits in registers,
-  // kSmallR per thread, so the selection is ONE register-resident radix threshold (csl::kth32, coarse_select.cuh) +
-  // a rank ordering of the k survivors instead of the append / compact / sort machinery of BlockSelect, which was 80 %
-  // of this kernel's instructions at 2.7 k entries per query.  Ties resolve to the lowest stream position exactly as in
-  // the general path (take_k_strided); same arithmetic, same bits.
-  constexpr int kSmallR = 16, kSmallB = 4;
-  if (!LONG && use_owner && !a.no_small && total <= kSmallR * Q_THREADS && a.k <= a.sel_cap) {  // block-uniform
-    // stream position of key[r] = r * Q_THREADS + t: adjacent threads read adjacent entries of a list, every thread has
-    // work (a C2 query has ~1800 entries: 7 rows of 256), and the loads of kSmallB rows are in flight together
-    uint32_t key[kSmallR];
-#pragma unroll
-    for (int r = 0; r < kSmallR; r++) key[r] = csl::kInf32;
-#pragma unroll
-    for (int r0 = 0; r0 < kSmallR; r0 += kSmallB) {
-      if (r0 * Q_THREADS >= total) break;  // block-uniform
-      CodeRegs<M_T> cr[kSmallB];
-      uint8_t lq[kSmallB];
-      float kp[kSmallB];
-      int lo_[kSmallB];
-#pragma unroll
-      for (int u = 0; u < kSmallB; u++) {
-        const int pos = (r0 + u) * Q_THREADS + (int)threadIdx.x;
-        lq[u] = 0;
-        kp[u] = 0.f;
-        lo_[u] = 0;
-        if (pos < total) {
-          const int lo = owner[pos];
-          const int pl = pos - prefix[lo];
-          const int64_t ent = lstart[lo] + pl;
-          cr[u].load(a.codes + ent * M, pl);
-          lq[u] = a.lamq[ent];
-          kp[u] = a.kappa[ent];
-          lo_[u] = lo;
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < kSmallB; u++) {
-        const int pos = (r0 + u) * Q_THREADS + (int)threadIdx.x;
-        if (pos < total) {
-          const int lo = lo_[u];
-          const float la = lcb[lq[u]];
-          const float base_d = lt1[lo] + la * lt6[lo] + (la * la - la) * lt5[lo];
-          const float dist = (kp[u] + cr[u].adc(T3, M, ksub)) + base_d;
-          key[r0 + u] = csl::key32(dist);
-        }
-      }
-    }
-    uint64_t* skeys = reinterpret_cast<uint64_t*>(smem);  // the BlockSelect key area: <= k survivors
-    int* shist = reinterpret_cast<int*>(skeys + a.sel_cap);
-    int* smeta = shist + 256;
-    int* swsum = reinterpret_cast<int*>(owner + ((a.owner_cap + 1) & ~1));  // 16 ints behind the owner table
-    if (threadIdx.x == 0) swsum[8] = 0;
-    const csl::Kth kt = csl::kth32<kSmallR>(key, a.k, shist, smeta);
-    bool take[kSmallR];
-    csl::take_k_strided<kSmallR>(key, kt, a.k, swsum, take);
-#pragma unroll
-    for (int r = 0; r < kSmallR; r++)
-      if (take[r]) skeys[atomicAdd(&swsum[8], 1)] = ((uint64_t)key[r] << 32) | (uint32_t)(r * Q_THREADS + (int)threadIdx.x);
-    for (int i = threadIdx.x; i < a.k; i += Q_THREADS) {
-      a.outD[qi * a.k + i] = FLT_MAX;
-      a.outI[qi * a.k + i] = -1;
-    }
-    __syncthreads();
-    const int ns = swsum[8];  // <= k
-    if (ns > 128 && ns <= Q_THREADS) {  // block-uniform: one survivor per thread, bitonic sort (coarse_select.cuh);
-                                        // up to 128 survivors the rank loop below is cheaper (4 warps x ns compares)
-      uint64_t mykey = (int)threadIdx.x < ns ? skeys[threadIdx.x] : ~0ull;
-      __syncthreads();  // skeys[] becomes the exchange buffer (sel_cap >= 256 keys)
-      mykey = csl::block_sort256(mykey, skeys);
-      if ((int)threadIdx.x < ns) {
-        const int pos = (int)key_payload(mykey);
-        const int lo = owner[pos];
-        a.outD[qi * a.k + threadIdx.x] = ord2f((uint32_t)(mykey >> 32));
-        const int64_t e = lstart[lo] + (pos - prefix[lo]);
-        a.outI[qi * a.k + threadIdx.x] = a.ids ? a.ids[e] : e;
-      }
-      return;
-    }
-    for (int i = threadIdx.x; i < ns; i += Q_THREADS) {
-      const uint64_t mykey = skeys[i];
-      int rank = 0;
-      for (int j = 0; j < ns; j++) rank += skeys[j] < mykey;
-      const int pos = (int)key_payload(mykey);
-      const int lo = owner[pos];
-      a.outD[qi * a.k + rank] = ord2f((uint32_t)(mykey >> 32));
-      const int64_t e = lstart[lo] + (pos - prefix[lo]);
-      a.outI[qi * a.k + rank] = a.ids ? a.ids[e] : e;
-    }
-    return;
   }
 
   for (int base = 0; !LONG && base < total; base += Q_BATCH * Q_THREADS) {
@@ -562,10 +472,7 @@ __global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel
       float dist = 0.f;
       if (valid) {
         const int lo = lo_[b];
-        const float la = lcb[lq[b]];
-        const float base_d = lt1[lo] + la * lt6[lo] + (la * la - la) * lt5[lo];
-        const float acc = cr[b].adc(T3, M, ksub);
-        dist = (kp[b] + acc) + base_d;
+        dist = entry_dist(kp[b], cr[b].adc(T3, M, ksub), lcb[lq[b]], lt1[lo], lt6[lo], lt5[lo]);
       }
       any |= sel.offer_f(valid, dist, (uint32_t)pos);
     }
@@ -589,6 +496,219 @@ __global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel
     }
     a.outD[qi * a.k + i] = dv;
     a.outI[qi * a.k + i] = id;
+  }
+}
+
+// a.qlist: CTA j scans query a.qlist[1 + j] of the overflow list of scan_short_kernel.  3 CTAs per SM at M = 16 (ptxas,
+// sm_100a, CUDA 12.9: 80 registers, 40 bytes of spill stores); measured at C2 before the small queries had a kernel of
+// their own: 2 CTAs 1.03 ms per 10 k queries, 3 CTAs 0.86, 4 CTAs (spills) 1.63.
+template <int M_T, bool LONG>
+__global__ void __launch_bounds__(Q_THREADS, M_T == 16 ? 3 : 2) scan_topk_kernel(ScanArgs a) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  if (a.qlist && (int)blockIdx.x >= a.qlist[0]) return;
+  scan_query<M_T, LONG>(a, a.qlist ? (int64_t)a.qlist[1 + blockIdx.x] : (int64_t)blockIdx.x, smem);
+}
+
+// ------------------------------------------------------------------------------------------------ short-list scan
+// The flattened-stream queries of the C2 regime (a few thousand entries each): every distance of the query fits in
+// registers, kShortR per thread, so the selection is ONE register-resident radix threshold (csl::kth32,
+// coarse_select.cuh) + a rank ordering of the <= k survivors instead of BlockSelect's append / compact / sort machinery.
+// A kernel of its own so that it is sized for this path alone -- no 16 KiB BlockSelect buffer, <= 64 registers, four
+// CTAs per SM where the general kernel fits three -- and with a short per-query chain: the term-3 row arrives through
+// one bulk copy issued first, while the line descriptors are read; the prefix over the lines is a block scan.
+// A query of more than kShortCap entries is appended to the overflow list {n, q_0 .. q_n-1} and scanned by
+// scan_topk_kernel afterwards.  Same distance (entry_dist) and the same rule -- the k smallest (key32(dist), stream
+// position), NaN never selected -- as the general path: same bits.
+constexpr int kShortR = 16, kShortB = 4, kShortCap = kShortR * Q_THREADS;
+
+__host__ __device__ inline size_t align16(size_t b) { return (b + 15) & ~size_t(15); }
+
+struct ShortSmem {  // byte offsets in dynamic shared memory (host and device agree through this constructor)
+  size_t t3, lcb, lstart, prefix, t1, t6, t5, owner, keys, ints, end;
+  __host__ __device__ ShortSmem(int M, int nL, int W, int k) {
+    t3 = 0;
+    lcb = t3 + align16(sizeof(float) * M * 256);
+    lstart = lcb + align16(sizeof(float) * nL);
+    prefix = lstart + align16(sizeof(int64_t) * W);
+    t1 = prefix + align16(sizeof(int) * (W + 1));
+    t6 = t1 + align16(sizeof(float) * W);
+    t5 = t6 + align16(sizeof(float) * W);
+    owner = t5 + align16(sizeof(float) * W);
+    keys = owner + align16(sizeof(uint16_t) * kShortCap);
+    ints = keys + sizeof(uint64_t) * (k > Q_THREADS ? k : Q_THREADS);  // survivors; >= 256 for block_sort256
+    end = ints + sizeof(int) * (256 + 8 + 16);                          // histogram, kth32 meta, warp sums + counter
+  }
+};
+
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+  uint32_t done = 0;
+  while (!done)
+    asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
+                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+}
+
+// 4 CTAs per SM.  ptxas (sm_100a, CUDA 12.9): 62 registers at M = 16 (60 at M = 8, 64 generic), no spills; dynamic
+// shared memory 34 928 bytes at M = 16, W = 256, k = 100, nL = 256 (+ 16 bytes static for the mbarrier).
+template <int M_T>
+__global__ void __launch_bounds__(Q_THREADS, 4) scan_short_kernel(ScanArgs a, int* __restrict__ overflow) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  __shared__ __align__(8) uint64_t t3_bar;
+  const int M = a.M, ksub = a.ksub, W = a.W;
+  const ShortSmem L(M, a.nL, W, a.k);
+  float* T3 = reinterpret_cast<float*>(smem + L.t3);
+  float* lcb = reinterpret_cast<float*>(smem + L.lcb);
+  int64_t* lstart = reinterpret_cast<int64_t*>(smem + L.lstart);
+  int* prefix = reinterpret_cast<int*>(smem + L.prefix);
+  float* lt1 = reinterpret_cast<float*>(smem + L.t1);
+  float* lt6 = reinterpret_cast<float*>(smem + L.t6);
+  float* lt5 = reinterpret_cast<float*>(smem + L.t5);
+  uint16_t* owner = reinterpret_cast<uint16_t*>(smem + L.owner);  // line slot of every stream position
+  uint64_t* skeys = reinterpret_cast<uint64_t*>(smem + L.keys);
+  int* shist = reinterpret_cast<int*>(smem + L.ints);
+  int* smeta = shist + 256;
+  int* swsum = smeta + 8;
+  const int64_t qi = blockIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+
+  const uint32_t bar = (uint32_t)__cvta_generic_to_shared(&t3_bar);
+  if (tid == 0) {  // term-3 row of the query (a.t3, 16-byte aligned): nothing waits for it before the first ADC
+    const uint32_t bytes = (uint32_t)(sizeof(float) * M * ksub);
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar) : "memory");
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"((uint32_t)__cvta_generic_to_shared(T3)), "l"(a.t3 + (size_t)qi * M * ksub), "r"(bytes), "r"(bar)
+                 : "memory");
+  }
+  for (int i = tid; i < a.nL; i += Q_THREADS) lcb[i] = a.lambda_cb[i];
+  // line descriptors (lengths capped like gpu/impl/IVFUtils.cu:87); thread t owns the consecutive lines [w0, w1)
+  const int chunk = (W + Q_THREADS - 1) / Q_THREADS;
+  const int w0 = min(W, tid * chunk), w1 = min(W, w0 + chunk);
+  int mine = 0;
+  for (int w = w0; w < w1; w++) {
+    const int list = a.line_list[qi * W + w];
+    int len = 0;
+    int64_t st = 0;
+    float t5 = 0.f;
+    if (list >= 0) {
+      st = a.offsets[list];
+      const int64_t l = a.offsets[list + 1] - st;
+      len = (int)(l < a.cap ? l : a.cap);
+      t5 = a.edge_d2 ? a.edge_d2[list] : 0.f;
+    }
+    lstart[w] = st;
+    prefix[w + 1] = len;
+    lt1[w] = a.term1[qi * W + w];
+    lt6[w] = a.term6[qi * W + w];
+    lt5[w] = t5;
+    mine += len;
+  }
+  // block-wide exclusive scan of the per-thread entry counts: warp scans + 8 warp totals
+  int inc = mine;
+#pragma unroll
+  for (int o = 1; o < kWarp; o <<= 1) {
+    const int t = __shfl_up_sync(kFull, inc, o);
+    if (lane >= o) inc += t;
+  }
+  if (lane == kWarp - 1) swsum[warp] = inc;
+  __syncthreads();
+  int run = inc - mine, total = 0;
+#pragma unroll
+  for (int w = 0; w < Q_THREADS / kWarp; w++) {
+    const int c = swsum[w];
+    if (w < warp) run += c;
+    total += c;
+  }
+  if (total > kShortCap) {  // block-uniform: the general kernel takes this query
+    if (tid == 0) {
+      overflow[1 + atomicAdd(overflow, 1)] = (int)qi;
+      mbar_wait(bar, 0);  // the bulk copy must land before the CTA's shared memory is released
+    }
+    return;
+  }
+  if (tid == 0) prefix[0] = 0;
+  for (int w = w0; w < w1; w++) {  // stream positions of the thread's lines -> prefix and owner table
+    const int len = prefix[w + 1];
+    for (int p = run; p < run + len; p++) owner[p] = (uint16_t)w;
+    run += len;
+    prefix[w + 1] = run;
+  }
+  if (tid == 0) swsum[8] = 0;  // survivor counter (swsum[0..7] are free again after the barrier)
+  __syncthreads();
+
+  // stream position of key[r] = r * Q_THREADS + t: adjacent threads read adjacent entries of a list, every thread has
+  // work (a C2 query has ~1800 entries: 7 rows of 256), and the loads of kShortB rows are in flight together
+  uint32_t key[kShortR];
+#pragma unroll
+  for (int r = 0; r < kShortR; r++) key[r] = csl::kInf32;
+#pragma unroll
+  for (int r0 = 0; r0 < kShortR; r0 += kShortB) {
+    if (r0 > 0 && r0 * Q_THREADS >= total) break;  // block-uniform (the first round always runs: it waits for T3)
+    CodeRegs<M_T> cr[kShortB];
+    uint8_t lq[kShortB];
+    float kp[kShortB];
+    int lo_[kShortB];
+#pragma unroll
+    for (int u = 0; u < kShortB; u++) {
+      const int pos = (r0 + u) * Q_THREADS + tid;
+      lq[u] = 0;
+      kp[u] = 0.f;
+      lo_[u] = 0;
+      if (pos < total) {
+        const int lo = owner[pos];
+        const int pl = pos - prefix[lo];
+        const int64_t ent = lstart[lo] + pl;
+        cr[u].load(a.codes + ent * M, pl);
+        lq[u] = a.lamq[ent];
+        kp[u] = a.kappa[ent];
+        lo_[u] = lo;
+      }
+    }
+    if (r0 == 0) mbar_wait(bar, 0);
+#pragma unroll
+    for (int u = 0; u < kShortB; u++) {
+      const int pos = (r0 + u) * Q_THREADS + tid;
+      if (pos < total) {
+        const int lo = lo_[u];
+        key[r0 + u] = csl::key32(entry_dist(kp[u], cr[u].adc(T3, M, ksub), lcb[lq[u]], lt1[lo], lt6[lo], lt5[lo]));
+      }
+    }
+  }
+  const csl::Kth kt = csl::kth32<kShortR>(key, a.k, shist, smeta);
+  bool take[kShortR];
+  csl::take_k_strided<kShortR>(key, kt, a.k, swsum, take);
+#pragma unroll
+  for (int r = 0; r < kShortR; r++)
+    if (take[r]) skeys[atomicAdd(&swsum[8], 1)] = ((uint64_t)key[r] << 32) | (uint32_t)(r * Q_THREADS + tid);
+  for (int i = tid; i < a.k; i += Q_THREADS) {
+    a.outD[qi * a.k + i] = FLT_MAX;
+    a.outI[qi * a.k + i] = -1;
+  }
+  __syncthreads();
+  const int ns = swsum[8];  // <= k
+  if (ns > 128 && ns <= Q_THREADS) {  // block-uniform: one survivor per thread, bitonic sort (coarse_select.cuh);
+                                      // up to 128 survivors the rank loop below is cheaper (4 warps x ns compares)
+    uint64_t mykey = tid < ns ? skeys[tid] : ~0ull;
+    __syncthreads();  // skeys[] becomes the exchange buffer (>= 256 keys)
+    mykey = csl::block_sort256(mykey, skeys);
+    if (tid < ns) {
+      const int pos = (int)key_payload(mykey);
+      const int lo = owner[pos];
+      a.outD[qi * a.k + tid] = ord2f((uint32_t)(mykey >> 32));
+      const int64_t e = lstart[lo] + (pos - prefix[lo]);
+      a.outI[qi * a.k + tid] = a.ids ? a.ids[e] : e;
+    }
+    return;
+  }
+  for (int i = tid; i < ns; i += Q_THREADS) {
+    const uint64_t mykey = skeys[i];
+    int rank = 0;
+    for (int j = 0; j < ns; j++) rank += skeys[j] < mykey;
+    const int pos = (int)key_payload(mykey);
+    const int lo = owner[pos];
+    a.outD[qi * a.k + rank] = ord2f((uint32_t)(mykey >> 32));
+    const int64_t e = lstart[lo] + (pos - prefix[lo]);
+    a.outI[qi * a.k + rank] = a.ids ? a.ids[e] : e;
   }
 }
 
@@ -1006,7 +1126,7 @@ static size_t scan_smem_bytes(int sel_cap, int M, int ksub, int nL, int W, int o
   off += sizeof(int64_t) * W;
   off += sizeof(int) * ((W + 1 + 3) & ~3);
   off += sizeof(float) * W * 3;
-  off += sizeof(uint16_t) * ((owner_cap + 1) & ~1) + sizeof(int) * 16;  // owner table + scratch of the small-query path
+  off += sizeof(uint16_t) * ((owner_cap + 1) & ~1);  // owner table
   return off;
 }
 
@@ -1290,8 +1410,12 @@ int vlq_coarse_lines(const float* q, int64_t nq, int d, const float* cent, const
   return vlq_select_lines(D, nq, C, cidx, P, edge, edge_d2, E, W, out_list, out_term1, out_term6, stream);
 }
 
-// term-3 tables of the batch (+ 256 spare bytes)
-size_t vlq_scan_topk_workspace_bytes(int64_t nq, int M) { return (size_t)(nq > 0 ? nq : 0) * M * 256 * sizeof(float) + 256; }
+// term-3 tables of the batch, the overflow list of the short-list scan {n, q_0 .. q_nq-1} (+ 256 spare bytes)
+static size_t scan_overflow_bytes(int64_t nq) { return ((size_t)(nq > 0 ? nq : 0) + 1) * sizeof(int); }
+
+size_t vlq_scan_topk_workspace_bytes(int64_t nq, int M) {
+  return (size_t)(nq > 0 ? nq : 0) * M * 256 * sizeof(float) + ((scan_overflow_bytes(nq) + 255) & ~size_t(255)) + 256;
+}
 
 int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
                   const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
@@ -1352,7 +1476,6 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
     a.t3 = t3;
   }
   a.owner_cap = (int)((long long)W * cap < 4096 ? (long long)W * cap : 4096);
-  a.no_small = getenv("VLQ_SCAN_NO_SMALL") != nullptr;  // read per call: tests flip it between calls
   if (use_long) return launch_scan_long(a, nq, as_stream(stream));
   if (use_async) {
     cudaStream_t st_ = as_stream(stream);
@@ -1376,6 +1499,27 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
   if (long_lists) a.sel_cap = select_capacity(k, Q_THREADS, 2, (long long)W * cap);
   size_t smem = scan_smem_bytes(a.sel_cap, M, a.ksub, nL, W, a.owner_cap);
   cudaStream_t st = as_stream(stream);
+  // short lists: scan_short_kernel takes every query of <= kShortCap entries and lists the others for the general
+  // kernel, whose CTA j then scans listed query j (CTAs past the list's length exit at once; a persistent grid walking
+  // the list made ptxas spill 240 bytes in that kernel).  VLQ_SCAN_NO_SMALL (read per call: tests flip it between
+  // calls) sends every query to the general kernel, the reference the short-list kernel is tested against.
+  const bool use_short = !long_lists && have_t3 && workspace_bytes >= t3_bytes + scan_overflow_bytes(nq) &&
+                         getenv("VLQ_SCAN_NO_SMALL") == nullptr;
+  if (use_short) {
+    int* overflow = reinterpret_cast<int*>(static_cast<unsigned char*>(workspace) + t3_bytes);
+    VLQ_CUDA_TRY(cudaMemsetAsync(overflow, 0, sizeof(int), st));
+    const size_t ssmem = ShortSmem(M, nL, W, k).end;
+#define VLQ_SHORT_LAUNCH(MT)                                                                                           \
+  do {                                                                                                                 \
+    VLQ_CUDA_TRY(cudaFuncSetAttribute(scan_short_kernel<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssmem)); \
+    VLQ_LAUNCH((scan_short_kernel<MT>), (unsigned)nq, Q_THREADS, ssmem, st, a, overflow);                             \
+  } while (0)
+    if (M == 16 && al16) VLQ_SHORT_LAUNCH(16);
+    else if (M == 8 && al16) VLQ_SHORT_LAUNCH(8);
+    else VLQ_SHORT_LAUNCH(0);
+#undef VLQ_SHORT_LAUNCH
+    a.qlist = overflow;
+  }
 #define VLQ_SCAN_LAUNCH(MT, LG)                                                                                        \
   do {                                                                                                                 \
     VLQ_CUDA_TRY(cudaFuncSetAttribute(scan_topk_kernel<MT, LG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
