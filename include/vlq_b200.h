@@ -167,6 +167,23 @@ int vlq_remove_ids_apply(int64_t nlists, int M, int64_t n, const int64_t* offset
                          const uint8_t* lamq, const float* kappa, const int64_t* ids, const int64_t* out_offsets,
                          uint8_t* out_codes, uint8_t* out_lamq, float* out_kappa, int64_t* out_ids,
                          const void* workspace, size_t workspace_bytes, vlq_stream_t stream);
+/* a9 with an auxiliary per-entry byte column (GpuIndexIVFPQR's refinement codes): vlq_build_lists / vlq_remove_ids_apply
+ *     plus aux [n][aux_width] bytes, moved with their entry to the same slab position (canonical byte order: the column
+ *     is NOT rotated like the PQ codes).  The placement is computed once, by the same kernels; the entry points above are
+ *     these with aux_width = 0.  0 <= aux_width <= 64; with aux_width > 0 the aux arrays of the non-empty sides must be
+ *     non-NULL. */
+int vlq_build_lists_aux(int64_t nlists, int M, int aux_width, int64_t n_old, const int64_t* old_offsets,
+                        const uint8_t* old_codes, const uint8_t* old_lamq, const float* old_kappa,
+                        const int64_t* old_ids, const uint8_t* old_aux, int64_t n_new, const int* new_list,
+                        const uint8_t* new_codes, const uint8_t* new_lamq, const float* new_kappa,
+                        const int64_t* new_ids, const uint8_t* new_aux, int64_t* out_offsets, uint8_t* out_codes,
+                        uint8_t* out_lamq, float* out_kappa, int64_t* out_ids, uint8_t* out_aux, void* workspace,
+                        size_t workspace_bytes, vlq_stream_t stream);
+int vlq_remove_ids_apply_aux(int64_t nlists, int M, int aux_width, int64_t n, const int64_t* offsets,
+                             const uint8_t* codes, const uint8_t* lamq, const float* kappa, const int64_t* ids,
+                             const uint8_t* aux, const int64_t* out_offsets, uint8_t* out_codes, uint8_t* out_lamq,
+                             float* out_kappa, int64_t* out_ids, uint8_t* out_aux, const void* workspace,
+                             size_t workspace_bytes, vlq_stream_t stream);
 
 /* a9 (read-back): id lookup and decode of stored entries (Index::reconstruct / reconstruct_n / search_and_reconstruct,
  *     IndexIVFPQ::reconstruct_from_offset in the reference).
@@ -204,6 +221,37 @@ int vlq_imi_decode_entries(int64_t n, const int64_t* pos, const int64_t* offsets
  *       n = 0 is a no-op; out_kappa must not alias kappa.
  *     vlq_filter_results: D[i] = FLT_MAX, I[i] = -1 wherever D[i] is +inf in the rows x k results of a scan: a query
  *       with fewer than k members among its candidates gets the usual padding.  Rows stay sorted. */
+/* a9-refine: the refinement stage of GpuIndexIVFPQR (faiss IndexIVFPQR, IndexIVFPQR.cpp): a second 8-bit PQ code
+ *     (pq2: (M2, 256, d / M2) fp32) of the residual the first level leaves.  Definitions:
+ *       x1 = the first-level decode of vlq_decode_entries (the same device function, decode.cuh)
+ *       r2 = x - x1, one fp32 subtraction per component
+ *       code2[m] = argmin_j ||r2_m - pq2[m][j]||^2, lowest j on ties
+ *       x2 = x1 + pq2[m][code2_m][j - m dsub2], one fp32 add per component
+ *     M2 <= 64, d % M2 == 0 (VLQ_EINVAL); d <= 512 (VLQ_EUNSUPPORTED: one row lives in shared memory).  Every argument
+ *     is checked before the first launch.
+ *     vlq_refine_encode: for n rows x in arrival order with their vlq_line_encode outputs (list, lamq, canonical codes
+ *       [n][M]), code2 [n][M2] and (nullable) r2 [n][d].  pq2 == NULL: only r2 (training the refinement codebook); then
+ *       out_r2 must be non-NULL.  A row with list < 0 (NaN input, dropped at commit) reads nothing and gets zeros.
+ *     vlq_refine_topk: re-rank.  cand [nq][kc] are slab indexes of the lists (-1 = no candidate; repeats allowed),
+ *       1 <= k <= kc <= VLQ_MAX_K.  Per query the k candidates with the smallest ||q - x2||^2 (the FULL squared L2,
+ *       fp32, as fvec_L2sqr in IndexIVFPQR::search), ascending; ties keep candidate order; padding (FLT_MAX, -1) where
+ *       fewer than k candidates hold an entry (a NaN distance counts as none).  outI = ids[slab index]; ids == NULL:
+ *       the slab index itself (search_and_reconstruct decodes it).  code2 is the aux column of vlq_build_lists_aux.
+ *       outI may alias cand when k == kc (re-rank in place); the slab arrays are only read at valid candidates.
+ *     vlq_refine_decode: vlq_decode_entries with x2 instead of x1 (the same kernel, p2 added last). */
+int vlq_refine_encode(const float* x, int64_t n, int d, const int* list, const uint8_t* lamq, const uint8_t* codes,
+                      int M, const float* pq, const float* cent, const int* edge, int E, const float* lambda_cb, int nL,
+                      const float* pq2, int M2, uint8_t* out_code2, float* out_r2, vlq_stream_t stream);
+int vlq_refine_topk(const float* q, int64_t nq, int d, const int64_t* cand, int kc, int k, int64_t nlists,
+                    const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const int64_t* ids,
+                    const uint8_t* code2, int M, const float* pq, const float* cent, const int* edge, int E,
+                    const float* lambda_cb, int nL, const float* pq2, int M2, float* outD, int64_t* outI,
+                    vlq_stream_t stream);
+int vlq_refine_decode(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets, const uint8_t* codes,
+                      const uint8_t* lamq, const int64_t* ids, const uint8_t* code2, int M, int d, const float* pq,
+                      const float* cent, const int* edge, int E, const float* lambda_cb, int nL, const float* pq2, int M2,
+                      float* out_x, int64_t* out_ids, vlq_stream_t stream);
+
 int vlq_filter_kappa(int64_t n, const int64_t* ids, const float* kappa, int64_t range_lo, int64_t range_hi,
                      const int64_t* batch, int64_t n_batch, const uint8_t* bitmap, int64_t bitmap_bytes, int invert,
                      float* out_kappa, vlq_stream_t stream);

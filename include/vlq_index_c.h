@@ -101,6 +101,20 @@ int vlq_host_vlq_read_codebook(void* index, const char* name);
 int vlq_host_vlq_write_db(void* index, const char* name);
 int vlq_host_vlq_read_db(void* index, const char* name, int pronum, int rank);
 
+/* GpuIndexIVFPQR (faiss IndexIVFPQR): the VLQ index plus an 8-bit PQ code of M_refine sub-quantizers of each entry's
+   residual, which search re-ranks the scan's min(1024, max(k, floor(k * k_factor))) candidates with.  Train / add /
+   search / reconstruct / remove_ids / reset through the vlq_host_index_* calls and the vlq_host_vlq_* calls above;
+   search distances are FULL squared L2 (||q - x2||^2, as IndexIVFPQR), unlike GpuIndexIVFPQ's.  range_search,
+   copy_from / copy_to and the .db* files fail (-1).  Refinement codebook: (M_refine, 256, d / M_refine) floats; list
+   refine codes: [list length][M_refine] bytes. */
+int vlq_host_ivfpqr_new(void* res, int d, int nlist, int M, int M_refine, int bits, int nedge, int nlambda,
+                        int use_tensor_cores, void** out);
+int vlq_host_ivfpqr_set_k_factor(void* index, float k_factor); /* k_factor >= 1 (default 4) */
+int vlq_host_ivfpqr_get_k_factor(void* index, float* out);
+int vlq_host_ivfpqr_set_refine_codebook(void* index, const float* pq2);
+int vlq_host_ivfpqr_get_refine_codebook(void* index, float* pq2);
+int vlq_host_ivfpqr_get_list_refine_codes(void* index, int list, unsigned char* codes);
+
 /* the permutation Clustering::train subsamples and initialises with (rand_perm, utils.cpp:307-317, on the glibc random_r
  * generator of utils.cpp:135-160): host-only, exposed so that CPU tests can pin it against the reference library */
 int vlq_host_rand_perm(int* perm, long n, long seed);

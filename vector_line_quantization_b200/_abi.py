@@ -42,9 +42,16 @@ SIGNATURES = {
     "vlq_remove_ids_workspace_bytes": (_z, [_l, _l]),
     "vlq_remove_ids_plan": (_i, [_l, _l, _p, _p, _l, _l, _p, _l, _p, _p, _z, _p]),
     "vlq_remove_ids_apply": (_i, [_l, _i, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _z, _p]),
+    "vlq_build_lists_aux": (_i, [_l, _i, _i, _l, _p, _p, _p, _p, _p, _p, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p,
+                                 _p, _p, _z, _p]),
+    "vlq_remove_ids_apply_aux": (_i, [_l, _i, _i, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _z, _p]),
     "vlq_lookup_ids": (_i, [_l, _p, _l, _p, _l, _p, _p, _p]),
     "vlq_decode_entries": (_i, [_l, _p, _l, _p, _p, _p, _p, _i, _i, _p, _p, _p, _i, _p, _i, _p, _p, _p]),
     "vlq_imi_decode_entries": (_i, [_l, _p, _p, _p, _p, _i, _i, _p, _p, _p, _i, _p, _p, _p]),
+    "vlq_refine_encode": (_i, [_p, _l, _i, _p, _p, _p, _i, _p, _p, _p, _i, _p, _i, _p, _i, _p, _p, _p]),
+    "vlq_refine_topk": (_i, [_p, _l, _i, _p, _i, _i, _l, _p, _p, _p, _p, _p, _i, _p, _p, _p, _i, _p, _i, _p, _i, _p, _p,
+                             _p]),
+    "vlq_refine_decode": (_i, [_l, _p, _l, _p, _p, _p, _p, _p, _i, _i, _p, _p, _p, _i, _p, _i, _p, _i, _p, _p, _p]),
     "vlq_filter_kappa": (_i, [_l, _p, _p, _l, _l, _p, _l, _p, _l, _i, _p, _p]),
     "vlq_filter_results": (_i, [_l, _i, _p, _p, _p]),
     "vlq_recompute_kappa": (_i, [_l, _l, _p, _p, _p, _p, _i, _p, _i, _p, _p, _i, _p, _p]),

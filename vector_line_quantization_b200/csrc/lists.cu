@@ -12,6 +12,7 @@
 //   5. old entries are copied to their new place; new entries are gathered behind them.
 #include <cfloat>
 
+#include "decode.cuh"
 #include "scan.cuh"
 
 namespace vlq {
@@ -217,22 +218,27 @@ __device__ __forceinline__ void copy_code(uint8_t* dst, const uint8_t* src, int 
   }
 }
 
+// aux: an optional per-entry byte column of aux_w bytes (a refinement code), moved with its entry without rotation;
+// aux_w = 0: no column (aux unused)
 struct ListArrays {
   uint8_t* codes;
   uint8_t* lamq;
   float* kappa;
   int64_t* ids;
+  uint8_t* aux;
 };
 struct ConstListArrays {
   const uint8_t* codes;
   const uint8_t* lamq;
   const float* kappa;
   const int64_t* ids;
+  const uint8_t* aux;
 };
 
 __global__ void gather_new_kernel(const uint32_t* __restrict__ perm, int64_t nlists, const int* __restrict__ new_list,
                                   const int64_t* __restrict__ new_base, const int64_t* __restrict__ old_offsets,
-                                  const int64_t* __restrict__ out_offsets, ConstListArrays src, ListArrays dst, int M) {
+                                  const int64_t* __restrict__ out_offsets, ConstListArrays src, ListArrays dst, int M,
+                                  int aux_w) {
   int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   int64_t stride = (int64_t)gridDim.x * blockDim.x;
   const int64_t live = new_base[nlists];  // entries with list id < 0 (invalid vectors) were never scattered
@@ -246,11 +252,13 @@ __global__ void gather_new_kernel(const uint32_t* __restrict__ perm, int64_t nli
     dst.lamq[o] = src.lamq[s];
     dst.kappa[o] = src.kappa[s];
     dst.ids[o] = src.ids[s];
+    if (aux_w) copy_code(dst.aux + o * aux_w, src.aux + (int64_t)s * aux_w, aux_w);
   }
 }
 
 __global__ void copy_old_kernel(int64_t n_old, int64_t nlists, const int64_t* __restrict__ old_offsets,
-                                const int64_t* __restrict__ out_offsets, ConstListArrays src, ListArrays dst, int M) {
+                                const int64_t* __restrict__ out_offsets, ConstListArrays src, ListArrays dst, int M,
+                                int aux_w) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (; i < n_old; i += stride) {
@@ -265,6 +273,7 @@ __global__ void copy_old_kernel(int64_t n_old, int64_t nlists, const int64_t* __
     dst.lamq[o] = src.lamq[i];
     dst.kappa[o] = src.kappa[i];
     dst.ids[o] = src.ids[i];
+    if (aux_w) copy_code(dst.aux + o * aux_w, src.aux + i * aux_w, aux_w);
   }
 }
 
@@ -413,15 +422,6 @@ __device__ __forceinline__ bool removed_id(int64_t id, int64_t lo, int64_t hi, c
   return batch_slot(id, batch, nb) >= 0;
 }
 
-// largest l in [lo, hi] with offsets[l] <= p (offsets[lo] <= p)
-__device__ __forceinline__ int64_t list_of(const int64_t* offsets, int64_t lo, int64_t hi, int64_t p) {
-  while (lo < hi) {
-    const int64_t mid = (lo + hi + 1) >> 1;
-    if (offsets[mid] <= p) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
-
 // pass 1: keep mask, survivors per tile (tile_sums), and for every list that starts inside the tile its survivor prefix
 // relative to the tile (rem_offsets_kernel adds the tile's base once the tile totals are scanned)
 __global__ void __launch_bounds__(SCAN_THREADS)
@@ -478,11 +478,13 @@ __global__ void rem_offsets_kernel(int64_t n, int64_t nlists, const int64_t* __r
 }
 
 // pass 2: the in-tile prefix is rebuilt from the mask; every survivor is copied to its prefix and its code word re-rotated
-// from its old list position p to its new one p' (store_code_rotated by (p' - p) mod M)
+// from its old list position p to its new one p' (store_code_rotated by (p' - p) mod M).  AUX: the aux column moves
+// too (a template parameter: the kernel without it keeps its registers)
+template <bool AUX>
 __global__ void __launch_bounds__(SCAN_THREADS)
 rem_apply_kernel(int64_t n, int64_t nlists, int M, const int64_t* __restrict__ offsets,
                  const int64_t* __restrict__ out_offsets, const uint32_t* __restrict__ mask,
-                 const int64_t* __restrict__ tile_sums, ConstListArrays src, ListArrays dst) {
+                 const int64_t* __restrict__ tile_sums, ConstListArrays src, ListArrays dst, int aux_w) {
   __shared__ uint32_t sword[REM_WORDS];
   __shared__ int64_t spre[REM_WORDS];
   __shared__ int64_t soff[REM_LISTS], sout[REM_LISTS];
@@ -529,6 +531,7 @@ rem_apply_kernel(int64_t n, int64_t nlists, int M, const int64_t* __restrict__ o
     dst.lamq[o] = src.lamq[e];
     dst.kappa[o] = src.kappa[e];
     dst.ids[o] = src.ids[e];
+    if constexpr (AUX) for (int t = 0; t < aux_w; t++) dst.aux[o * aux_w + t] = src.aux[e * aux_w + t];
   }
 }
 
@@ -609,6 +612,7 @@ lookup_finish_kernel(int64_t* __restrict__ out_pos, int64_t nslots, unsigned lon
 //   VLQ:    anchor = (1 - lh) c + lh s,  c = cent[l / E], s = cent[edge[l]], lh = lambda_cb[lamq[p]]
 //   IMI-PQ: anchor = [cb1[i1] | cb2[i2]],  l = i1 | i2 << nbits
 // fp32, every operation rounded as written (no contraction), in the order shown: lh = 0 gives exactly c + p.
+// With a refinement codebook (pq2 != NULL, VLQ only) the entry's refinement code adds p2: x2 = x1 + pq2[m][code2_m][..].
 struct DecodeAnchor {
   const float* cent;       // VLQ: [C][d]
   const int* edge;         // VLQ: [nlists]
@@ -618,6 +622,9 @@ struct DecodeAnchor {
   const float* cb1;        // IMI: [K][d / 2]
   const float* cb2;
   int nbits;
+  const uint8_t* code2;    // refinement: [n entries][M2], canonical order
+  const float* pq2;        // refinement: (M2, 256, d / M2); NULL = first level only
+  int M2;
 };
 
 template <bool IMI>
@@ -641,27 +648,24 @@ decode_entries_kernel(int64_t n, const int64_t* pos, int64_t nlists, const int64
     const int64_t l = list_of(offsets, 0, nlists - 1, p);
     const int rot = (int)((p - offsets[l]) % M);
     const uint8_t* cw = codes + p * M;
-    const float *a0, *a1;
-    float lh = 0.f, oml = 1.f;
     if constexpr (IMI) {
       const int h = d / 2;
-      a0 = an.cb1 + (l & ((1 << an.nbits) - 1)) * h;
-      a1 = an.cb2 + (l >> an.nbits) * h;
+      const float* a0 = an.cb1 + (l & ((1 << an.nbits) - 1)) * h;
+      const float* a1 = an.cb2 + (l >> an.nbits) * h;
+      for (int j = lane; j < d; j += kWarp)
+        o[j] = __fadd_rn(*(j < h ? a0 + j : a1 + (j - h)), pq_component(pq, cw, M, dsub, rot, j));
     } else {
-      a0 = an.cent + (l / an.E) * d;
-      a1 = an.cent + (int64_t)an.edge[l] * d;
-      lh = an.lambda_cb[an.lamq[p]];
-      oml = __fsub_rn(1.f, lh);
-    }
-    for (int j = lane; j < d; j += kWarp) {
-      const int m = j / dsub;
-      int sb = m - rot;  // stored[(m - pos) mod M] = code[m]
-      if (sb < 0) sb += M;
-      const float pv = pq[((int64_t)m * 256 + cw[sb]) * dsub + (j - m * dsub)];
-      float a;
-      if constexpr (IMI) a = *(j < d / 2 ? a0 + j : a1 + (j - d / 2));
-      else a = __fadd_rn(__fmul_rn(oml, a0[j]), __fmul_rn(lh, a1[j]));
-      o[j] = __fadd_rn(a, pv);
+      const float* a0 = an.cent + (l / an.E) * d;
+      const float* a1 = an.cent + (int64_t)an.edge[l] * d;
+      const float lh = an.lambda_cb[an.lamq[p]];
+      const float oml = __fsub_rn(1.f, lh);
+      const uint8_t* c2 = an.pq2 ? an.code2 + p * an.M2 : nullptr;
+      const int dsub2 = an.pq2 ? d / an.M2 : 1;
+      for (int j = lane; j < d; j += kWarp) {
+        float v = vlq_decode_component(a0, a1, lh, oml, pq, cw, M, dsub, rot, j);
+        if (c2) v = __fadd_rn(v, pq_component(an.pq2, c2, an.M2, dsub2, 0, j));
+        o[j] = v;
+      }
     }
     if (out_ids && lane == 0) out_ids[r] = ids[p];
   }
@@ -778,7 +782,22 @@ extern "C" int vlq_build_lists(int64_t nlists, int M, int64_t n_old, const int64
                                const uint8_t* new_lamq, const float* new_kappa, const int64_t* new_ids,
                                int64_t* out_offsets, uint8_t* out_codes, uint8_t* out_lamq, float* out_kappa,
                                int64_t* out_ids, void* workspace, size_t workspace_bytes, vlq_stream_t stream) {
+  return vlq_build_lists_aux(nlists, M, 0, n_old, old_offsets, old_codes, old_lamq, old_kappa, old_ids, nullptr, n_new,
+                             new_list, new_codes, new_lamq, new_kappa, new_ids, nullptr, out_offsets, out_codes,
+                             out_lamq, out_kappa, out_ids, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int vlq_build_lists_aux(int64_t nlists, int M, int aux_width, int64_t n_old, const int64_t* old_offsets,
+                                   const uint8_t* old_codes, const uint8_t* old_lamq, const float* old_kappa,
+                                   const int64_t* old_ids, const uint8_t* old_aux, int64_t n_new, const int* new_list,
+                                   const uint8_t* new_codes, const uint8_t* new_lamq, const float* new_kappa,
+                                   const int64_t* new_ids, const uint8_t* new_aux, int64_t* out_offsets,
+                                   uint8_t* out_codes, uint8_t* out_lamq, float* out_kappa, int64_t* out_ids,
+                                   uint8_t* out_aux, void* workspace, size_t workspace_bytes, vlq_stream_t stream) {
   if (nlists <= 0 || M <= 0 || n_old < 0 || n_new < 0 || !out_offsets || !workspace) return VLQ_EINVAL;
+  if (aux_width < 0 || aux_width > 64) return VLQ_EINVAL;
+  if (aux_width > 0 && ((n_old > 0 && !old_aux) || (n_new > 0 && !new_aux) || (n_old + n_new > 0 && !out_aux)))
+    return VLQ_EINVAL;
   if (n_new >= (int64_t)0xffffffffll) return VLQ_EINVAL;
   if (n_old > 0 && (!old_offsets || !old_codes || !old_lamq || !old_kappa || !old_ids)) return VLQ_EINVAL;
   if (n_new > 0 && (!new_list || !new_codes || !new_lamq || !new_kappa || !new_ids)) return VLQ_EINVAL;
@@ -797,17 +816,18 @@ extern "C" int vlq_build_lists(int64_t nlists, int M, int64_t n_old, const int64
   VLQ_LAUNCH(scan_tile_offsets_kernel, 1, SCAN_THREADS, 0, st, w.tile_sums, ntiles);
   VLQ_LAUNCH(scan_finish_kernel, (unsigned)ntiles, SCAN_THREADS, 0, st, w.counts, nlists, w.tile_sums, oo, w.new_base,
              out_offsets);
-  ConstListArrays osrc{old_codes, old_lamq, old_kappa, old_ids};
-  ConstListArrays nsrc{new_codes, new_lamq, new_kappa, new_ids};
-  ListArrays dst{out_codes, out_lamq, out_kappa, out_ids};
+  ConstListArrays osrc{old_codes, old_lamq, old_kappa, old_ids, old_aux};
+  ConstListArrays nsrc{new_codes, new_lamq, new_kappa, new_ids, new_aux};
+  ListArrays dst{out_codes, out_lamq, out_kappa, out_ids, out_aux};
   if (n_new > 0) {
     VLQ_LAUNCH(scatter_ordinals_kernel, wide, 256, 0, st, new_list, n_new, w.new_base, w.cursor, w.perm);
     unsigned sgrid = (unsigned)(nlists < 148 * 64 ? nlists : 148 * 64);
     VLQ_LAUNCH(seg_sort_kernel, sgrid, SEG_THREADS, 0, st, w.new_base, nlists, w.perm);
   }
-  if (n_old > 0) VLQ_LAUNCH(copy_old_kernel, wide, 256, 0, st, n_old, nlists, oo, out_offsets, osrc, dst, M);
+  if (n_old > 0) VLQ_LAUNCH(copy_old_kernel, wide, 256, 0, st, n_old, nlists, oo, out_offsets, osrc, dst, M, aux_width);
   if (n_new > 0) {
-    VLQ_LAUNCH(gather_new_kernel, wide, 256, 0, st, w.perm, nlists, new_list, w.new_base, oo, out_offsets, nsrc, dst, M);
+    VLQ_LAUNCH(gather_new_kernel, wide, 256, 0, st, w.perm, nlists, new_list, w.new_base, oo, out_offsets, nsrc, dst, M,
+               aux_width);
   }
   return last_error();
 }
@@ -841,14 +861,30 @@ extern "C" int vlq_remove_ids_apply(int64_t nlists, int M, int64_t n, const int6
                                     const uint8_t* lamq, const float* kappa, const int64_t* ids, const int64_t* out_offsets,
                                     uint8_t* out_codes, uint8_t* out_lamq, float* out_kappa, int64_t* out_ids,
                                     const void* workspace, size_t workspace_bytes, vlq_stream_t stream) {
+  return vlq_remove_ids_apply_aux(nlists, M, 0, n, offsets, codes, lamq, kappa, ids, nullptr, out_offsets, out_codes,
+                                  out_lamq, out_kappa, out_ids, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int vlq_remove_ids_apply_aux(int64_t nlists, int M, int aux_width, int64_t n, const int64_t* offsets,
+                                        const uint8_t* codes, const uint8_t* lamq, const float* kappa, const int64_t* ids,
+                                        const uint8_t* aux, const int64_t* out_offsets, uint8_t* out_codes,
+                                        uint8_t* out_lamq, float* out_kappa, int64_t* out_ids, uint8_t* out_aux,
+                                        const void* workspace, size_t workspace_bytes, vlq_stream_t stream) {
   if (nlists < 1 || M < 1 || M > 64 || n < 0 || !offsets || !out_offsets || !workspace) return VLQ_EINVAL;
+  if (aux_width < 0 || aux_width > 64) return VLQ_EINVAL;
   if (n > 0 && (!codes || !lamq || !kappa || !ids || !out_codes || !out_lamq || !out_kappa || !out_ids)) return VLQ_EINVAL;
+  if (n > 0 && aux_width > 0 && (!aux || !out_aux)) return VLQ_EINVAL;
   RemWs w = carve_rem(const_cast<void*>(workspace), n);
   if (workspace_bytes < w.bytes) return VLQ_EWORKSPACE;
   if (n == 0) return VLQ_OK;
-  VLQ_LAUNCH(rem_apply_kernel, (unsigned)w.ntiles, SCAN_THREADS, 0, as_stream(stream), n, nlists, M, offsets,
-             out_offsets, w.mask, w.tile_sums, ConstListArrays{codes, lamq, kappa, ids},
-             ListArrays{out_codes, out_lamq, out_kappa, out_ids});
+  const ConstListArrays src{codes, lamq, kappa, ids, aux};
+  const ListArrays dst{out_codes, out_lamq, out_kappa, out_ids, out_aux};
+  if (aux_width > 0)
+    VLQ_LAUNCH(rem_apply_kernel<true>, (unsigned)w.ntiles, SCAN_THREADS, 0, as_stream(stream), n, nlists, M, offsets,
+               out_offsets, w.mask, w.tile_sums, src, dst, aux_width);
+  else
+    VLQ_LAUNCH(rem_apply_kernel<false>, (unsigned)w.ntiles, SCAN_THREADS, 0, as_stream(stream), n, nlists, M, offsets,
+               out_offsets, w.mask, w.tile_sums, src, dst, 0);
   return last_error();
 }
 
@@ -895,6 +931,19 @@ extern "C" int vlq_decode_entries(int64_t n, const int64_t* pos, int64_t nlists,
   if (n > 0 && (!lamq || !cent || !edge || !lambda_cb)) return VLQ_EINVAL;
   DecodeAnchor an{};
   an.cent = cent; an.edge = edge; an.lamq = lamq; an.lambda_cb = lambda_cb; an.E = E;
+  return decode_launch(false, n, pos, nlists, offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
+}
+
+extern "C" int vlq_refine_decode(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
+                                 const uint8_t* codes, const uint8_t* lamq, const int64_t* ids, const uint8_t* code2,
+                                 int M, int d, const float* pq, const float* cent, const int* edge, int E,
+                                 const float* lambda_cb, int nL, const float* pq2, int M2, float* out_x, int64_t* out_ids,
+                                 vlq_stream_t stream) {
+  if (E < 1 || nlists % E != 0 || nL < 1 || nL > 256 || M2 < 1 || M2 > 64 || d < 1 || d % M2 != 0) return VLQ_EINVAL;
+  if (n > 0 && (!lamq || !cent || !edge || !lambda_cb || !code2 || !pq2)) return VLQ_EINVAL;
+  DecodeAnchor an{};
+  an.cent = cent; an.edge = edge; an.lamq = lamq; an.lambda_cb = lambda_cb; an.E = E;
+  an.code2 = code2; an.pq2 = pq2; an.M2 = M2;
   return decode_launch(false, n, pos, nlists, offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
 }
 

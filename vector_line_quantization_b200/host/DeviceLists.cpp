@@ -8,7 +8,10 @@
 namespace faiss {
 namespace gpu {
 
-DeviceLists::DeviceLists(GpuResources* res, int64_t nlists, int M) : res_(res), nlists_(nlists), M_(M) {}
+DeviceLists::DeviceLists(GpuResources* res, int64_t nlists, int M, int auxWidth)
+    : res_(res), nlists_(nlists), M_(M), auxWidth_(auxWidth) {
+  VLQ_THROW_IF_NOT_MSG(auxWidth >= 0 && auxWidth <= 64, "aux column width must be in [0, 64]");
+}
 
 DeviceLists::Slots DeviceLists::makeRoom(size_t n) {
   const size_t need = nPending_ + n;
@@ -16,13 +19,14 @@ DeviceLists::Slots DeviceLists::makeRoom(size_t n) {
     vlq_stream_t st = res_->getDefaultStream();
     const size_t cap = std::max({need, 2 * capPending_, reserveVecs_, (size_t)1 << 16});
     DeviceBuffer nl(cap * sizeof(int));
-    Columns nc(cap, M_);
+    Columns nc(cap, M_, auxWidth_);
     if (nPending_) {
       VLQ_CALL(vlq_memcpy_d2d(nl.get(), pList_.get(), nPending_ * sizeof(int), st));
       VLQ_CALL(vlq_memcpy_d2d(nc.codes.get(), pending_.codes.get(), nPending_ * M_, st));
       VLQ_CALL(vlq_memcpy_d2d(nc.lamq.get(), pending_.lamq.get(), nPending_, st));
       VLQ_CALL(vlq_memcpy_d2d(nc.kappa.get(), pending_.kappa.get(), nPending_ * sizeof(float), st));
       VLQ_CALL(vlq_memcpy_d2d(nc.ids.get(), pending_.ids.get(), nPending_ * sizeof(int64_t), st));
+      if (auxWidth_) VLQ_CALL(vlq_memcpy_d2d(nc.aux.get(), pending_.aux.get(), nPending_ * auxWidth_, st));
       res_->syncDefaultStream();
     }
     pList_ = std::move(nl);
@@ -31,7 +35,8 @@ DeviceLists::Slots DeviceLists::makeRoom(size_t n) {
   }
   const size_t o = nPending_;
   return Slots{pList_.as<int>() + o, pending_.codes.as<uint8_t>() + o * M_, pending_.lamq.as<uint8_t>() + o,
-               pending_.kappa.as<float>() + o, pending_.ids.as<int64_t>() + o};
+               pending_.kappa.as<float>() + o, pending_.ids.as<int64_t>() + o,
+               auxWidth_ ? pending_.aux.as<uint8_t>() + o * auxWidth_ : nullptr};
 }
 
 void DeviceLists::appended(size_t n) {
@@ -44,14 +49,15 @@ void DeviceLists::commit(DeviceBuffer& workspace) {
   vlq_stream_t st = res_->getDefaultStream();
   const size_t tot = n_ + nPending_;
   DeviceBuffer no((size_t)(nlists_ + 1) * sizeof(int64_t));
-  Columns nc(tot, M_);
+  Columns nc(tot, M_, auxWidth_);
   workspace.reserve(vlq_build_lists_workspace_bytes((int64_t)nPending_, nlists_));
-  VLQ_CALL(vlq_build_lists(nlists_, M_, (int64_t)n_, offsets_.as<int64_t>(), slab_.codes.as<uint8_t>(),
-                           slab_.lamq.as<uint8_t>(), slab_.kappa.as<float>(), slab_.ids.as<int64_t>(),
-                           (int64_t)nPending_, pList_.as<int>(), pending_.codes.as<uint8_t>(),
-                           pending_.lamq.as<uint8_t>(), pending_.kappa.as<float>(), pending_.ids.as<int64_t>(),
-                           no.as<int64_t>(), nc.codes.as<uint8_t>(), nc.lamq.as<uint8_t>(), nc.kappa.as<float>(),
-                           nc.ids.as<int64_t>(), workspace.get(), workspace.bytes(), st));
+  VLQ_CALL(vlq_build_lists_aux(nlists_, M_, auxWidth_, (int64_t)n_, offsets_.as<int64_t>(), slab_.codes.as<uint8_t>(),
+                               slab_.lamq.as<uint8_t>(), slab_.kappa.as<float>(), slab_.ids.as<int64_t>(),
+                               slab_.aux.as<uint8_t>(), (int64_t)nPending_, pList_.as<int>(),
+                               pending_.codes.as<uint8_t>(), pending_.lamq.as<uint8_t>(), pending_.kappa.as<float>(),
+                               pending_.ids.as<int64_t>(), pending_.aux.as<uint8_t>(), no.as<int64_t>(),
+                               nc.codes.as<uint8_t>(), nc.lamq.as<uint8_t>(), nc.kappa.as<float>(), nc.ids.as<int64_t>(),
+                               nc.aux.as<uint8_t>(), workspace.get(), workspace.bytes(), st));
   // entries the encoder skipped (list id < 0) are not stored: the live count is offsets[nlists]
   int64_t live = 0;
   VLQ_CALL(vlq_memcpy_d2h(&live, no.as<int64_t>() + nlists_, sizeof(int64_t), st));
@@ -89,11 +95,12 @@ long DeviceLists::remove(const IDSelector& sel) {
   VLQ_CALL(vlq_memcpy_d2h(&live, no.as<int64_t>() + nlists_, sizeof(int64_t), st));
   res_->syncDefaultStream();
   if (live == n) return 0;  // nothing selected: the slab stays as it is
-  Columns nc(std::max<size_t>(1, (size_t)live), M_);
-  VLQ_CALL(vlq_remove_ids_apply(nlists_, M_, n, offsets_.as<int64_t>(), slab_.codes.as<uint8_t>(),
-                                slab_.lamq.as<uint8_t>(), slab_.kappa.as<float>(), slab_.ids.as<int64_t>(),
-                                no.as<int64_t>(), nc.codes.as<uint8_t>(), nc.lamq.as<uint8_t>(), nc.kappa.as<float>(),
-                                nc.ids.as<int64_t>(), ws.get(), ws.bytes(), st));
+  Columns nc(std::max<size_t>(1, (size_t)live), M_, auxWidth_);
+  VLQ_CALL(vlq_remove_ids_apply_aux(nlists_, M_, auxWidth_, n, offsets_.as<int64_t>(), slab_.codes.as<uint8_t>(),
+                                    slab_.lamq.as<uint8_t>(), slab_.kappa.as<float>(), slab_.ids.as<int64_t>(),
+                                    slab_.aux.as<uint8_t>(), no.as<int64_t>(), nc.codes.as<uint8_t>(),
+                                    nc.lamq.as<uint8_t>(), nc.kappa.as<float>(), nc.ids.as<int64_t>(),
+                                    nc.aux.as<uint8_t>(), ws.get(), ws.bytes(), st));
   res_->syncDefaultStream();
   offsets_ = std::move(no);
   slab_ = std::move(nc);
@@ -138,11 +145,12 @@ int64_t DeviceLists::listLength(int64_t l) const {
 float* DeviceLists::install(const std::vector<int64_t>& offsets, const std::vector<uint8_t>& codes,
                             const std::vector<uint8_t>& lamq, const std::vector<long>& ids) {
   VLQ_THROW_IF_NOT(offsets.size() == (size_t)nlists_ + 1);
+  VLQ_THROW_IF_NOT_MSG(auxWidth_ == 0, "lists with an aux column cannot be installed from codes alone");
   const size_t tot = (size_t)offsets.back();
   reset();
   vlq_stream_t st = res_->getDefaultStream();
   offsets_.resize(offsets.size() * sizeof(int64_t));
-  slab_ = Columns(std::max<size_t>(1, tot), M_);
+  slab_ = Columns(std::max<size_t>(1, tot), M_, 0);
   VLQ_CALL(vlq_memcpy_h2d(offsets_.get(), offsets.data(), offsets.size() * sizeof(int64_t), st));
   if (tot) {
     VLQ_CALL(vlq_memcpy_h2d(slab_.codes.get(), codes.data(), codes.size(), st));

@@ -5,7 +5,12 @@
 // list-major, in insertion order inside a list.  The M code bytes of the entry at list position pos are stored rotated
 // by pos mod M (stored[j] = code[(j + pos) mod M], csrc/scan.cuh).
 //
-// Pending arena: encoded entries in arrival order (list id | codes | lamq | kappa | id), written by the index's encoder.
+// Optional aux column: auxWidth bytes per entry (GpuIndexIVFPQR's refinement code), in canonical byte order (not
+// rotated), beside the other columns in the slab and the arena; it moves with its entry through commit and remove.
+// auxWidth = 0 (GpuIndexIVFPQ, GpuIndexIMIPQ): nothing is allocated and the launches are those without the column.
+//
+// Pending arena: encoded entries in arrival order (list id | codes | lamq | kappa | id | aux), written by the index's
+// encoder.
 // commit() merges them into the slab with vlq_build_lists (stable counting sort) at the first read after adds; entries
 // the encoder skipped (list id < 0: NaN input) are dropped there.
 //
@@ -23,15 +28,17 @@ namespace gpu {
 
 class DeviceLists {
  public:
-  DeviceLists(GpuResources* res, int64_t nlists, int M);
+  DeviceLists(GpuResources* res, int64_t nlists, int M, int auxWidth = 0);
 
-  /// device pointers to the next free arena slots (list id, M code bytes, lambda byte, kappa, id per entry)
+  /// device pointers to the next free arena slots (list id, M code bytes, lambda byte, kappa, id, auxWidth aux bytes per
+  /// entry; aux is null when auxWidth = 0)
   struct Slots {
     int* list;
     uint8_t* codes;
     uint8_t* lamq;
     float* kappa;
     int64_t* ids;
+    uint8_t* aux;
   };
   /// room for n more pending entries: the arena grows to max(need, 2 x capacity, the reserve() hint, 65 536) entries,
   /// keeping its contents
@@ -60,6 +67,7 @@ class DeviceLists {
   /// replaces the lists by a finished slab from host memory: offsets [nlists + 1], stored-order codes, lambda bytes and
   /// ids of offsets[nlists] entries.  Returns the kappa column for the caller to compute (it depends on the index's
   /// tables).  The uploads are enqueued: the host arrays must outlive the caller's next sync of the default stream.
+  /// Lists with an aux column cannot be installed (the formats behind install carry no aux bytes): throws.
   float* install(const std::vector<int64_t>& offsets, const std::vector<uint8_t>& codes,
                  const std::vector<uint8_t>& lamq, const std::vector<long>& ids);
   /// syncs the default stream, then frees the slab, the arena and the masked kappa
@@ -67,22 +75,26 @@ class DeviceLists {
 
   int64_t nlists() const { return nlists_; }
   int M() const { return M_; }
+  int auxWidth() const { return auxWidth_; }
   size_t size() const { return n_; }  ///< entries in the committed slab
   const int64_t* offsets() const { return offsets_.as<int64_t>(); }
   const uint8_t* codes() const { return slab_.codes.as<uint8_t>(); }
   const uint8_t* lamq() const { return slab_.lamq.as<uint8_t>(); }
   const int64_t* ids() const { return slab_.ids.as<int64_t>(); }
+  const uint8_t* aux() const { return slab_.aux.as<uint8_t>(); }
 
  private:
-  struct Columns {  // codes [n][M] | lamq [n] | kappa [n] | ids [n]
-    DeviceBuffer codes, lamq, kappa, ids;
+  struct Columns {  // codes [n][M] | lamq [n] | kappa [n] | ids [n] | aux [n][R]
+    DeviceBuffer codes, lamq, kappa, ids, aux;
     Columns() = default;
-    Columns(size_t n, int M) : codes(n * M), lamq(n), kappa(n * sizeof(float)), ids(n * sizeof(int64_t)) {}
+    Columns(size_t n, int M, int R)
+        : codes(n * M), lamq(n), kappa(n * sizeof(float)), ids(n * sizeof(int64_t)), aux(n * R) {}
   };
 
   GpuResources* res_;
   int64_t nlists_;
   int M_;
+  int auxWidth_;
   DeviceBuffer offsets_;  // committed slab: offsets_ + slab_
   Columns slab_;
   size_t n_ = 0;

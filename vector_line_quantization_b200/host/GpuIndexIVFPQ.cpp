@@ -52,10 +52,14 @@ void GpuIndexIVF::trainQuantizer_(Index::idx_t n, const float* x) {
 // ================================================================================================ GpuIndexIVFPQ (VLQ)
 GpuIndexIVFPQ::GpuIndexIVFPQ(GpuResources* resources, int dims, int nlist, int subQuantizers, int bitsPerCode,
                              int nedge, int nLambda, faiss::MetricType metric, GpuIndexIVFPQConfig config)
+    : GpuIndexIVFPQ(resources, dims, nlist, subQuantizers, bitsPerCode, nedge, nLambda, metric, config, 0) {}
+
+GpuIndexIVFPQ::GpuIndexIVFPQ(GpuResources* resources, int dims, int nlist, int subQuantizers, int bitsPerCode,
+                             int nedge, int nLambda, faiss::MetricType metric, GpuIndexIVFPQConfig config, int auxWidth)
     : GpuIndexIVF(resources, dims, metric, nlist, config), nLambda_(nLambda), numedge_(nedge), begin_(0), end_(nlist),
       w1_(256), edgeInfo_(nullptr), edgeDistInfo_(nullptr), lambdaInfo_(nullptr), constInfo_(nullptr), listCap_(VLQ_LIST_CAP),
       ivfpqConfig_(config), subQuantizers_(subQuantizers), bitsPerCode_(bitsPerCode),
-      lists_(resources, (int64_t)nlist * nedge, subQuantizers), populatedLists_((size_t)nlist * nedge) {
+      lists_(resources, (int64_t)nlist * nedge, subQuantizers, auxWidth), populatedLists_((size_t)nlist * nedge) {
   VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8, "the scan kernels are written for 8-bit PQ codes");
   VLQ_THROW_IF_NOT_MSG(subQuantizers > 0 && subQuantizers <= 64 && dims % subQuantizers == 0,
                        "number of sub-quantizers must divide the dimension (and be <= 64)");
@@ -219,6 +223,7 @@ void GpuIndexIVFPQ::addTiles_(Index::idx_t n, const void* xv, bool isU8, const l
     VLQ_CALL(vlq_line_encode(dx, m, d, dA.as<int>(), quantizer_->deviceVectors(), dEdge_.as<int>(),
                              dEdgeDist_.as<float>(), numedge_, dLambda_.as<float>(), nLambda_, dPq_.as<float>(), M,
                              out.list + s, nullptr, out.lamq + s, out.codes + (size_t)s * M, out.kappa + s, nullptr, st));
+    encodeAux_(dx, m, out, s, st);
     if (xids) {
       if (vlq_pointer_is_device(xids) == 1)
         VLQ_CALL(vlq_memcpy_d2d(out.ids + s, xids + s, (size_t)m * sizeof(int64_t), st));
@@ -311,13 +316,13 @@ void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, R
 // picks the route (fp32 matrix, tcgen05 matrix, matrix-free) and lays out its workspace.
 void GpuIndexIVFPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels) const {
   DeviceScope scope(ivfConfig_.device);
-  searchTiles_(n, x, k, distances, labels, false, nullptr, nullptr);
+  searchTiles_(n, x, k, k, distances, labels, false, nullptr, nullptr);
 }
 
 void GpuIndexIVFPQ::search(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
                            const SearchParameters* params) const {
   DeviceScope scope(ivfConfig_.device);
-  searchTiles_(n, x, k, distances, labels, false, nullptr, searchSelector(params));
+  searchTiles_(n, x, k, k, distances, labels, false, nullptr, searchSelector(params));
 }
 
 // search() whose scan reports slab indexes: each tile's labels are decoded (vlq_decode_entries turns them into ids in
@@ -331,18 +336,21 @@ void GpuIndexIVFPQ::search_and_reconstruct(Index::idx_t n, const float* x, Index
                                            Index::idx_t* labels, float* recons, const SearchParameters* params) const {
   VLQ_THROW_IF_NOT_MSG(n == 0 || recons != nullptr, "search_and_reconstruct: recons is null");
   DeviceScope scope(ivfConfig_.device);
-  const TileEpilogue decode = [&](Index::idx_t row0, Index::idx_t m, float*, int64_t* dI, vlq_stream_t st) {
+  const TileEpilogue decode = [&](Index::idx_t row0, Index::idx_t m, const float*, float*, int64_t* dI, float*, int64_t*,
+                                  vlq_stream_t st) {
     decodeToOutput(d, dI, (int64_t)m * k, recons + (size_t)row0 * k * d, dI,
                    [this](const int64_t* p, int64_t c, float* o, int64_t* oi, vlq_stream_t s) { decode_(p, c, o, oi, s); },
                    recStage_, st);
   };
-  searchTiles_(n, x, k, distances, labels, true, &decode, searchSelector(params));
+  searchTiles_(n, x, k, k, distances, labels, true, &decode, searchSelector(params));
 }
 
-void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
-                                 bool slabIndex, const TileEpilogue* epilogue, const IDSelector* sel) const {
+void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, Index::idx_t kc, float* distances,
+                                 Index::idx_t* labels, bool slabIndex, const TileEpilogue* epilogue,
+                                 const IDSelector* sel) const {
   VLQ_THROW_IF_NOT_MSG(is_trained, "Index not trained");
   VLQ_THROW_IF_NOT_MSG(k >= 1 && k <= VLQ_MAX_K, "k must be in [1, 1024]");
+  VLQ_THROW_IF_NOT(kc >= k && kc <= VLQ_MAX_K && (kc == k || epilogue));
   VLQ_THROW_IF_NOT_MSG(w1_ >= 1 && w1_ <= VLQ_MAX_K, "w1_ must be in [1, 1024]");
   if (sel) checkSearchSelector(sel);
   if (n == 0) return;
@@ -369,6 +377,10 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
   const size_t lineBytes = ((size_t)tileCap * W * sizeof(float) + 255) & ~size_t(255);
   scratchB_.reserve(2 * 3 * lineBytes);
   t3ws_.reserve(vlq_scan_topk_workspace_bytes(tileCap, M));
+  if (kc > k) {  // the scan's kc candidates of a tile; the epilogue of the tile reads them before the next scan (stream order)
+    candD_.reserve((size_t)tileCap * kc * sizeof(float));
+    candI_.reserve((size_t)tileCap * kc * sizeof(int64_t));
+  }
   // Host buffers: the queries of tile i+1 go up on the copy stream and the results of tile i-1 come down on the download
   // stream while tile i is computed (cross-stream order by vlq_stream_wait: the compute stream only ever waits for
   // uploads); device buffers are used in place (the scan writes straight into the caller's arrays).
@@ -430,12 +442,14 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
       const bool inPlace = dOnDevice && lOnDevice;
       float* oD = inPlace ? hD : outD.as<float>() + (size_t)s * k;
       int64_t* oI = inPlace ? reinterpret_cast<int64_t*>(hI) : outI.as<int64_t>() + (size_t)s * k;
+      float* sD = kc == k ? oD : candD_.as<float>();
+      int64_t* sI = kc == k ? oI : candI_.as<int64_t>();
       VLQ_CALL(vlq_scan_topk(q, m, d, dPq_.as<float>(), M, dLambda_.as<float>(), nLambda_, lline, t1, t6,
                              dEdgeDist_.as<float>(), W, lists_.offsets(), lists_.codes(), lists_.lamq(), kappa, ids,
-                             (int)k, listCap_, (int)std::min<size_t>(lists_.size() / populatedLists_, 1 << 20), oD, oI,
+                             (int)kc, listCap_, (int)std::min<size_t>(lists_.size() / populatedLists_, 1 << 20), sD, sI,
                              t3ws_.get(), t3ws_.bytes(), sb));
-      if (sel) VLQ_CALL(vlq_filter_results(m, (int)k, oD, oI, sb));  // (+inf, id) of masked entries -> padding
-      if (epilogue) (*epilogue)(p0 + s, m, oD, oI, sb);
+      if (sel) VLQ_CALL(vlq_filter_results(m, (int)kc, sD, sI, sb));  // (+inf, id) of masked entries -> padding
+      if (epilogue) (*epilogue)(p0 + s, m, q, sD, sI, oD, oI, sb);
       if (overlap) VLQ_CALL(vlq_event_record(evScan_[slot], sb));
       if (!inPlace) {
         VLQ_CALL(vlq_stream_wait(ds, sb));  // results of this tile are complete
@@ -498,6 +512,12 @@ std::vector<unsigned char> GpuIndexIVFPQ::getListLambdas(int listId) const {
   commit_();
   return fetchList<unsigned char>(lists_.offsets(), lists_.lamq(), listId, 1, resources_);
 }
+std::vector<unsigned char> GpuIndexIVFPQ::listAux_(int listId) const {
+  VLQ_THROW_IF_NOT(listId >= 0 && listId < nlist_ * numedge_);
+  DeviceScope scope(ivfConfig_.device);
+  commit_();
+  return fetchList<unsigned char>(lists_.offsets(), lists_.aux(), listId, lists_.auxWidth(), resources_);
+}
 std::vector<long> GpuIndexIVFPQ::getListIndices(int listId) const {
   VLQ_THROW_IF_NOT(listId >= 0 && listId < nlist_ * numedge_);
   DeviceScope scope(ivfConfig_.device);
@@ -556,6 +576,7 @@ void GpuIndexIVFPQ::readCodebookFromFile(const std::string& name) {  // gpu/GpuI
 }
 
 void GpuIndexIVFPQ::writeDbToFile(const std::string& name) {  // .dbIdx .dbcodes .dbcount .dblas, :1813-1844
+  VLQ_THROW_IF_NOT_MSG(lists_.auxWidth() == 0, "writeDbToFile: the .db* files have no place for refinement codes");
   DeviceScope scope(ivfConfig_.device);
   commit_();
   vlq_stream_t st = resources_->getDefaultStream();
@@ -609,6 +630,7 @@ void GpuIndexIVFPQ::readDbFromFile(const std::string& name) { readDbFromFile(nam
 
 // rank keeps the lists [L/P*rank, L/P*(rank+1)) and zeroes the other counts (gpu/GpuIndexIVFPQ.cu:2106-2163)
 void GpuIndexIVFPQ::readDbFromFile(const std::string& name, int pronum, int rank) {
+  VLQ_THROW_IF_NOT_MSG(lists_.auxWidth() == 0, "readDbFromFile: the .db* files have no place for refinement codes");
   VLQ_THROW_IF_NOT_MSG(is_trained, "read the codebook first");
   VLQ_THROW_IF_NOT(pronum >= 1 && rank >= 0 && rank < pronum);
   DeviceScope scope(ivfConfig_.device);
@@ -658,6 +680,7 @@ namespace gpu {
 // ---------------------------------------------------------------------------------------------- f4: CPU index exchange
 void GpuIndexIVFPQ::copyFrom(const faiss::IndexIVFPQ* index) {
   VLQ_THROW_IF_NOT_MSG(index != nullptr, "null index");
+  VLQ_THROW_IF_NOT_MSG(lists_.auxWidth() == 0, "copyFrom: an IndexIVFPQ has no refinement codes");
   VLQ_THROW_IF_NOT_MSG(index->metric_type == faiss::METRIC_L2, "inner product unsupported");
   VLQ_THROW_IF_NOT_MSG(index->d == d && (int)index->nlist == nlist_, "copyFrom: d / nlist differ from this index");
   VLQ_THROW_IF_NOT_MSG((int)index->pq.M == subQuantizers_ && (int)index->pq.nbits == bitsPerCode_,
@@ -705,6 +728,7 @@ void GpuIndexIVFPQ::copyFrom(const faiss::IndexIVFPQ* index) {
 
 void GpuIndexIVFPQ::copyTo(faiss::IndexIVFPQ* index) const {
   VLQ_THROW_IF_NOT_MSG(index != nullptr, "null index");
+  VLQ_THROW_IF_NOT_MSG(lists_.auxWidth() == 0, "copyTo: an IndexIVFPQ has no place for refinement codes");
   for (int j = 0; j < nLambda_; j++)
     VLQ_THROW_IF_NOT_MSG(lambdaInfo_[j] == 0.f,
                          "copyTo: entries of a VLQ index are residuals of line points, not of centroids; only an index "

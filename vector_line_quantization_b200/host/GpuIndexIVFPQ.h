@@ -131,7 +131,9 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   void merge(faiss::Index::idx_t* nns, float* dist, int k, int nq, int nprocess, float* distances,
              faiss::Index::idx_t* labels) const;
 
-  // reference on-disk formats (gpu/GpuIndexIVFPQ.cu:1731-1844, 2106-2242)
+  // reference on-disk formats (gpu/GpuIndexIVFPQ.cu:1731-1844, 2106-2242); the .db* files hold no aux column, so
+  // writeDbToFile / readDbFromFile throw for a GpuIndexIVFPQR
+
   void writeCodebookToFile(const std::string& name);
   void readCodebookFromFile(const std::string& name);
   void writeDbToFile(const std::string& name);
@@ -145,6 +147,7 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   /// (every line of the probed centroids) search() then returns exactly IndexIVFPQ::search(nprobe), distances without
   /// the ||q||^2 term.  copyTo needs an index whose lambda codebook is all zero (it throws otherwise: entries on a line
   /// are not residuals of a centroid) and merges the numedge_ lines of every centroid back into one list.
+  /// Both throw for an index whose lists carry an aux column (GpuIndexIVFPQR): IndexIVFPQ has no place for it.
   void copyFrom(const faiss::IndexIVFPQ* index);
   void copyTo(faiss::IndexIVFPQ* index) const;
   /// Candidate lists (reference search1 / searchImpl1_, gpu/GpuIndexIVFPQ.cu:1593-1670): labels[q][0..k) = ids of the
@@ -162,17 +165,30 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   /// maximum entries scanned per list (reference: 1024, gpu/impl/IVFUtils.cu:87)
   int listCap_;
 
- private:
+ protected:
+  /// the constructor of an index whose lists carry auxWidth bytes per entry beside the codes (GpuIndexIVFPQR)
+  GpuIndexIVFPQ(GpuResources* resources, int dims, int nlist, int subQuantizers, int bitsPerCode, int nedge,
+                int nLambda, faiss::MetricType metric, GpuIndexIVFPQConfig config, int auxWidth);
   void uploadTables_();
   void commit_() const { lists_.commit(scratch_); }  ///< lazy: first search / list access after adds
-  /// the query tile pipeline of search(): slabIndex makes the scan report slab indexes instead of ids; `epilogue`
-  /// (nullable) runs on the scan stream after each tile's scan with (first row, rows, device D [m][k], device I [m][k],
-  /// stream), before the tile's results are copied out.  sel (nullable): the scan reads the masked kappa and each
-  /// tile's +inf results become padding (vlq_filter_results) before the epilogue.
-  using TileEpilogue = std::function<void(Index::idx_t row0, Index::idx_t m, float* dD, int64_t* dI, vlq_stream_t st)>;
-  void searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, float* distances, Index::idx_t* labels,
-                    bool slabIndex, const TileEpilogue* epilogue, const IDSelector* sel) const;
-  void decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const;
+  /// the query tile pipeline of search(): the scan keeps kc >= k candidates per query, slabIndex makes it report slab
+  /// indexes instead of ids.  `epilogue` (nullable; required when kc > k) runs on the scan stream after each tile's scan
+  /// with (first row, rows, device queries [m][d], scan results D / I [m][kc], tile outputs D / I [m][k], stream),
+  /// before the tile's results are copied out; at kc == k the scan results ARE the tile outputs (same pointers).
+  /// sel (nullable): the scan reads the masked kappa and each tile's +inf results become padding (vlq_filter_results)
+  /// before the epilogue.
+  using TileEpilogue = std::function<void(Index::idx_t row0, Index::idx_t m, const float* dq, float* scanD,
+                                          int64_t* scanI, float* outD, int64_t* outI, vlq_stream_t st)>;
+  void searchTiles_(Index::idx_t n, const float* x, Index::idx_t k, Index::idx_t kc, float* distances,
+                    Index::idx_t* labels, bool slabIndex, const TileEpilogue* epilogue, const IDSelector* sel) const;
+  /// decode of the entries at slab indexes pos (vlq_decode_entries): what reconstruct* and search_and_reconstruct return
+  virtual void decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const;
+  /// writes the aux column of the rows [s, s + m) of an add into the arena slots `out` (their first-level list, lambda
+  /// byte and codes are written): dx are those m rows on the device.  No aux column: nothing.
+  virtual void encodeAux_(const float* dx, Index::idx_t m, const DeviceLists::Slots& out, Index::idx_t s,
+                          vlq_stream_t st) {}
+  /// aux bytes of list listId in list order (auxWidth per entry)
+  std::vector<unsigned char> listAux_(int listId) const;
   void readBack_(Index::idx_t n, const Index::idx_t* keys, Index::idx_t i0, float* recons) const;
   void addTiles_(Index::idx_t n, const void* x, bool isU8, const long* xids);
   void installLists_(const std::vector<int>& counts, const std::vector<uint8_t>& codes, const std::vector<uint8_t>& las,
@@ -188,8 +204,8 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   mutable DeviceLists lists_;  // over the nlist * numedge lines
   size_t populatedLists_;  ///< lists that can hold entries (all of them; the slice of readDbFromFile(name, pronum, rank))
   mutable vlq_event_t evCoarse_[2] = {nullptr, nullptr}, evScan_[2] = {nullptr, nullptr};  // search(): two-stream tile pipeline
-  mutable DeviceBuffer scratch_, scratchB_, qIn_, outD_, outI_, addIn_[2], addA_, addF32_, t3ws_,
-      recStage_;  // grow-only staging / workspace
+  mutable DeviceBuffer scratch_, scratchB_, qIn_, outD_, outI_, addIn_[2], addA_, addF32_, t3ws_, recStage_, candD_,
+      candI_;  // grow-only staging / workspace
 };
 
 }  // namespace gpu

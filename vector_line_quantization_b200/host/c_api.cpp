@@ -8,6 +8,7 @@
 #include "Clustering.h"
 #include "GpuIndexIMIPQ.h"
 #include "GpuIndexIVFPQ.h"
+#include "GpuIndexIVFPQR.h"
 #include "IndexProxy.h"
 #include "filehelper.h"
 
@@ -32,6 +33,11 @@ static Index* I(void* h) { return static_cast<Index*>(h); }
 static GpuIndexIVFPQ* V(void* h) {
   GpuIndexIVFPQ* p = dynamic_cast<GpuIndexIVFPQ*>(static_cast<Index*>(h));
   if (!p) throw FaissException("handle is not a VLQ index");
+  return p;
+}
+static GpuIndexIVFPQR* VR(void* h) {
+  GpuIndexIVFPQR* p = dynamic_cast<GpuIndexIVFPQR*>(static_cast<Index*>(h));
+  if (!p) throw FaissException("handle is not a GpuIndexIVFPQR");
   return p;
 }
 static GpuIndexFlat* F(void* h) {
@@ -277,6 +283,38 @@ int vlq_host_vlq_read_codebook(void* index, const char* name) { GUARD(V(index)->
 int vlq_host_vlq_write_db(void* index, const char* name) { GUARD(V(index)->writeDbToFile(name)) }
 int vlq_host_vlq_read_db(void* index, const char* name, int pronum, int rank) {
   GUARD(V(index)->readDbFromFile(name, pronum, rank))
+}
+
+int vlq_host_ivfpqr_new(void* res, int d, int nlist, int M, int M_refine, int bits, int nedge, int nlambda,
+                        int use_tensor_cores, void** out) {
+  GUARD({
+    GpuResources* r = static_cast<GpuResources*>(res);
+    GpuIndexIVFPQConfig cfg;
+    cfg.device = r->getDevice();
+    cfg.flatConfig.useTensorCores = use_tensor_cores != 0;
+    *out = static_cast<Index*>(new GpuIndexIVFPQR(r, d, nlist, M, M_refine, bits, nedge, nlambda, METRIC_L2, cfg));
+  })
+}
+int vlq_host_ivfpqr_set_k_factor(void* index, float k_factor) {
+  GUARD({
+    VLQ_THROW_IF_NOT_MSG(k_factor >= 1.f, "k_factor must be >= 1");
+    VR(index)->k_factor = k_factor;
+  })
+}
+int vlq_host_ivfpqr_get_k_factor(void* index, float* out) { GUARD(*out = VR(index)->k_factor) }
+int vlq_host_ivfpqr_set_refine_codebook(void* index, const float* pq2) { GUARD(VR(index)->setRefineCodebook(pq2)) }
+int vlq_host_ivfpqr_get_refine_codebook(void* index, float* pq2) {
+  GUARD({
+    const std::vector<float>& cb = VR(index)->refineCodebook();
+    VLQ_THROW_IF_NOT_MSG(!cb.empty(), "GpuIndexIVFPQR: no refinement codebook");
+    std::memcpy(pq2, cb.data(), cb.size() * sizeof(float));
+  })
+}
+int vlq_host_ivfpqr_get_list_refine_codes(void* index, int list, unsigned char* codes) {
+  GUARD({
+    auto c = VR(index)->getListRefineCodes(list);
+    if (codes && !c.empty()) std::memcpy(codes, c.data(), c.size());
+  })
 }
 
 /* host-side pieces of k-means that never touch the GPU (reference utils.cpp:135-160,307-317) */

@@ -534,6 +534,52 @@ class GpuIndexIVFPQ(_ReadBack, Index):
         return dists, nns
 
 
+class GpuIndexIVFPQR(GpuIndexIVFPQ):
+    """GpuIndexIVFPQ plus a refinement stage (faiss IndexIVFPQR, host/GpuIndexIVFPQR.h): every entry also stores an
+    8-bit PQ code of M_refine sub-quantizers of the residual its first-level code leaves, and search re-ranks the
+    scan's min(1024, max(k, floor(k * k_factor))) candidates by the two-level reconstruction.  search distances are
+    FULL squared L2 ||q - x2||^2 (as IndexIVFPQR), not GpuIndexIVFPQ's ||q||^2-less values; reconstruct* return x2.
+    range_search, copyFrom / copyTo and the .db* files raise FaissException."""
+
+    def __init__(self, res, d, nlist, M, M_refine, bits=8, nedge=32, nLambda=256, use_tensor_cores=True):
+        M_refine = int(M_refine)
+        if not 1 <= M_refine <= 64 or d % M_refine != 0:
+            raise ValueError("M_refine must be in [1, 64] and divide d = %d, got %d" % (d, M_refine))
+        Index.__init__(self, d)
+        self.res, self.nlist, self.M, self.nedge, self.nLambda, self.M_refine = res, nlist, M, nedge, nLambda, M_refine
+        _call("vlq_host_ivfpqr_new", res.h, d, nlist, M, M_refine, bits, nedge, nLambda, int(use_tensor_cores),
+              C.byref(self.h))
+        self._w1 = 256
+
+    @property
+    def k_factor(self):
+        out = C.c_float()
+        _call("vlq_host_ivfpqr_get_k_factor", self.h, C.byref(out))
+        return out.value
+
+    @k_factor.setter
+    def k_factor(self, v):
+        _call("vlq_host_ivfpqr_set_k_factor", self.h, C.c_float(v))
+
+    def setRefineCodebook(self, pq2):
+        """pq2: (M_refine, 256, d / M_refine) float32"""
+        pq2 = np.ascontiguousarray(pq2, np.float32)
+        if pq2.size != 256 * self.d:
+            raise ValueError("refinement codebook must hold (M_refine, 256, d / M_refine) floats")
+        _call("vlq_host_ivfpqr_set_refine_codebook", self.h, C.c_void_p(pq2.ctypes.data))
+
+    def refineCodebook(self):
+        out = np.empty((self.M_refine, 256, self.d // self.M_refine), np.float32)
+        _call("vlq_host_ivfpqr_get_refine_codebook", self.h, C.c_void_p(out.ctypes.data))
+        return out
+
+    def getListRefineCodes(self, l):
+        """code2 of the entries of list l in list order -> uint8 [len][M_refine]"""
+        out = np.empty((self.getListLength(l), self.M_refine), np.uint8)
+        _call("vlq_host_ivfpqr_get_list_refine_codes", self.h, int(l), C.c_void_p(out.ctypes.data))
+        return out
+
+
 class CpuIndexIVFPQ:
     """faiss::IndexIVFPQ as a CONTAINER (host/IndexIVFPQ.h): coarse centroids, PQ codebook, per-list ids + codes -- what
     GpuIndexIVFPQ.copyFrom / copyTo exchange with a CPU index"""

@@ -235,6 +235,60 @@ def decode_entries(lists, pos, pq, cent=None, edge=None, lambda_cb=None, cb=None
     return (out, oid) if want_ids else out
 
 
+def _refine_tables(pq, cent, edge, lambda_cb, pq2):
+    return (_chk(pq, torch.float32, "pq"), _chk(cent, torch.float32, "cent"), _chk(edge, torch.int32, "edge"),
+            _chk(lambda_cb, torch.float32, "lambda_cb"), _chk(pq2, torch.float32, "pq2"))
+
+
+def refine_encode(x, enc, pq, cent, edge, lambda_cb, pq2=None, want_residual=False):
+    """refinement code of rows x from their line_encode outputs enc (list, lamq, canonical codes) (vlq_refine_encode)
+    -> (code2 uint8 [n][M2] or None, r2 f32 [n][d] or None); r2 = x - x1, code2 = PQ2(r2).  pq2=None: r2 only."""
+    x = _chk(x, torch.float32, "x")
+    pq, cent, edge, lambda_cb, pq2 = _refine_tables(pq, cent, edge, lambda_cb, pq2)
+    n, d = x.shape
+    M2 = pq2.shape[0] if pq2 is not None else 0
+    code2 = torch.empty((n, M2), dtype=torch.uint8, device=x.device) if pq2 is not None else None
+    r2 = torch.empty((n, d), dtype=torch.float32, device=x.device) if (want_residual or pq2 is None) else None
+    _abi.call("vlq_refine_encode", _ptr(x), n, d, _ptr(_chk(enc.list, torch.int32, "list")),
+              _ptr(_chk(enc.lamq, torch.uint8, "lamq")), _ptr(_chk(enc.codes, torch.uint8, "codes")), pq.shape[0],
+              _ptr(pq), _ptr(cent), _ptr(edge), edge.shape[-1], _ptr(lambda_cb), lambda_cb.shape[0], _ptr(pq2), M2,
+              _ptr(code2), _ptr(r2), _stream())
+    return code2, r2
+
+
+def refine_topk(q, cand, k, lists, code2, pq, cent, edge, lambda_cb, pq2, labels=True):
+    """re-rank (vlq_refine_topk): cand int64 [nq][kc] slab indexes (-1 = none) -> (D f32 [nq][k] = ||q - x2||^2
+    ascending, I int64 [nq][k] ids, or slab indexes with labels=False); ties keep candidate order, (FLT_MAX, -1) pad"""
+    q = _chk(q, torch.float32, "q")
+    cand = _chk(cand, torch.int64, "cand")
+    pq, cent, edge, lambda_cb, pq2 = _refine_tables(pq, cent, edge, lambda_cb, pq2)
+    offsets = _chk(lists.offsets, torch.int64, "offsets")
+    nq, d = q.shape
+    kc = cand.shape[1]
+    D = torch.empty((nq, k), dtype=torch.float32, device=q.device)
+    I = torch.empty((nq, k), dtype=torch.int64, device=q.device)
+    _abi.call("vlq_refine_topk", _ptr(q), nq, d, _ptr(cand), kc, k, offsets.shape[0] - 1, _ptr(offsets),
+              _ptr(lists.codes), _ptr(lists.lamq), _ptr(lists.ids) if labels else 0, _ptr(code2), pq.shape[0], _ptr(pq),
+              _ptr(cent), _ptr(edge), edge.shape[-1], _ptr(lambda_cb), lambda_cb.shape[0], _ptr(pq2), pq2.shape[0],
+              _ptr(D), _ptr(I), _stream())
+    return D, I
+
+
+def refine_decode(lists, code2, pos, pq, cent, edge, lambda_cb, pq2):
+    """x2 = x1 + p2(code2) of the entries at the slab indexes pos (vlq_refine_decode) -> f32 [n][d] (-1: NaN row)"""
+    pq, cent, edge, lambda_cb, pq2 = _refine_tables(pq, cent, edge, lambda_cb, pq2)
+    offsets = _chk(lists.offsets, torch.int64, "offsets")
+    pos = _chk(pos, torch.int64, "pos")
+    M, d = pq.shape[0], pq.shape[0] * pq.shape[2]
+    n = pos.numel()
+    out = torch.empty((n, d), dtype=torch.float32, device=offsets.device)
+    _abi.call("vlq_refine_decode", n, _ptr(pos), offsets.shape[0] - 1, _ptr(offsets), _ptr(lists.codes),
+              _ptr(lists.lamq), _ptr(lists.ids), _ptr(_chk(code2, torch.uint8, "code2")), M, d, _ptr(pq), _ptr(cent),
+              _ptr(edge), edge.shape[-1], _ptr(lambda_cb), lambda_cb.shape[0], _ptr(pq2), pq2.shape[0], _ptr(out), 0,
+              _stream())
+    return out
+
+
 def filter_kappa(lists, id_range=None, ids=None, bitmap=None, invert=False, out=None):
     """masked kappa of filtered search (vlq_filter_kappa) -> f32 CUDA tensor [n]: lists.kappa where the entry's id is a
     member, +inf elsewhere.  member = id in the half-open id_range (lo, hi) OR in `ids` (int64, any order, duplicates
