@@ -511,7 +511,10 @@ __global__ void __launch_bounds__(THREADS, 1) l2_tc_kernel(const Params p) {
                   mn[b] = fminf(mn[b], __shfl_xor_sync(0xffffffffu, mn[b], 1));
                   mn[b] = fminf(mn[b], __shfl_xor_sync(0xffffffffu, mn[b], 2));
                 }
-                if (row_ok && p.bmin && qd < 2) p.bmin[row * nb + t * 4 + col_half * 2 + qd] = mn[qd];
+                // a select, not mn[qd]: indexed by a lane value, mn would live in local memory (8 bytes of stack, 32
+                // local loads and stores in the sweep's epilogue; the sweep took 0.69 instead of 0.62 ms per 10 k
+                // C2 queries, profiles/r10_overlap.md)
+                if (row_ok && p.bmin && qd < 2) p.bmin[row * nb + t * 4 + col_half * 2 + qd] = qd ? mn[1] : mn[0];
               }
             }
           }
