@@ -382,6 +382,53 @@ int vlq_range_gather(const float* q, int64_t nq, int d, const float* pq, int M, 
                      float* outD, int64_t* outI, const void* workspace, size_t workspace_bytes, vlq_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
+ * 4-bit PQ codes (faiss ProductQuantizer(d, M, 4)), two codes per stored byte.  pq is (M, 16, dsub) fp32; M even,
+ *     2 <= M <= 64, d % M == 0, d <= 256 (VLQ_EINVAL otherwise).  An entry's codes are stored packed in Mb = M / 2 bytes,
+ *       byte j = code[2j] | code[2j + 1] << 4                (faiss's low-nibble-first order)
+ *     and the packed word is an 8-bit word of Mb "sub-quantizers" to every list routine: vlq_build_lists[_aux],
+ *     vlq_remove_ids_*, vlq_filter_kappa, vlq_gather_candidates take M = Mb and rotate it by pos mod Mb.
+ *     The scans read PAIR tables, one of 256 entries per stored byte:
+ *       T3'[m'][b] = T3[2m'][b & 15] + T3[2m' + 1][b >> 4],  T3[m][j] = -2 q_m . p_mj   (one fp32 add)
+ *       dist = term1 + l term6 + (l^2 - l) term5 + kappa + sum_m' T3'[m'][byte_m']
+ *     so their per-entry work is that of an 8-bit index with Mb sub-quantizers; the sum runs over pair tables and can
+ *     differ from a sum of the M 16-entry tables in the last ulp.
+ *     vlq_line_encode_pq4:      vlq_line_encode with the 16-centroid codebook; out_codes [n][M / 2] packed.
+ *     vlq_scan_topk_pq4:        vlq_scan_topk over packed lists; the workspace is REQUIRED (the tables are built into
+ *                               it; there is no in-kernel build): >= vlq_scan_topk_workspace_bytes(nq, M / 2), else
+ *                               VLQ_EWORKSPACE; workspace and pq 16-byte aligned.
+ *     vlq_range_count_pq4 / vlq_range_gather_pq4: the radius passes, workspace vlq_range_workspace_bytes(nq, M / 2, W, cap).
+ *     vlq_decode_entries_pq4 / vlq_recompute_kappa_pq4: vlq_decode_entries / vlq_recompute_kappa of packed entries.
+ *     Every other argument is as in the 8-bit entry point of the same name.
+ * ---------------------------------------------------------------------------------------------------------------- */
+int vlq_line_encode_pq4(const float* x, int64_t n, int d, const int* assign, const float* cent, const int* edge,
+                        const float* edge_d2, int E, const float* lambda_cb, int nL, const float* pq, int M,
+                        int* out_list, float* out_lambda, uint8_t* out_lamq, uint8_t* out_codes, float* out_kappa,
+                        float* out_residual, vlq_stream_t stream);
+int vlq_scan_topk_pq4(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                      const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                      const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa,
+                      const int64_t* ids, int k, int cap, int list_len_hint, float* outD, int64_t* outI, void* workspace,
+                      size_t workspace_bytes, vlq_stream_t stream);
+int vlq_range_count_pq4(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                        const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                        const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
+                        const float* row_add, float radius, int64_t* out_lims, void* workspace, size_t workspace_bytes,
+                        vlq_stream_t stream);
+int vlq_range_gather_pq4(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                         const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                         const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
+                         const float* row_add, float radius, const int64_t* ids, const int64_t* lims, int64_t q0,
+                         int64_t q1, float* outD, int64_t* outI, const void* workspace, size_t workspace_bytes,
+                         vlq_stream_t stream);
+int vlq_decode_entries_pq4(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets, const uint8_t* codes,
+                           const uint8_t* lamq, const int64_t* ids, int M, int d, const float* pq, const float* cent,
+                           const int* edge, int E, const float* lambda_cb, int nL, float* out_x, int64_t* out_ids,
+                           vlq_stream_t stream);
+int vlq_recompute_kappa_pq4(int64_t n, int64_t nlists, const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq,
+                            const float* cent, int d, const int* edge, int E, const float* lambda_cb, const float* pq,
+                            int M, float* kappa, vlq_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------------------------
  * a16 shard merge: k smallest of R*k candidates per query; D, I are [R][nq][k] (the all-gather layout); shards with
  *     fewer than k results pad with (FLT_MAX, -1), as vlq_scan_topk does.
  *     replaces GpuIndexIVFPQ::merge / mergekernel, gpu/GpuIndexIVFPQ.cu:1467-1591 (CPU twin MetaIndexes.cpp:290-347).

@@ -79,7 +79,10 @@ int vlq_host_flat_build_graph(void* flat, int nedge, float* distances, int* labe
 /* Clustering::train over a GpuIndexFlatL2 assigner */
 int vlq_host_kmeans(void* res, int d, int k, long n, const float* x, int niter, int seed, float* centroids_out);
 
-/* GpuIndexIVFPQ with the VLQ constructor (res, d, nlist, M, bits, nedge, nLambda, METRIC_L2) */
+/* GpuIndexIVFPQ with the VLQ constructor (res, d, nlist, M, bits, nedge, nLambda, METRIC_L2).  bits 8, or 4 with an
+   even M (two codes per stored byte on the device; list codes, the codebook exchange and the .db* files keep one byte
+   per code, pq (M, 2^bits, d / M) floats).  The code format is checked before res is used; GpuIndexIVFPQR and
+   GpuIndexIMIPQ take bits = 8 only. */
 int vlq_host_vlq_new(void* res, int d, int nlist, int M, int bits, int nedge, int nlambda, int use_tensor_cores,
                      void** out);
 int vlq_host_vlq_set_nprobe(void* index, int nprobe);

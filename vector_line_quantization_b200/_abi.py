@@ -70,6 +70,15 @@ SIGNATURES = {
     "vlq_range_count": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i, _p, _f, _p, _p, _z, _p]),
     "vlq_range_gather": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i, _p, _f, _p, _p, _l, _l,
                               _p, _p, _p, _z, _p]),
+    "vlq_line_encode_pq4": (_i, [_p, _l, _i, _p, _p, _p, _p, _i, _p, _i, _p, _i, _p, _p, _p, _p, _p, _p, _p]),
+    "vlq_scan_topk_pq4": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p,
+                               _z, _p]),
+    "vlq_range_count_pq4": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i, _p, _f, _p, _p, _z,
+                                 _p]),
+    "vlq_range_gather_pq4": (_i, [_p, _l, _i, _p, _i, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i, _p, _f, _p, _p, _l,
+                                  _l, _p, _p, _p, _z, _p]),
+    "vlq_decode_entries_pq4": (_i, [_l, _p, _l, _p, _p, _p, _p, _i, _i, _p, _p, _p, _i, _p, _i, _p, _p, _p]),
+    "vlq_recompute_kappa_pq4": (_i, [_l, _l, _p, _p, _p, _p, _i, _p, _i, _p, _p, _i, _p, _p]),
     "vlq_merge_topk": (_i, [_p, _p, _i, _l, _i, _p, _p, _p]),
     "vlq_merge_topk_peers": (_i, [_p, _z, _z, _i, _l, _i, _p, _p, _p]),
     "vlq_gather_peer_slices": (_i, [_p, _i, _i, _p, _i, _l, _l, _p]),

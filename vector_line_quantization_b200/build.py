@@ -77,7 +77,9 @@ def build_host(force=False, verbose=False):
     srcs = sorted(glob.glob(os.path.join(HOST, "*.cpp")))
     if not srcs:
         return None
-    hdrs = glob.glob(os.path.join(HOST, "*.h")) + glob.glob(os.path.join(INCLUDE, "*.h")) + [__file__]
+    # the host layer includes csrc/pq4.cuh (the 4-bit code format is shared with the device code)
+    hdrs = (glob.glob(os.path.join(HOST, "*.h")) + glob.glob(os.path.join(INCLUDE, "*.h")) +
+            [os.path.join(CSRC, "pq4.cuh"), __file__])
     lib = os.path.join(LIBDIR, "libvlq_host.so")
     cuda_lib = os.path.join(LIBDIR, "libvlq_b200.so")
     if force or _newer(lib, srcs + hdrs + [cuda_lib]):

@@ -3,6 +3,7 @@
 // the value the re-rank and reconstruct add it to are the same bits.
 #pragma once
 #include "common.cuh"
+#include "pq4.cuh"
 
 namespace vlq {
 
@@ -41,13 +42,25 @@ __device__ __forceinline__ float pq_component(const float* __restrict__ pq, cons
   return pq[((int64_t)m * 256 + cw[sb]) * dsub + (j - m * dsub)];
 }
 
+// the same for a packed 4-bit code (pq4.cuh): pq is (M, 16, dsub), the Mb = M / 2 stored bytes are rotated by rot
+// (stored[(b - rot) mod Mb] = packed[b]), code m is nibble m & 1 of packed byte m / 2
+__device__ __forceinline__ float pq4_component(const float* __restrict__ pq, const uint8_t* cw, int M, int dsub, int rot,
+                                               int j) {
+  const int m = j / dsub, Mb = M / 2;
+  int sb = (m >> 1) - rot;
+  if (sb < 0) sb += Mb;
+  const int code = (cw[sb] >> ((m & 1) * 4)) & 15;
+  return pq[((int64_t)m * kPq4Ksub + code) * dsub + (j - m * dsub)];
+}
+
 // x1[j] = ((1 - lh) c[j] + lh s[j]) + pq[m][code_m][j - m dsub]: fp32, each operation rounded as written (no fma
-// contraction), oml = 1 - lh rounded; lh = 0 gives exactly c + p (IndexIVFPQ's decode)
+// contraction), oml = 1 - lh rounded; lh = 0 gives exactly c + p (IndexIVFPQ's decode).  pq4: cw is a packed 4-bit code
+// of M / 2 bytes and rot is taken mod M / 2.
 __device__ __forceinline__ float vlq_decode_component(const float* c, const float* s, float lh, float oml,
                                                       const float* __restrict__ pq, const uint8_t* cw, int M, int dsub,
-                                                      int rot, int j) {
+                                                      int rot, int j, bool pq4 = false) {
   const float a = __fadd_rn(__fmul_rn(oml, c[j]), __fmul_rn(lh, s[j]));
-  return __fadd_rn(a, pq_component(pq, cw, M, dsub, rot, j));
+  return __fadd_rn(a, pq4 ? pq4_component(pq, cw, M, dsub, rot, j) : pq_component(pq, cw, M, dsub, rot, j));
 }
 
 }  // namespace vlq

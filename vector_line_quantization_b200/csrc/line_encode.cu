@@ -13,6 +13,7 @@
 //      (ProductQuantizer.cpp:311-336), and emits kappa = ||p||^2 + 2 anchor.p for the scan.
 // Nothing but the final list id / lambda byte / M code bytes / kappa leaves the SM.
 #include "common.cuh"
+#include "pq4.cuh"
 
 namespace vlq {
 
@@ -262,6 +263,35 @@ __global__ void __launch_bounds__(LE_THREADS, 1) line_encode_kernel(LineEncodeAr
           }
           kc[v] = make_key(bd, (uint32_t)(lane + 32 * bc));
         }
+      } else if (ksub == kPq4Ksub) {
+        // 4-bit codebook (pq4_in_smem always holds, 16 d floats): lane = (h, j) scores codeword j = lane & 15 of
+        // sub-quantizer m + h, h = lane >> 4, for all LE_V vectors -- two sub-quantizers per pass, no idle lane.  The
+        // arg-min over the 16 lanes of a half takes the lowest (distance, j): the lowest codeword wins ties.
+        const int h = lane >> 4, j = lane & 15, mh = m + h;
+        float dis[LE_V];
+#pragma unroll
+        for (int v = 0; v < LE_V; v++) dis[v] = 0.f;
+        const float* pp = pqs + (size_t)mh * dsub * kPq4Ksub + j;
+        for (int t = 0; t < dsub; t++) {
+          const float pc = pp[t * kPq4Ksub];
+#pragma unroll
+          for (int v = 0; v < LE_V; v++) {
+            const float df = r_w[v * d + mh * dsub + t] - pc;
+            dis[v] = fmaf(df, df, dis[v]);
+          }
+        }
+#pragma unroll
+        for (int v = 0; v < LE_V; v++) {
+          uint64_t key = make_key(dis[v], (uint32_t)j);
+#pragma unroll
+          for (int o = 8; o > 0; o >>= 1) {
+            const uint64_t other = __shfl_xor_sync(kFull, key, o);
+            key = other < key ? other : key;
+          }
+          if (j == 0) code_w[v * 64 + mh] = (uint8_t)key_payload(key);
+        }
+        m++;  // the pass covered m and m + 1 (M is even)
+        continue;
       } else {
 #pragma unroll
         for (int v = 0; v < LE_V; v++) {
@@ -316,8 +346,11 @@ __global__ void __launch_bounds__(LE_THREADS, 1) line_encode_kernel(LineEncodeAr
         if (a.out_lamq) a.out_lamq[i] = (uint8_t)lq;
         if (a.out_kappa) a.out_kappa[i] = kp;
       }
-      if (a.out_codes)
+      if (a.out_codes && ksub == kPq4Ksub) {  // packed, M / 2 bytes (pq4.cuh)
+        for (int b = lane; b < M / 2; b += kWarp) a.out_codes[i * (M / 2) + b] = pq4_pack_byte(code_s[2 * b], code_s[2 * b + 1]);
+      } else if (a.out_codes) {
         for (int m = lane; m < M; m += kWarp) a.out_codes[i * M + m] = code_s[m];
+      }
     }
     __syncwarp();
   }
@@ -405,13 +438,14 @@ extern "C" int vlq_i32_to_i64(const int* src, int64_t n, int64_t* dst, vlq_strea
   return last_error();
 }
 
-extern "C" int vlq_line_encode(const float* x, int64_t n, int d, const int* assign, const float* cent,
-                               const int* edge, const float* edge_d2, int E, const float* lambda_cb, int nL,
-                               const float* pq, int M, int* out_list, float* out_lambda, uint8_t* out_lamq,
-                               uint8_t* out_codes, float* out_kappa, float* out_residual, vlq_stream_t stream) {
+// vlq_line_encode (ksub = 256) and vlq_line_encode_pq4 (ksub = 16: packed output, M even)
+static int line_encode(int ksub, const float* x, int64_t n, int d, const int* assign, const float* cent,
+                       const int* edge, const float* edge_d2, int E, const float* lambda_cb, int nL, const float* pq,
+                       int M, int* out_list, float* out_lambda, uint8_t* out_lamq, uint8_t* out_codes,
+                       float* out_kappa, float* out_residual, vlq_stream_t stream) {
   if (n < 0 || d <= 0 || d > 256 || E <= 0 || E > LE_MAX_E) return VLQ_EINVAL;
   if (n > 0 && (!x || !assign || !cent || !edge || !edge_d2 || !out_list)) return VLQ_EINVAL;
-  const int ksub = 256;
+  if (ksub == kPq4Ksub && !pq4_shape_ok(d, M)) return VLQ_EINVAL;
   LineEncodeArgs a{};
   a.x = x; a.n = n; a.d = d; a.assign = assign; a.cent = cent; a.edge = edge; a.edge_d2 = edge_d2; a.E = E;
   a.lambda_cb = lambda_cb; a.nL = nL; a.pq = pq; a.M = M; a.ksub = ksub; a.dsub = M > 0 ? d / M : 0;
@@ -453,4 +487,20 @@ extern "C" int vlq_line_encode(const float* x, int64_t n, int d, const int* assi
   }
 #undef VLQ_LE_CASE
   return last_error();
+}
+
+extern "C" int vlq_line_encode(const float* x, int64_t n, int d, const int* assign, const float* cent,
+                               const int* edge, const float* edge_d2, int E, const float* lambda_cb, int nL,
+                               const float* pq, int M, int* out_list, float* out_lambda, uint8_t* out_lamq,
+                               uint8_t* out_codes, float* out_kappa, float* out_residual, vlq_stream_t stream) {
+  return line_encode(256, x, n, d, assign, cent, edge, edge_d2, E, lambda_cb, nL, pq, M, out_list, out_lambda, out_lamq,
+                     out_codes, out_kappa, out_residual, stream);
+}
+
+extern "C" int vlq_line_encode_pq4(const float* x, int64_t n, int d, const int* assign, const float* cent,
+                                   const int* edge, const float* edge_d2, int E, const float* lambda_cb, int nL,
+                                   const float* pq, int M, int* out_list, float* out_lambda, uint8_t* out_lamq,
+                                   uint8_t* out_codes, float* out_kappa, float* out_residual, vlq_stream_t stream) {
+  return line_encode(kPq4Ksub, x, n, d, assign, cent, edge, edge_d2, E, lambda_cb, nL, pq, M, out_list, out_lambda,
+                     out_lamq, out_codes, out_kappa, out_residual, stream);
 }

@@ -306,9 +306,10 @@ __global__ void recompute_kappa_kernel(int64_t n, int64_t nlists, const int64_t*
                                        const uint8_t* __restrict__ codes, const uint8_t* __restrict__ lamq,
                                        const float* __restrict__ cent, int d, const int* __restrict__ edge, int E,
                                        const float* __restrict__ lambda_cb, const float* __restrict__ pq, int M,
-                                       float* __restrict__ kappa) {
+                                       bool pq4, float* __restrict__ kappa) {
   const int lane = threadIdx.x % kWarp;
   const int dsub = d / M;
+  const int CB = pq4 ? M / 2 : M;  // code bytes per entry
   for (int64_t i = (int64_t)blockIdx.x * (blockDim.x / kWarp) + threadIdx.x / kWarp; i < n;
        i += (int64_t)gridDim.x * (blockDim.x / kWarp)) {
     int64_t lo = 0, hi = nlists;  // list of entry i: largest l with offsets[l] <= i
@@ -318,14 +319,15 @@ __global__ void recompute_kappa_kernel(int64_t n, int64_t nlists, const int64_t*
     }
     const int A = (int)(lo / E);
     const int s = edge[lo];
-    const int rot = (int)((i - offsets[lo]) % M);  // stored[j] = code[(j + pos) mod M]
+    const int rot = (int)((i - offsets[lo]) % CB);  // stored[j] = code[(j + pos) mod CB]
     const float lh = lambda_cb[lamq[i]];
     const float oml = 1.f - lh;
     float kp = 0.f;
     for (int j = lane; j < d; j += kWarp) {
       const float anc = __fadd_rn(__fmul_rn(oml, cent[(int64_t)A * d + j]), __fmul_rn(lh, cent[(int64_t)s * d + j]));
       const int m = j / dsub, tt = j % dsub;
-      const float pv = pq[((size_t)m * 256 + codes[i * M + (m - rot + M) % M]) * dsub + tt];
+      const float pv = pq4 ? pq4_component(pq, codes + i * CB, M, dsub, rot, j)
+                           : pq[((size_t)m * 256 + codes[i * M + (m - rot + M) % M]) * dsub + tt];
       kp = fmaf(pv, pv, kp);
       kp = fmaf(2.f * anc, pv, kp);
     }
@@ -627,7 +629,7 @@ struct DecodeAnchor {
   int M2;
 };
 
-template <bool IMI>
+template <bool IMI, bool PQ4 = false>
 __global__ void __launch_bounds__(SCAN_THREADS)
 decode_entries_kernel(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* __restrict__ offsets,
                       const uint8_t* __restrict__ codes, const int64_t* __restrict__ ids, int M, int d,
@@ -636,6 +638,7 @@ decode_entries_kernel(int64_t n, const int64_t* pos, int64_t nlists, const int64
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) / kWarp;
   const int64_t nslab = offsets[nlists];
   const int dsub = d / M;
+  const int CB = PQ4 ? M / 2 : M;  // code bytes per entry
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / kWarp; r < n; r += nwarps) {
     const int64_t p = pos[r];
     __syncwarp();  // out_ids may alias pos: every lane has read pos[r] before lane 0 overwrites it
@@ -646,8 +649,8 @@ decode_entries_kernel(int64_t n, const int64_t* pos, int64_t nlists, const int64
       continue;
     }
     const int64_t l = list_of(offsets, 0, nlists - 1, p);
-    const int rot = (int)((p - offsets[l]) % M);
-    const uint8_t* cw = codes + p * M;
+    const int rot = (int)((p - offsets[l]) % CB);
+    const uint8_t* cw = codes + p * CB;
     if constexpr (IMI) {
       const int h = d / 2;
       const float* a0 = an.cb1 + (l & ((1 << an.nbits) - 1)) * h;
@@ -662,7 +665,7 @@ decode_entries_kernel(int64_t n, const int64_t* pos, int64_t nlists, const int64
       const uint8_t* c2 = an.pq2 ? an.code2 + p * an.M2 : nullptr;
       const int dsub2 = an.pq2 ? d / an.M2 : 1;
       for (int j = lane; j < d; j += kWarp) {
-        float v = vlq_decode_component(a0, a1, lh, oml, pq, cw, M, dsub, rot, j);
+        float v = vlq_decode_component(a0, a1, lh, oml, pq, cw, M, dsub, rot, j, PQ4);
         if (c2) v = __fadd_rn(v, pq_component(an.pq2, c2, an.M2, dsub2, 0, j));
         o[j] = v;
       }
@@ -735,15 +738,28 @@ int launch_exclusive_scan_i64(int64_t* v, int64_t n, cudaStream_t st) {
 
 using namespace vlq;
 
-extern "C" int vlq_recompute_kappa(int64_t n, int64_t nlists, const int64_t* offsets, const uint8_t* codes,
-                                   const uint8_t* lamq, const float* cent, int d, const int* edge, int E,
-                                   const float* lambda_cb, const float* pq, int M, float* kappa, vlq_stream_t stream) {
-  if (n < 0 || nlists <= 0 || d <= 0 || E <= 0 || M <= 0 || d % M != 0) return VLQ_EINVAL;
+static int recompute_kappa(bool pq4, int64_t n, int64_t nlists, const int64_t* offsets, const uint8_t* codes,
+                           const uint8_t* lamq, const float* cent, int d, const int* edge, int E,
+                           const float* lambda_cb, const float* pq, int M, float* kappa, vlq_stream_t stream) {
+  if (n < 0 || nlists <= 0 || d <= 0 || E <= 0 || M <= 0 || d % M != 0 || (pq4 && !pq4_shape_ok(d, M))) return VLQ_EINVAL;
   if (n == 0) return VLQ_OK;
   if (!offsets || !codes || !lamq || !cent || !edge || !lambda_cb || !pq || !kappa) return VLQ_EINVAL;
   VLQ_LAUNCH(recompute_kappa_kernel, 148 * 8, 256, 0, as_stream(stream), n, nlists, offsets, codes, lamq, cent, d, edge,
-             E, lambda_cb, pq, M, kappa);
+             E, lambda_cb, pq, M, pq4, kappa);
   return last_error();
+}
+
+extern "C" int vlq_recompute_kappa(int64_t n, int64_t nlists, const int64_t* offsets, const uint8_t* codes,
+                                   const uint8_t* lamq, const float* cent, int d, const int* edge, int E,
+                                   const float* lambda_cb, const float* pq, int M, float* kappa, vlq_stream_t stream) {
+  return recompute_kappa(false, n, nlists, offsets, codes, lamq, cent, d, edge, E, lambda_cb, pq, M, kappa, stream);
+}
+
+extern "C" int vlq_recompute_kappa_pq4(int64_t n, int64_t nlists, const int64_t* offsets, const uint8_t* codes,
+                                       const uint8_t* lamq, const float* cent, int d, const int* edge, int E,
+                                       const float* lambda_cb, const float* pq, int M, float* kappa,
+                                       vlq_stream_t stream) {
+  return recompute_kappa(true, n, nlists, offsets, codes, lamq, cent, d, edge, E, lambda_cb, pq, M, kappa, stream);
 }
 
 extern "C" size_t vlq_km_update_workspace_bytes(int64_t n, int k) { return carve(nullptr, n, k).bytes; }
@@ -907,31 +923,53 @@ extern "C" int vlq_lookup_ids(int64_t n, const int64_t* ids, int64_t range_lo, c
   return last_error();
 }
 
-static int decode_launch(bool imi, int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
+// kind: 0 VLQ, 1 IMI-PQ, 2 VLQ with packed 4-bit codes
+static int decode_launch(int kind, int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
                          const uint8_t* codes, const int64_t* ids, int M, int d, const float* pq, const DecodeAnchor& an,
                          float* out_x, int64_t* out_ids, vlq_stream_t stream) {
-  if (n < 0 || nlists < 1 || M < 1 || M > 64 || d < 1 || d % M != 0) return VLQ_EINVAL;
+  if (n < 0 || nlists < 1 || M < 1 || M > 64 || d < 1 || d % M != 0 || (kind == 2 && !pq4_shape_ok(d, M)))
+    return VLQ_EINVAL;
   if (n > 0 && (!pos || !offsets || !codes || !pq || !out_x || (out_ids && !ids))) return VLQ_EINVAL;
   if (n == 0) return VLQ_OK;
   const unsigned grid = grid_for(n, SCAN_THREADS / kWarp);
-  if (imi)
+  if (kind == 1)
     VLQ_LAUNCH(decode_entries_kernel<true>, grid, SCAN_THREADS, 0, as_stream(stream), n, pos, nlists, offsets, codes, ids, M,
                d, pq, an, out_x, out_ids);
+  else if (kind == 2)
+    VLQ_LAUNCH((decode_entries_kernel<false, true>), grid, SCAN_THREADS, 0, as_stream(stream), n, pos, nlists, offsets,
+               codes, ids, M, d, pq, an, out_x, out_ids);
   else
     VLQ_LAUNCH(decode_entries_kernel<false>, grid, SCAN_THREADS, 0, as_stream(stream), n, pos, nlists, offsets, codes, ids,
                M, d, pq, an, out_x, out_ids);
   return last_error();
 }
 
-extern "C" int vlq_decode_entries(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
-                                  const uint8_t* codes, const uint8_t* lamq, const int64_t* ids, int M, int d,
-                                  const float* pq, const float* cent, const int* edge, int E, const float* lambda_cb,
-                                  int nL, float* out_x, int64_t* out_ids, vlq_stream_t stream) {
+static int decode_vlq(bool pq4, int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
+                      const uint8_t* codes, const uint8_t* lamq, const int64_t* ids, int M, int d, const float* pq,
+                      const float* cent, const int* edge, int E, const float* lambda_cb, int nL, float* out_x,
+                      int64_t* out_ids, vlq_stream_t stream) {
   if (E < 1 || nlists % E != 0 || nL < 1 || nL > 256) return VLQ_EINVAL;
   if (n > 0 && (!lamq || !cent || !edge || !lambda_cb)) return VLQ_EINVAL;
   DecodeAnchor an{};
   an.cent = cent; an.edge = edge; an.lamq = lamq; an.lambda_cb = lambda_cb; an.E = E;
-  return decode_launch(false, n, pos, nlists, offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
+  return decode_launch(pq4 ? 2 : 0, n, pos, nlists, offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
+}
+
+extern "C" int vlq_decode_entries(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
+                                  const uint8_t* codes, const uint8_t* lamq, const int64_t* ids, int M, int d,
+                                  const float* pq, const float* cent, const int* edge, int E, const float* lambda_cb,
+                                  int nL, float* out_x, int64_t* out_ids, vlq_stream_t stream) {
+  return decode_vlq(false, n, pos, nlists, offsets, codes, lamq, ids, M, d, pq, cent, edge, E, lambda_cb, nL, out_x,
+                    out_ids, stream);
+}
+
+extern "C" int vlq_decode_entries_pq4(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
+                                      const uint8_t* codes, const uint8_t* lamq, const int64_t* ids, int M, int d,
+                                      const float* pq, const float* cent, const int* edge, int E,
+                                      const float* lambda_cb, int nL, float* out_x, int64_t* out_ids,
+                                      vlq_stream_t stream) {
+  return decode_vlq(true, n, pos, nlists, offsets, codes, lamq, ids, M, d, pq, cent, edge, E, lambda_cb, nL, out_x,
+                    out_ids, stream);
 }
 
 extern "C" int vlq_refine_decode(int64_t n, const int64_t* pos, int64_t nlists, const int64_t* offsets,
@@ -944,7 +982,7 @@ extern "C" int vlq_refine_decode(int64_t n, const int64_t* pos, int64_t nlists, 
   DecodeAnchor an{};
   an.cent = cent; an.edge = edge; an.lamq = lamq; an.lambda_cb = lambda_cb; an.E = E;
   an.code2 = code2; an.pq2 = pq2; an.M2 = M2;
-  return decode_launch(false, n, pos, nlists, offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
+  return decode_launch(0, n, pos, nlists, offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
 }
 
 extern "C" int vlq_imi_decode_entries(int64_t n, const int64_t* pos, const int64_t* offsets, const uint8_t* codes,
@@ -954,7 +992,7 @@ extern "C" int vlq_imi_decode_entries(int64_t n, const int64_t* pos, const int64
   if (n > 0 && (!cb1 || !cb2)) return VLQ_EINVAL;
   DecodeAnchor an{};
   an.cb1 = cb1; an.cb2 = cb2; an.nbits = nbits;
-  return decode_launch(true, n, pos, (int64_t)1 << (2 * nbits), offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
+  return decode_launch(1, n, pos, (int64_t)1 << (2 * nbits), offsets, codes, ids, M, d, pq, an, out_x, out_ids, stream);
 }
 
 extern "C" int vlq_filter_kappa(int64_t n, const int64_t* ids, const float* kappa, int64_t range_lo, int64_t range_hi,

@@ -11,6 +11,7 @@
 #include <cmath>
 
 #include "scan.cuh"
+#include "pq4.cuh"
 
 namespace vlq {
 
@@ -264,24 +265,33 @@ static int dispatch_range(bool gather, const RangeArgs& a, unsigned grid, cudaSt
   return launch_range<0>(gather, a, grid, smem, st);
 }
 
-// the checks both passes share; VLQ_OK with a.nq == 0 means "nothing to launch"
-static int range_args(RangeArgs& a, const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb,
-                      int nL, const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
-                      const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
-                      const float* row_add, float radius, const void* workspace, size_t workspace_bytes) {
-  if (nq < 0 || d <= 0 || M <= 0 || M > 64 || d % M != 0 || nL <= 0 || nL > 256 || W <= 0 || W > VLQ_MAX_K ||
+// the term-3 tables of the 8-bit codebook (M, 256, dsub) or the pair tables of the 4-bit one (M, 16, dsub)
+static TableBuild range_tables(bool pq4, int d, int M) {
+  return pq4 ? TableBuild{launch_pair_tables, true, true} : TableBuild{launch_term3, term3_supported(d, M), true};
+}
+
+// the checks both passes share; VLQ_OK with a.nq == 0 means "nothing to launch".  M is the number of sub-quantizers;
+// a.M the number of code bytes per entry (M / 2 for 4-bit codes)
+static int range_args(RangeArgs& a, bool pq4, const float* q, int64_t nq, int d, const float* pq, int M,
+                      const float* lambda_cb, int nL, const int* line_list, const float* term1, const float* term6,
+                      const float* edge_d2, int W, const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq,
+                      const float* kappa, int cap, const float* row_add, float radius, const void* workspace,
+                      size_t workspace_bytes) {
+  const bool shape_ok = pq4 ? pq4_shape_ok(d, M) && d <= 256 : d > 0 && M > 0 && M <= 64 && d % M == 0;
+  if (nq < 0 || !shape_ok || nL <= 0 || nL > 256 || W <= 0 || W > VLQ_MAX_K ||
       cap <= 0 || cap > (1 << 20) || (int64_t)W * cap > (int64_t)0x7fffffff || std::isnan(radius))
     return VLQ_EINVAL;
+  const int Mb = pq4 ? M / 2 : M;
   a = RangeArgs{};
   a.nq = nq;
   if (nq == 0) return VLQ_OK;
   if (!q || !pq || !lambda_cb || !line_list || !term1 || !term6 || !offsets || !codes || !lamq || !kappa || !workspace)
     return VLQ_EINVAL;
   if ((reinterpret_cast<uintptr_t>(pq) | reinterpret_cast<uintptr_t>(workspace)) & 15) return VLQ_EINVAL;
-  if (!term3_supported(d, M)) return VLQ_EUNSUPPORTED;
-  if (workspace_bytes < vlq_range_workspace_bytes(nq, M, W, cap)) return VLQ_EWORKSPACE;
+  if (!range_tables(pq4, d, M).supported) return VLQ_EUNSUPPORTED;
+  if (workspace_bytes < vlq_range_workspace_bytes(nq, Mb, W, cap)) return VLQ_EWORKSPACE;
   a.t3 = static_cast<const float*>(workspace);
-  a.M = M; a.nL = nL; a.lambda_cb = lambda_cb; a.line_list = line_list; a.term1 = term1; a.term6 = term6;
+  a.M = Mb; a.nL = nL; a.lambda_cb = lambda_cb; a.line_list = line_list; a.term1 = term1; a.term6 = term6;
   a.edge_d2 = edge_d2; a.W = W; a.cap = cap; a.offsets = offsets; a.codes = codes; a.lamq = lamq; a.kappa = kappa;
   a.row_add = row_add; a.radius = radius;
   return VLQ_OK;
@@ -299,22 +309,25 @@ size_t vlq_range_workspace_bytes(int64_t nq, int M, int /*W*/, int /*cap*/) {
   return (n * m * 256 * sizeof(float) + 255) & ~size_t(255);
 }
 
-int vlq_range_count(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
-                    const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
-                    const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
-                    const float* row_add, float radius, int64_t* out_lims, void* workspace, size_t workspace_bytes,
-                    vlq_stream_t stream) {
+}  // extern "C"
+
+// both passes of both codebooks: pq4 selects the table build and the code width, nothing else differs
+static int range_count(bool pq4, const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb,
+                       int nL, const int* line_list, const float* term1, const float* term6, const float* edge_d2,
+                       int W, const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa,
+                       int cap, const float* row_add, float radius, int64_t* out_lims, void* workspace,
+                       size_t workspace_bytes, vlq_stream_t stream) {
   if (!out_lims) return VLQ_EINVAL;
   RangeArgs a;
-  const int rc = range_args(a, q, nq, d, pq, M, lambda_cb, nL, line_list, term1, term6, edge_d2, W, offsets, codes, lamq,
-                            kappa, cap, row_add, radius, workspace, workspace_bytes);
+  const int rc = range_args(a, pq4, q, nq, d, pq, M, lambda_cb, nL, line_list, term1, term6, edge_d2, W, offsets, codes,
+                            lamq, kappa, cap, row_add, radius, workspace, workspace_bytes);
   if (rc) return rc;
   cudaStream_t st = as_stream(stream);
   if (nq == 0) {
     VLQ_CUDA_TRY(cudaMemsetAsync(out_lims, 0, sizeof(int64_t), st));
     return VLQ_OK;
   }
-  int r = launch_term3(q, nq, d, pq, M, static_cast<float*>(workspace), false, st);
+  int r = range_tables(pq4, d, M).launch(q, nq, d, pq, a.M, static_cast<float*>(workspace), false, st);
   if (r) return r;
   a.counts = out_lims;
   r = dispatch_range(false, a, (unsigned)nq, st);
@@ -322,14 +335,15 @@ int vlq_range_count(const float* q, int64_t nq, int d, const float* pq, int M, c
   return launch_exclusive_scan_i64(out_lims, nq + 1, st);
 }
 
-int vlq_range_gather(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
-                     const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
-                     const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
-                     const float* row_add, float radius, const int64_t* ids, const int64_t* lims, int64_t q0, int64_t q1,
-                     float* outD, int64_t* outI, const void* workspace, size_t workspace_bytes, vlq_stream_t stream) {
+static int range_gather(bool pq4, const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb,
+                        int nL, const int* line_list, const float* term1, const float* term6, const float* edge_d2,
+                        int W, const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa,
+                        int cap, const float* row_add, float radius, const int64_t* ids, const int64_t* lims,
+                        int64_t q0, int64_t q1, float* outD, int64_t* outI, const void* workspace,
+                        size_t workspace_bytes, vlq_stream_t stream) {
   RangeArgs a;
-  const int rc = range_args(a, q, nq, d, pq, M, lambda_cb, nL, line_list, term1, term6, edge_d2, W, offsets, codes, lamq,
-                            kappa, cap, row_add, radius, workspace, workspace_bytes);
+  const int rc = range_args(a, pq4, q, nq, d, pq, M, lambda_cb, nL, line_list, term1, term6, edge_d2, W, offsets, codes,
+                            lamq, kappa, cap, row_add, radius, workspace, workspace_bytes);
   if (rc) return rc;
   if (q0 < 0 || q1 < q0 || q1 > nq) return VLQ_EINVAL;
   if (q1 == q0) return VLQ_OK;
@@ -341,5 +355,50 @@ int vlq_range_gather(const float* q, int64_t nq, int d, const float* pq, int M, 
   a.outI = outI;
   return dispatch_range(true, a, (unsigned)(q1 - q0), as_stream(stream));
 }
+
+extern "C" {
+
+#define VLQ_RANGE_COUNT_ARGS                                                                                          \
+  q, nq, d, pq, M, lambda_cb, nL, line_list, term1, term6, edge_d2, W, offsets, codes, lamq, kappa, cap, row_add,    \
+      radius, out_lims, workspace, workspace_bytes, stream
+#define VLQ_RANGE_GATHER_ARGS                                                                                         \
+  q, nq, d, pq, M, lambda_cb, nL, line_list, term1, term6, edge_d2, W, offsets, codes, lamq, kappa, cap, row_add,    \
+      radius, ids, lims, q0, q1, outD, outI, workspace, workspace_bytes, stream
+
+int vlq_range_count(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                    const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                    const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
+                    const float* row_add, float radius, int64_t* out_lims, void* workspace, size_t workspace_bytes,
+                    vlq_stream_t stream) {
+  return range_count(false, VLQ_RANGE_COUNT_ARGS);
+}
+
+int vlq_range_count_pq4(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                        const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                        const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
+                        const float* row_add, float radius, int64_t* out_lims, void* workspace, size_t workspace_bytes,
+                        vlq_stream_t stream) {
+  return range_count(true, VLQ_RANGE_COUNT_ARGS);
+}
+
+int vlq_range_gather(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                     const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                     const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
+                     const float* row_add, float radius, const int64_t* ids, const int64_t* lims, int64_t q0, int64_t q1,
+                     float* outD, int64_t* outI, const void* workspace, size_t workspace_bytes, vlq_stream_t stream) {
+  return range_gather(false, VLQ_RANGE_GATHER_ARGS);
+}
+
+int vlq_range_gather_pq4(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                         const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                         const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa, int cap,
+                         const float* row_add, float radius, const int64_t* ids, const int64_t* lims, int64_t q0,
+                         int64_t q1, float* outD, int64_t* outI, const void* workspace, size_t workspace_bytes,
+                         vlq_stream_t stream) {
+  return range_gather(true, VLQ_RANGE_GATHER_ARGS);
+}
+
+#undef VLQ_RANGE_COUNT_ARGS
+#undef VLQ_RANGE_GATHER_ARGS
 
 }  // extern "C"

@@ -116,6 +116,17 @@ bool scan_long_supported(const ScanArgs& a);
 // the shapes those kernels take (d % 4 == 0, the PQ codebook fits their shared memory); pq and t3 16-byte aligned.
 bool term3_supported(int d, int M);
 int launch_term3(const float* q, int64_t nq, int d, const float* pq, int M, float* t3, bool code_major, cudaStream_t st);
+// the same tables for a 4-bit codebook (M = 2 Mb, 16, dsub): the Mb pair tables of pq4.cuh in either layout, so the scans
+// run unmodified with M = Mb.  Any pq4_shape_ok shape with d <= 256; t3 16-byte aligned.
+int launch_pair_tables(const float* q, int64_t nq, int d, const float* pq, int Mb, float* t3, bool code_major,
+                       cudaStream_t st);
+// how a scan or range entry point gets its term-3 tables: the 8-bit kernels above, or the pair tables (`required`: there
+// is no in-kernel table build for that codebook, so the workspace must hold the tables)
+struct TableBuild {
+  int (*launch)(const float* q, int64_t nq, int d, const float* pq, int M, float* t3, bool code_major, cudaStream_t st);
+  bool supported;
+  bool required;
+};
 
 // in-place exclusive scan of n int64 values by one block (lists.cu)
 int launch_exclusive_scan_i64(int64_t* v, int64_t n, cudaStream_t st);

@@ -19,6 +19,7 @@
 #include <cstdlib>
 
 #include "scan.cuh"
+#include "pq4.cuh"
 #include "topk.cuh"
 #include "coarse_select.cuh"
 
@@ -836,6 +837,51 @@ int launch_term3(const float* q, int64_t nq, int d, const float* pq, int M, floa
   return VLQ_OK;
 }
 
+// Pair tables of a 4-bit codebook (pq4.cuh): per query the M x 16 term-3 values T3[m][j] = -2 q_m . p_mj (the same fmaf
+// chain, t ascending, as the 8-bit kernels), then the Mb = M / 2 tables T3'[m'][b] = T3[2m'][b & 15] + T3[2m'+1][b >> 4]
+// of 256 entries, written in the layout the scan reads: row-major [Mb][256] or the code-major rows [256][Mb] of the
+// bank-skewed and long-list scans.  Persistent CTAs keep the 16 d-float codebook in shared memory; thread b owns table
+// column b, so both layouts are written coalesced.
+__global__ void __launch_bounds__(T3_THREADS)
+pair_tables_kernel(const float* __restrict__ q, int64_t nq, int d, const float* __restrict__ pq, int Mb,
+                   float* __restrict__ t3, bool code_major) {
+  extern __shared__ __align__(16) float pts[];
+  const int M = 2 * Mb, dsub = d / M;
+  float* pqs = pts;                       // [M][16][dsub]
+  float* qs = pqs + (size_t)M * 16 * dsub;  // [d]
+  float* t16 = qs + d;                      // [M][16]
+  for (int i = threadIdx.x; i < M * 16 * dsub; i += T3_THREADS) pqs[i] = pq[i];
+  for (int64_t qi = blockIdx.x; qi < nq; qi += gridDim.x) {
+    __syncthreads();
+    for (int j = threadIdx.x; j < d; j += T3_THREADS) qs[j] = q[qi * d + j];
+    __syncthreads();
+    for (int i = threadIdx.x; i < M * 16; i += T3_THREADS) {
+      const float* p = pqs + (size_t)i * dsub;
+      const float* qm = qs + (i / 16) * dsub;
+      float ip = 0.f;
+      for (int t = 0; t < dsub; t++) ip = fmaf(qm[t], p[t], ip);
+      t16[i] = -2.f * ip;
+    }
+    __syncthreads();
+    float* out = t3 + (size_t)qi * Mb * 256;
+    const int b = threadIdx.x, lo = b & 15, hi = b >> 4;
+    if (code_major) {  // row b: Mb consecutive floats (Mb % 4 == 0 wherever the scans read this layout)
+      for (int m = 0; m < Mb; m++) out[(size_t)b * Mb + m] = __fadd_rn(t16[(2 * m) * 16 + lo], t16[(2 * m + 1) * 16 + hi]);
+    } else {
+      for (int m = 0; m < Mb; m++) out[(size_t)m * 256 + b] = __fadd_rn(t16[(2 * m) * 16 + lo], t16[(2 * m + 1) * 16 + hi]);
+    }
+  }
+}
+
+int launch_pair_tables(const float* q, int64_t nq, int d, const float* pq, int Mb, float* t3, bool code_major,
+                       cudaStream_t st) {
+  const unsigned grid = (unsigned)(nq < 148 ? nq : 148);
+  const size_t smem = sizeof(float) * ((size_t)16 * d + d + 2 * Mb * 16);
+  VLQ_CUDA_TRY(cudaFuncSetAttribute(pair_tables_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  VLQ_LAUNCH(pair_tables_kernel, grid, T3_THREADS, smem, st, q, nq, d, pq, Mb, t3, code_major);
+  return VLQ_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ asynchronous scan
 // The 1B-scale variant of scan_topk_kernel (k <= 128): one CTA per query, but every WARP runs on its own -- it grabs the
 // next selected list from a shared counter, strides its entries (2 per lane per step, loads first), and keeps its own
@@ -1417,11 +1463,16 @@ size_t vlq_scan_topk_workspace_bytes(int64_t nq, int M) {
   return (size_t)(nq > 0 ? nq : 0) * M * 256 * sizeof(float) + ((scan_overflow_bytes(nq) + 255) & ~size_t(255)) + 256;
 }
 
-int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
-                  const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
-                  const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa,
-                  const int64_t* ids, int k, int cap, int list_len_hint, float* outD, int64_t* outI, void* workspace,
-                  size_t workspace_bytes, vlq_stream_t stream) {
+}  // extern "C"
+
+// The scan dispatch of vlq_scan_topk and vlq_scan_topk_pq4: M is the number of code BYTES per entry (tables of 256
+// entries each), tb how the term-3 tables of the batch are made.  Everything after the table build is the same for both.
+static int scan_topk_dispatch(const TableBuild& tb, const float* q, int64_t nq, int d, const float* pq, int M,
+                              const float* lambda_cb, int nL, const int* line_list, const float* term1,
+                              const float* term6, const float* edge_d2, int W, const int64_t* offsets,
+                              const uint8_t* codes, const uint8_t* lamq, const float* kappa, const int64_t* ids, int k,
+                              int cap, int list_len_hint, float* outD, int64_t* outI, void* workspace,
+                              size_t workspace_bytes, vlq_stream_t stream) {
   if (nq > 0 && (!q || !pq || !lambda_cb || !line_list || !term1 || !term6 || !offsets || !outD || !outI))
     return VLQ_EINVAL;
   if (nq < 0 || d <= 0 || M <= 0 || M > 64 || d % M != 0 || nL <= 0 || nL > 256 || W <= 0 || W > VLQ_MAX_K ||
@@ -1437,8 +1488,9 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
   const size_t t3_bytes = (size_t)nq * M * 256 * sizeof(float);
   const bool long_lists = list_len_hint >= 24;  // average list length of the index: warp-per-list pays off
   const bool al16 = (reinterpret_cast<uintptr_t>(codes) % 16) == 0;
-  const bool have_t3 = workspace && workspace_bytes >= t3_bytes + 256 && term3_supported(d, M) &&
+  const bool have_t3 = workspace && workspace_bytes >= t3_bytes + 256 && tb.supported &&
                        ((reinterpret_cast<uintptr_t>(workspace) | reinterpret_cast<uintptr_t>(pq)) & 15) == 0;
+  if (tb.required && !have_t3) return VLQ_EWORKSPACE;
   const bool use_async = long_lists && k <= kWarpSelMaxK && have_t3 && (M * 256) % 4 == 0;  // warp-autonomous scan
   // bank-skewed tables pay off once the lists are long enough to amortise the 64 KB table fill and the four extra
   // warps per query (measured on the C2 geometry, average list length -> speed-up over the plain tables:
@@ -1471,7 +1523,7 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
   const bool skew = use_long || (use_async && al16 && (M == 16 || M == 8) && list_len_hint >= skew_min_len);
   if (have_t3) {
     float* t3 = static_cast<float*>(workspace);
-    const int rc = launch_term3(q, nq, d, pq, M, t3, skew, as_stream(stream));
+    const int rc = tb.launch(q, nq, d, pq, M, t3, skew, as_stream(stream));
     if (rc) return rc;
     a.t3 = t3;
   }
@@ -1534,6 +1586,31 @@ int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, con
   }
 #undef VLQ_SCAN_LAUNCH
   return last_error();
+}
+
+extern "C" {
+
+int vlq_scan_topk(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                  const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                  const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa,
+                  const int64_t* ids, int k, int cap, int list_len_hint, float* outD, int64_t* outI, void* workspace,
+                  size_t workspace_bytes, vlq_stream_t stream) {
+  const TableBuild tb{launch_term3, M > 0 && term3_supported(d, M), false};
+  return scan_topk_dispatch(tb, q, nq, d, pq, M, lambda_cb, nL, line_list, term1, term6, edge_d2, W, offsets, codes,
+                            lamq, kappa, ids, k, cap, list_len_hint, outD, outI, workspace, workspace_bytes, stream);
+}
+
+int vlq_scan_topk_pq4(const float* q, int64_t nq, int d, const float* pq, int M, const float* lambda_cb, int nL,
+                      const int* line_list, const float* term1, const float* term6, const float* edge_d2, int W,
+                      const int64_t* offsets, const uint8_t* codes, const uint8_t* lamq, const float* kappa,
+                      const int64_t* ids, int k, int cap, int list_len_hint, float* outD, int64_t* outI, void* workspace,
+                      size_t workspace_bytes, vlq_stream_t stream) {
+  if (nq < 0 || !pq4_shape_ok(d, M) || d > 256) return VLQ_EINVAL;
+  if (!workspace || workspace_bytes < vlq_scan_topk_workspace_bytes(nq, M / 2)) return VLQ_EWORKSPACE;
+  if ((reinterpret_cast<uintptr_t>(workspace) | reinterpret_cast<uintptr_t>(pq)) & 15) return VLQ_EINVAL;
+  const TableBuild tb{launch_pair_tables, true, true};
+  return scan_topk_dispatch(tb, q, nq, d, pq, M / 2, lambda_cb, nL, line_list, term1, term6, edge_d2, W, offsets, codes,
+                            lamq, kappa, ids, k, cap, list_len_hint, outD, outI, workspace, workspace_bytes, stream);
 }
 
 int vlq_merge_topk(const float* D, const int64_t* I, int R, int64_t nq, int k, float* outD, int64_t* outI,

@@ -16,7 +16,7 @@ GpuIndexIMIPQ::GpuIndexIMIPQ(GpuResources* resources, int dims, int nbitsCoarse,
       lists_(resources, (int64_t)1 << (2 * nbitsCoarse), subQuantizers) {
   VLQ_THROW_IF_NOT_MSG(dims % 2 == 0 && dims % subQuantizers == 0 && (dims / 2) % (dims / subQuantizers) == 0,
                        "d must be even and every PQ sub-space must lie inside one half");
-  VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8, "only 8-bit PQ codes (as the VLQ index)");
+  VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8, "GpuIndexIMIPQ takes 8-bit PQ codes only (the IMI-PQ baseline of BASELINE configs[4])");
   VLQ_THROW_IF_NOT_MSG(nbitsCoarse >= 1 && nbitsCoarse <= 15, "nbitsCoarse must be in [1, 15]");
   is_trained = false;
   cp_.niter = 10;

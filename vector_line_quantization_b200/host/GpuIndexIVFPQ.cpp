@@ -10,6 +10,8 @@
 #include <cstring>
 #include <fstream>
 
+#include "../csrc/pq4.cuh"
+
 namespace faiss {
 namespace gpu {
 
@@ -50,6 +52,14 @@ void GpuIndexIVF::trainQuantizer_(Index::idx_t n, const float* x) {
 }
 
 // ================================================================================================ GpuIndexIVFPQ (VLQ)
+int GpuIndexIVFPQ::storedCodeBytes(int bitsPerCode, int M, int auxWidth) {
+  VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8 || bitsPerCode == 4, "bitsPerCode must be 4 or 8");
+  VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8 || M % 2 == 0, "4-bit PQ codes need an even number of sub-quantizers");
+  // the re-rank and refinement encode of GpuIndexIVFPQR (csrc/refine.cu) read one byte per first-level code
+  VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8 || auxWidth == 0, "GpuIndexIVFPQR takes 8-bit PQ codes only");
+  return bitsPerCode == 4 ? M / 2 : M;
+}
+
 GpuIndexIVFPQ::GpuIndexIVFPQ(GpuResources* resources, int dims, int nlist, int subQuantizers, int bitsPerCode,
                              int nedge, int nLambda, faiss::MetricType metric, GpuIndexIVFPQConfig config)
     : GpuIndexIVFPQ(resources, dims, nlist, subQuantizers, bitsPerCode, nedge, nLambda, metric, config, 0) {}
@@ -59,8 +69,8 @@ GpuIndexIVFPQ::GpuIndexIVFPQ(GpuResources* resources, int dims, int nlist, int s
     : GpuIndexIVF(resources, dims, metric, nlist, config), nLambda_(nLambda), numedge_(nedge), begin_(0), end_(nlist),
       w1_(256), edgeInfo_(nullptr), edgeDistInfo_(nullptr), lambdaInfo_(nullptr), constInfo_(nullptr), listCap_(VLQ_LIST_CAP),
       ivfpqConfig_(config), subQuantizers_(subQuantizers), bitsPerCode_(bitsPerCode),
-      lists_(resources, (int64_t)nlist * nedge, subQuantizers, auxWidth), populatedLists_((size_t)nlist * nedge) {
-  VLQ_THROW_IF_NOT_MSG(bitsPerCode == 8, "the scan kernels are written for 8-bit PQ codes");
+      codeBytes_(storedCodeBytes(bitsPerCode, subQuantizers, auxWidth)), lists_(resources, (int64_t)nlist * nedge, codeBytes_, auxWidth),
+      populatedLists_((size_t)nlist * nedge) {
   VLQ_THROW_IF_NOT_MSG(subQuantizers > 0 && subQuantizers <= 64 && dims % subQuantizers == 0,
                        "number of sub-quantizers must divide the dimension (and be <= 64)");
   VLQ_THROW_IF_NOT_MSG(nedge >= 1 && nedge <= 64 && nedge < nlist, "nedge must be in [1, 64] and < nlist");
@@ -71,7 +81,7 @@ GpuIndexIVFPQ::GpuIndexIVFPQ(GpuResources* resources, int dims, int nlist, int s
   edgeDistInfo_ = new float[(size_t)nlist * nedge]();
   lambdaInfo_ = new float[256]();
   constInfo_ = new float[256]();
-  pqHost_.resize((size_t)256 * dims);
+  pqHost_.resize(((size_t)1 << bitsPerCode) * dims);
 }
 
 GpuIndexIVFPQ::~GpuIndexIVFPQ() {
@@ -220,9 +230,10 @@ void GpuIndexIVFPQ::addTiles_(Index::idx_t n, const void* xv, bool isU8, const l
     }
     dA.reserve((size_t)m * sizeof(int));
     quantizer_->assignDevice(dx, m, dA.as<int>(), nullptr, false);
-    VLQ_CALL(vlq_line_encode(dx, m, d, dA.as<int>(), quantizer_->deviceVectors(), dEdge_.as<int>(),
-                             dEdgeDist_.as<float>(), numedge_, dLambda_.as<float>(), nLambda_, dPq_.as<float>(), M,
-                             out.list + s, nullptr, out.lamq + s, out.codes + (size_t)s * M, out.kappa + s, nullptr, st));
+    VLQ_CALL((pq4() ? vlq_line_encode_pq4 : vlq_line_encode)(
+        dx, m, d, dA.as<int>(), quantizer_->deviceVectors(), dEdge_.as<int>(), dEdgeDist_.as<float>(), numedge_,
+        dLambda_.as<float>(), nLambda_, dPq_.as<float>(), M, out.list + s, nullptr, out.lamq + s,
+        out.codes + (size_t)s * codeBytes_, out.kappa + s, nullptr, st));
     encodeAux_(dx, m, out, s, st);
     if (xids) {
       if (vlq_pointer_is_device(xids) == 1)
@@ -252,7 +263,7 @@ long GpuIndexIVFPQ::remove_ids(const IDSelector& sel) {
 
 // ------------------------------------------------------------------------------------------------ read-back
 void GpuIndexIVFPQ::decode_(const int64_t* pos, int64_t n, float* out, int64_t* outIds, vlq_stream_t st) const {
-  VLQ_CALL(vlq_decode_entries(n, pos, lists_.nlists(), lists_.offsets(), lists_.codes(), lists_.lamq(), lists_.ids(),
+  VLQ_CALL((pq4() ? vlq_decode_entries_pq4 : vlq_decode_entries)(n, pos, lists_.nlists(), lists_.offsets(), lists_.codes(), lists_.lamq(), lists_.ids(),
                               subQuantizers_, d, dPq_.as<float>(), quantizer_->deviceVectors(), dEdge_.as<int>(),
                               numedge_, dLambda_.as<float>(), nLambda_, out, outIds, st));
 }
@@ -298,7 +309,7 @@ void GpuIndexIVFPQ::range_search(Index::idx_t n, const float* x, float radius, R
   const Index::idx_t tile = std::max<Index::idx_t>(64, std::min<Index::idx_t>(5120, ((Index::idx_t)5 << 26) / nlist_));
   DeviceBuffer coarseWs;
   RangeLists lists{dPq_.as<float>(), subQuantizers_, dLambda_.as<float>(), nLambda_, dEdgeDist_.as<float>(), W, listCap_,
-                   &lists_, kappa, true, tile};
+                   &lists_, kappa, true, tile, pq4()};
   rangeSearchLists(resources_, d, n, x, radius, lists,
                    [&](const float* dq, Index::idx_t m, int* lines, float* t1, float* t6) {
                      coarseWs.reserve(vlq_coarse_lines_workspace_bytes(m, d, nlist_, P, numedge_, W,
@@ -376,7 +387,7 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
   // coarse stage of tile i + 1 (default stream) fills the other one
   const size_t lineBytes = ((size_t)tileCap * W * sizeof(float) + 255) & ~size_t(255);
   scratchB_.reserve(2 * 3 * lineBytes);
-  t3ws_.reserve(vlq_scan_topk_workspace_bytes(tileCap, M));
+  t3ws_.reserve(vlq_scan_topk_workspace_bytes(tileCap, codeBytes_));
   if (kc > k) {  // the scan's kc candidates of a tile; the epilogue of the tile reads them before the next scan (stream order)
     candD_.reserve((size_t)tileCap * kc * sizeof(float));
     candI_.reserve((size_t)tileCap * kc * sizeof(int64_t));
@@ -444,7 +455,7 @@ void GpuIndexIVFPQ::searchTiles_(Index::idx_t n, const float* x, Index::idx_t k,
       int64_t* oI = inPlace ? reinterpret_cast<int64_t*>(hI) : outI.as<int64_t>() + (size_t)s * k;
       float* sD = kc == k ? oD : candD_.as<float>();
       int64_t* sI = kc == k ? oI : candI_.as<int64_t>();
-      VLQ_CALL(vlq_scan_topk(q, m, d, dPq_.as<float>(), M, dLambda_.as<float>(), nLambda_, lline, t1, t6,
+      VLQ_CALL((pq4() ? vlq_scan_topk_pq4 : vlq_scan_topk)(q, m, d, dPq_.as<float>(), M, dLambda_.as<float>(), nLambda_, lline, t1, t6,
                              dEdgeDist_.as<float>(), W, lists_.offsets(), lists_.codes(), lists_.lamq(), kappa, ids,
                              (int)kc, listCap_, (int)std::min<size_t>(lists_.size() / populatedLists_, 1 << 20), sD, sI,
                              t3ws_.get(), t3ws_.bytes(), sb));
@@ -501,10 +512,24 @@ std::vector<unsigned char> GpuIndexIVFPQ::getListCodes(int listId) const {
   VLQ_THROW_IF_NOT(listId >= 0 && listId < nlist_ * numedge_);
   DeviceScope scope(ivfConfig_.device);
   commit_();
-  std::vector<unsigned char> codes =
-      fetchList<unsigned char>(lists_.offsets(), lists_.codes(), listId, subQuantizers_, resources_);
-  rotateListCodes(codes.data(), codes.size() / subQuantizers_, subQuantizers_, false);
-  return codes;
+  std::vector<unsigned char> codes = fetchList<unsigned char>(lists_.offsets(), lists_.codes(), listId, codeBytes_, resources_);
+  rotateListCodes(codes.data(), codes.size() / codeBytes_, codeBytes_, false);
+  return unpackedCodes_(codes);
+}
+
+// one byte per code, as the reference's formats hold them (byte_per_idx = 1): 4-bit codes are unpacked / packed here
+std::vector<uint8_t> GpuIndexIVFPQ::unpackedCodes_(const std::vector<uint8_t>& stored) const {
+  if (!pq4()) return stored;
+  std::vector<uint8_t> out(stored.size() * 2);
+  vlq::pq4_unpack(stored.data(), (int64_t)(stored.size() / codeBytes_), subQuantizers_, out.data());
+  return out;
+}
+std::vector<uint8_t> GpuIndexIVFPQ::packedCodes_(const std::vector<uint8_t>& codes) const {
+  if (!pq4()) return codes;
+  for (uint8_t c : codes) VLQ_THROW_IF_NOT_MSG(c < 16, "a 4-bit PQ code is >= 16");
+  std::vector<uint8_t> out(codes.size() / 2);
+  vlq::pq4_pack(codes.data(), (int64_t)(codes.size() / subQuantizers_), subQuantizers_, out.data());
+  return out;
 }
 std::vector<unsigned char> GpuIndexIVFPQ::getListLambdas(int listId) const {
   VLQ_THROW_IF_NOT(listId >= 0 && listId < nlist_ * numedge_);
@@ -584,7 +609,7 @@ void GpuIndexIVFPQ::writeDbToFile(const std::string& name) {  // .dbIdx .dbcodes
   std::vector<int64_t> off(L + 1);
   const size_t n = lists_.size();
   std::vector<long> ids(n);
-  std::vector<uint8_t> codes(n * subQuantizers_), las(n);
+  std::vector<uint8_t> codes(n * codeBytes_), las(n);
   VLQ_CALL(vlq_memcpy_d2h(off.data(), lists_.offsets(), off.size() * sizeof(int64_t), st));
   if (n) {
     VLQ_CALL(vlq_memcpy_d2h(ids.data(), lists_.ids(), ids.size() * sizeof(long), st));
@@ -595,8 +620,9 @@ void GpuIndexIVFPQ::writeDbToFile(const std::string& name) {  // .dbIdx .dbcodes
   std::vector<int> counts(L);
   for (size_t l = 0; l < L; l++) {
     counts[l] = (int)(off[l + 1] - off[l]);
-    rotateListCodes(codes.data() + (size_t)off[l] * subQuantizers_, (size_t)counts[l], subQuantizers_, false);
+    rotateListCodes(codes.data() + (size_t)off[l] * codeBytes_, (size_t)counts[l], codeBytes_, false);
   }
+  codes = unpackedCodes_(codes);
   std::ofstream fi((name + ".dbIdx").c_str(), std::ofstream::binary), fc((name + ".dbcodes").c_str(), std::ofstream::binary),
       fn((name + ".dbcount").c_str(), std::ofstream::binary), fl((name + ".dblas").c_str(), std::ofstream::binary);
   VLQ_THROW_IF_NOT_MSG(fi.good() && fc.good() && fn.good() && fl.good(), "cannot open database files for writing");
@@ -614,12 +640,12 @@ void GpuIndexIVFPQ::installLists_(const std::vector<int>& counts, const std::vec
   for (size_t l = 0; l < L; l++) off[l + 1] = off[l] + counts[l];
   const size_t tot = (size_t)off[L];
   VLQ_THROW_IF_NOT(ids.size() == tot && las.size() == tot && codes.size() == tot * subQuantizers_);
-  std::vector<uint8_t> stored = codes;  // outlives the copy (freed after the stream sync below)
+  std::vector<uint8_t> stored = packedCodes_(codes);  // outlives the copy (freed after the stream sync below)
   for (size_t l = 0; l < L; l++)
-    rotateListCodes(stored.data() + (size_t)off[l] * subQuantizers_, (size_t)counts[l], subQuantizers_, true);
+    rotateListCodes(stored.data() + (size_t)off[l] * codeBytes_, (size_t)counts[l], codeBytes_, true);
   float* kappa = lists_.install(off, stored, las, ids);
   if (tot)
-    VLQ_CALL(vlq_recompute_kappa((int64_t)tot, (int64_t)L, lists_.offsets(), lists_.codes(), lists_.lamq(),
+    VLQ_CALL((pq4() ? vlq_recompute_kappa_pq4 : vlq_recompute_kappa)((int64_t)tot, (int64_t)L, lists_.offsets(), lists_.codes(), lists_.lamq(),
                                  quantizer_->deviceVectors(), d, dEdge_.as<int>(), numedge_, dLambda_.as<float>(),
                                  dPq_.as<float>(), subQuantizers_, kappa, st));
   resources_->syncDefaultStream();

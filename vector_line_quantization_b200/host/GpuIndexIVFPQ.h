@@ -159,7 +159,10 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   void add_with_ids2(Index::idx_t n, Index::idx_t nq, unsigned kgt, const float* x, const float* xq, const Index::idx_t* ids,
                      Index::idx_t* nns, float* dists);
 
-  /// install externally trained codebooks (tests / multi-GPU broadcast): pq is (M, 256, dsub)
+  /// bytes per stored entry code for bitsPerCode 8 (M) or 4 (M / 2, two codes per byte, M even); throws for any other
+  /// format, and for 4-bit codes in lists with an aux column (GpuIndexIVFPQR).  Touches no device.
+  static int storedCodeBytes(int bitsPerCode, int M, int auxWidth = 0);
+  /// install externally trained codebooks (tests / multi-GPU broadcast): pq is (M, 2^bitsPerCode, dsub)
   void setCodebooks(const float* coarse, const int* edge, const float* edgeDist, const float* lambdaCb, const float* pq);
   const std::vector<float>& pqCentroids() const { return pqHost_; }
   /// maximum entries scanned per list (reference: 1024, gpu/impl/IVFUtils.cu:87)
@@ -194,10 +197,16 @@ class GpuIndexIVFPQ : public GpuIndexIVF {
   void installLists_(const std::vector<int>& counts, const std::vector<uint8_t>& codes, const std::vector<uint8_t>& las,
                      const std::vector<long>& ids);
 
+  bool pq4() const { return bitsPerCode_ == 4; }
+  /// one-byte-per-code rows [n][M] from the stored rows [n][codeBytes_] and back (the identity at 8 bits)
+  std::vector<uint8_t> unpackedCodes_(const std::vector<uint8_t>& stored) const;
+  std::vector<uint8_t> packedCodes_(const std::vector<uint8_t>& codes) const;
+
   GpuIndexIVFPQConfig ivfpqConfig_;
   int subQuantizers_;
   int bitsPerCode_;
-  std::vector<float> pqHost_;  // (M, 256, dsub)
+  int codeBytes_;  ///< bytes per stored entry code: M, or M / 2 for 4-bit codes (two per byte, csrc/pq4.cuh)
+  std::vector<float> pqHost_;  // (M, 2^bitsPerCode, dsub)
 
   // device tables
   DeviceBuffer dEdge_, dEdgeDist_, dLambda_, dPq_;

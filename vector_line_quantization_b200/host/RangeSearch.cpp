@@ -32,7 +32,7 @@ void rangeSearchLists(GpuResources* res, int d, Index::idx_t n, const float* x, 
     const int64_t budget = stagingResults();
     DeviceBuffer xin, lines((size_t)tile * W * sizeof(int)), t1((size_t)tile * W * sizeof(float)),
         t6((size_t)tile * W * sizeof(float)), qn((size_t)tile * sizeof(float)), lims((size_t)(tile + 1) * sizeof(int64_t)),
-        ws(vlq_range_workspace_bytes(tile, L.M, W, L.cap)), stage;
+        ws(vlq_range_workspace_bytes(tile, L.pq4 ? L.M / 2 : L.M, W, L.cap)), stage;
     if (!xOnDevice) xin.resize((size_t)tile * d * sizeof(float));
     std::vector<int64_t> hl((size_t)tile + 1);
     for (Index::idx_t s = 0; s < n; s += tile) {
@@ -45,7 +45,7 @@ void rangeSearchLists(GpuResources* res, int d, Index::idx_t n, const float* x, 
       coarse(q, m, lines.as<int>(), t1.as<float>(), t6.as<float>());
       if (L.addQueryNorm) VLQ_CALL(vlq_row_norms(q, m, d, qn.as<float>(), st));
       const float* rowAdd = L.addQueryNorm ? qn.as<float>() : nullptr;
-      VLQ_CALL(vlq_range_count(q, m, d, L.pq, L.M, L.lambdaCb, L.nLambda, lines.as<int>(), t1.as<float>(), t6.as<float>(),
+      VLQ_CALL((L.pq4 ? vlq_range_count_pq4 : vlq_range_count)(q, m, d, L.pq, L.M, L.lambdaCb, L.nLambda, lines.as<int>(), t1.as<float>(), t6.as<float>(),
                                L.edgeDist, W, L.lists->offsets(), L.lists->codes(), L.lists->lamq(), L.kappa, L.cap,
                                rowAdd, radius, lims.as<int64_t>(), ws.get(), ws.bytes(), st));
       // the one host synchronisation of a tile: its result sizes decide the sub-ranges and the host arrays
@@ -73,7 +73,7 @@ void rangeSearchLists(GpuResources* res, int d, Index::idx_t n, const float* x, 
       for (const auto& p : parts) {
         const int64_t cnt = hl[p.second] - hl[p.first];
         if (cnt == 0) continue;
-        VLQ_CALL(vlq_range_gather(q, m, d, L.pq, L.M, L.lambdaCb, L.nLambda, lines.as<int>(), t1.as<float>(),
+        VLQ_CALL((L.pq4 ? vlq_range_gather_pq4 : vlq_range_gather)(q, m, d, L.pq, L.M, L.lambdaCb, L.nLambda, lines.as<int>(), t1.as<float>(),
                                   t6.as<float>(), L.edgeDist, W, L.lists->offsets(), L.lists->codes(), L.lists->lamq(),
                                   L.kappa, L.cap, rowAdd, radius, L.lists->ids(), lims.as<int64_t>(), p.first, p.second,
                                   sD, sI, ws.get(), ws.bytes(), st));

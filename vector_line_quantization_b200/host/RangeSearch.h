@@ -16,8 +16,8 @@ namespace gpu {
 
 /// the committed lists and the scan tables of an index (device pointers)
 struct RangeLists {
-  const float* pq;        ///< (M, 256, d / M)
-  int M;
+  const float* pq;        ///< (M, 256, d / M), or (M, 16, d / M) with pq4
+  int M;                  ///< sub-quantizers
   const float* lambdaCb;  ///< [nLambda]
   int nLambda;
   const float* edgeDist;  ///< per-list squared edge length (term5); nullptr = 0 (IMI-PQ)
@@ -27,6 +27,7 @@ struct RangeLists {
   const float* kappa;        ///< lists->kappa(sel) of the call
   bool addQueryNorm;      ///< term1 excludes ||q||^2 (the VLQ coarse stage): add it back for the full distance
   Index::idx_t tile;      ///< queries per coarse stage at most
+  bool pq4 = false;       ///< 4-bit codes, M / 2 packed bytes per entry (vlq_range_*_pq4)
 };
 
 /// lines / term1 / term6 [m][W] of the m queries at the device pointer dq, on the resource's default stream

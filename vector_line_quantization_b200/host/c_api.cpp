@@ -220,6 +220,8 @@ int vlq_host_kmeans(void* res, int d, int k, long n, const float* x, int niter, 
 int vlq_host_vlq_new(void* res, int d, int nlist, int M, int bits, int nedge, int nlambda, int use_tensor_cores,
                      void** out) {
   GUARD({
+    GpuIndexIVFPQ::storedCodeBytes(bits, M);  // the code format is checked before anything touches a device
+    VLQ_THROW_IF_NOT_MSG(res != nullptr, "GpuResources must not be null");
     GpuResources* r = static_cast<GpuResources*>(res);
     GpuIndexIVFPQConfig cfg;
     cfg.device = r->getDevice();
@@ -288,6 +290,8 @@ int vlq_host_vlq_read_db(void* index, const char* name, int pronum, int rank) {
 int vlq_host_ivfpqr_new(void* res, int d, int nlist, int M, int M_refine, int bits, int nedge, int nlambda,
                         int use_tensor_cores, void** out) {
   GUARD({
+    GpuIndexIVFPQ::storedCodeBytes(bits, M, M_refine > 0 ? M_refine : 1);
+    VLQ_THROW_IF_NOT_MSG(res != nullptr, "GpuResources must not be null");
     GpuResources* r = static_cast<GpuResources*>(res);
     GpuIndexIVFPQConfig cfg;
     cfg.device = r->getDevice();

@@ -410,11 +410,13 @@ def kmeans(res, x, k, niter=10, seed=1234):
 
 
 class GpuIndexIVFPQ(_ReadBack, Index):
-    """The VLQ index: GpuIndexIVFPQ(res, d, nlist, M, bitsPerCode, nedge, nLambda) (gpu/GpuIndexIVFPQ.h:59-67)."""
+    """The VLQ index: GpuIndexIVFPQ(res, d, nlist, M, bitsPerCode, nedge, nLambda) (gpu/GpuIndexIVFPQ.h:59-67).
+    bits = 8, or 4 with an even M: two codes per stored byte on the device; getList, copyFrom / copyTo and the .db*
+    files still see one byte per code."""
 
     def __init__(self, res, d, nlist, M, bits=8, nedge=32, nLambda=256, use_tensor_cores=True):
         super().__init__(d)
-        self.res, self.nlist, self.M, self.nedge, self.nLambda = res, nlist, M, nedge, nLambda
+        self.res, self.nlist, self.M, self.nedge, self.nLambda, self.bits = res, nlist, M, nedge, nLambda, bits
         _call("vlq_host_vlq_new", res.h, d, nlist, M, bits, nedge, nLambda, int(use_tensor_cores), C.byref(self.h))
         self._w1 = 256
 
@@ -456,7 +458,7 @@ class GpuIndexIVFPQ(_ReadBack, Index):
         L = self.nlist * self.nedge
         out = dict(cent=np.empty((self.nlist, self.d), np.float32), edge=np.empty((self.nlist, self.nedge), np.int32),
                    edge_d2=np.empty((self.nlist, self.nedge), np.float32), lambda_cb=np.empty(self.nLambda, np.float32),
-                   pq=np.empty((self.M, 256, self.d // self.M), np.float32))
+                   pq=np.empty((self.M, 1 << self.bits, self.d // self.M), np.float32))
         _call("vlq_host_vlq_get_codebooks", self.h, *(C.c_void_p(out[k].ctypes.data) for k in
                                                       ("cent", "edge", "edge_d2", "lambda_cb", "pq")))
         assert out["edge"].size == L
@@ -547,6 +549,7 @@ class GpuIndexIVFPQR(GpuIndexIVFPQ):
             raise ValueError("M_refine must be in [1, 64] and divide d = %d, got %d" % (d, M_refine))
         Index.__init__(self, d)
         self.res, self.nlist, self.M, self.nedge, self.nLambda, self.M_refine = res, nlist, M, nedge, nLambda, M_refine
+        self.bits = bits
         _call("vlq_host_ivfpqr_new", res.h, d, nlist, M, M_refine, bits, nedge, nLambda, int(use_tensor_cores),
               C.byref(self.h))
         self._w1 = 256

@@ -100,6 +100,23 @@ def knn_graph(cent, E, cnorm=None):
 Encoded = namedtuple("Encoded", "list lam lamq codes kappa residual")
 
 
+# 4-bit PQ codes (include/vlq_b200.h, csrc/pq4.cuh): a codebook (M, 16, dsub) selects the *_pq4 entry points of
+# line_encode, scan_topk, range_scan_lines and decode_entries, whose lists hold M / 2 packed bytes per entry,
+# byte j = code[2j] | code[2j + 1] << 4.
+def is_pq4(pq):
+    return pq.shape[1] == 16
+
+
+def pack_pq4(codes):
+    """one byte per 4-bit code [n][M] (M even) -> the stored form [n][M / 2]"""
+    return (codes[:, 0::2] | (codes[:, 1::2] << 4)).contiguous()
+
+
+def unpack_pq4(packed):
+    """[n][M / 2] packed bytes -> [n][M] codes"""
+    return torch.stack((packed & 15, packed >> 4), dim=2).reshape(packed.shape[0], -1).contiguous()
+
+
 def line_encode(x, assign, cent, edge, edge_d2, lambda_cb=None, pq=None, want_residual=False):
     """fused line stage (+ lambda quantiser + residual + PQ encode when lambda_cb/pq are given) (a5-a8)"""
     x = _chk(x, torch.float32, "x")
@@ -119,11 +136,11 @@ def line_encode(x, assign, cent, edge, edge_d2, lambda_cb=None, pq=None, want_re
         pq = _chk(pq, torch.float32, "pq")
         M, nL = pq.shape[0], lambda_cb.shape[0]
         lamq = torch.empty(n, dtype=torch.uint8, device=dev)
-        codes = torch.empty((n, M), dtype=torch.uint8, device=dev)
+        codes = torch.empty((n, M // 2 if is_pq4(pq) else M), dtype=torch.uint8, device=dev)
         kappa = torch.empty(n, dtype=torch.float32, device=dev)
         if want_residual:
             resid = torch.empty((n, d), dtype=torch.float32, device=dev)
-    _abi.call("vlq_line_encode", _ptr(x), n, d, _ptr(assign), _ptr(cent), _ptr(edge), _ptr(edge_d2), E,
+    _abi.call("vlq_line_encode_pq4" if pq is not None and is_pq4(pq) else "vlq_line_encode", _ptr(x), n, d, _ptr(assign), _ptr(cent), _ptr(edge), _ptr(edge_d2), E,
               _ptr(lambda_cb), nL, _ptr(pq), M, _ptr(out_list), _ptr(out_lam), _ptr(lamq), _ptr(codes), _ptr(kappa),
               _ptr(resid), _stream())
     return Encoded(out_list, out_lam, lamq, codes, kappa, resid)
@@ -216,6 +233,7 @@ def decode_entries(lists, pos, pq, cent=None, edge=None, lambda_cb=None, cb=None
     pq = _chk(pq, torch.float32, "pq")
     pos = _chk(pos, torch.int64, "pos")
     M, d = pq.shape[0], pq.shape[0] * pq.shape[2]
+    pq4 = is_pq4(pq)
     n = pos.numel()
     out = torch.empty((n, d), dtype=torch.float32, device=offsets.device)
     oid = torch.empty(n, dtype=torch.int64, device=offsets.device) if want_ids else None
@@ -224,7 +242,7 @@ def decode_entries(lists, pos, pq, cent=None, edge=None, lambda_cb=None, cb=None
     if cb is None:
         edge = _chk(edge, torch.int32, "edge")
         lambda_cb = _chk(lambda_cb, torch.float32, "lambda_cb")
-        _abi.call("vlq_decode_entries", n, _ptr(pos), offsets.shape[0] - 1, _ptr(offsets), _ptr(codes),
+        _abi.call("vlq_decode_entries_pq4" if pq4 else "vlq_decode_entries", n, _ptr(pos), offsets.shape[0] - 1, _ptr(offsets), _ptr(codes),
                   _ptr(_chk(lists.lamq, torch.uint8, "lamq")), _ptr(ids), M, d, _ptr(pq),
                   _ptr(_chk(cent, torch.float32, "cent")), _ptr(edge), edge.shape[-1], _ptr(lambda_cb),
                   lambda_cb.shape[0], _ptr(out), _ptr(oid), _stream())
@@ -280,6 +298,7 @@ def refine_decode(lists, code2, pos, pq, cent, edge, lambda_cb, pq2):
     offsets = _chk(lists.offsets, torch.int64, "offsets")
     pos = _chk(pos, torch.int64, "pos")
     M, d = pq.shape[0], pq.shape[0] * pq.shape[2]
+    pq4 = is_pq4(pq)
     n = pos.numel()
     out = torch.empty((n, d), dtype=torch.float32, device=offsets.device)
     _abi.call("vlq_refine_decode", n, _ptr(pos), offsets.shape[0] - 1, _ptr(offsets), _ptr(lists.codes),
@@ -365,11 +384,13 @@ def scan_topk(q, pq, lambda_cb, line_list, term1, term6, edge_d2, lists, k, cap=
               list_len_hint=None, out=None, slab_index=False, kappa=None):
     """ADC scan of the selected lists fused with exact top-k (a13-a15): -> (D f32 [nq][k], I int64 [nq][k]).
     slab_index=True: I holds each result's slab index (its row in lists.codes) instead of its id (ids = NULL).
-    kappa: per-entry kappa to read instead of lists.kappa (filter_kappa's mask)."""
+    kappa: per-entry kappa to read instead of lists.kappa (filter_kappa's mask).
+    A 4-bit codebook (M, 16, dsub) scans packed lists through pair tables (vlq_scan_topk_pq4: use_workspace required)."""
     q = _chk(q, torch.float32, "q")
     pq = _chk(pq, torch.float32, "pq")
     nq, d = q.shape
     M = pq.shape[0]
+    pq4 = is_pq4(pq)
     W = line_list.shape[1]
     if out is not None:  # contiguous (nq, k) f32 / int64 destinations (e.g. row slices of the caller's result arrays)
         outD, outI = _chk(out[0], torch.float32, "out D"), _chk(out[1], torch.int64, "out I")
@@ -381,12 +402,12 @@ def scan_topk(q, pq, lambda_cb, line_list, term1, term6, edge_d2, lists, k, cap=
     ws = None
     wsb = 0
     if use_workspace:  # term-3 tables of the batch (grow-only cache per device)
-        wsb = _abi.lib().vlq_scan_topk_workspace_bytes(nq, M)
+        wsb = _abi.lib().vlq_scan_topk_workspace_bytes(nq, M // 2 if pq4 else M)
         ws = _scan_ws.get(q.device)
         if ws is None or ws.numel() < wsb:
             ws = torch.empty(max(wsb, 16), dtype=torch.uint8, device=q.device)
             _scan_ws[q.device] = ws
-    _abi.call("vlq_scan_topk", _ptr(q), nq, d, _ptr(pq), M, _ptr(lambda_cb), lambda_cb.shape[0],
+    _abi.call("vlq_scan_topk_pq4" if pq4 else "vlq_scan_topk", _ptr(q), nq, d, _ptr(pq), M, _ptr(lambda_cb), lambda_cb.shape[0],
               _ptr(_chk(line_list, torch.int32, "line_list")), _ptr(term1), _ptr(term6), _ptr(edge_d2), W,
               _ptr(lists.offsets), _ptr(lists.codes), _ptr(lists.lamq),
               _ptr(lists.kappa if kappa is None else _chk(kappa, torch.float32, "kappa")),
@@ -407,6 +428,8 @@ def range_scan_lines(q, pq, lambda_cb, lines, edge_d2, lists, radius, cap=1024, 
     pq = _chk(pq, torch.float32, "pq")
     nq, d = q.shape
     M = pq.shape[0]
+    pq4 = is_pq4(pq)
+    count, gather = ("vlq_range_count_pq4", "vlq_range_gather_pq4") if pq4 else ("vlq_range_count", "vlq_range_gather")
     lst, t1, t6 = lines
     W = lst.shape[1]
     dev = q.device
@@ -414,7 +437,7 @@ def range_scan_lines(q, pq, lambda_cb, lines, edge_d2, lists, radius, cap=1024, 
     lims = [torch.zeros(1, dtype=torch.int64, device=dev)]
     outD, outI = [], []
     tile = _tile_rows(nq, tile)
-    ws = torch.empty(max(_abi.lib().vlq_range_workspace_bytes(tile, M, W, cap), 256), dtype=torch.uint8, device=dev)
+    ws = torch.empty(max(_abi.lib().vlq_range_workspace_bytes(tile, M // 2 if pq4 else M, W, cap), 256), dtype=torch.uint8, device=dev)
     lt = torch.empty(tile + 1, dtype=torch.int64, device=dev)
     done = 0
     for s in range(0, nq, tile):
@@ -424,7 +447,7 @@ def range_scan_lines(q, pq, lambda_cb, lines, edge_d2, lists, radius, cap=1024, 
                 _ptr(_chk(lst[s:e], torch.int32, "line_list")), _ptr(t1[s:e]), _ptr(t6[s:e]), _ptr(ed2), W,
                 _ptr(lists.offsets), _ptr(lists.codes), _ptr(lists.lamq), _ptr(lists.kappa), cap,
                 _ptr(None if row_add is None else row_add[s:e]), float(radius))
-        _abi.call("vlq_range_count", *args, _ptr(lt), _ptr(ws), ws.numel(), _stream())
+        _abi.call(count, *args, _ptr(lt), _ptr(ws), ws.numel(), _stream())
         hl = lt[:m + 1].cpu()
         total = int(hl[m])
         D = torch.empty(max(total, 1), dtype=torch.float32, device=dev)
@@ -440,7 +463,7 @@ def range_scan_lines(q, pq, lambda_cb, lines, edge_d2, lists, radius, cap=1024, 
             if int(hl[q1]) == o:  # no results in [q0, q1): nothing to write (and an empty slice has no address)
                 q0 = q1
                 continue
-            _abi.call("vlq_range_gather", *args, _ptr(lists.ids), _ptr(lt), q0, q1, _ptr(D[o:]), _ptr(I[o:]), _ptr(ws),
+            _abi.call(gather, *args, _ptr(lists.ids), _ptr(lt), q0, q1, _ptr(D[o:]), _ptr(I[o:]), _ptr(ws),
                       ws.numel(), _stream())
             q0 = q1
         lims.append(hl[1:].to(dev) + done)

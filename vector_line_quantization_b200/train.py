@@ -109,8 +109,9 @@ def kmeans(x, k, niter=10, seed=1234, max_points_per_centroid=256, exact_perm=Tr
 
 
 def train_vlq(xt, nlist, E, M, nL, nbits=8, niter=10, pq_niter=25, seed=1234, exact_perm=True, verbose=False):
-    """-> dict(cent, cnorm, edge, edge_d2, lambda_cb, pq) of device tensors"""
-    assert nbits == 8, "the scan kernels are written for 8-bit PQ codes (ksub = 256)"
+    """-> dict(cent, cnorm, edge, edge_d2, lambda_cb, pq) of device tensors; pq is (M, 2^nbits, d / M), nbits 8 or 4
+    (two codes per stored byte, M even: the ops entry points take the 4-bit form from the codebook's shape)"""
+    assert nbits in (4, 8) and (nbits == 8 or M % 2 == 0), "PQ codes are 8-bit, or 4-bit with an even M"
     d = xt.shape[1]
     cent, _ = kmeans(xt, nlist, niter=niter, seed=seed, exact_perm=exact_perm, verbose=verbose)
     cnorm = ops.row_norms(cent)
@@ -127,8 +128,9 @@ def train_vlq(xt, nlist, E, M, nL, nbits=8, niter=10, pq_niter=25, seed=1234, ex
     dummy = torch.zeros((M, 256, dsub), dtype=torch.float32, device=xt.device)
     enc = ops.line_encode(x2, A, cent, edge, ed2, lcb, dummy, want_residual=True)
     r = enc.residual
-    pq = torch.empty((M, 256, dsub), dtype=torch.float32, device=xt.device)
+    ksub = 1 << nbits
+    pq = torch.empty((M, ksub, dsub), dtype=torch.float32, device=xt.device)
     for m in range(M):
         sub = r[:, m * dsub:(m + 1) * dsub].contiguous()
-        pq[m], _ = kmeans(sub, 256, niter=pq_niter, seed=seed, exact_perm=exact_perm)
+        pq[m], _ = kmeans(sub, ksub, niter=pq_niter, seed=seed, exact_perm=exact_perm)
     return dict(cent=cent, cnorm=cnorm, edge=edge, edge_d2=ed2, lambda_cb=lcb, pq=pq, pack=pack)
